@@ -1,15 +1,21 @@
 #!/usr/bin/env python
 """bench.py -- spectrograms/s of the VirtualRadar forward pass (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch of BASELINE config 2
 (N=256 NTU-shaped sequences, 3x300x25x2 -> 256x19) per GPU, synthetic input.
 
-Every device-timed figure is measured the same way (`timed_reps`): the K-step loop -- bracketed by a barrier +
-synchronize on both sides, CUDA events on the launching stream, max over ranks -- is REPEATED until at least 50 ms
-have been timed, and the median repetition is reported; K=20 steps of a 15 us kernel alone would be a 0.3 ms sample.
+The K-step figures (value, stream_ordered, module_forward) are measured the same way (`timed_steps`): one untimed step
+that loads the kernels, then at least W untimed steps, and at least 50 ms of them so that the clocks have risen, then
+exactly K steps between two CUDA events on the launching stream, max over ranks.  The figures with a fixed size of
+their own (large_batch, sweep) repeat their loop until at least 50 ms have been timed and report the median
+repetition (`timed_reps`).
+
+--dump-outputs DIR writes the spectrograms of the last timed step, (256, 256, 19) float32, to DIR/spectrograms.npy
+(DIR/spectrograms_rank<r>.npy per rank on several GPUs).  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 
   value          sequences/s, whole job, inputs resident in HBM, one fused launch per step, steps = independent batches
                  in distinct buffers (a pool larger than the 126 MB L2) launched with VR_FLAG_INPUTS_READY, so that
@@ -40,6 +46,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 BATCH, T, V, M = 256, 300, 25, 2
 N_FFT, HOP = 256, 16
@@ -51,6 +58,7 @@ FLOPS_PER_SPEC = 55 * T * 24 * M + F * (5 * N_FFT * 8 + 8 * N_FFT)   # 1 025 472
 WAVELENGTH = 5e-4
 WORKLOAD = "synthetic NTU-60 batch N=256, C=3, T=300, V=25, M=2 (BASELINE configs[1]), wavelength 5e-4, default 24-bone skeleton"
 MIN_TIMED_MS = 50.0
+MIN_WARM_MS = 50.0
 
 
 def synth_batch(n, seed):
@@ -195,10 +203,11 @@ def run_reference(args, rank, world):
 def run_ours(args, rank, world, local_rank):
     import ctypes
     import torch
+    import numpy as np
     import torch.distributed as dist
-    import __graft_entry__ as ge
-    ge.build_product()
+    # the library __graft_entry__.build() left in the tree; nothing is compiled here (_cabi fails loudly if it is missing)
     from skeleton_action_recognition_b200 import VirtualRadar, _cabi, shard_bounds
+    assert _cabi.lib().vr_abi_version() == _cabi.ABI_VERSION
 
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (no CPU fallback)"
     torch.cuda.set_device(local_rank)
@@ -219,7 +228,27 @@ def run_ours(args, rank, world, local_rank):
         return [float(v) for v in t.tolist()]
 
     stream = torch.cuda.current_stream(dev)
-    launches = [0]
+
+    def timed_steps(step, k):
+        """(milliseconds of exactly k steps, max over ranks; number of warm-up steps).  Warm-up: one step and a
+        synchronize (a kernel's first launch loads its module, which must not count as warm-up time), then steps until
+        at least args.warmup of them have been launched over at least MIN_WARM_MS.  The window then opens behind them
+        without a synchronize, so the first timed step does not wait for its launch.  Warm-up steps have indices
+        counting from 0, the timed steps 0..k-1: what the timed steps compute does not depend on the warm-up."""
+        barrier()
+        step(0)
+        barrier()
+        n, t0 = 1, time.perf_counter()
+        while n < args.warmup or (time.perf_counter() - t0) * 1e3 < MIN_WARM_MS:
+            step(n)
+            n += 1
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        for i in range(k):
+            step(i)
+        e1.record(stream)
+        barrier()
+        return max_over_ranks([e0.elapsed_time(e1)])[0], n
 
     def timed_reps(step, k, min_ms=MIN_TIMED_MS, max_reps=400, warm=3):
         """Median (over repetitions, after max over ranks) milliseconds of a k-step loop; repetitions until >= min_ms
@@ -254,7 +283,7 @@ def run_ours(args, rank, world, local_rank):
     s_ptr = ctypes.c_void_p(stream.cuda_stream)
     lam_ptr, loc_ptr = layer.wavelength.data_ptr(), layer.radar_location.data_ptr()
     E = len(layer.src)
-    K = max(1, args.steps)
+    K = args.steps
 
     def raw_step(i, flags):
         # the module's forward minus torch.empty: the same C-ABI call on preallocated buffers
@@ -262,7 +291,6 @@ def run_ours(args, rank, world, local_rank):
                                 lam_ptr, loc_ptr, N_FFT, HOP, flags, outs[i % pool].data_ptr(), s_ptr)
         if rc:
             _cabi.check(rc)
-        launches[0] += 1
 
     sampler = ClockSampler(physical_gpu_index(local_rank))
     sampler.start()
@@ -270,12 +298,8 @@ def run_ours(args, rank, world, local_rank):
     frac = lambda n, ms: BYTES_PER_SPEC * n / (ms * 1e-3) / 1e9 / peak     # noqa: E731
 
     # ---- headline: device-resident throughput, independent batches ----------------------------
-    for i in range(max(args.warmup, 3)):
-        raw_step(i, _cabi.VR_FLAG_INPUTS_READY)
     sampler.active.set()
-    launches[0] = 0
-    ms_k, reps, timed_ms = timed_reps(lambda i: raw_step(i, _cabi.VR_FLAG_INPUTS_READY), K, warm=0)
-    gpu_launches = launches[0]
+    ms_k, warm_n = timed_steps(lambda i: raw_step(i, _cabi.VR_FLAG_INPUTS_READY), K)
     sampler.active.clear()
     ms_per_step = ms_k / K
     value = world * BATCH / (ms_per_step * 1e-3)
@@ -283,17 +307,21 @@ def run_ours(args, rank, world, local_rank):
     torch.cuda.synchronize(dev)
     for i in {0, (K - 1) % pool, K % pool}:
         assert torch.equal(outs[i], layer(xs[i])), "timed path != VirtualRadar.forward"
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "spectrograms.npy" if world == 1 else "spectrograms_rank%d.npy" % rank
+        np.save(os.path.join(args.dump_outputs, name), outs[(K - 1) % pool].cpu().numpy())
 
     # ---- the same loop in plain stream order (what the module does by default) ----------------
     sampler.active.set()
-    so_k, so_reps, _ = timed_reps(lambda i: raw_step(i, 0), K)
+    so_k, so_warm = timed_steps(lambda i: raw_step(i, 0), K)
     so_ms = so_k / K
     # ---- the drop-in module itself: eager, and one forward captured in a CUDA graph ------------
     holder = [None]
 
     def module_step(i):
         holder[0] = layer(xs[i % pool])
-    me_k, _, _ = timed_reps(module_step, K)
+    me_k, _ = timed_steps(module_step, K)
     me_ms = me_k / K
     static_x = xs[0].clone()
     side = torch.cuda.Stream(dev)
@@ -305,7 +333,7 @@ def run_ours(args, rank, world, local_rank):
     graph = torch.cuda.CUDAGraph()
     with torch.cuda.graph(graph):
         static_y = layer(static_x)
-    mg_k, _, _ = timed_reps(lambda i: graph.replay(), K)
+    mg_k, _ = timed_steps(lambda i: graph.replay(), K)
     mg_ms = mg_k / K
     assert torch.equal(static_y, layer(static_x))
     sampler.active.clear()
@@ -555,18 +583,18 @@ def run_ours(args, rank, world, local_rank):
         traffic, traffic_src = ncu_traffic("dram_bytes_per_launch_n256")
         line = {
             "metric": "spectrograms/sec (NTU 3x300x25x2)", "value": value, "unit": "spectrograms/s",
-            "n_gpus": world, "steps": K, "warmup": max(args.warmup, 3), "ms_per_step": ms_per_step,
+            "n_gpus": world, "steps": K, "warmup": warm_n, "ms_per_step": ms_per_step,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": WORKLOAD, "batch_per_gpu": BATCH, "sharding": "by sequence, no collective on the path",
                        "l2": "steps rotate over %d input/output buffer pairs (%.0f MB > 126 MB L2)" % (pool, pool * BATCH * BYTES_PER_SPEC / 1e6),
-                       "timing": "the %d-step loop repeated %d times (%.0f ms timed in total, >= %.0f ms), median repetition, max over ranks per repetition"
-                                 % (K, reps, timed_ms, MIN_TIMED_MS),
+                       "timing": "one window of exactly %d steps between CUDA events, max over ranks, after %d warm-up steps "
+                                 "(>= --warmup %d, launched over >= %.0f ms)" % (K, warm_n, args.warmup, MIN_WARM_MS),
                        "launch": {"cooperative": plan, "team_jobs": plan_team,
                                   "schedule": "team jobs for overlapping or large batches, cooperative otherwise (vr_set_schedule)"},
                        "overlap": "value: steps are independent batches, programmatic dependent launches with VR_FLAG_INPUTS_READY "
                                   "(a step's reads may start while the previous step's last CTAs finish; writes wait); "
                                   "stream_ordered: the same loop without the flag, the module's default"},
-            "stream_ordered": {"value": world * BATCH / (so_ms * 1e-3), "ms_per_step": so_ms, "steps": K, "reps": so_reps,
+            "stream_ordered": {"value": world * BATCH / (so_ms * 1e-3), "ms_per_step": so_ms, "steps": K, "warmup": so_warm,
                                "hbm_frac": frac(BATCH, so_ms),
                                "note": "same loop without the flag: every step waits for the previous kernel to finish"},
             "module_forward": module_forward,
@@ -584,7 +612,7 @@ def run_ours(args, rank, world, local_rank):
                     "d2h_bytes_per_step": BATCH * BYTES_OUT, "steps": e2e_steps,
                     "api": "VirtualRadar.forward_host (C ABI vr_forward_host_f32), pinned host buffers"},
             "e2e_upsampled": e2e_upsampled,
-            "gpu_launches": gpu_launches,
+            "gpu_launches": K,
             "source_hash": source_hash(),
             "clocks": sampler.summary(),
         }
@@ -604,16 +632,21 @@ def main():
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the spectrograms of the last timed step to DIR/spectrograms.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if world == 1 and args.gpus > 1 and args.impl == "ours":
-        # convenience: relaunch under torchrun
+        # convenience: relaunch under torchrun, with every argument of this call
         import subprocess
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(args.gpus),
-               "--master-addr", "127.0.0.1", "--master-port", "29517", os.path.abspath(__file__),
-               "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup)]
+               "--master-addr", "127.0.0.1", "--master-port", "29517", os.path.abspath(__file__)] + sys.argv[1:]
         sys.exit(subprocess.call(cmd))
     # exactly ONE line on stdout: libraries (NCCL's version banner, torch warnings) write to fd 1 too, so
     # everything except the final JSON line is sent to stderr
