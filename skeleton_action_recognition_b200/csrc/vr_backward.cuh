@@ -17,6 +17,7 @@
 // against the float64 autograd of the oracle (tests/test_backward_gpu.py).
 #pragma once
 #include "vr_kernels.cuh"
+#include "vr_pad_frames.cuh"
 
 namespace vr {
 
@@ -33,6 +34,9 @@ struct BwdParams {
     int V, M, E, F, hop, VM;
     int fma_range;
     float inv_E;
+    const double* coef;          // vr_synth_adjoint_ups_kernel: (N, ups_T-1, 4, 3*V*M) cubics of vr_pad_frames_kernel; T = ups_K * ups_T
+    double ups_ratio;
+    int ups_T;
     uint16_t src[NG * MAX_EG], dst[NG * MAX_EG];
 };
 
@@ -145,108 +149,100 @@ __device__ __forceinline__ void bwd_range_phase(float jx, float jy, float jz, bo
     th = div_rn_fast(__fmul_rn(12.566370614359172f, d), lam, lam_rcp);
 }
 
-__global__ void __launch_bounds__(128) vr_synth_adjoint_kernel(const __grid_constant__ BwdParams p) {
-    const int T = (int)p.T;
-    const long long total = p.N * (long long)T;
-    const float lam = __ldg(p.lam_ptr);
-    const float Lx = __ldg(p.loc_ptr), Ly = __ldg(p.loc_ptr + 1), Lz = __ldg(p.loc_ptr + 2);
-    const float lam_rcp = rcp_refined(lam);
+// The adjoint of one (sequence, time step, body): mean bone length, then per bone the forward geometry (range and phase
+// with the forward's exact float32 rounding, the rest in float64) and the analytic derivatives of
+// z = sum amp * exp(j theta), accumulated in float64.  `pos(v, m, c)` is coordinate c of joint v of body m at this step:
+// read from x, or evaluated from the up-sampling spline -- equal positions and equal (gI, gQ) give equal results.
+// gx0 (optional): this step's x-plane row of dL/dx.
+template <class Pos>
+__device__ __forceinline__ void synth_adjoint_body(const BwdParams& p, const Pos& pos, int m, double gI, double gQ,
+                                                   float lam, float lam_rcp, float Lx, float Ly, float Lz,
+                                                   double& g_lam, double& g_lx, double& g_ly, double& g_lz,
+                                                   float* gx0, long long ps) {
     const double PI = 3.14159265358979323846;
-    double g_lam = 0.0, g_lx = 0.0, g_ly = 0.0, g_lz = 0.0;
-    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
-        const long long n = idx / T;
-        const int t = (int)(idx - n * T);
-        const double gI = (double)__ldg(p.gz + idx * 2), gQ = (double)__ldg(p.gz + idx * 2 + 1);
-        if (gI == 0.0 && gQ == 0.0) continue;
-        const float* x0 = p.x + (n * 3 * T + t) * (long long)p.VM;       // x-plane row of this time step
-        const long long ps = (long long)T * p.VM;                         // floats between coordinate planes
-        for (int m = 0; m < p.M; ++m) {
-            // mean bone length (:110-113), float32 like the forward
-            float sumB = 0.f;
-            for (int e = 0; e < p.E; ++e) {
-                const float* s = x0 + p.src[e] * p.M + m;
-                const float* d = x0 + p.dst[e] * p.M + m;
-                const float bx = __fsub_rn(__ldg(d), __ldg(s)), by = __fsub_rn(__ldg(d + ps), __ldg(s + ps)),
-                            bz = __fsub_rn(__ldg(d + 2 * ps), __ldg(s + 2 * ps));
-                const float bb = p.fma_range ? __fmaf_rn(bz, bz, __fmaf_rn(by, by, __fmul_rn(bx, bx)))
-                                             : __fadd_rn(__fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by)), __fmul_rn(bz, bz));
-                sumB = __fadd_rn(sumB, sqrt_rn_fast(bb));
+    // mean bone length (:110-113), float32 like the forward
+    float sumB = 0.f;
+    for (int e = 0; e < p.E; ++e) {
+        const int si = p.src[e], di = p.dst[e];
+        const float bx = __fsub_rn(pos(di, m, 0), pos(si, m, 0)), by = __fsub_rn(pos(di, m, 1), pos(si, m, 1)),
+                    bz = __fsub_rn(pos(di, m, 2), pos(si, m, 2));
+        const float bb = p.fma_range ? __fmaf_rn(bz, bz, __fmaf_rn(by, by, __fmul_rn(bx, bx)))
+                                     : __fadd_rn(__fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by)), __fmul_rn(bz, bz));
+        sumB = __fadd_rn(sumB, sqrt_rn_fast(bb));
+    }
+    if (sumB == 0.f) return;                                           // absent body: contributes exactly 0
+    const double cbar = (double)__fmul_rn(sumB, p.inv_E);
+    const double c = cbar * cbar, K = sqrt(PI) * cbar;
+    double G_c = 0.0;                                                  // dL/d(mean bone length), over this body's bones
+    for (int e = 0; e < p.E; ++e) {
+        const int si = p.src[e], di = p.dst[e];
+        const float sx = pos(si, m, 0), sy = pos(si, m, 1), sz = pos(si, m, 2);
+        const float dx = pos(di, m, 0), dy = pos(di, m, 1), dz = pos(di, m, 2);
+        // range, phase: the forward's float32 values
+        float rng, th;
+        bwd_range_phase(__fsub_rn(sx, Lx), __fsub_rn(sy, Ly), __fsub_rn(sz, Lz), p.fma_range != 0, lam, lam_rcp, rng, th);
+        double sn, cs;
+        sincos((double)th, &sn, &cs);
+        // aspect cosine and amplitude, float64 from the float32 inputs
+        const double Bx = (double)dx - sx, By = (double)dy - sy, Bz = (double)dz - sz;
+        const double Ax = (double)Lx - 0.5 * ((double)sx + dx), Ay = (double)Ly - 0.5 * ((double)sy + dy),
+                     Az = (double)Lz - 0.5 * ((double)sz + dz);
+        const double na = sqrt(Ax * Ax + Ay * Ay + Az * Az), nb = sqrt(Bx * Bx + By * By + Bz * Bz);
+        const double dot = Ax * Bx + Ay * By + Az * Bz;
+        const double q = na * nb + 1e-6;
+        const double u = dot / q;
+        const double den = 1.0 + (c - 1.0) * u * u;
+        const double amp = K / den;
+        const double dL_dth = amp * (gQ * cs - gI * sn);
+        const double dL_damp = gI * cs + gQ * sn;
+        g_lam += dL_dth * (-(double)th / (double)lam);
+        double gsx = 0.0, gsy = 0.0, gsz = 0.0, gdx = 0.0, gdy = 0.0, gdz = 0.0;   // dL/dS, dL/dD of this bone
+        if (rng > 0.f) {
+            const double kth = dL_dth * (4.0 * PI / (double)lam) / (double)rng;
+            g_lx += kth * ((double)Lx - sx); g_ly += kth * ((double)Ly - sy); g_lz += kth * ((double)Lz - sz);
+            gsx = kth * ((double)sx - Lx); gsy = kth * ((double)sy - Ly); gsz = kth * ((double)sz - Lz);
+        }
+        const double kamp = dL_damp * (-K * 2.0 * u * (c - 1.0) / (den * den));
+        if (na > 0.0) {
+            const double r2 = dot * nb / (na * q * q);
+            const double ax = kamp * (Bx / q - r2 * Ax), ay = kamp * (By / q - r2 * Ay), az = kamp * (Bz / q - r2 * Az);   // dL/dA
+            g_lx += ax; g_ly += ay; g_lz += az;
+            gsx -= 0.5 * ax; gsy -= 0.5 * ay; gsz -= 0.5 * az;
+            gdx -= 0.5 * ax; gdy -= 0.5 * ay; gdz -= 0.5 * az;
+        }
+        if (gx0) {
+            if (nb > 0.0) {
+                const double r3 = dot * na / (nb * q * q);
+                const double bx = kamp * (Ax / q - r3 * Bx), by = kamp * (Ay / q - r3 * By), bz = kamp * (Az / q - r3 * Bz);  // dL/dB via u
+                gsx -= bx; gsy -= by; gsz -= bz;
+                gdx += bx; gdy += by; gdz += bz;
             }
-            if (sumB == 0.f) continue;                                    // absent body: contributes exactly 0
-            const double cbar = (double)__fmul_rn(sumB, p.inv_E);
-            const double c = cbar * cbar, K = sqrt(PI) * cbar;
-            float* gx0 = p.gx ? p.gx + (n * 3 * T + t) * (long long)p.VM : nullptr;   // this thread's own rows of dL/dx
-            double G_c = 0.0;                                              // dL/d(mean bone length), over this body's bones
-            for (int e = 0; e < p.E; ++e) {
-                const float* s = x0 + p.src[e] * p.M + m;
-                const float* d = x0 + p.dst[e] * p.M + m;
-                const float sx = __ldg(s), sy = __ldg(s + ps), sz = __ldg(s + 2 * ps);
-                const float dx = __ldg(d), dy = __ldg(d + ps), dz = __ldg(d + 2 * ps);
-                // range, phase: the forward's float32 values
-                float rng, th;
-                bwd_range_phase(__fsub_rn(sx, Lx), __fsub_rn(sy, Ly), __fsub_rn(sz, Lz), p.fma_range != 0, lam, lam_rcp, rng, th);
-                double sn, cs;
-                sincos((double)th, &sn, &cs);
-                // aspect cosine and amplitude, float64 from the float32 inputs
-                const double Bx = (double)dx - sx, By = (double)dy - sy, Bz = (double)dz - sz;
-                const double Ax = (double)Lx - 0.5 * ((double)sx + dx), Ay = (double)Ly - 0.5 * ((double)sy + dy),
-                             Az = (double)Lz - 0.5 * ((double)sz + dz);
-                const double na = sqrt(Ax * Ax + Ay * Ay + Az * Az), nb = sqrt(Bx * Bx + By * By + Bz * Bz);
-                const double dot = Ax * Bx + Ay * By + Az * Bz;
-                const double q = na * nb + 1e-6;
-                const double u = dot / q;
-                const double den = 1.0 + (c - 1.0) * u * u;
-                const double amp = K / den;
-                const double dL_dth = amp * (gQ * cs - gI * sn);
-                const double dL_damp = gI * cs + gQ * sn;
-                g_lam += dL_dth * (-(double)th / (double)lam);
-                double gsx = 0.0, gsy = 0.0, gsz = 0.0, gdx = 0.0, gdy = 0.0, gdz = 0.0;   // dL/dS, dL/dD of this bone
-                if (rng > 0.f) {
-                    const double kth = dL_dth * (4.0 * PI / (double)lam) / (double)rng;
-                    g_lx += kth * ((double)Lx - sx); g_ly += kth * ((double)Ly - sy); g_lz += kth * ((double)Lz - sz);
-                    gsx = kth * ((double)sx - Lx); gsy = kth * ((double)sy - Ly); gsz = kth * ((double)sz - Lz);
-                }
-                const double kamp = dL_damp * (-K * 2.0 * u * (c - 1.0) / (den * den));
-                if (na > 0.0) {
-                    const double r2 = dot * nb / (na * q * q);
-                    const double ax = kamp * (Bx / q - r2 * Ax), ay = kamp * (By / q - r2 * Ay), az = kamp * (Bz / q - r2 * Az);   // dL/dA
-                    g_lx += ax; g_ly += ay; g_lz += az;
-                    gsx -= 0.5 * ax; gsy -= 0.5 * ay; gsz -= 0.5 * az;
-                    gdx -= 0.5 * ax; gdy -= 0.5 * ay; gdz -= 0.5 * az;
-                }
-                if (gx0) {
-                    if (nb > 0.0) {
-                        const double r3 = dot * na / (nb * q * q);
-                        const double bx = kamp * (Ax / q - r3 * Bx), by = kamp * (Ay / q - r3 * By), bz = kamp * (Az / q - r3 * Bz);  // dL/dB via u
-                        gsx -= bx; gsy -= by; gsz -= bz;
-                        gdx += bx; gdy += by; gdz += bz;
-                    }
-                    G_c += dL_damp * sqrt(PI) * (1.0 / den - 2.0 * c * u * u / (den * den));
-                    float* gs = gx0 + p.src[e] * p.M + m;
-                    float* gd = gx0 + p.dst[e] * p.M + m;
-                    gs[0] += (float)gsx; gs[ps] += (float)gsy; gs[2 * ps] += (float)gsz;
-                    gd[0] += (float)gdx; gd[ps] += (float)gdy; gd[2 * ps] += (float)gdz;
-                }
-            }
-            if (gx0) {                                                     // through the mean bone length (:110-113)
-                for (int e = 0; e < p.E; ++e) {
-                    const float* s = x0 + p.src[e] * p.M + m;
-                    const float* d = x0 + p.dst[e] * p.M + m;
-                    const double Bx = (double)__ldg(d) - __ldg(s), By = (double)__ldg(d + ps) - __ldg(s + ps),
-                                 Bz = (double)__ldg(d + 2 * ps) - __ldg(s + 2 * ps);
-                    const double nb = sqrt(Bx * Bx + By * By + Bz * Bz);
-                    if (nb > 0.0) {
-                        const double kc = G_c * (double)p.inv_E / nb;
-                        float* gs = gx0 + p.src[e] * p.M + m;
-                        float* gd = gx0 + p.dst[e] * p.M + m;
-                        gs[0] -= (float)(kc * Bx); gs[ps] -= (float)(kc * By); gs[2 * ps] -= (float)(kc * Bz);
-                        gd[0] += (float)(kc * Bx); gd[ps] += (float)(kc * By); gd[2 * ps] += (float)(kc * Bz);
-                    }
-                }
+            G_c += dL_damp * sqrt(PI) * (1.0 / den - 2.0 * c * u * u / (den * den));
+            float* gs = gx0 + si * p.M + m;
+            float* gd = gx0 + di * p.M + m;
+            gs[0] += (float)gsx; gs[ps] += (float)gsy; gs[2 * ps] += (float)gsz;
+            gd[0] += (float)gdx; gd[ps] += (float)gdy; gd[2 * ps] += (float)gdz;
+        }
+    }
+    if (gx0) {                                                         // through the mean bone length (:110-113)
+        for (int e = 0; e < p.E; ++e) {
+            const int si = p.src[e], di = p.dst[e];
+            const double Bx = (double)pos(di, m, 0) - pos(si, m, 0), By = (double)pos(di, m, 1) - pos(si, m, 1),
+                         Bz = (double)pos(di, m, 2) - pos(si, m, 2);
+            const double nb = sqrt(Bx * Bx + By * By + Bz * Bz);
+            if (nb > 0.0) {
+                const double kc = G_c * (double)p.inv_E / nb;
+                float* gs = gx0 + si * p.M + m;
+                float* gd = gx0 + di * p.M + m;
+                gs[0] -= (float)(kc * Bx); gs[ps] -= (float)(kc * By); gs[2 * ps] -= (float)(kc * Bz);
+                gd[0] += (float)(kc * Bx); gd[ps] += (float)(kc * By); gd[2 * ps] += (float)(kc * Bz);
             }
         }
     }
-    // block reduction, then one float64 atomic per block and parameter
+}
+
+// block reduction of the four parameter gradients, then one float64 atomic per block and parameter
+__device__ __forceinline__ void synth_adjoint_reduce(const BwdParams& p, double g_lam, double g_lx, double g_ly, double g_lz) {
     __shared__ double red[4][4];
     double vals[4] = {g_lam, g_lx, g_ly, g_lz};
 #pragma unroll
@@ -260,6 +256,61 @@ __global__ void __launch_bounds__(128) vr_synth_adjoint_kernel(const __grid_cons
         const double v = (red[threadIdx.x][0] + red[threadIdx.x][1]) + (red[threadIdx.x][2] + red[threadIdx.x][3]);
         if (v != 0.0) atomicAdd(p.gparams + threadIdx.x, v);
     }
+}
+
+__global__ void __launch_bounds__(128) vr_synth_adjoint_kernel(const __grid_constant__ BwdParams p) {
+    const int T = (int)p.T;
+    const long long total = p.N * (long long)T;
+    const float lam = __ldg(p.lam_ptr);
+    const float Lx = __ldg(p.loc_ptr), Ly = __ldg(p.loc_ptr + 1), Lz = __ldg(p.loc_ptr + 2);
+    const float lam_rcp = rcp_refined(lam);
+    double g_lam = 0.0, g_lx = 0.0, g_ly = 0.0, g_lz = 0.0;
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
+        const long long n = idx / T;
+        const int t = (int)(idx - n * T);
+        const double gI = (double)__ldg(p.gz + idx * 2), gQ = (double)__ldg(p.gz + idx * 2 + 1);
+        if (gI == 0.0 && gQ == 0.0) continue;
+        const float* x0 = p.x + (n * 3 * T + t) * (long long)p.VM;       // x-plane row of this time step
+        const long long ps = (long long)T * p.VM;                         // floats between coordinate planes
+        const int M = p.M;
+        auto pos = [&](int v, int m, int c) { return __ldg(x0 + v * M + m + c * ps); };
+        float* gx0 = p.gx ? p.gx + (n * 3 * T + t) * (long long)p.VM : nullptr;   // this thread's own rows of dL/dx
+        for (int m = 0; m < p.M; ++m)
+            synth_adjoint_body(p, pos, m, gI, gQ, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz, gx0, ps);
+    }
+    synth_adjoint_reduce(p, g_lam, g_lx, g_ly, g_lz);
+}
+
+// The same adjoint at the up-sampled steps of vr_forward_upsampled_f32 (T = ups_K * ups_T): the joint positions of step
+// i come from the per-interval cubics (pf_locate + pf_eval on p.coef), bit-identical to what vr_pad_frames_f32 writes.
+// Parameter gradients only.  (Staging the positions of a block's steps in shared memory first was measured slower on a
+// B200: 54.7 vs 38.6 ms per fwd+bwd step at N = 256, k = 250 -- occupancy drops to two blocks per SM.)
+__global__ void __launch_bounds__(128) vr_synth_adjoint_ups_kernel(const __grid_constant__ BwdParams p) {
+    const long long KT = p.T;
+    const long long total = p.N * KT;
+    const float lam = __ldg(p.lam_ptr);
+    const float Lx = __ldg(p.loc_ptr), Ly = __ldg(p.loc_ptr + 1), Lz = __ldg(p.loc_ptr + 2);
+    const float lam_rcp = rcp_refined(lam);
+    const int C3 = 3 * p.VM;
+    double g_lam = 0.0, g_lx = 0.0, g_ly = 0.0, g_lz = 0.0;
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
+        const long long n = idx / KT;
+        const long long i = idx - n * KT;
+        const double gI = (double)__ldg(p.gz + idx * 2), gQ = (double)__ldg(p.gz + idx * 2 + 1);
+        if (gI == 0.0 && gQ == 0.0) continue;
+        int j;
+        double tt;
+        pf_locate(i, p.ups_ratio, p.ups_T, j, tt);
+        const double* cf = p.coef + ((size_t)n * (p.ups_T - 1) + j) * 4 * C3;   // a0..a3 of interval j, C3 apart
+        const int M = p.M, VM = p.VM;
+        auto pos = [&](int v, int m, int c) {
+            const double* a = cf + c * VM + v * M + m;
+            return pf_eval(tt, __ldg(a), __ldg(a + C3), __ldg(a + 2 * C3), __ldg(a + 3 * C3));
+        };
+        for (int m = 0; m < p.M; ++m)
+            synth_adjoint_body(p, pos, m, gI, gQ, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz, nullptr, 0);
+    }
+    synth_adjoint_reduce(p, g_lam, g_lx, g_ly, g_lz);
 }
 #endif  // __CUDACC__
 

@@ -601,32 +601,43 @@ int vr_forward_host_f32(const float* x_host, int64_t N, int64_t T, int32_t V, in
 
 }  // extern "C"
 namespace {
-// Dataset.pad_frames on the device.  out_dev: the up-sampled batch, and/or coef_dev: only the spline
-// (per-interval cubics) for the fused radar kernel.
-int pad_launch(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M, int32_t num_pad_frames,
-               float sigma, float* out_dev, double* coef_dev, void* stream) {
-    if (!x_dev || (!out_dev && !coef_dev)) return fail(VR_ERR_ARG, "x_dev and out_dev must not be null");
+// scipy.ndimage._filters._gaussian_kernel1d(sigma, 0, radius), radius = int(4 * sigma + 0.5), float64; w[0] = centre
+int gaussian_weights(float sigma, int& radius, double* w) {
+    const double sd = (double)sigma;
+    radius = (int)(4.0 * sd + 0.5);
+    if (radius > vr::PF_MAX_RADIUS) return fail(VR_ERR_UNSUPPORTED, "sigma=%g needs a Gaussian radius of %d > %d", sd, radius, vr::PF_MAX_RADIUS);
+    double phi[2 * vr::PF_MAX_RADIUS + 1], sum = 0.0;
+    const double sigma2 = sd * sd;
+    for (int i = -radius; i <= radius; ++i) phi[i + radius] = exp(-0.5 / sigma2 * (double)(i * i));
+    for (int i = 0; i <= 2 * radius; ++i) sum += phi[i];
+    for (int j = 0; j <= radius; ++j) w[j] = phi[radius + j] / sum;
+    return VR_OK;
+}
+
+// the arguments vr_pad_frames_f32 and its backward pass accept
+int pad_check(int64_t N, int64_t T, int32_t V, int32_t M, int32_t num_pad_frames, float sigma) {
     if (N <= 0 || V <= 0 || M <= 0) return fail(VR_ERR_SHAPE, "N, V, M must be positive (got %lld, %d, %d)", (long long)N, V, M);
     if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames (scipy interp1d raises ValueError)", (long long)T);
     if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
     if (!(sigma > 0.f)) return fail(VR_ERR_SHAPE, "sigma must be positive, got %g", (double)sigma);
     if ((double)T * num_pad_frames > 2.0e9) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
+    return VR_OK;
+}
+
+// Dataset.pad_frames on the device.  out_dev: the up-sampled batch, and/or coef_dev: only the spline
+// (per-interval cubics) for the fused radar kernel.
+int pad_launch(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M, int32_t num_pad_frames,
+               float sigma, float* out_dev, double* coef_dev, void* stream) {
+    if (!x_dev || (!out_dev && !coef_dev)) return fail(VR_ERR_ARG, "x_dev and out_dev must not be null");
+    int rc = pad_check(N, T, V, M, num_pad_frames, sigma);
+    if (rc) return rc;
     int dev, sm_count;
-    int rc = device_setup(dev, sm_count);
+    rc = device_setup(dev, sm_count);
     if (rc) return rc;
     vr::PadParams p;
     memset(&p, 0, sizeof(p));
-    // scipy.ndimage._filters._gaussian_kernel1d(sigma, 0, radius), radius = int(4 * sigma + 0.5), float64
-    const double sd = (double)sigma;
-    p.radius = (int)(4.0 * sd + 0.5);
-    if (p.radius > vr::PF_MAX_RADIUS) return fail(VR_ERR_UNSUPPORTED, "sigma=%g needs a Gaussian radius of %d > %d", sd, p.radius, vr::PF_MAX_RADIUS);
-    {
-        double phi[2 * vr::PF_MAX_RADIUS + 1], sum = 0.0;
-        const double sigma2 = sd * sd;
-        for (int i = -p.radius; i <= p.radius; ++i) phi[i + p.radius] = exp(-0.5 / sigma2 * (double)(i * i));
-        for (int i = 0; i <= 2 * p.radius; ++i) sum += phi[i];
-        for (int j = 0; j <= p.radius; ++j) p.w[j] = phi[p.radius + j] / sum;
-    }
+    rc = gaussian_weights(sigma, p.radius, p.w);
+    if (rc) return rc;
     p.x = x_dev; p.out = out_dev; p.coef = coef_dev;
     p.planes = N * 3; p.T = (int)T; p.VM = V * M; p.K = num_pad_frames;
     p.ratio = (double)(T - 1) / (double)((long long)num_pad_frames * T - 1);
@@ -663,6 +674,50 @@ int vr_pad_frames_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32
     return pad_launch(x_dev, N, T, V, M, num_pad_frames, sigma, out_dev, nullptr, stream);
 }
 
+int vr_pad_frames_backward_f32(const float* grad_out_dev, int64_t N, int64_t T, int32_t V, int32_t M, int32_t num_pad_frames,
+                               float sigma, float* grad_x_dev, void* stream) {
+    if (!grad_out_dev || !grad_x_dev) return fail(VR_ERR_ARG, "grad_out_dev and grad_x_dev must not be null");
+    int rc = pad_check(N, T, V, M, num_pad_frames, sigma);
+    if (rc) return rc;
+    int dev, sm_count;
+    rc = device_setup(dev, sm_count);
+    if (rc) return rc;
+    vr::PadBwdParams p;
+    memset(&p, 0, sizeof(p));
+    rc = gaussian_weights(sigma, p.radius, p.w);
+    if (rc) return rc;
+    if (T > 200 * 1024 / 20)                                     // the forward's limit (vr_pad_frames_f32)
+        return fail(VR_ERR_UNSUPPORTED, "T=%lld too long for the shared-memory spline solve (max %d frames)", (long long)T, 200 * 1024 / 20);
+    {
+        double c = 0.0;                                          // the forward's Thomas recurrence, bit for bit
+        for (int i = 2; i < vr::PF_CP_N; ++i) { c = 1.0 / (4.0 - c); p.cp[i] = c; }
+        if (1.0 / (4.0 - c) != c) return fail(VR_ERR_UNSUPPORTED, "Thomas coefficients did not reach their fixed point");
+    }
+    p.g = grad_out_dev; p.gx = grad_x_dev;
+    p.planes = N * 3; p.T = (int)T; p.VM = V * M; p.K = num_pad_frames;
+    p.ratio = (double)(T - 1) / (double)((long long)num_pad_frames * T - 1);
+    // columns per CTA: 16 bytes per (frame, column) of shared memory (dL/dys and dL/dM in float64)
+    long long nc = (200 * 1024) / (16ll * T);
+    nc = std::min<long long>(std::min<long long>(nc, p.VM), 1024);
+    p.ncb = (int)((p.VM + nc - 1) / nc);
+    p.nc = (int)((p.VM + p.ncb - 1) / p.ncb);
+    const size_t smem = (size_t)p.T * p.nc * 16;
+    static std::mutex mu;
+    static bool attr_done[64] = {false};
+    {
+        std::lock_guard<std::mutex> lk(mu);
+        if (!attr_done[dev]) {
+            CUDA_TRY(cudaFuncSetAttribute(vr::vr_pad_frames_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            attr_done[dev] = true;
+        }
+    }
+    const long long units = p.planes * p.ncb;
+    const int grid = (int)std::min<long long>(units, (long long)sm_count * 4);
+    vr::vr_pad_frames_backward_kernel<<<grid, 1024, smem, (cudaStream_t)stream>>>(p);
+    CUDA_TRY(cudaGetLastError());
+    return VR_OK;
+}
+
 int vr_pad_frames_joints(const void* x_dev, int32_t x_is_f64, int64_t N, int64_t T, int32_t V, int32_t C,
                          int32_t num_pad_frames, float sigma, int32_t planar_out, float* out_dev, void* stream) {
     if (!x_dev || !out_dev) return fail(VR_ERR_ARG, "x_dev and out_dev must not be null");
@@ -676,16 +731,8 @@ int vr_pad_frames_joints(const void* x_dev, int32_t x_is_f64, int64_t N, int64_t
     if (rc) return rc;
     vr::PadNbParams p;
     memset(&p, 0, sizeof(p));
-    const double sd = (double)sigma;
-    p.radius = (int)(4.0 * sd + 0.5);
-    if (p.radius > vr::PF_MAX_RADIUS) return fail(VR_ERR_UNSUPPORTED, "sigma=%g needs a Gaussian radius of %d > %d", sd, p.radius, vr::PF_MAX_RADIUS);
-    {
-        double phi[2 * vr::PF_MAX_RADIUS + 1], sum = 0.0;
-        const double sigma2 = sd * sd;
-        for (int i = -p.radius; i <= p.radius; ++i) phi[i + p.radius] = exp(-0.5 / sigma2 * (double)(i * i));
-        for (int i = 0; i <= 2 * p.radius; ++i) sum += phi[i];
-        for (int j = 0; j <= p.radius; ++j) p.w[j] = phi[p.radius + j] / sum;
-    }
+    rc = gaussian_weights(sigma, p.radius, p.w);
+    if (rc) return rc;
     p.x = x_dev; p.out = out_dev; p.N = N; p.T = (int)T; p.V = V; p.C = C; p.K = num_pad_frames; p.planar = planar_out ? 1 : 0;
     p.ratio = (double)(T - 1) / (double)((long long)num_pad_frames * T - 1);
     const long long VC = (long long)V * C;
@@ -730,12 +777,14 @@ int64_t vr_upsampled_workspace_bytes(int64_t N, int64_t T, int32_t V, int32_t M)
     return N * (T - 1) * 4 * 3 * (int64_t)V * M * (int64_t)sizeof(double);
 }
 
-int vr_forward_upsampled_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
-                             const int32_t* src_host, const int32_t* dst_host, int32_t E,
-                             const float* wavelength_dev, const float* radar_loc_dev,
-                             int32_t n_fft, int32_t hop, uint32_t flags,
-                             int32_t num_pad_frames, float sigma, int32_t image_size,
-                             void* workspace_dev, int64_t workspace_bytes, float* out_dev, void* stream) {
+}  // extern "C"
+namespace {
+int upsampled_impl(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
+                   const int32_t* src_host, const int32_t* dst_host, int32_t E,
+                   const float* wavelength_dev, const float* radar_loc_dev,
+                   int32_t n_fft, int32_t hop, uint32_t flags,
+                   int32_t num_pad_frames, float sigma, int32_t image_size,
+                   void* workspace_dev, int64_t workspace_bytes, float* out_dev, float* iq_dev, void* stream) {
     if (!wavelength_dev || !radar_loc_dev) return fail(VR_ERR_ARG, "wavelength_dev and radar_loc_dev must not be null");
     if (!x_dev || !out_dev || !workspace_dev) return fail(VR_ERR_ARG, "x_dev, out_dev and workspace_dev must not be null");
     if (image_size < 0) return fail(VR_ERR_SHAPE, "image_size must be >= 0, got %d", image_size);
@@ -751,7 +800,29 @@ int vr_forward_upsampled_f32(const float* x_dev, int64_t N, int64_t T, int32_t V
     int rc = pad_launch(x_dev, N, T, V, M, num_pad_frames, sigma, nullptr, coef, stream);
     if (rc) return rc;
     return launch(x_dev, N, T * num_pad_frames, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
-                  n_fft, hop, flags, image_size, out_dev, nullptr, (cudaStream_t)stream, coef, (int)T, num_pad_frames);
+                  n_fft, hop, flags, image_size, out_dev, iq_dev, (cudaStream_t)stream, coef, (int)T, num_pad_frames);
+}
+}  // namespace
+extern "C" {
+
+int vr_forward_upsampled_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
+                             const int32_t* src_host, const int32_t* dst_host, int32_t E,
+                             const float* wavelength_dev, const float* radar_loc_dev,
+                             int32_t n_fft, int32_t hop, uint32_t flags,
+                             int32_t num_pad_frames, float sigma, int32_t image_size,
+                             void* workspace_dev, int64_t workspace_bytes, float* out_dev, void* stream) {
+    return upsampled_impl(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, n_fft, hop, flags,
+                          num_pad_frames, sigma, image_size, workspace_dev, workspace_bytes, out_dev, nullptr, stream);
+}
+
+int vr_forward_upsampled_debug_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
+                                   const int32_t* src_host, const int32_t* dst_host, int32_t E,
+                                   const float* wavelength_dev, const float* radar_loc_dev,
+                                   int32_t n_fft, int32_t hop, uint32_t flags, int32_t num_pad_frames, float sigma,
+                                   void* workspace_dev, int64_t workspace_bytes, float* out_dev, float* iq_dev, void* stream) {
+    if (!iq_dev) return fail(VR_ERR_ARG, "iq_dev must not be null");
+    return upsampled_impl(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, n_fft, hop, flags,
+                          num_pad_frames, sigma, 0, workspace_dev, workspace_bytes, out_dev, iq_dev, stream);
 }
 
 int vr_backward_params_f32(const float* x_dev, const float* iq_dev, const float* grad_out_dev,
@@ -771,7 +842,8 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
                   const int32_t* src_host, const int32_t* dst_host, int32_t E,
                   const float* wavelength_dev, const float* radar_loc_dev,
                   int32_t n_fft, int32_t hop, uint32_t flags, bool synth_only,
-                  float* gz_work_dev, double* grad_params_dev, float* grad_x_dev, void* stream);
+                  float* gz_work_dev, double* grad_params_dev, float* grad_x_dev, void* stream,
+                  const double* coef = nullptr, int ups_T = 0, int ups_K = 0);
 }  // namespace
 extern "C" {
 
@@ -794,6 +866,22 @@ int vr_backward_f32(const float* x_dev, const float* iq_dev, const float* grad_o
                          n_fft, hop, flags, false, gz_work_dev, grad_params_dev, grad_x_dev, stream);
 }
 
+int vr_backward_upsampled_params_f32(const void* workspace_dev, const float* iq_dev, const float* grad_out_dev,
+                                     int64_t N, int64_t T, int32_t V, int32_t M,
+                                     const int32_t* src_host, const int32_t* dst_host, int32_t E,
+                                     const float* wavelength_dev, const float* radar_loc_dev,
+                                     int32_t n_fft, int32_t hop, uint32_t flags, int32_t num_pad_frames,
+                                     float* gz_work_dev, double* grad_params_dev, void* stream) {
+    if (!workspace_dev) return fail(VR_ERR_ARG, "workspace_dev must not be null");
+    if (((uintptr_t)workspace_dev & 7) != 0) return fail(VR_ERR_ARG, "workspace_dev must be 8-byte aligned");
+    if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames", (long long)T);
+    if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
+    if ((double)T * num_pad_frames > (double)(1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
+    return backward_impl(nullptr, iq_dev, grad_out_dev, N, T * num_pad_frames, V, M, src_host, dst_host, E, wavelength_dev,
+                         radar_loc_dev, n_fft, hop, flags, false, gz_work_dev, grad_params_dev, nullptr, stream,
+                         static_cast<const double*>(workspace_dev), (int)T, num_pad_frames);
+}
+
 }  // extern "C"
 namespace {
 int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out_dev,
@@ -801,9 +889,11 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
                   const int32_t* src_host, const int32_t* dst_host, int32_t E,
                   const float* wavelength_dev, const float* radar_loc_dev,
                   int32_t n_fft, int32_t hop, uint32_t flags, bool synth_only,
-                  float* gz_work_dev, double* grad_params_dev, float* grad_x_dev, void* stream) {
-    // synth_only: gz_work_dev already holds dL/d(iq); the adjoint STFT is skipped
-    if (!x_dev || !gz_work_dev || !grad_params_dev || !wavelength_dev || !radar_loc_dev || (!synth_only && (!iq_dev || !grad_out_dev)))
+                  float* gz_work_dev, double* grad_params_dev, float* grad_x_dev, void* stream,
+                  const double* coef, int ups_T, int ups_K) {
+    // synth_only: gz_work_dev already holds dL/d(iq); the adjoint STFT is skipped.  coef != nullptr: the joint positions are
+    // the up-sampling spline's (T = ups_K * ups_T steps, x_dev unused), parameter gradients only
+    if ((!x_dev && !coef) || !gz_work_dev || !grad_params_dev || !wavelength_dev || !radar_loc_dev || (!synth_only && (!iq_dev || !grad_out_dev)))
         return fail(VR_ERR_ARG, "device pointers must not be null");
     if (flags & ~VR_FLAG_RANGE_FMA) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
     if (N <= 0 || T <= 0 || V <= 0 || M <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M, hop must be positive");
@@ -829,6 +919,8 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     p.F = (int)(T / hop) + 1;
     p.fma_range = (flags & VR_FLAG_RANGE_FMA) ? 1 : 0;
     p.inv_E = 1.0f / (float)E;
+    p.coef = coef; p.ups_T = ups_T;
+    p.ups_ratio = coef ? (double)(ups_T - 1) / (double)((long long)ups_K * ups_T - 1) : 0.0;
     cudaStream_t st = (cudaStream_t)stream;
     if (grad_x_dev) CUDA_TRY(cudaMemsetAsync(grad_x_dev, 0, (size_t)N * 3 * T * V * M * sizeof(float), st));
     if (!synth_only) {
@@ -840,7 +932,8 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     }
     const long long steps = N * T;
     const int grid2 = (int)std::min<long long>((steps + 127) / 128, (long long)sm_count * 16);
-    vr::vr_synth_adjoint_kernel<<<grid2, 128, 0, st>>>(p);
+    if (coef) vr::vr_synth_adjoint_ups_kernel<<<grid2, 128, 0, st>>>(p);
+    else vr::vr_synth_adjoint_kernel<<<grid2, 128, 0, st>>>(p);
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
 }

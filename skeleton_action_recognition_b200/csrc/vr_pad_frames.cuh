@@ -162,6 +162,177 @@ __global__ void __launch_bounds__(1024, 1) vr_pad_frames_kernel(const __grid_con
 #endif  // __CUDACC__
 
 // ------------------------------------------------------------------------------------------------
+// Backward pass of vr_pad_frames_kernel: dL/d(out) (N,3,k*T,V,M) -> dL/dx (N,3,T,V,M), both float32.
+//
+// Definition: the gradient is the transpose of the float64 linear operator the forward evaluates (Gaussian ->
+// not-a-knot spline solve -> per-interval cubics -> Horner evaluation at the k*T positions).  The two float32
+// roundings of the forward (the smoothed samples ys and the output) pass the gradient through unchanged, as autograd
+// treats a dtype cast.  Everything is float64 and rounded to float32 once, at the end; no atomics, so the result is
+// bitwise reproducible.  Stages, in reverse order of the forward's:
+//   (1) evaluation: ga_q[j] = sum over the output rows i of interval j of tt_i^q g_i, q = 0..3, with the forward's own
+//       pf_locate (the last row is clamped into interval T-2 there too).  The rows of an interval are contiguous: one warp,
+//       lanes = columns, walks them in order (coalesced, fixed summation order);
+//   (2) pf_cubic: (ga0..ga3) of interval j -> gy_j, gy_{j+1}, gM_j, gM_{j+1} (even intervals first, then odd ones: no two
+//       intervals of a pass share an end point);
+//   (3) the spline solve run backwards, one thread per column: end extrapolations, back substitution, forward sweep, the
+//       direct rows M1 = rhs1 / 6 and M(T-2) = rhs(T-2) / 6, and the second differences of the right-hand sides;
+//   (4) the reflect-padded Gaussian transposed: dL/dx[s] gathers w[|u - t|] gys[t] over every u that pf_reflect folds
+//       onto s (a radius larger than T folds several times, exactly as the forward does).
+// Shared memory: 16 bytes per (frame, column).  The Thomas coefficients c'_i reach their float64 fixed point at i = 15;
+// the host computes them (the forward's recurrence) into `cp` and the kernel reads c'_i = cp[min(i, PF_CP_N - 1)].
+constexpr int PF_CP_N = 32;
+
+struct PadBwdParams {
+    const float* g;              // (N,3,k*T,V,M) dL/d(out)
+    float* gx;                   // (N,3,T,V,M)   dL/dx, overwritten
+    long long planes;            // N*3
+    int T, VM, K, nc, ncb;
+    int radius;
+    double ratio;                // as PadParams::ratio
+    double w[PF_MAX_RADIUS + 1];
+    double cp[PF_CP_N];          // c'_i of the forward's Thomas sweep, i < PF_CP_N (entries 0, 1 unused)
+};
+
+#ifdef __CUDACC__
+// first output row of interval j (rows i with pf_locate(i) == j are [pf_first_row(j), pf_first_row(j+1)))
+__device__ __forceinline__ long long pf_first_row(int j, double ratio, int T, long long KT) {
+    if (j <= 0) return 0;
+    if (j > T - 2) return KT;
+    long long i = (long long)((double)j / ratio);
+    i = i < 2 ? 0 : i - 2;
+    int jj;
+    double tt;
+    for (;; ++i) {                                               // pf_locate is monotone in i: the first row not below j
+        pf_locate(i, ratio, T, jj, tt);
+        if (jj >= j) break;
+    }
+    while (i > 0) {
+        pf_locate(i - 1, ratio, T, jj, tt);
+        if (jj < j) break;
+        --i;
+    }
+    return i;
+}
+
+__global__ void __launch_bounds__(1024, 1) vr_pad_frames_backward_kernel(const __grid_constant__ PadBwdParams p) {
+    extern __shared__ __align__(16) unsigned char pf_smem[];
+    const int T = p.T, nc = p.nc;
+    double* Y = reinterpret_cast<double*>(pf_smem);               // [T][nc] dL/dys
+    double* G = Y + (size_t)T * nc;                               // [T][nc] dL/dM, then dL/d(rhs), then dL/dx
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
+    const long long KT = (long long)p.K * T;
+    auto cp = [&](int i) { return p.cp[i < PF_CP_N ? i : PF_CP_N - 1]; };
+
+    for (long long unit = blockIdx.x; unit < p.planes * p.ncb; unit += gridDim.x) {
+        const long long plane = unit / p.ncb;
+        const int col0 = (int)(unit - plane * p.ncb) * nc;
+        const int ncl = (p.VM - col0 < nc) ? (p.VM - col0) : nc;
+        const int ngr = (ncl + 31) >> 5;                          // 32-column groups
+        const float* gp = p.g + plane * KT * p.VM + col0;
+        __syncthreads();                                          // previous unit's gather has finished with shared memory
+        for (int idx = tid; idx < 2 * T * nc; idx += blockDim.x) Y[idx] = 0.0;
+        __syncthreads();
+
+        // (1) + (2): interval sums, mapped through pf_cubic; even intervals, then odd ones
+        for (int parity = 0; parity < 2; ++parity) {
+            const int nint = (T - 1 - parity + 1) / 2;            // intervals j = parity, parity + 2, ... <= T - 2
+            for (int task = warp; task < nint * ngr; task += nwarps) {
+                const int j = parity + 2 * (task / ngr);
+                const int c = (task - (task / ngr) * ngr) * 32 + lane;
+                const long long lo = pf_first_row(j, p.ratio, T, KT), hi = pf_first_row(j + 1, p.ratio, T, KT);
+                double ga0 = 0.0, ga1 = 0.0, ga2 = 0.0, ga3 = 0.0;
+                if (c < ncl) {
+                    const float* gc = gp + c;
+                    long long i = lo;
+                    for (; i + 4 <= hi; i += 4) {                 // four loads in flight ahead of the FP64 chain
+                        float v[4];
+#pragma unroll
+                        for (int u = 0; u < 4; ++u) v[u] = __ldg(gc + (i + u) * p.VM);
+#pragma unroll
+                        for (int u = 0; u < 4; ++u) {
+                            int jj;
+                            double tt;
+                            pf_locate(i + u, p.ratio, T, jj, tt);
+                            const double gv = (double)v[u], t2 = tt * tt;
+                            ga0 += gv; ga1 += tt * gv; ga2 += t2 * gv; ga3 += (t2 * tt) * gv;
+                        }
+                    }
+                    for (; i < hi; ++i) {
+                        int jj;
+                        double tt;
+                        pf_locate(i, p.ratio, T, jj, tt);
+                        const double gv = (double)__ldg(gc + i * p.VM), t2 = tt * tt;
+                        ga0 += gv; ga1 += tt * gv; ga2 += t2 * gv; ga3 += (t2 * tt) * gv;
+                    }
+                    // a0 = y0, a1 = (y1 - y0) - (2 m0 + m1) / 6, a2 = m0 / 2, a3 = (m1 - m0) / 6
+                    Y[j * nc + c] += ga0 - ga1;
+                    Y[(j + 1) * nc + c] += ga1;
+                    G[j * nc + c] += (0.5 * ga2 - (2.0 / 6.0) * ga1) - (1.0 / 6.0) * ga3;
+                    G[(j + 1) * nc + c] += (1.0 / 6.0) * (ga3 - ga1);
+                }
+            }
+            __syncthreads();
+        }
+
+        // (3) the not-a-knot solve backwards, one thread per column (in place in G)
+        if (tid < ncl) {
+            const int c = tid;
+            double* g = G + c;
+            // M(T-1) = 2 M(T-2) - M(T-3), M0 = 2 M1 - M2 (the forward's last two statements, reversed)
+            g[(T - 2) * nc] += 2.0 * g[(T - 1) * nc];
+            g[(T - 3) * nc] -= g[(T - 1) * nc];
+            g[1 * nc] += 2.0 * g[0];
+            g[2 * nc] -= g[0];
+            g[0] = 0.0;
+            g[(T - 1) * nc] = 0.0;
+            // back substitution M_i = d_i - c'_i M_{i+1}, i = T-4 .. 2 (and M(T-3) = d(T-3)): g[i] becomes dL/dd_i
+            for (int i = 2; i <= T - 4; ++i) g[(i + 1) * nc] -= cp(i) * g[i * nc];
+            // forward sweep d_i = (r_i - d_{i-1}) c'_i, i = 2 .. T-3: g[i] becomes dL/dr_i = dL/d(rhs_i);
+            // r_2 -= M1, r(T-3) -= M(T-2)
+            for (int i = T - 3; i >= 2; --i) {
+                const double gr = g[i * nc] * cp(i);
+                g[i * nc] = gr;
+                if (i > 2) g[(i - 1) * nc] -= gr;
+            }
+            if (T >= 5) {
+                g[1 * nc] -= g[2 * nc];
+                g[(T - 2) * nc] -= g[(T - 3) * nc];
+            }
+            // M1 = rhs1 / 6, M(T-2) = rhs(T-2) / 6
+            g[1 * nc] /= 6.0;
+            g[(T - 2) * nc] /= 6.0;
+        }
+        __syncthreads();
+        // rhs_i = 6 ((ys_{i-1} - 2 ys_i) + ys_{i+1}), i = 1 .. T-2 (G[0] = G[T-1] = 0)
+        for (int idx = tid; idx < T * ncl; idx += blockDim.x) {
+            const int t = idx / ncl, c = idx - t * ncl;
+            const double gm = t > 0 ? G[(t - 1) * nc + c] : 0.0, gq = t < T - 1 ? G[(t + 1) * nc + c] : 0.0;
+            Y[t * nc + c] += 6.0 * ((gm + gq) - 2.0 * G[t * nc + c]);
+        }
+        __syncthreads();
+
+        // (4) transposed Gaussian: ys[t] = sum_{|u - t| <= r} w[|u - t|] x[pf_reflect(u)]; dL/dx[s] sums over the u that
+        // fold onto s -- they lie in {s + 2Tm} and {2Tm - 1 - s} (the folds map each family onto itself)
+        float* gxp = p.gx + plane * (long long)T * p.VM + col0;
+        const int r = p.radius, mlim = r / (2 * T) + 1;
+        for (int idx = tid; idx < T * ncl; idx += blockDim.x) {
+            const int s = idx / ncl, c = idx - s * ncl;
+            double acc = 0.0;
+            for (int m = -mlim; m <= mlim; ++m) {
+                for (int fam = 0; fam < 2; ++fam) {
+                    const int u = fam == 0 ? s + 2 * T * m : 2 * T * m - 1 - s;
+                    if (u < -r || u > T - 1 + r || pf_reflect(u, T) != s) continue;
+                    const int t0 = u - r > 0 ? u - r : 0, t1 = u + r < T - 1 ? u + r : T - 1;
+                    for (int t = t0; t <= t1; ++t) acc += p.w[t > u ? t - u : u - t] * Y[t * nc + c];
+                }
+            }
+            gxp[(size_t)s * p.VM + c] = (float)acc;
+        }
+    }
+}
+#endif  // __CUDACC__
+
+// ------------------------------------------------------------------------------------------------
 // The notebook's variant: `utils.pad_frames` (reference utils.py:82-89), used by virtual_radar_example.ipynb
 // cells 2-4 on (T, V, C) arrays of ONE body:
 //

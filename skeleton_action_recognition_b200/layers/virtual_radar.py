@@ -208,6 +208,51 @@ class _SynthFunction(torch.autograd.Function):
         return g_lam, g_loc, gx, None, None
 
 
+class _UpsampledRadarFunction(torch.autograd.Function):
+    """forward_upsampled() with gradients for `wavelength` and `radar_location`, without the up-sampled batch: the forward
+    is the fused up-sampling + radar launch, asked to also save the complex baseband signal (vr_forward_upsampled_debug_f32);
+    the spline's per-interval cubics stay in the workspace, from which the backward (vr_backward_upsampled_params_f32)
+    re-evaluates the joint positions of every up-sampled step."""
+
+    @staticmethod
+    def forward(ctx, lam, loc, xc, layer, k, sigma):
+        N, _, T, V, M = xc.shape
+        L = _cabi.lib()
+        nbytes = int(L.vr_upsampled_workspace_bytes(N, T, V, M))
+        work = torch.empty(max(nbytes, 8) // 8, dtype=torch.float64, device=xc.device)
+        out = torch.empty((N, layer.n_fft, (k * T) // layer.hop_length + 1), dtype=torch.float32, device=xc.device)
+        iq = torch.empty((N, k * T, 2), dtype=torch.float32, device=xc.device)
+        with torch.cuda.device(xc.device):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
+            rc = L.vr_forward_upsampled_debug_f32(xc.data_ptr(), N, T, V, M, layer._src_c, layer._dst_c, len(layer.src),
+                                                  lam.data_ptr(), loc.data_ptr(), layer.n_fft, layer.hop_length, 0,
+                                                  k, ctypes.c_float(float(sigma)), work.data_ptr(), nbytes,
+                                                  out.data_ptr(), iq.data_ptr(), stream)
+        _cabi.check(rc)
+        ctx.save_for_backward(lam, loc, work, iq)
+        ctx.layer, ctx.dims = layer, (N, T, V, M, k)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        lam, loc, work, iq = ctx.saved_tensors
+        layer = ctx.layer
+        N, T, V, M, k = ctx.dims
+        g = grad_out.contiguous().to(torch.float32)
+        gz = torch.empty_like(iq)
+        gp = torch.zeros(4, dtype=torch.float64, device=iq.device)
+        with torch.cuda.device(iq.device):
+            stream = torch.cuda.current_stream(iq.device).cuda_stream
+            rc = _cabi.lib().vr_backward_upsampled_params_f32(work.data_ptr(), iq.data_ptr(), g.data_ptr(), N, T, V, M,
+                                                              layer._src_c, layer._dst_c, len(layer.src),
+                                                              lam.data_ptr(), loc.data_ptr(), layer.n_fft, layer.hop_length,
+                                                              0, k, gz.data_ptr(), gp.data_ptr(), ctypes.c_void_p(stream))
+        _cabi.check(rc)
+        g_lam = gp[0].to(torch.float32).reshape(lam.shape) if ctx.needs_input_grad[0] else None
+        g_loc = gp[1:4].to(torch.float32).reshape(loc.shape) if ctx.needs_input_grad[1] else None
+        return g_lam, g_loc, None, None, None, None
+
+
 class VirtualRadar(torch.nn.Module):
     """Skeleton sequences -> micro-Doppler log-spectrograms on a B200 (see module docstring)."""
 
@@ -405,7 +450,10 @@ class VirtualRadar(torch.nn.Module):
         `self.forward_image(pad_frames(...), image_size)` when `image_size` is given -- bit for bit,
         without the `num_pad_frames`-times larger batch ever existing in HBM (C ABI
         vr_forward_upsampled_f32; replaces reference utils.py:128-140 + layers/virtual_radar.py:79-134
-        [+ models/resnet.py:24-26])."""
+        [+ models/resnet.py:24-26]).  Trainable `wavelength` / `radar_location` keep the fused path
+        (vr_forward_upsampled_debug_f32 + vr_backward_upsampled_params_f32); with `image_size` the
+        spectrogram is then resized by `F.interpolate`, as `forward_image` does under grad.  Gradients
+        with respect to x itself go through `self(pad_frames(x, num_pad_frames, sigma))`."""
         self._check_input(x)
         lam, loc = self._check_device(x)
         xc = x.contiguous()
@@ -415,12 +463,15 @@ class VirtualRadar(torch.nn.Module):
         if image_size is not None and img < 1:
             raise ValueError("image_size must be positive, got %d" % img)
         if x.requires_grad and torch.is_grad_enabled():
-            raise NotImplementedError("the temporal up-sampling has no backward pass: detach x, or differentiate "
-                                      "forward() on an already up-sampled batch")
-        if self._needs_grad() or self._general_stft():      # trainable parameters / general STFT kernels: materialise the up-sampled batch
+            raise NotImplementedError("forward_upsampled has no gradient with respect to x: detach x, or differentiate "
+                                      "layer(pad_frames(x, num_pad_frames, sigma)), which materialises the up-sampled batch")
+        if self._general_stft():      # general STFT kernels: materialise the up-sampled batch
             from ..upsample import pad_frames
             up = pad_frames(xc, k, sigma)
             return self.forward_image(up, img) if img else self.forward(up)
+        if self._needs_grad() and N > 0:
+            out = _UpsampledRadarFunction.apply(lam, loc, xc, self, k, sigma)
+            return torch.nn.functional.interpolate(out.unsqueeze(1), img) if img else out
         shape = (N, 1, img, img) if img else (N, self.n_fft, (k * T) // self.hop_length + 1)
         out = torch.empty(shape, dtype=torch.float32, device=x.device)
         if N == 0:

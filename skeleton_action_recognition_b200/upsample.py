@@ -3,7 +3,9 @@ replacement for the reference data loader's `Dataset.pad_frames` (utils.py:134-1
 cast of `Dataset.__getitem__` (utils.py:128-132): Gaussian smoothing along time (scipy
 `gaussian_filter1d`, reflect boundary, float64 accumulation, float32 result) followed by not-a-knot
 cubic interpolation (scipy `interp1d(..., 'cubic')`) to `num_pad_frames * T` frames, evaluated in
-float64 and rounded to float32.  One CUDA kernel through the C ABI (`vr_pad_frames_f32`); no CPU path."""
+float64 and rounded to float32.  One CUDA kernel through the C ABI (`vr_pad_frames_f32`); no CPU path.
+Differentiable: under grad mode, an `x` that requires grad gets dL/dx from `vr_pad_frames_backward_f32` (the transpose
+of the float64 linear operator; the float32 roundings pass the gradient through as a dtype cast does)."""
 import ctypes
 
 import torch
@@ -11,9 +13,43 @@ import torch
 from . import _cabi
 
 
+def _launch(xb, k, sigma, out):
+    N, _, T, V, M = xb.shape
+    with torch.cuda.device(xb.device):
+        stream = torch.cuda.current_stream(xb.device).cuda_stream
+        rc = _cabi.lib().vr_pad_frames_f32(xb.data_ptr(), N, T, V, M, k, ctypes.c_float(float(sigma)),
+                                           out.data_ptr(), ctypes.c_void_p(stream))
+    _cabi.check(rc)
+
+
+class _PadFramesFunction(torch.autograd.Function):
+    """pad_frames with a backward pass (C ABI vr_pad_frames_backward_f32).  `out` is written in place and marked dirty,
+    so that the `out=` form carries the graph too."""
+
+    @staticmethod
+    def forward(ctx, xb, k, sigma, out):
+        _launch(xb, k, sigma, out)
+        ctx.mark_dirty(out)
+        ctx.dims = (tuple(xb.shape), k, sigma)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        (N, C, T, V, M), k, sigma = ctx.dims
+        g = grad_out.contiguous().to(torch.float32)
+        gx = torch.empty((N, C, T, V, M), dtype=torch.float32, device=g.device)
+        with torch.cuda.device(g.device):
+            stream = torch.cuda.current_stream(g.device).cuda_stream
+            rc = _cabi.lib().vr_pad_frames_backward_f32(g.data_ptr(), N, T, V, M, k, ctypes.c_float(float(sigma)),
+                                                        gx.data_ptr(), ctypes.c_void_p(stream))
+        _cabi.check(rc)
+        return gx, None, None, None
+
+
 def pad_frames(x, num_pad_frames=250, sigma=3, out=None):
     """x: (N,3,T,V,M) or a single sample (3,T,V,M), float32 CUDA tensor -> same rank with
-    `num_pad_frames * T` frames.  Defaults are the reference's (utils.py:105)."""
+    `num_pad_frames * T` frames.  Defaults are the reference's (utils.py:105).  Differentiable with
+    respect to x (also through `out=`); without grad the result carries no graph."""
     if not isinstance(x, torch.Tensor) or x.dim() not in (4, 5):
         raise ValueError("expected a (N,3,T,V,M) or (3,T,V,M) tensor")
     if x.dtype != torch.float32:
@@ -33,11 +69,10 @@ def pad_frames(x, num_pad_frames=250, sigma=3, out=None):
         raise ValueError("expected 3 coordinate planes, got %d" % C)
     if N == 0:
         return out[0] if single else out
-    with torch.cuda.device(x.device):
-        stream = torch.cuda.current_stream(x.device).cuda_stream
-        rc = _cabi.lib().vr_pad_frames_f32(xb.data_ptr(), N, T, V, M, k, ctypes.c_float(float(sigma)),
-                                           out.data_ptr(), ctypes.c_void_p(stream))
-    _cabi.check(rc)
+    if torch.is_grad_enabled() and x.requires_grad:
+        out = _PadFramesFunction.apply(xb, k, sigma, out)
+    else:
+        _launch(xb, k, sigma, out)
     return out[0] if single else out
 
 
