@@ -9,6 +9,10 @@ Two independent routes, both on the CPU:
   analytic_grads   the closed form the CUDA kernels implement (csrc/vr_backward.cuh), written with numpy in
                    float64: adjoint of the windowed STFT + log magnitude, then the derivatives of
                    z = sum amp * exp(j theta).  tests/test_oracle.py pins it to autograd_grads.
+  synth_adjoint    the second stage alone (dL/d(iq) -> parameter and skeleton gradients) with the CUDA kernel's
+                   deliberate roundings: float32 range, phase and mean bone length, float64 everything else, in the
+                   kernel's order of operations.  It returns each path of the gradient separately, and the sums of
+                   absolute terms from which tests/test_backward_property_gpu.py derives its tolerances.
 """
 import numpy as np
 import torch
@@ -103,3 +107,119 @@ def analytic_grads(x, grad_out, edges=vro.NTU_EDGES, wavelength=1e-3, radar_loca
         gx[:, :, :, si] += gS[:, :, :, e]
         gx[:, :, :, di] += gD[:, :, :, e]
     return float(g_lam), g_loc, gx
+
+
+PATHS = ("phase", "u", "length")
+
+
+def _bone_lengths_f32(S, D, mode):
+    """|D - S| of every bone in float32 as the kernel rounds it: float32 B = D - S, norm in the layout's mode."""
+    loc0 = np.zeros(3, np.float32)
+    _, ln = vro.aspect_cosine_c(torch.from_numpy(np.ascontiguousarray(S)), torch.from_numpy(np.ascontiguousarray(D)),
+                                loc0, mode)
+    return ln.numpy()
+
+
+def synth_adjoint(x, giq, edges=vro.NTU_EDGES, wavelength=1e-3, radar_location=(0., 0., 0.), mode="seq",
+                  theta32=True, cbar32=True):
+    """The synthesis adjoint of csrc/vr_backward.cuh (synth_adjoint_body) in numpy.
+
+    x (N,3,T,V,M) float32, giq = dL/d(iq) (N,T,2), mode "seq" / "fma": the range rounding of the layout
+    (VR_FLAG_RANGE_FMA).  Roundings as in the kernel:
+      * range d and phase theta: float32, bit-exact (range_phase_c), unless theta32=False (float64 norm and phase);
+      * mean bone length: float32 B = D - S, norm in `mode`, float32 sum in edge order, times f32(1/E), unless
+        cbar32=False (float64 mean; the derivative then uses 1/E instead of f32(1/E));
+      * the aspect cosine u, the amplitude and every derivative: float64 from the float32 inputs, in the kernel's order
+        of operations, with its guards (d > 0, |A| > 0, |B| > 0) and the absent-body rule (float32 sum of the bone
+        lengths == 0: the body contributes exactly 0).  A time step whose dL/d(iq) is exactly 0 contributes 0.
+
+    Returns a dict, all float64:
+      "lam", "loc" (3,), "x" (N,3,T,V,M)   the gradients;
+      "paths"[p][k]                          the part of gradient k ("lam", "loc", "x") through path p: "phase" (the
+                                             range d), "u" (the aspect cosine), "length" (the mean bone length);
+      "scale"[p][k]                          the sum of |term| of path p: per parameter over all (sequence, step,
+                                             bone, body) terms, per dL/dx entry over the bones that touch it.
+    """
+    x = np.asarray(x, np.float32)
+    g = np.asarray(giq, np.float64)
+    N, _, T, V, M = x.shape
+    src, dst = map(list, zip(*edges))
+    E = len(src)
+    lam32 = np.float32(wavelength)
+    lam = float(lam32)
+    loc32 = np.asarray(radar_location, np.float32)
+    L = loc32.astype(np.float64)[:, None, None, None]
+    inv_E = float(np.float32(1) / np.float32(E)) if cbar32 else 1.0 / E
+    PI = np.pi
+    sqrt_pi = np.sqrt(PI)
+    zeros = lambda *s: np.zeros(s)                                              # noqa: E731
+    out = {"paths": {p: {"lam": 0.0, "loc": zeros(3), "x": zeros(*x.shape)} for p in PATHS},
+           "scale": {p: {"lam": 0.0, "loc": zeros(3), "x": zeros(*x.shape)} for p in PATHS}}
+    for n in range(N):
+        S32, D32 = x[n][:, :, src], x[n][:, :, dst]                             # (3,T,E,M)
+        if theta32:
+            d, th = vro.range_phase_c(torch.from_numpy(S32[None]), loc32, lam32, mode)
+            rng, th = d.numpy()[0].astype(np.float64), th.numpy()[0].astype(np.float64)
+        else:
+            rng = np.sqrt(((S32.astype(np.float64) - L) ** 2).sum(0))
+            th = 4 * PI * rng / lam
+        if cbar32:
+            ln = _bone_lengths_f32(S32[None], D32[None], mode)[0]               # (T,E,M) float32
+            sumB = np.zeros((T, M), np.float32)
+            for e in range(E):
+                sumB = sumB + ln[:, e]
+            cbar = (sumB * np.float32(inv_E)).astype(np.float64)[:, None]       # (T,1,M)
+            absent = (sumB == 0)[:, None]
+        else:
+            nb64 = np.sqrt(((D32.astype(np.float64) - S32) ** 2).sum(0))
+            cbar = nb64.sum(1, keepdims=True) * inv_E
+            absent = cbar == 0
+        gI, gQ = g[n, :, 0][:, None, None], g[n, :, 1][:, None, None]
+        active = ~absent & ~((gI == 0) & (gQ == 0))                             # (T,E or 1,M)
+        S, D = S32.astype(np.float64), D32.astype(np.float64)
+        c = cbar * cbar
+        K = sqrt_pi * cbar
+        sn, cs = np.sin(th), np.cos(th)
+        B = D - S
+        A = L - 0.5 * (S + D)
+        na = np.sqrt(A[0] * A[0] + A[1] * A[1] + A[2] * A[2])
+        nb = np.sqrt(B[0] * B[0] + B[1] * B[1] + B[2] * B[2])
+        dot = A[0] * B[0] + A[1] * B[1] + A[2] * B[2]
+        q = na * nb + 1e-6
+        u = dot / q
+        den = 1.0 + (c - 1.0) * u * u
+        amp = K / den
+        dth = amp * (gQ * cs - gI * sn)
+        damp = gI * cs + gQ * sn
+        with np.errstate(divide="ignore", invalid="ignore"):
+            t_lam = np.where(active, dth * (-th / lam), 0)
+            kth = np.where(active & (rng > 0), dth * (4.0 * PI / lam) / rng, 0)
+            kamp = np.where(active, damp * (-K * 2.0 * u * (c - 1.0) / (den * den)), 0)
+            r2 = dot * nb / (na * q * q)
+            dA = np.where(na > 0, kamp * (B / q - r2 * A), 0)                   # dL/dA through u
+            r3 = dot * na / (nb * q * q)
+            dB = np.where(nb > 0, kamp * (A / q - r3 * B), 0)                   # dL/dB through u
+            G_c = np.where(active, damp * sqrt_pi * (1.0 / den - 2.0 * c * u * u / (den * den)), 0).sum(1, keepdims=True)
+            kc = np.where(nb > 0, G_c * inv_E / nb, 0)
+        ph_loc = kth * (L - S)
+        # per bone: (dL/dS, dL/dD) of each path
+        parts = {"phase": (kth * (S - L), np.zeros_like(S)),
+                 "u": (-0.5 * dA - dB, -0.5 * dA + dB),
+                 "length": (-kc * B, kc * B)}
+        P, C = out["paths"], out["scale"]
+        P["phase"]["lam"] += t_lam.sum()
+        C["phase"]["lam"] += np.abs(t_lam).sum()
+        P["phase"]["loc"] += ph_loc.sum((1, 2, 3))
+        C["phase"]["loc"] += np.abs(ph_loc).sum((1, 2, 3))
+        P["u"]["loc"] += dA.sum((1, 2, 3))
+        C["u"]["loc"] += np.abs(dA).sum((1, 2, 3))
+        for p, (gS, gD) in parts.items():
+            px, cx = P[p]["x"][n], C[p]["x"][n]
+            for e, (si, di) in enumerate(zip(src, dst)):
+                px[:, :, si] += gS[:, :, e]
+                px[:, :, di] += gD[:, :, e]
+                cx[:, :, si] += np.abs(gS[:, :, e])
+                cx[:, :, di] += np.abs(gD[:, :, e])
+    for k in ("lam", "loc", "x"):
+        out[k] = sum(out["paths"][p][k] for p in PATHS)
+    return out
