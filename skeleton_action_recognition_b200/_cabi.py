@@ -19,7 +19,9 @@ SYMBOLS = ("vr_abi_version", "vr_last_error", "vr_forward_f32", "vr_forward_debu
            "vr_forward_image_f32", "vr_plan_image", "vr_forward_upsampled_f32", "vr_upsampled_workspace_bytes", "vr_backward_params_f32", "vr_backward_f32", "vr_synth_adjoint_f32", "vr_job_geometry",
            "vr_set_schedule", "vr_plan_team", "vr_pad_frames_joints",
            "vr_pad_frames_backward_f32", "vr_forward_upsampled_debug_f32", "vr_backward_upsampled_params_f32",
-           "vr_stft_general_workspace_floats", "vr_stft_general_f32", "vr_stft_general_backward_f32")
+           "vr_stft_general_workspace_floats", "vr_stft_general_f32", "vr_stft_general_backward_f32",
+           "vr_synth_f32", "vr_synth_upsampled_f32", "vr_synth_adjoint_upsampled_f32",
+           "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32")
 
 _lib = None
 
@@ -52,6 +54,12 @@ def lib():
     L.vr_backward_upsampled_params_f32.argtypes = [vp, vp, vp, i64, i64, i32, i32, c_i32p, c_i32p, i32, vp, vp, i32, i32, u32,
                                                    i32, vp, vp, vp]
     L.vr_backward_upsampled_params_f32.restype = ctypes.c_int
+    L.vr_synth_f32.argtypes = common + [vp, vp, u32, vp, vp]
+    L.vr_synth_f32.restype = ctypes.c_int
+    L.vr_synth_upsampled_f32.argtypes = common + [vp, vp, u32, i32, f32, vp, i64, vp, vp]
+    L.vr_synth_upsampled_f32.restype = ctypes.c_int
+    L.vr_synth_adjoint_upsampled_f32.argtypes = [vp, vp, i64, i64, i32, i32, c_i32p, c_i32p, i32, vp, vp, u32, i32, vp, vp]
+    L.vr_synth_adjoint_upsampled_f32.restype = ctypes.c_int
     L.vr_upsampled_workspace_bytes.argtypes = [i64, i64, i32, i32]
     L.vr_upsampled_workspace_bytes.restype = i64
     L.vr_backward_params_f32.argtypes = [vp, vp, vp, i64, i64, i32, i32, c_i32p, c_i32p, i32, vp, vp, i32, i32, u32, vp, vp, vp]
@@ -83,6 +91,12 @@ def lib():
     L.vr_stft_general_f32.restype = ctypes.c_int
     L.vr_stft_general_backward_f32.argtypes = [vp, vp, vp, vp, i64, i64, i32, i32, vp, vp, vp, vp, vp, vp, vp]
     L.vr_stft_general_backward_f32.restype = ctypes.c_int
+    L.vr_stft_general_frames_workspace_floats.argtypes = [i64, i64, i32, ctypes.POINTER(i64)]
+    L.vr_stft_general_frames_workspace_floats.restype = i64
+    L.vr_stft_general_frames_f32.argtypes = [vp, i64, i64, i32, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp]
+    L.vr_stft_general_frames_f32.restype = ctypes.c_int
+    L.vr_stft_general_frames_backward_f32.argtypes = [vp, vp, vp, vp, i64, i64, i32, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp]
+    L.vr_stft_general_frames_backward_f32.restype = ctypes.c_int
     L.vr_set_timeline_buffer.argtypes = [vp]
     L.vr_set_timeline_buffer.restype = ctypes.c_int
     L.vr_selftest_rounding.argtypes = [ctypes.c_uint64, f32, ctypes.POINTER(ctypes.c_uint64)]

@@ -103,13 +103,15 @@ int partition_edges(const int32_t* src, const int32_t* dst, int E, int V, Partit
 int round_up(int v, int a) { return (v + a - 1) / a * a; }
 
 int make_plan_z(int64_t N, int64_t T, int V, int M, const int32_t* src, const int32_t* dst, int E,
-                int n_fft, int hop, int img, bool ups, int sm_count, bool x_aligned, int ZCAP_MAX, bool park,
+                int n_fft, int hop, int img, bool ups, bool iq_only, int sm_count, bool x_aligned, int ZCAP_MAX, bool park,
                 vr::Params& p, int& grid, int& ctas_per_sm) {
+    // iq_only: synthesis only; n_fft, hop and img are ignored (no frames, no output tile)
     if (img < 0 || img > 4096) return fail(VR_ERR_SHAPE, "image_size must be in [1, 4096], got %d", img);
     if (N <= 0 || T <= 0 || V <= 0 || M <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M must be positive (got %lld, %lld, %d, %d)", (long long)N, (long long)T, V, M);
+    if (iq_only) { n_fft = vr::NFFT; hop = 1; img = 0; }
     if (hop <= 0) return fail(VR_ERR_SHAPE, "hop_length must be positive, got %d", hop);
     if (n_fft != vr::NFFT) return fail(VR_ERR_UNSUPPORTED, "this ABI version implements n_fft=256 only (got %d)", n_fft);
-    if (T <= n_fft / 2)
+    if (!iq_only && T <= n_fft / 2)
         return fail(VR_ERR_SHAPE, "T=%lld must exceed n_fft/2=%d: reflect padding needs it (the reference raises 'Padding size should be less than the corresponding input dimension')", (long long)T, n_fft / 2);
     if (T > (1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T=%lld too long", (long long)T);
     if ((int64_t)V * M * 4 > 65535) return fail(VR_ERR_UNSUPPORTED, "V*M=%lld too large", (long long)V * M);
@@ -119,7 +121,8 @@ int make_plan_z(int64_t N, int64_t T, int V, int M, const int32_t* src, const in
 
     memset(&p, 0, sizeof(p));
     p.N = N; p.T = T; p.V = V; p.M = M; p.E = E; p.hop = hop; p.VM = V * M;
-    p.F = (int)(T / hop) + 1;
+    p.F = iq_only ? 0 : (int)(T / hop) + 1;
+    p.iq_only = iq_only ? 1 : 0;
     p.inv_E = 1.0f / (float)E;
     p.negzero = -0.0f;
     p.plane_floats = vr::TL * p.VM;
@@ -170,7 +173,13 @@ int make_plan_z(int64_t N, int64_t T, int V, int M, const int32_t* src, const in
     int fj_max = (ZCAP_MAX - vr::NFFT - 2 * vr::TL - 2) / hop + 1;     // frames whose span fits the z buffer
     if (fj_max < 1) return fail(VR_ERR_UNSUPPORTED, "hop_length=%d too large", hop);
     int zspan = 0, cmax = 0, slots = 0;
-    if (!img) {
+    if (iq_only) {
+        // samples per job: whole chunks, as many as the z buffer holds, evened out over the jobs of a sequence
+        const int cap = ZCAP_MAX / vr::TL * vr::TL;
+        const long long jps = (T + cap - 1) / cap;
+        p.FJ = round_up((int)((T + jps - 1) / jps), vr::TL);
+        p.jobs_per_seq = (int)((T + p.FJ - 1) / p.FJ);
+    } else if (!img) {
         p.jobs_per_seq = (p.F + fj_max - 1) / fj_max;
         p.FJ = (p.F + p.jobs_per_seq - 1) / p.jobs_per_seq;
     } else {
@@ -188,16 +197,18 @@ int make_plan_z(int64_t N, int64_t T, int V, int M, const int32_t* src, const in
         if (zspan > ZCAP_MAX) return fail(VR_ERR_UNSUPPORTED, "no job split fits the z buffer (T=%lld, hop=%d, image_size=%d)", (long long)T, hop, img);
         p.FJ = CJ;
     }
-    p.jobs_per_seq = (p.ncols + p.FJ - 1) / p.FJ;
+    if (!iq_only) p.jobs_per_seq = (p.ncols + p.FJ - 1) / p.FJ;
     p.n_jobs = N * (long long)p.jobs_per_seq;
     if (p.n_jobs >= (1ll << 31) / 2) return fail(VR_ERR_UNSUPPORTED, "N*jobs_per_seq=%lld too large for one launch; split the batch", p.n_jobs);
-    span_of(p.FJ, zspan, cmax, slots);
+    if (iq_only) { zspan = p.FJ; cmax = p.FJ / vr::TL; }
+    else span_of(p.FJ, zspan, cmax, slots);
     p.zcap = round_up(zspan, 16);
     p.cmax = cmax;
 
     // output tile
     const int FB_BULK_MAX = 20;
-    if (!img && p.jobs_per_seq == 1 && p.F <= FB_BULK_MAX) { p.FB = p.F; p.ostride = p.F; p.bulk_out = 1; }
+    if (iq_only) { p.FB = 0; p.ostride = 0; p.bulk_out = 0; }        // no output tile in shared memory
+    else if (!img && p.jobs_per_seq == 1 && p.F <= FB_BULK_MAX) { p.FB = p.F; p.ostride = p.F; p.bulk_out = 1; }
     else if (img && slots <= FB_BULK_MAX) { p.FB = slots; p.ostride = slots | 1; p.bulk_out = 0; }
     else { p.FB = 16; p.ostride = 17; p.bulk_out = 0; }
 
@@ -247,21 +258,22 @@ int make_plan_z(int64_t N, int64_t T, int V, int M, const int32_t* src, const in
 // per SM; two CTAs matter more (the kernel is latency-bound with one), so take the largest buffer that
 // still leaves room for two.
 int make_plan(int64_t N, int64_t T, int V, int M, const int32_t* src, const int32_t* dst, int E,
-              int n_fft, int hop, int img, bool ups, int sm_count, bool x_aligned, vr::Params& p, int& grid, int& ctas_per_sm) {
+              int n_fft, int hop, int img, bool ups, int sm_count, bool x_aligned, vr::Params& p, int& grid, int& ctas_per_sm,
+              bool iq_only = false) {
     const int want = g_tuning.ctas_per_sm > 0 ? g_tuning.ctas_per_sm : 2;
     const int caps[] = {2304, 1920, 1664, 1408, 1152};
-    int rc = make_plan_z(N, T, V, M, src, dst, E, n_fft, hop, img, ups, sm_count, x_aligned, caps[0], ups, p, grid, ctas_per_sm);
+    int rc = make_plan_z(N, T, V, M, src, dst, E, n_fft, hop, img, ups, iq_only, sm_count, x_aligned, caps[0], ups, p, grid, ctas_per_sm);
     if (rc || (!ups && ctas_per_sm >= want && p.jobs_per_seq == 1)) return rc;
     for (int zc : caps) {
         vr::Params q;
         int g2, c2;
-        if (make_plan_z(N, T, V, M, src, dst, E, n_fft, hop, img, ups, sm_count, x_aligned, zc, true, q, g2, c2) == VR_OK && c2 >= want) {
+        if (make_plan_z(N, T, V, M, src, dst, E, n_fft, hop, img, ups, iq_only, sm_count, x_aligned, zc, true, q, g2, c2) == VR_OK && c2 >= want) {
             p = q; grid = g2; ctas_per_sm = c2;
             return VR_OK;
         }
     }
     g_err[0] = 0;
-    return make_plan_z(N, T, V, M, src, dst, E, n_fft, hop, img, ups, sm_count, x_aligned, caps[0], true, p, grid, ctas_per_sm);
+    return make_plan_z(N, T, V, M, src, dst, E, n_fft, hop, img, ups, iq_only, sm_count, x_aligned, caps[0], true, p, grid, ctas_per_sm);
 }
 
 // ---- team-job schedule (vr_team_kernel) -----------------------------------------------------------
@@ -380,7 +392,7 @@ struct PlanCache {
     bool valid = false;
     int64_t N = 0, T = 0;
     int V = 0, M = 0, E = 0, n_fft = 0, hop = 0, img = 0, sm_count = 0, grid = 0, cps = 0;
-    bool aligned = false, ups = false;
+    bool aligned = false, ups = false, iq_only = false;
     Tuning tuning;
     std::vector<int32_t> src, dst;
     vr::Params p;
@@ -388,9 +400,10 @@ struct PlanCache {
 thread_local PlanCache t_plan;
 
 int cached_plan(int64_t N, int64_t T, int V, int M, const int32_t* src, const int32_t* dst, int E,
-                int n_fft, int hop, int img, bool ups, int sm_count, bool aligned, vr::Params& p, int& grid, int& cps) {
+                int n_fft, int hop, int img, bool ups, bool iq_only, int sm_count, bool aligned, vr::Params& p, int& grid, int& cps) {
     PlanCache& c = t_plan;
     if (c.valid && c.N == N && c.T == T && c.V == V && c.M == M && c.E == E && c.n_fft == n_fft && c.hop == hop && c.img == img && c.ups == ups &&
+        c.iq_only == iq_only &&
         c.sm_count == sm_count && c.aligned == aligned && src && dst &&
         c.tuning.warps == g_tuning.warps && c.tuning.ctas_per_sm == g_tuning.ctas_per_sm && c.tuning.stages == g_tuning.stages &&
         memcmp(c.src.data(), src, sizeof(int32_t) * E) == 0 && memcmp(c.dst.data(), dst, sizeof(int32_t) * E) == 0) {
@@ -398,9 +411,10 @@ int cached_plan(int64_t N, int64_t T, int V, int M, const int32_t* src, const in
         return VR_OK;
     }
     c.valid = false;
-    int rc = make_plan(N, T, V, M, src, dst, E, n_fft, hop, img, ups, sm_count, aligned, p, grid, cps);
+    int rc = make_plan(N, T, V, M, src, dst, E, n_fft, hop, img, ups, sm_count, aligned, p, grid, cps, iq_only);
     if (rc) return rc;
-    c.N = N; c.T = T; c.V = V; c.M = M; c.E = E; c.n_fft = n_fft; c.hop = hop; c.img = img; c.ups = ups; c.sm_count = sm_count; c.aligned = aligned;
+    c.N = N; c.T = T; c.V = V; c.M = M; c.E = E; c.n_fft = n_fft; c.hop = hop; c.img = img; c.ups = ups; c.iq_only = iq_only;
+    c.sm_count = sm_count; c.aligned = aligned;
     c.tuning = g_tuning;
     c.src.assign(src, src + E); c.dst.assign(dst, dst + E);
     c.p = p; c.grid = grid; c.cps = cps; c.valid = true;
@@ -412,8 +426,9 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
            int n_fft, int hop, uint32_t flags, int img, float* out, float* iq, cudaStream_t stream,
            const double* coef = nullptr, int ups_T = 0, int ups_K = 0) {
     // coef != nullptr: fused temporal up-sampling; T is then the UP-SAMPLED length ups_K * ups_T and x is only
-    // used for its alignment (the kernel reads the spline coefficients instead)
-    if (!x || !out) return fail(VR_ERR_ARG, "x and out must not be null");
+    // used for its alignment (the kernel reads the spline coefficients instead).  out == nullptr: synthesis only (iq)
+    const bool iq_only = out == nullptr;
+    if (!x || (!out && !iq)) return fail(VR_ERR_ARG, "x and out (or iq) must not be null");
     if ((lam_dev == nullptr) != (loc_dev == nullptr)) return fail(VR_ERR_ARG, "wavelength and radar_location must both be device pointers or both be null");
     if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_INPUTS_READY)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
     int dev, sm_count;
@@ -421,7 +436,7 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
     if (rc) return rc;
     vr::Params p;
     int grid, cps;
-    rc = cached_plan(N, T, V, M, src, dst, E, n_fft, hop, img, coef != nullptr, sm_count, ((uintptr_t)x & 15) == 0, p, grid, cps);
+    rc = cached_plan(N, T, V, M, src, dst, E, n_fft, hop, img, coef != nullptr, iq_only, sm_count, ((uintptr_t)x & 15) == 0, p, grid, cps);
     if (rc) return rc;
     // schedule: batches with several sequences per team slot take the team-job kernel (no CTA-wide barriers, a double
     // buffer per team); small batches keep the cooperative kernel, whose latency per sequence is half
@@ -511,6 +526,15 @@ int vr_forward_debug_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, in
     if (!iq_dev) return fail(VR_ERR_ARG, "iq_dev must not be null");
     return launch(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
                   n_fft, hop, flags, 0, out_dev, iq_dev, (cudaStream_t)stream);
+}
+
+int vr_synth_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
+                 const int32_t* src_host, const int32_t* dst_host, int32_t E,
+                 const float* wavelength_dev, const float* radar_loc_dev, uint32_t flags, float* iq_dev, void* stream) {
+    if (!wavelength_dev || !radar_loc_dev) return fail(VR_ERR_ARG, "wavelength_dev and radar_loc_dev must not be null");
+    if (!iq_dev) return fail(VR_ERR_ARG, "iq_dev must not be null");
+    return launch(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
+                  vr::NFFT, 1, flags, 0, nullptr, iq_dev, (cudaStream_t)stream);
 }
 
 int vr_forward_image_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
@@ -786,7 +810,7 @@ int upsampled_impl(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t 
                    int32_t num_pad_frames, float sigma, int32_t image_size,
                    void* workspace_dev, int64_t workspace_bytes, float* out_dev, float* iq_dev, void* stream) {
     if (!wavelength_dev || !radar_loc_dev) return fail(VR_ERR_ARG, "wavelength_dev and radar_loc_dev must not be null");
-    if (!x_dev || !out_dev || !workspace_dev) return fail(VR_ERR_ARG, "x_dev, out_dev and workspace_dev must not be null");
+    if (!x_dev || (!out_dev && !iq_dev) || !workspace_dev) return fail(VR_ERR_ARG, "x_dev, out_dev and workspace_dev must not be null");
     if (image_size < 0) return fail(VR_ERR_SHAPE, "image_size must be >= 0, got %d", image_size);
     if (N <= 0 || V <= 0 || M <= 0) return fail(VR_ERR_SHAPE, "N, V, M must be positive (got %lld, %d, %d)", (long long)N, V, M);
     if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames (scipy interp1d raises ValueError)", (long long)T);
@@ -825,6 +849,16 @@ int vr_forward_upsampled_debug_f32(const float* x_dev, int64_t N, int64_t T, int
                           num_pad_frames, sigma, 0, workspace_dev, workspace_bytes, out_dev, iq_dev, stream);
 }
 
+int vr_synth_upsampled_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
+                           const int32_t* src_host, const int32_t* dst_host, int32_t E,
+                           const float* wavelength_dev, const float* radar_loc_dev, uint32_t flags,
+                           int32_t num_pad_frames, float sigma, void* workspace_dev, int64_t workspace_bytes,
+                           float* iq_dev, void* stream) {
+    if (!iq_dev) return fail(VR_ERR_ARG, "iq_dev must not be null");
+    return upsampled_impl(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, vr::NFFT, 1, flags,
+                          num_pad_frames, sigma, 0, workspace_dev, workspace_bytes, nullptr, iq_dev, stream);
+}
+
 int vr_backward_params_f32(const float* x_dev, const float* iq_dev, const float* grad_out_dev,
                            int64_t N, int64_t T, int32_t V, int32_t M,
                            const int32_t* src_host, const int32_t* dst_host, int32_t E,
@@ -844,6 +878,21 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
                   int32_t n_fft, int32_t hop, uint32_t flags, bool synth_only,
                   float* gz_work_dev, double* grad_params_dev, float* grad_x_dev, void* stream,
                   const double* coef = nullptr, int ups_T = 0, int ups_K = 0);
+// backward_impl with the joint positions of the up-sampling spline whose cubics vr_forward_upsampled_debug_f32 /
+// vr_synth_upsampled_f32 left in workspace_dev; T is the RAW length
+int backward_ups_impl(const void* workspace_dev, const float* iq_dev, const float* grad_out_dev,
+                      int64_t N, int64_t T, int32_t V, int32_t M, const int32_t* src_host, const int32_t* dst_host, int32_t E,
+                      const float* wavelength_dev, const float* radar_loc_dev, int32_t n_fft, int32_t hop, uint32_t flags,
+                      int32_t num_pad_frames, bool synth_only, float* gz_work_dev, double* grad_params_dev, void* stream) {
+    if (!workspace_dev) return fail(VR_ERR_ARG, "workspace_dev must not be null");
+    if (((uintptr_t)workspace_dev & 7) != 0) return fail(VR_ERR_ARG, "workspace_dev must be 8-byte aligned");
+    if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames", (long long)T);
+    if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
+    if ((double)T * num_pad_frames > (double)(1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
+    return backward_impl(nullptr, iq_dev, grad_out_dev, N, T * num_pad_frames, V, M, src_host, dst_host, E, wavelength_dev,
+                         radar_loc_dev, n_fft, hop, flags, synth_only, gz_work_dev, grad_params_dev, nullptr, stream,
+                         static_cast<const double*>(workspace_dev), (int)T, num_pad_frames);
+}
 }  // namespace
 extern "C" {
 
@@ -872,14 +921,8 @@ int vr_backward_upsampled_params_f32(const void* workspace_dev, const float* iq_
                                      const float* wavelength_dev, const float* radar_loc_dev,
                                      int32_t n_fft, int32_t hop, uint32_t flags, int32_t num_pad_frames,
                                      float* gz_work_dev, double* grad_params_dev, void* stream) {
-    if (!workspace_dev) return fail(VR_ERR_ARG, "workspace_dev must not be null");
-    if (((uintptr_t)workspace_dev & 7) != 0) return fail(VR_ERR_ARG, "workspace_dev must be 8-byte aligned");
-    if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames", (long long)T);
-    if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
-    if ((double)T * num_pad_frames > (double)(1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
-    return backward_impl(nullptr, iq_dev, grad_out_dev, N, T * num_pad_frames, V, M, src_host, dst_host, E, wavelength_dev,
-                         radar_loc_dev, n_fft, hop, flags, false, gz_work_dev, grad_params_dev, nullptr, stream,
-                         static_cast<const double*>(workspace_dev), (int)T, num_pad_frames);
+    return backward_ups_impl(workspace_dev, iq_dev, grad_out_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev,
+                             n_fft, hop, flags, num_pad_frames, false, gz_work_dev, grad_params_dev, stream);
 }
 
 }  // extern "C"
@@ -939,6 +982,16 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
 }
 }  // namespace
 extern "C" {
+
+int vr_synth_adjoint_upsampled_f32(const void* workspace_dev, const float* grad_iq_dev,
+                                   int64_t N, int64_t T, int32_t V, int32_t M,
+                                   const int32_t* src_host, const int32_t* dst_host, int32_t E,
+                                   const float* wavelength_dev, const float* radar_loc_dev, uint32_t flags,
+                                   int32_t num_pad_frames, double* grad_params_dev, void* stream) {
+    // the second stage of vr_backward_upsampled_params_f32 alone: dL/d(iq) comes from the caller (a general STFT)
+    return backward_ups_impl(workspace_dev, nullptr, nullptr, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev,
+                             vr::NFFT, 16, flags, num_pad_frames, true, const_cast<float*>(grad_iq_dev), grad_params_dev, stream);
+}
 
 int vr_release_host_staging(void) {
     int cur = 0;
@@ -1056,38 +1109,21 @@ static long long stft_bimg_floats(int n_fft) {
 }
 static long long stft_lp(long long T, int n_fft) { return (T + n_fft + 3) & ~3ll; }     // padded signal length, 16-byte rows
 
-int64_t vr_stft_general_workspace_floats(int64_t N, int64_t T, int32_t n_fft, int32_t hop, int64_t parts[3]) {
-    if (N <= 0 || T <= 0 || hop <= 0 || n_fft <= 0) return 0;
-    const int64_t M = N * (T / hop + 1), K = 2ll * n_fft;
-    const int64_t a = 2 * N * stft_lp(T, n_fft), b = 2 * stft_bimg_floats(n_fft), c = K * stft_ldm(M);   // padded planar signal (the frames are views of it);       // C / dC: column-major, leading dimension a multiple of 4
-    if (parts) { parts[0] = a; parts[1] = b; parts[2] = c; }
-    return a + b + c;
-}
-
-int vr_stft_general_f32(const float* iq_dev, int64_t N, int64_t T, int32_t n_fft, int32_t hop,
-                        const float* wsin_dev, const float* wcos_dev, float* frames_work, float* bt_work,
-                        float* c_save /* may be NULL */, float* out_dev, void* stream) {
-    if (!iq_dev || !wsin_dev || !wcos_dev || !frames_work || !bt_work || !out_dev) return fail(VR_ERR_ARG, "device pointers must not be null");
-    if (!aligned16(bt_work) || !aligned16(c_save) || (reinterpret_cast<uintptr_t>(iq_dev) & 7))     // bulk copies, 16-byte column accesses, float2 samples
-        return fail(VR_ERR_ARG, "bt_work and c_save must be 16-byte aligned, iq_dev 8-byte aligned");
-    int rc = stft_check(N, T, n_fft, hop);
-    if (rc) return rc;
-    int dev, sm_count;
-    rc = device_setup(dev, sm_count);
-    if (rc) return rc;
-    rc = gemm_setup(dev);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int F = (int)(T / hop) + 1, nb = stft_nb(n_fft), K = 2 * n_fft;
+}  // extern "C"
+namespace {
+// The GEMM part of the forward, over a planar padded signal P (S, 2, Lp) whose frame f starts at P[.. + f hop]: the full
+// route passes the reflect-padded signal (hop, F = T / hop + 1), the kept-frames route its compact copy of the kept frames
+// (hop = n_fft, F = F_kept).  Each output column is one GEMM row with the same K order and B tiles in both.
+int stft_forward_gemm(const float* P, long long Lp, int hop, int F, int64_t N, int n_fft, const float* wsin_dev,
+                      const float* wcos_dev, float* bt_work, float* c_save, float* out_dev, cudaStream_t st) {
+    const int nb = stft_nb(n_fft), K = 2 * n_fft;
     const long long M = N * (long long)F;
-    const long long Lp = stft_lp(T, n_fft);
-    vr::vr_stft_pad_kernel<<<(unsigned)std::min<long long>((N * Lp + 255) / 256, sm_count * 16ll), 256, 0, st>>>(iq_dev, frames_work, N, (int)T, Lp, n_fft);
     const long long img = stft_bimg_floats(n_fft);
     if (K % vr::GN) CUDA_TRY(cudaMemsetAsync(bt_work, 0, (size_t)(2 * img) * sizeof(float), st));      // rows past K of the one tile
     vr::vr_stft_bt_kernel<<<(n_fft * n_fft + 255) / 256, 256, 0, st>>>(wsin_dev, wcos_dev, bt_work, bt_work + img, n_fft, nb, (K + vr::GK - 1) / vr::GK);
     vr::GemmParams g;
     memset(&g, 0, sizeof(g));
-    g.P = frames_work; g.Lp = Lp; g.hop = hop;       // A = the frames, read as views of the padded signal
+    g.P = P; g.Lp = Lp; g.hop = hop;                 // A = the frames, read as views of the padded signal
     g.Bimg = bt_work;                                // B = the kernel matrix, pre-split and pre-tiled: bulk copies
     g.M = (int)M; g.N = K; g.K = K; g.kb_per_split = (K + vr::GK - 1) / vr::GK;
     g.out = out_dev; g.csave = c_save; g.ldc = stft_ldm(M); g.F = F; g.n_fft = n_fft; g.nb = nb;
@@ -1097,25 +1133,12 @@ int vr_stft_general_f32(const float* iq_dev, int64_t N, int64_t T, int32_t n_fft
     return VR_OK;
 }
 
-int vr_stft_general_backward_f32(const float* grad_out_dev, const float* frames_work, const float* bt_work, const float* c_save,
-                                 int64_t N, int64_t T, int32_t n_fft, int32_t hop,
-                                 float* dc_work, float* da_work /* NULL: no grad_iq */, float* dbt_work /* NULL: no kernel grads */,
-                                 float* grad_iq_dev, float* grad_wsin_dev, float* grad_wcos_dev, void* stream) {
-    if (!grad_out_dev || !frames_work || !bt_work || !c_save || !dc_work) return fail(VR_ERR_ARG, "device pointers must not be null");
-    if (!aligned16(bt_work) || !aligned16(c_save) || !aligned16(dc_work) || (reinterpret_cast<uintptr_t>(grad_iq_dev) & 7))
-        return fail(VR_ERR_ARG, "bt_work, c_save and dc_work must be 16-byte aligned, grad_iq_dev 8-byte aligned");
-    if ((da_work == nullptr) != (grad_iq_dev == nullptr)) return fail(VR_ERR_ARG, "da_work and grad_iq_dev go together");
-    if ((dbt_work == nullptr) != (grad_wsin_dev == nullptr) || (dbt_work == nullptr) != (grad_wcos_dev == nullptr))
-        return fail(VR_ERR_ARG, "dbt_work, grad_wsin_dev and grad_wcos_dev go together");
-    int rc = stft_check(N, T, n_fft, hop);
-    if (rc) return rc;
-    int dev, sm_count;
-    rc = device_setup(dev, sm_count);
-    if (rc) return rc;
-    rc = gemm_setup(dev);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int F = (int)(T / hop) + 1, nb = stft_nb(n_fft), K = 2 * n_fft;
+// The GEMM part of the backward over the same (P, Lp, hop, F): dC, then dA (frame gradients, folded by the caller) and dBt
+// (kernel gradients, reduced over every frame of the batch)
+int stft_backward_gemm(const float* grad_out_dev, const float* P, long long Lp, int hop, int F, int64_t N, int n_fft,
+                       const float* bt_work, const float* c_save, float* dc_work, float* da_work, float* dbt_work,
+                       float* grad_wsin_dev, float* grad_wcos_dev, int sm_count, cudaStream_t st) {
+    const int nb = stft_nb(n_fft), K = 2 * n_fft;
     const long long M = N * (long long)F;
     const long long ldm = stft_ldm(M);
     vr::vr_stft_dc_kernel<<<dim3((unsigned)std::min<long long>((M / 4 + 256) / 256, sm_count * 4ll), (unsigned)n_fft), 256, 0, st>>>(grad_out_dev, c_save, dc_work, (int)M, ldm, F, n_fft, nb);
@@ -1127,12 +1150,11 @@ int vr_stft_general_backward_f32(const float* grad_out_dev, const float* frames_
         g.M = (int)M; g.N = K; g.K = K; g.C = da_work; g.ldc = K; g.kb_per_split = (K + vr::GK - 1) / vr::GK;
         dim3 grid((unsigned)(((M + vr::GM - 1) / vr::GM) * ((K + vr::GN - 1) / vr::GN)));
         vr::vr_gemm_tf32x3_kernel<0, vr::G_STRIDED, vr::G_TILED><<<grid, vr::G_THREADS, vr::G_SMEM_BYTES, st>>>(g);
-        vr::vr_stft_fold_kernel<<<(unsigned)std::min<long long>((N * T + 255) / 256, sm_count * 16ll), 256, 0, st>>>(da_work, grad_iq_dev, N, (int)T, F, n_fft, hop);
     }
     if (dbt_work) {                                  // dBt[n, k] = sum_m dC[m, n] A[m, k]
         memset(&g, 0, sizeof(g));
         g.A = dc_work; g.sAm = ldm; g.sAk = 1;       // A'(m' = n, k' = m) = dC(m, n) = dc[n * ldm + m]: rows of 16-byte aligned chunks
-        g.P = frames_work; g.Lp = stft_lp(T, n_fft); g.hop = hop; g.F = F; g.n_fft = n_fft;     // B'(n' = k, k' = m) = A[m][k], a view
+        g.P = P; g.Lp = Lp; g.hop = hop; g.F = F; g.n_fft = n_fft;     // B'(n' = k, k' = m) = A[m][k], a view
         g.M = K; g.N = K; g.K = (int)M; g.C = dbt_work; g.ldc = K;
         // the reduction runs over all frames of the batch: split it over gridDim.z so that the (2 n_fft / 128)^2 output
         // tiles fill the machine; the slices add into the zeroed result with float atomics
@@ -1148,6 +1170,130 @@ int vr_stft_general_backward_f32(const float* grad_out_dev, const float* frames_
         vr::vr_gemm_tf32x3_kernel<0, vr::G_STRIDED, vr::G_FRAME_COLS><<<grid, vr::G_THREADS, vr::G_SMEM_BYTES, st>>>(g);
         vr::vr_stft_dw_kernel<<<(n_fft * n_fft + 255) / 256, 256, 0, st>>>(dbt_work, grad_wsin_dev, grad_wcos_dev, n_fft, nb);
     }
+    CUDA_TRY(cudaGetLastError());
+    return VR_OK;
+}
+
+// the argument checks of both forward entries (F: frames of the GEMM, T / hop + 1 or F_kept)
+int stft_forward_args(const float* iq_dev, const float* wsin_dev, const float* wcos_dev, const float* frames_work,
+                      const float* bt_work, const float* c_save, const float* out_dev, int64_t N, int64_t T, int n_fft, int hop,
+                      int& dev, int& sm_count) {
+    if (!iq_dev || !wsin_dev || !wcos_dev || !frames_work || !bt_work || !out_dev) return fail(VR_ERR_ARG, "device pointers must not be null");
+    if (!aligned16(bt_work) || !aligned16(c_save) || (reinterpret_cast<uintptr_t>(iq_dev) & 7))     // bulk copies, 16-byte column accesses, float2 samples
+        return fail(VR_ERR_ARG, "bt_work and c_save must be 16-byte aligned, iq_dev 8-byte aligned");
+    int rc = stft_check(N, T, n_fft, hop);
+    if (rc) return rc;
+    rc = device_setup(dev, sm_count);
+    if (rc) return rc;
+    return gemm_setup(dev);
+}
+
+// the argument checks of both backward entries
+int stft_backward_args(const float* grad_out_dev, const float* frames_work, const float* bt_work, const float* c_save,
+                       const float* dc_work, const float* da_work, const float* dbt_work, const float* grad_iq_dev,
+                       const float* grad_wsin_dev, const float* grad_wcos_dev, int64_t N, int64_t T, int n_fft, int hop,
+                       int& dev, int& sm_count) {
+    if (!grad_out_dev || !frames_work || !bt_work || !c_save || !dc_work) return fail(VR_ERR_ARG, "device pointers must not be null");
+    if (!aligned16(bt_work) || !aligned16(c_save) || !aligned16(dc_work) || (reinterpret_cast<uintptr_t>(grad_iq_dev) & 7))
+        return fail(VR_ERR_ARG, "bt_work, c_save and dc_work must be 16-byte aligned, grad_iq_dev 8-byte aligned");
+    if ((da_work == nullptr) != (grad_iq_dev == nullptr)) return fail(VR_ERR_ARG, "da_work and grad_iq_dev go together");
+    if ((dbt_work == nullptr) != (grad_wsin_dev == nullptr) || (dbt_work == nullptr) != (grad_wcos_dev == nullptr))
+        return fail(VR_ERR_ARG, "dbt_work, grad_wsin_dev and grad_wcos_dev go together");
+    int rc = stft_check(N, T, n_fft, hop);
+    if (rc) return rc;
+    rc = device_setup(dev, sm_count);
+    if (rc) return rc;
+    return gemm_setup(dev);
+}
+
+// the frame table of the kept-frames entries: F_kept in [1, T / hop + 1] (the table's contents stay on the device: strictly
+// increasing indices in [0, T / hop + 1) are the caller's contract)
+int stft_kept_check(const int32_t* frames_dev, int64_t N, int64_t T, int hop, int64_t F_kept) {
+    if (!frames_dev) return fail(VR_ERR_ARG, "frames_dev must not be null");
+    if (hop <= 0 || T <= 0) return fail(VR_ERR_SHAPE, "T, hop must be positive");
+    if (F_kept < 1 || F_kept > T / hop + 1) return fail(VR_ERR_SHAPE, "F_kept=%lld outside [1, T/hop+1 = %lld]", (long long)F_kept, (long long)(T / hop + 1));
+    if (N * F_kept >= (1ll << 31) / 2) return fail(VR_ERR_UNSUPPORTED, "too many frames for one launch; split the batch");
+    return VR_OK;
+}
+}  // namespace
+extern "C" {
+
+int64_t vr_stft_general_workspace_floats(int64_t N, int64_t T, int32_t n_fft, int32_t hop, int64_t parts[3]) {
+    if (N <= 0 || T <= 0 || hop <= 0 || n_fft <= 0) return 0;
+    const int64_t M = N * (T / hop + 1), K = 2ll * n_fft;
+    const int64_t a = 2 * N * stft_lp(T, n_fft), b = 2 * stft_bimg_floats(n_fft), c = K * stft_ldm(M);   // padded planar signal (the frames are views of it);       // C / dC: column-major, leading dimension a multiple of 4
+    if (parts) { parts[0] = a; parts[1] = b; parts[2] = c; }
+    return a + b + c;
+}
+
+int vr_stft_general_f32(const float* iq_dev, int64_t N, int64_t T, int32_t n_fft, int32_t hop,
+                        const float* wsin_dev, const float* wcos_dev, float* frames_work, float* bt_work,
+                        float* c_save /* may be NULL */, float* out_dev, void* stream) {
+    int dev, sm_count;
+    int rc = stft_forward_args(iq_dev, wsin_dev, wcos_dev, frames_work, bt_work, c_save, out_dev, N, T, n_fft, hop, dev, sm_count);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long Lp = stft_lp(T, n_fft);
+    vr::vr_stft_pad_kernel<<<(unsigned)std::min<long long>((N * Lp + 255) / 256, sm_count * 16ll), 256, 0, st>>>(iq_dev, frames_work, N, (int)T, Lp, n_fft);
+    return stft_forward_gemm(frames_work, Lp, hop, (int)(T / hop) + 1, N, n_fft, wsin_dev, wcos_dev, bt_work, c_save, out_dev, st);
+}
+
+int vr_stft_general_backward_f32(const float* grad_out_dev, const float* frames_work, const float* bt_work, const float* c_save,
+                                 int64_t N, int64_t T, int32_t n_fft, int32_t hop,
+                                 float* dc_work, float* da_work /* NULL: no grad_iq */, float* dbt_work /* NULL: no kernel grads */,
+                                 float* grad_iq_dev, float* grad_wsin_dev, float* grad_wcos_dev, void* stream) {
+    int dev, sm_count;
+    int rc = stft_backward_args(grad_out_dev, frames_work, bt_work, c_save, dc_work, da_work, dbt_work, grad_iq_dev,
+                                grad_wsin_dev, grad_wcos_dev, N, T, n_fft, hop, dev, sm_count);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int F = (int)(T / hop) + 1;
+    rc = stft_backward_gemm(grad_out_dev, frames_work, stft_lp(T, n_fft), hop, F, N, n_fft, bt_work, c_save, dc_work, da_work,
+                            dbt_work, grad_wsin_dev, grad_wcos_dev, sm_count, st);
+    if (rc || !da_work) return rc;
+    vr::vr_stft_fold_kernel<<<(unsigned)std::min<long long>((N * T + 255) / 256, sm_count * 16ll), 256, 0, st>>>(da_work, grad_iq_dev, N, (int)T, F, n_fft, hop);
+    CUDA_TRY(cudaGetLastError());
+    return VR_OK;
+}
+
+int64_t vr_stft_general_frames_workspace_floats(int64_t N, int64_t F_kept, int32_t n_fft, int64_t parts[3]) {
+    if (N <= 0 || F_kept <= 0 || n_fft <= 0) return 0;
+    const int64_t M = N * F_kept, K = 2ll * n_fft;
+    const int64_t a = 2 * N * F_kept * n_fft, b = 2 * stft_bimg_floats(n_fft), c = K * stft_ldm(M);    // compact kept frames; B images; C / dC
+    if (parts) { parts[0] = a; parts[1] = b; parts[2] = c; }
+    return a + b + c;
+}
+
+int vr_stft_general_frames_f32(const float* iq_dev, int64_t N, int64_t T, int32_t n_fft, int32_t hop,
+                               const int32_t* frames_dev, int64_t F_kept,
+                               const float* wsin_dev, const float* wcos_dev, float* frames_work, float* bt_work,
+                               float* c_save /* may be NULL */, float* out_dev, void* stream) {
+    int dev, sm_count;
+    int rc = stft_forward_args(iq_dev, wsin_dev, wcos_dev, frames_work, bt_work, c_save, out_dev, N, T, n_fft, hop, dev, sm_count);
+    if (rc) return rc;
+    rc = stft_kept_check(frames_dev, N, T, hop, F_kept);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long Lp = F_kept * (long long)n_fft;
+    vr::vr_stft_gather_kernel<<<(unsigned)std::min<long long>((N * Lp + 255) / 256, sm_count * 16ll), 256, 0, st>>>(iq_dev, frames_dev, frames_work, N, (int)T, (int)F_kept, n_fft, hop);
+    return stft_forward_gemm(frames_work, Lp, n_fft, (int)F_kept, N, n_fft, wsin_dev, wcos_dev, bt_work, c_save, out_dev, st);
+}
+
+int vr_stft_general_frames_backward_f32(const float* grad_out_dev, const float* frames_work, const float* bt_work, const float* c_save,
+                                        int64_t N, int64_t T, int32_t n_fft, int32_t hop, const int32_t* frames_dev, int64_t F_kept,
+                                        float* dc_work, float* da_work, float* dbt_work,
+                                        float* grad_iq_dev, float* grad_wsin_dev, float* grad_wcos_dev, void* stream) {
+    int dev, sm_count;
+    int rc = stft_backward_args(grad_out_dev, frames_work, bt_work, c_save, dc_work, da_work, dbt_work, grad_iq_dev,
+                                grad_wsin_dev, grad_wcos_dev, N, T, n_fft, hop, dev, sm_count);
+    if (rc) return rc;
+    rc = stft_kept_check(frames_dev, N, T, hop, F_kept);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = stft_backward_gemm(grad_out_dev, frames_work, F_kept * (long long)n_fft, n_fft, (int)F_kept, N, n_fft, bt_work, c_save,
+                            dc_work, da_work, dbt_work, grad_wsin_dev, grad_wcos_dev, sm_count, st);
+    if (rc || !da_work) return rc;
+    vr::vr_stft_fold_kept_kernel<<<(unsigned)std::min<long long>((N * T + 255) / 256, sm_count * 16ll), 256, 0, st>>>(da_work, frames_dev, grad_iq_dev, N, (int)T, (int)F_kept, n_fft, hop);
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
 }

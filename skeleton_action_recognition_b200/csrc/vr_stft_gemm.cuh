@@ -520,6 +520,12 @@ __global__ void __launch_bounds__(G_THREADS, 1) vr_gemm_tf32x3_kernel(const __gr
 }
 
 // ---- small kernels around the GEMM -------------------------------------------------------------------------------
+// nnAudio center=True, pad_mode='reflect': padded position j (0 <= j < T + n_fft) holds sample stft_reflect(j)
+__device__ __forceinline__ int stft_reflect(int j, int T, int n_fft) {
+    int t = j - n_fft / 2;
+    t = t < 0 ? -t : t;
+    return t >= T ? 2 * (T - 1) - t : t;
+}
 // the padded, planar signal the frame views read: iq (S, T, 2) -> P (S, 2, Lp), P[s][c][j] = iq[s][reflect(j - n_fft/2)][c]
 // for j < T + n_fft (nnAudio center=True, pad_mode='reflect'), 0 beyond.  Frame f of sequence s is P[s][c][f * hop ...].
 __global__ void vr_stft_pad_kernel(const float* __restrict__ iq, float* __restrict__ P, long long S, int T, long long Lp, int n_fft) {
@@ -528,14 +534,24 @@ __global__ void vr_stft_pad_kernel(const float* __restrict__ iq, float* __restri
         const long long sq = i / Lp;
         const int j = (int)(i - sq * Lp);
         float2 z = make_float2(0.f, 0.f);
-        if (j < T + n_fft) {
-            int t = j - n_fft / 2;
-            t = t < 0 ? -t : t;
-            t = t >= T ? 2 * (T - 1) - t : t;
-            z = __ldg(reinterpret_cast<const float2*>(iq) + sq * T + t);
-        }
+        if (j < T + n_fft) z = __ldg(reinterpret_cast<const float2*>(iq) + sq * T + stft_reflect(j, T, n_fft));
         P[sq * 2 * Lp + j] = z.x;
         P[(sq * 2 + 1) * Lp + j] = z.y;
+    }
+}
+// kept frames only: the frames listed in `frames` (Fk strictly increasing indices, the same for every sequence) copied end to
+// end into a compact planar buffer, P'[(s * 2 + c) * Fk n_fft + i n_fft + j] = padded[s][c][frames[i] hop + j], so that the
+// GEMMs read it as a frame view with hop' = n_fft and F' = Fk.
+__global__ void vr_stft_gather_kernel(const float* __restrict__ iq, const int* __restrict__ frames, float* __restrict__ P,
+                                      long long S, int T, int Fk, int n_fft, int hop) {
+    const long long Lp = (long long)Fk * n_fft, total = S * Lp;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const long long sq = i / Lp;
+        const int r = (int)(i - sq * Lp), fi = r / n_fft, j = r - fi * n_fft;
+        const int t = stft_reflect(__ldg(frames + fi) * hop + j, T, n_fft);
+        const float2 z = __ldg(reinterpret_cast<const float2*>(iq) + sq * T + t);
+        P[sq * 2 * Lp + r] = z.x;
+        P[(sq * 2 + 1) * Lp + r] = z.y;
     }
 }
 // row of Bt that holds Re / Im of `bin` under the column-tile layout [re block | im block] of nb bins
@@ -627,6 +643,46 @@ __global__ void vr_stft_fold_kernel(const float* __restrict__ dA, float* __restr
             if (on && u >= 0 && u < U) {
                 g.x += stft_fold_at(dA, seq, 0, u, F, n_fft, hop);
                 g.y += stft_fold_at(dA, seq, 1, u, F, n_fft, hop);
+            }
+        }
+        reinterpret_cast<float2*>(giq)[i] = g;
+    }
+}
+// the same fold when dA holds only the kept frames (dA (S*Fk, 2 n_fft), row i = frame frames[i]): the kept frames covering
+// position u are a contiguous run of the sorted table, found by binary search; summed in increasing frame order like
+// stft_fold_at, so the result equals the full fold fed zero gradients for the frames that were not kept.  A sample that no
+// kept frame covers gets 0.
+__device__ __forceinline__ float stft_fold_kept_at(const float* __restrict__ dA, const int* __restrict__ frames, long long seq,
+                                                   int c, int u, int Fk, int n_fft, int hop) {
+    const int fmin = u - n_fft + 1 <= 0 ? 0 : (u - n_fft + hop) / hop;      // frames f with f hop <= u < f hop + n_fft
+    int a = 0, b = Fk;                                                      // first table entry >= fmin
+    while (a < b) {
+        const int mid = (a + b) >> 1;
+        if (__ldg(frames + mid) < fmin) a = mid + 1; else b = mid;
+    }
+    float acc = 0.f;
+    for (int i = a; i < Fk; ++i) {
+        const int f = __ldg(frames + i);
+        if (f * hop > u) break;
+        acc += __ldg(dA + ((seq * Fk + i) * 2 + c) * (long long)n_fft + (u - f * hop));
+    }
+    return acc;
+}
+__global__ void vr_stft_fold_kept_kernel(const float* __restrict__ dA, const int* __restrict__ frames, float* __restrict__ giq,
+                                         long long S, int T, int Fk, int n_fft, int hop) {
+    const long long total = S * T;
+    const int h = n_fft / 2, U = T + n_fft;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const long long seq = i / T;
+        const int t = (int)(i - seq * T);
+        float2 g = make_float2(0.f, 0.f);
+#pragma unroll
+        for (int side = 0; side < 3; ++side) {          // the direct position and the two mirrors, as vr_stft_fold_kernel
+            const int u = side == 0 ? t + h : (side == 1 ? h - t : h + 2 * (T - 1) - t);
+            const bool on = side == 0 || (side == 1 ? (t >= 1 && t <= h) : (t <= T - 2 && t >= T - 1 - h));
+            if (on && u >= 0 && u < U) {
+                g.x += stft_fold_kept_at(dA, frames, seq, 0, u, Fk, n_fft, hop);
+                g.y += stft_fold_kept_at(dA, frames, seq, 1, u, Fk, n_fft, hop);
             }
         }
         reinterpret_cast<float2*>(giq)[i] = g;

@@ -14,6 +14,7 @@ There is no CPU path and no PyTorch fallback: a CPU tensor, a missing shared obj
 kernels do not cover raises.
 """
 import ctypes
+import functools
 import math
 
 import numpy as np
@@ -63,15 +64,17 @@ class _STFTKernels(torch.nn.Module):
         if not self.is_dft():
             raise NotImplementedError("stft.wsin/wcos differ from the Hann-windowed Fourier kernels")
 
-    def logmag(self, iq):
+    def logmag(self, iq, frames=None):
         """General-kernel path (trained or trainable `wsin`/`wcos`, or an `n_fft` the fused FFT does not cover): what the
         reference computes at layers/virtual_radar.py:124-133 with nnAudio's conv1d STFT, as one float32-accurate GEMM per
         batch on the tensor cores (C ABI vr_stft_general_f32: tcgen05.mma kind::tf32, 3-term split, accumulator in tensor
         memory, magnitude / log / roll in the epilogue), differentiable with respect to `wsin`, `wcos` and `iq`
-        (vr_stft_general_backward_f32).  iq (N,T,2) CUDA float32 -> (N, n_fft, T//hop+1)."""
+        (vr_stft_general_backward_f32).  iq (N,T,2) CUDA float32 -> (N, n_fft, T//hop+1).  `frames` (optional): a strictly
+        increasing int32 CUDA tensor of frame indices; only those columns are computed (vr_stft_general_frames_f32), bit for
+        bit the same, -> (N, n_fft, len(frames))."""
         if not iq.is_cuda:
             raise RuntimeError("the general-kernel STFT (B200) has no CPU path")
-        return _GeneralSTFTFunction.apply(iq, self.wsin, self.wcos, self.n_fft, self.stride, torch.is_grad_enabled())
+        return _GeneralSTFTFunction.apply(iq, self.wsin, self.wcos, self.n_fft, self.stride, torch.is_grad_enabled(), frames)
 
     def _logmag_torch(self, iq):
         """TEST CROSS-CHECK ONLY (never called by forward): the same computation with torch ops (cuBLAS GEMM + autograd)."""
@@ -89,45 +92,54 @@ class _STFTKernels(torch.nn.Module):
 
 class _GeneralSTFTFunction(torch.autograd.Function):
     """STFT against general kernels + log-magnitude + roll: forward and backward are the tcgen05 GEMM kernels of
-    csrc/vr_stft_gemm.cuh behind vr_stft_general_f32 / vr_stft_general_backward_f32 (no library GEMM, no autograd graph)."""
+    csrc/vr_stft_gemm.cuh behind vr_stft_general_f32 / vr_stft_general_backward_f32 (no library GEMM, no autograd graph).
+    With a frame table, only the listed frames (vr_stft_general_frames_f32 / vr_stft_general_frames_backward_f32)."""
 
     @staticmethod
-    def forward(ctx, iq, wsin, wcos, n_fft, hop, grad_mode):
+    def forward(ctx, iq, wsin, wcos, n_fft, hop, grad_mode, frames=None):
         iq = iq.contiguous()
         if iq.dtype != torch.float32 or wsin.dtype != torch.float32:
             raise ValueError("the general-kernel STFT computes in float32")
         N, T, _ = iq.shape
         L = _cabi.lib()
         parts = (ctypes.c_int64 * 3)()
-        L.vr_stft_general_workspace_floats(N, T, n_fft, hop, parts)
+        if frames is None:
+            L.vr_stft_general_workspace_floats(N, T, n_fft, hop, parts)
+            ncols = T // hop + 1
+        else:
+            ncols = frames.numel()
+            L.vr_stft_general_frames_workspace_floats(N, ncols, n_fft, parts)
         dev = iq.device
-        frames = torch.empty(max(int(parts[0]), 1), dtype=torch.float32, device=dev)
+        work = torch.empty(max(int(parts[0]), 1), dtype=torch.float32, device=dev)       # the padded signal / the kept frames
         bt = torch.empty(max(int(parts[1]), 1), dtype=torch.float32, device=dev)
         # needs_input_grad ignores torch.no_grad(): the caller passes the grad mode, so that inference does not write Re / Im
         need = bool(grad_mode) and any(ctx.needs_input_grad[:3])
         csave = torch.empty(max(int(parts[2]), 1), dtype=torch.float32, device=dev) if need else None
-        out = torch.empty((N, n_fft, T // hop + 1), dtype=torch.float32, device=dev)
+        out = torch.empty((N, n_fft, ncols), dtype=torch.float32, device=dev)
         if N > 0:
             with torch.cuda.device(dev):
                 stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-                rc = L.vr_stft_general_f32(iq.data_ptr(), N, T, n_fft, hop, wsin.contiguous().data_ptr(), wcos.contiguous().data_ptr(),
-                                           frames.data_ptr(), bt.data_ptr(), csave.data_ptr() if need else None,
-                                           out.data_ptr(), stream)
+                args = (wsin.contiguous().data_ptr(), wcos.contiguous().data_ptr(), work.data_ptr(), bt.data_ptr(),
+                        csave.data_ptr() if need else None, out.data_ptr(), stream)
+                if frames is None:
+                    rc = L.vr_stft_general_f32(iq.data_ptr(), N, T, n_fft, hop, *args)
+                else:
+                    rc = L.vr_stft_general_frames_f32(iq.data_ptr(), N, T, n_fft, hop, frames.data_ptr(), ncols, *args)
             _cabi.check(rc)
         if need:
-            ctx.save_for_backward(frames, bt, csave)
-        ctx.dims = (N, T, n_fft, hop, tuple(wsin.shape))
+            ctx.save_for_backward(work, bt, csave, frames)
+        ctx.dims = (N, T, n_fft, hop, ncols, tuple(wsin.shape))
         return out
 
     @staticmethod
     def backward(ctx, gout):
-        frames, bt, csave = ctx.saved_tensors
-        N, T, n_fft, hop, wshape = ctx.dims
+        work, bt, csave, frames = ctx.saved_tensors
+        N, T, n_fft, hop, ncols, wshape = ctx.dims
         dev = gout.device
         need_iq, need_w = ctx.needs_input_grad[0], (ctx.needs_input_grad[1] or ctx.needs_input_grad[2])
         g = gout.contiguous().to(torch.float32)
         dc = torch.empty_like(csave)
-        da = torch.empty(N * (T // hop + 1) * 2 * n_fft, dtype=torch.float32, device=dev) if need_iq else None   # frame gradients
+        da = torch.empty(N * ncols * 2 * n_fft, dtype=torch.float32, device=dev) if need_iq else None   # frame gradients
         dbt = torch.empty_like(bt) if need_w else None
         giq = torch.empty((N, T, 2), dtype=torch.float32, device=dev) if need_iq else None
         gsin = torch.empty(wshape, dtype=torch.float32, device=dev) if need_w else None
@@ -136,11 +148,16 @@ class _GeneralSTFTFunction(torch.autograd.Function):
             ptr = lambda t: t.data_ptr() if t is not None else None     # noqa: E731
             with torch.cuda.device(dev):
                 stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-                rc = _cabi.lib().vr_stft_general_backward_f32(g.data_ptr(), frames.data_ptr(), bt.data_ptr(), csave.data_ptr(),
-                                                              N, T, n_fft, hop, dc.data_ptr(), ptr(da), ptr(dbt),
-                                                              ptr(giq), ptr(gsin), ptr(gcos), stream)
+                outs = (dc.data_ptr(), ptr(da), ptr(dbt), ptr(giq), ptr(gsin), ptr(gcos), stream)
+                if frames is None:
+                    rc = _cabi.lib().vr_stft_general_backward_f32(g.data_ptr(), work.data_ptr(), bt.data_ptr(), csave.data_ptr(),
+                                                                  N, T, n_fft, hop, *outs)
+                else:
+                    rc = _cabi.lib().vr_stft_general_frames_backward_f32(g.data_ptr(), work.data_ptr(), bt.data_ptr(),
+                                                                         csave.data_ptr(), N, T, n_fft, hop,
+                                                                         frames.data_ptr(), ncols, *outs)
             _cabi.check(rc)
-        return (giq, gsin if ctx.needs_input_grad[1] else None, gcos if ctx.needs_input_grad[2] else None, None, None, None)
+        return (giq, gsin if ctx.needs_input_grad[1] else None, gcos if ctx.needs_input_grad[2] else None, None, None, None, None)
 
 
 class _RadarFunction(torch.autograd.Function):
@@ -184,7 +201,7 @@ class _SynthFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, lam, loc, xc, layer, flags):
-        _, iq = layer._launch(xc, flags, want_iq=True)
+        iq = layer._synth(xc, flags)
         ctx.save_for_backward(lam, loc, xc)
         ctx.layer, ctx.flags = layer, flags
         return iq
@@ -251,6 +268,55 @@ class _UpsampledRadarFunction(torch.autograd.Function):
         g_lam = gp[0].to(torch.float32).reshape(lam.shape) if ctx.needs_input_grad[0] else None
         g_loc = gp[1:4].to(torch.float32).reshape(loc.shape) if ctx.needs_input_grad[1] else None
         return g_lam, g_loc, None, None, None, None
+
+
+class _UpsampledSynthFunction(torch.autograd.Function):
+    """Complex baseband synthesis of the up-sampled batch -> iq (N, k*T, 2), with gradients for `wavelength` and
+    `radar_location`, without the up-sampled batch: the forward (vr_synth_upsampled_f32) leaves the spline's per-interval
+    cubics in the workspace, from which the backward (vr_synth_adjoint_upsampled_f32) re-evaluates the joint positions.
+    Used by forward_upsampled when the STFT is general and therefore runs outside the fused kernel."""
+
+    @staticmethod
+    def forward(ctx, lam, loc, xc, layer, k, sigma):
+        iq, work = layer._synth_upsampled(xc, k, sigma)
+        ctx.save_for_backward(lam, loc, work)
+        ctx.layer, ctx.dims = layer, tuple(xc.shape) + (k,)
+        return iq
+
+    @staticmethod
+    def backward(ctx, grad_iq):
+        lam, loc, work = ctx.saved_tensors
+        layer = ctx.layer
+        N, _, T, V, M, k = ctx.dims
+        g = grad_iq.contiguous().to(torch.float32)
+        gp = torch.zeros(4, dtype=torch.float64, device=g.device)
+        with torch.cuda.device(g.device):
+            stream = torch.cuda.current_stream(g.device).cuda_stream
+            rc = _cabi.lib().vr_synth_adjoint_upsampled_f32(work.data_ptr(), g.data_ptr(), N, T, V, M, layer._src_c, layer._dst_c,
+                                                            len(layer.src), lam.data_ptr(), loc.data_ptr(), 0, k, gp.data_ptr(),
+                                                            ctypes.c_void_p(stream))
+        _cabi.check(rc)
+        g_lam = gp[0].to(torch.float32).reshape(lam.shape) if ctx.needs_input_grad[0] else None
+        g_loc = gp[1:4].to(torch.float32).reshape(loc.shape) if ctx.needs_input_grad[1] else None
+        return g_lam, g_loc, None, None, None, None
+
+
+def kept_frame_table(n_frames, image_size):
+    """The frames a nearest resize of `n_frames` spectrogram columns to `image_size` reads, by ATen's rule (column c reads
+    min(int(floorf(c * scale)), n_frames - 1), scale = float32(n_frames) / image_size): an int32 array of `image_size`
+    strictly increasing indices when n_frames > image_size, else None (every frame is read; the full STFT is computed)."""
+    if n_frames <= image_size:
+        return None
+    scale = np.float32(n_frames) / np.float32(image_size)
+    idx = np.minimum(np.floor(np.arange(image_size, dtype=np.float32) * scale).astype(np.int64), n_frames - 1)
+    if not (np.diff(idx) > 0).all():
+        raise AssertionError("nearest map from %d columns to %d frames is not strictly increasing" % (image_size, n_frames))
+    return idx.astype(np.int32)
+
+
+@functools.lru_cache(maxsize=64)
+def _kept_frames_on(n_frames, image_size, device):
+    return torch.from_numpy(kept_frame_table(n_frames, image_size)).to(device)
 
 
 class VirtualRadar(torch.nn.Module):
@@ -376,6 +442,60 @@ class VirtualRadar(torch.nn.Module):
         _cabi.check(rc)
         return out, iq
 
+    def _synth(self, xc, flags):
+        """Synthesis only (C ABI vr_synth_f32): the complex baseband signal (N,T,2) that the general-kernel STFT reads,
+        bit for bit forward_debug's, without any STFT work."""
+        N, _, T, V, M = xc.shape
+        if self.assume_inputs_ready:
+            flags |= _cabi.VR_FLAG_INPUTS_READY
+        iq = torch.empty((N, T, 2), dtype=torch.float32, device=xc.device)
+        if N == 0:
+            return iq
+        if self.nvtx_ranges:
+            torch.cuda.nvtx.range_push("VirtualRadar.synth N=%d T=%d" % (N, T))
+        try:
+            with torch.cuda.device(xc.device):
+                stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
+                rc = _cabi.lib().vr_synth_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
+                                              self.wavelength.data_ptr(), self.radar_location.data_ptr(), flags,
+                                              iq.data_ptr(), stream)
+        finally:
+            if self.nvtx_ranges:
+                torch.cuda.nvtx.range_pop()
+        _cabi.check(rc)
+        return iq
+
+    def _synth_upsampled(self, xc, k, sigma):
+        """Synthesis of pad_frames(xc, k, sigma) without the up-sampled batch (C ABI vr_synth_upsampled_f32) -> iq
+        (N, k*T, 2) and the workspace holding the spline's cubics.  The up-sampled tensor the reference's loader builds
+        is standard-contiguous: range rounding mode "seq" (flags 0)."""
+        N, _, T, V, M = xc.shape
+        L = _cabi.lib()
+        nbytes = int(L.vr_upsampled_workspace_bytes(N, T, V, M))
+        work = torch.empty(max(nbytes, 8) // 8, dtype=torch.float64, device=xc.device)
+        iq = torch.empty((N, k * T, 2), dtype=torch.float32, device=xc.device)
+        if N == 0:
+            return iq, work
+        with torch.cuda.device(xc.device):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
+            rc = L.vr_synth_upsampled_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
+                                          self.wavelength.data_ptr(), self.radar_location.data_ptr(), 0, k,
+                                          ctypes.c_float(float(sigma)), work.data_ptr(), nbytes, iq.data_ptr(), stream)
+        _cabi.check(rc)
+        return iq, work
+
+    def _check_general_length(self, T):
+        if T <= max(self.n_fft, self._FUSED_N_FFT) // 2:
+            raise ValueError("T=%d must exceed n_fft/2=%d: reflect padding needs it" % (T, max(self.n_fft, self._FUSED_N_FFT) // 2))
+
+    def _general_image(self, iq, image_size):
+        """`F.interpolate(self.stft.logmag(iq).unsqueeze(1), image_size)` (nearest) bit for bit.  When the spectrogram has
+        more frames than the image has columns, the resize reads exactly `image_size` distinct frames: only those are
+        transformed (kept-frames STFT), and resizing the compact spectrogram -- column scale 1 -- reads each once."""
+        n_frames = iq.shape[1] // self.hop_length + 1
+        frames = _kept_frames_on(n_frames, image_size, iq.device) if n_frames > image_size else None
+        return torch.nn.functional.interpolate(self.stft.logmag(iq, frames).unsqueeze(1), image_size)
+
     def _needs_grad(self, x=None):
         return torch.is_grad_enabled() and (self.wavelength.requires_grad or self.radar_location.requires_grad
                                             or (x is not None and x.requires_grad))
@@ -390,16 +510,17 @@ class VirtualRadar(torch.nn.Module):
         """forward() after the layout has been normalised: xc standard-contiguous, flags carry the range rounding mode."""
         lam, loc = self.wavelength, self.radar_location
         if self._general_stft():     # trained / trainable STFT kernels: synthesis on our kernels, STFT as a GEMM
-            if xc.shape[2] <= max(self.n_fft, self._FUSED_N_FFT) // 2:
-                raise ValueError("T=%d must exceed n_fft/2=%d: reflect padding needs it"
-                                 % (xc.shape[2], max(self.n_fft, self._FUSED_N_FFT) // 2))
+            self._check_general_length(xc.shape[2])
             if xc.shape[0] == 0:
                 return self._launch(xc, flags)[0]
-            iq = _SynthFunction.apply(lam, loc, xc, self, flags) if self._needs_grad(x) else self._launch(xc, flags, want_iq=True)[1]
-            return self.stft.logmag(iq)
+            return self.stft.logmag(self._general_iq(x, xc, flags))
         if self._needs_grad(x) and xc.shape[0] > 0:
             return _RadarFunction.apply(lam, loc, xc, self, flags)
         return self._launch(xc, flags)[0]
+
+    def _general_iq(self, x, xc, flags):
+        lam, loc = self.wavelength, self.radar_location
+        return _SynthFunction.apply(lam, loc, xc, self, flags) if self._needs_grad(x) else self._synth(xc, flags)
 
     def forward_notebook(self, data, num_pad_frames=1, sigma=3):
         """virtual_radar_example.ipynb cells 2-4 on the device: `data` is one body's (T, V, 3) array (or a batch
@@ -427,7 +548,11 @@ class VirtualRadar(torch.nn.Module):
         image_size = int(image_size)
         if image_size < 1:
             raise ValueError("image_size must be positive, got %d" % image_size)
-        if self._needs_grad(x) or self._general_stft():     # gradients wanted / general STFT kernels: spectrogram, then torch's resize
+        if self._general_stft():        # general STFT kernels: synthesis, then the STFT of the frames the resize keeps
+            xc, flags = self._prepare(x)
+            self._check_general_length(xc.shape[2])
+            return self._general_image(self._general_iq(x, xc, flags), image_size)
+        if self._needs_grad(x):         # gradients wanted: spectrogram, then torch's resize
             return torch.nn.functional.interpolate(self.forward(x).unsqueeze(1), image_size)
         xc, flags = self._prepare(x)
         if self.assume_inputs_ready:
@@ -465,10 +590,13 @@ class VirtualRadar(torch.nn.Module):
         if x.requires_grad and torch.is_grad_enabled():
             raise NotImplementedError("forward_upsampled has no gradient with respect to x: detach x, or differentiate "
                                       "layer(pad_frames(x, num_pad_frames, sigma)), which materialises the up-sampled batch")
-        if self._general_stft():      # general STFT kernels: materialise the up-sampled batch
-            from ..upsample import pad_frames
-            up = pad_frames(xc, k, sigma)
-            return self.forward_image(up, img) if img else self.forward(up)
+        if self._general_stft():      # general STFT kernels: synthesis without the up-sampled batch, then the GEMM STFT
+            if self._needs_grad() and N > 0:
+                iq = _UpsampledSynthFunction.apply(lam, loc, xc, self, k, sigma)
+            else:
+                iq = self._synth_upsampled(xc, k, sigma)[0]
+            self._check_general_length(k * T)
+            return self._general_image(iq, img) if img else self.stft.logmag(iq)
         if self._needs_grad() and N > 0:
             out = _UpsampledRadarFunction.apply(lam, loc, xc, self, k, sigma)
             return torch.nn.functional.interpolate(out.unsqueeze(1), img) if img else out
