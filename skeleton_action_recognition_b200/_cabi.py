@@ -21,7 +21,8 @@ SYMBOLS = ("vr_abi_version", "vr_last_error", "vr_forward_f32", "vr_forward_debu
            "vr_pad_frames_backward_f32", "vr_forward_upsampled_debug_f32", "vr_backward_upsampled_params_f32",
            "vr_stft_general_workspace_floats", "vr_stft_general_f32", "vr_stft_general_backward_f32",
            "vr_synth_f32", "vr_synth_upsampled_f32", "vr_synth_adjoint_upsampled_f32",
-           "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32")
+           "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32",
+           "vr_plan_adjoint_stft")
 
 _lib = None
 
@@ -97,6 +98,8 @@ def lib():
     L.vr_stft_general_frames_f32.restype = ctypes.c_int
     L.vr_stft_general_frames_backward_f32.argtypes = [vp, vp, vp, vp, i64, i64, i32, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp]
     L.vr_stft_general_frames_backward_f32.restype = ctypes.c_int
+    L.vr_plan_adjoint_stft.argtypes = [i64, i64, i32, i32, ctypes.POINTER(i64), ctypes.POINTER(i64), i64]
+    L.vr_plan_adjoint_stft.restype = ctypes.c_int
     L.vr_set_timeline_buffer.argtypes = [vp]
     L.vr_set_timeline_buffer.restype = ctypes.c_int
     L.vr_selftest_rounding.argtypes = [ctypes.c_uint64, f32, ctypes.POINTER(ctypes.c_uint64)]
@@ -158,6 +161,20 @@ def plan_team(N, T, V, M, src, dst, n_fft=256, hop=16, sm_count=148):
     out = (ctypes.c_int64 * 8)()
     check(lib().vr_plan_team(N, T, V, M, i32_array(src), i32_array(dst), len(src), n_fft, hop, sm_count, out))
     return dict(zip(TEAM_PLAN_FIELDS, [int(v) for v in out]))
+
+
+ADJOINT_PLAN_FIELDS = ("segment_length", "segments", "grid", "smem_bytes")
+
+
+def plan_adjoint_stft(N, T, hop=16, sm_count=148):
+    """The owner-form plan of the adjoint STFT -> (plan dict, [(first sample, end sample, first frame, last frame)] per
+    segment of a sequence)."""
+    out = (ctypes.c_int64 * 4)()
+    check(lib().vr_plan_adjoint_stft(N, T, hop, sm_count, out, None, 0))
+    plan = dict(zip(ADJOINT_PLAN_FIELDS, [int(v) for v in out]))
+    rows = (ctypes.c_int64 * (4 * plan["segments"]))()
+    check(lib().vr_plan_adjoint_stft(N, T, hop, sm_count, out, rows, plan["segments"]))
+    return plan, [tuple(int(v) for v in rows[4 * k:4 * k + 4]) for k in range(plan["segments"])]
 
 
 def set_schedule(mode):

@@ -6,11 +6,14 @@
 //   vr_stft_adjoint_kernel   grad_out (N, 256, F) and the saved complex baseband signal z (N, T, 2)
 //                            -> dL/dz (N, T, 2): per frame, X = FFT(hann * zp); G = g * X / (|X| (|X| + 1e-6))
 //                            (log-magnitude and fftshift, :126-133); dL/dzp = hann * conj(FFT(conj(G))) (the
-//                            adjoint of the windowed DFT, :124-125); overlap-add through the reflect padding.
+//                            adjoint of the windowed DFT, :124-125); overlap-add through the reflect padding, in
+//                            owner form: a CTA owns a segment of samples and adds every contribution to it in a fixed
+//                            order (adj_seg_frames), so dL/dz is bitwise reproducible and independent of the batch.
 //   vr_synth_adjoint_kernel  dL/dz and x -> dL/dwavelength, dL/dradar_location (and, on request, dL/dx): per (sequence, time step, body,
 //                            bone) the forward geometry is recomputed (range and phase with the forward's exact
 //                            float32 rounding, the rest in float64) and the analytic derivatives of
-//                            z = sum amp * exp(j theta) are accumulated in float64.
+//                            z = sum amp * exp(j theta) are accumulated in float64; the block partials of the
+//                            parameter gradients are added in block order by the last block (synth_adjoint_reduce).
 //
 // theta = 4 pi d / lambda reaches 1e4..1e5 rad, so dtheta/dlambda = -theta/lambda is of order 1e7..1e8: the
 // reference's float32 autograd result carries relative errors of 1e-3 and more; these kernels are checked
@@ -25,8 +28,11 @@ struct BwdParams {
     const float* x;              // (N,3,T,V,M)
     const float* iq;             // (N,T,2) saved by the forward (vr_forward_debug_f32)
     const float* gout;           // (N,256,F)
-    float* gz;                   // (N,T,2) work buffer, zeroed before the adjoint STFT
-    double* gparams;             // [dL/dlambda, dL/dLx, dL/dLy, dL/dLz], accumulated with atomics
+    float* gz;                   // (N,T,2) dL/dz: every sample written once by the adjoint STFT
+    double* gparams;             // [dL/dlambda, dL/dLx, dL/dLy, dL/dLz]: the launch's total is added by its last block
+    double* part;                // this launch's slot of g_param_partials: 4 partials per block
+    unsigned* count;             // and its counter of finished blocks (0 between launches)
+    int seg_len, segs;           // adjoint STFT: samples per segment, segments per sequence (adjoint_plan)
     float* gx;                   // optional dL/dx (N,3,T,V,M), zeroed before the launch; nullptr = not wanted
     const float* lam_ptr;
     const float* loc_ptr;
@@ -39,6 +45,45 @@ struct BwdParams {
     int ups_T;
     uint16_t src[NG * MAX_EG], dst[NG * MAX_EG];
 };
+
+// ---- owner-form plan of the adjoint STFT -----------------------------------------------------------------------------
+// The samples of a sequence are cut into segments of seg_len samples; one CTA at a time owns a segment.  Frame f covers the
+// padded positions u in [f hop, f hop + 256); sample t sits at u = t + 128, and through the reflect padding also at u = 128 - t
+// (1 <= t <= 128) and u = 128 + 2 (T - 1) - t (T - 129 <= t <= T - 2).  A segment transforms every frame that reaches one of
+// its samples by any of the three, including halo frames its neighbours transform as well, and adds each sample's
+// contributions frame by frame in increasing order, direct position before the mirrors: the order depends on neither the
+// segment cut nor the batch.
+constexpr int ADJ_SEG_MAX = 4096;          // samples per segment: the float2 accumulators live in shared memory (32 KB,
+                                           // 56 KB per CTA with the FFT buffers: four CTAs per SM)
+constexpr int ADJ_SEG_MIN = 1024;          // a cut costs 256 / hop - 1 halo frames; below this it would cost more than 1/5
+
+// the frames [lo, hi] that reach samples [s0, s1) (lo > hi: none)
+__host__ __device__ inline void adj_seg_frames(long long s0, long long s1, long long T, int F, int hop, int& lo, int& hi) {
+    long long ulo = s0 + 128, uhi = s1 - 1 + 128;                                           // direct positions
+    const long long a = s0 > 1 ? s0 : 1, b = s1 - 1 < 128 ? s1 - 1 : 128;                   // left mirror
+    if (a <= b) { ulo = ulo < 128 - b ? ulo : 128 - b; uhi = uhi > 128 - a ? uhi : 128 - a; }
+    const long long c = s0 > T - 129 ? s0 : T - 129, d = s1 - 1 < T - 2 ? s1 - 1 : T - 2;  // right mirror
+    if (c <= d) { ulo = ulo < 126 + 2 * T - d ? ulo : 126 + 2 * T - d; uhi = uhi > 126 + 2 * T - c ? uhi : 126 + 2 * T - c; }
+    const long long f0 = ulo - 255 <= 0 ? 0 : (ulo - 255 + hop - 1) / hop, f1 = uhi / hop;
+    lo = (int)f0;
+    hi = (int)(f1 < F - 1 ? f1 : F - 1);
+}
+
+// The host's choice: enough segments that the batch fills the machine (about four CTAs per SM), none shorter than
+// ADJ_SEG_MIN unless it is the whole sequence, none longer than ADJ_SEG_MAX.  The result does not depend on it.
+inline void adjoint_plan(long long N, long long T, int sm_count, int& seg_len, int& segs) {
+    const long long want = (4ll * sm_count + N - 1) / N;
+    long long s = (T + ADJ_SEG_MIN - 1) / ADJ_SEG_MIN;
+    s = want < s ? want : s;
+    const long long smin = (T + ADJ_SEG_MAX - 1) / ADJ_SEG_MAX;
+    s = s > smin ? s : smin;
+    s = s > 1 ? s : 1;
+    long long len = (T + s - 1) / s;
+    len = (len + 31) / 32 * 32;
+    if (len > ADJ_SEG_MAX) len = ADJ_SEG_MAX;
+    seg_len = (int)len;
+    segs = (int)((T + len - 1) / len);
+}
 
 #ifdef __CUDACC__
 // 256-point forward DFT (e^{-j...}) of one frame by one warp.  In: v[q] = sample lane + 32 q.  Out: v holds
@@ -83,11 +128,19 @@ __device__ __forceinline__ int bwd_reflect(int t, int T) {       // nnAudio cent
 
 constexpr int BWD_WARPS = 8;
 
+// One CTA per (sequence, segment) job.  Round after round, warp w transforms frame lo + round * BWD_WARPS + w and parks its
+// Hann-weighted contributions in its slot of shared memory (tr); after a barrier the segment's samples that the round reaches
+// take them from the slots in frame order into their float2 accumulators (acc, dynamic shared memory: seg_len entries).
+// Each sample of gz is written once at the end of its job; a sample no frame covers (hop > 256) gets exactly 0.
 __global__ void __launch_bounds__(BWD_WARPS * 32) vr_stft_adjoint_kernel(const __grid_constant__ BwdParams p) {
     __shared__ float4 tw1[7 * 32 + 7 * 4];
     __shared__ float hann[NFFT];
+    // per warp: the FFT exchange buffer, also the parking place of G between the two FFTs and, after the second, the
+    // frame's contribution slot that the gather reads (every use is separated from the next by a __syncwarp inside
+    // bwd_fft256 or the round's __syncthreads)
     __shared__ float2 xch_all[BWD_WARPS][8 * XCH_STRIDE];
-    __shared__ float2 tr_all[BWD_WARPS][NFFT];
+    static_assert(8 * XCH_STRIDE >= NFFT, "a frame's 256 values fit the exchange buffer");
+    extern __shared__ float2 acc[];
     float4* tw2 = tw1 + 7 * 32;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (int i = tid; i < 7 * 32 + 7 * 4; i += blockDim.x) {
@@ -99,44 +152,78 @@ __global__ void __launch_bounds__(BWD_WARPS * 32) vr_stft_adjoint_kernel(const _
     for (int i = tid; i < NFFT; i += blockDim.x) hann[i] = fmaf(-0.5f, cospif((float)i * (2.0f / NFFT)), 0.5f);
     __syncthreads();
     float2* xch = xch_all[warp];
-    float2* tr = tr_all[warp];
-    const int T = (int)p.T;
-    const long long frames = p.N * (long long)p.F;
-    for (long long fr = (long long)blockIdx.x * BWD_WARPS + warp; fr < frames; fr += (long long)gridDim.x * BWD_WARPS) {
-        const long long n = fr / p.F;
-        const int f = (int)(fr - n * p.F);
+    float2* tr = xch_all[warp];
+    const int T = (int)p.T, hop = p.hop, h = NFFT / 2;
+    const long long jobs = p.N * (long long)p.segs;
+    for (long long job = blockIdx.x; job < jobs; job += gridDim.x) {
+        const long long n = job / p.segs;
+        const int s0 = (int)(job - n * p.segs) * p.seg_len;
+        const int s1 = s0 + p.seg_len < T ? s0 + p.seg_len : T;
+        int flo, fhi;
+        adj_seg_frames(s0, s1, T, p.F, hop, flo, fhi);
+        for (int i = tid; i < s1 - s0; i += blockDim.x) acc[i] = make_float2(0.f, 0.f);
         const float2* z = reinterpret_cast<const float2*>(p.iq) + n * T;
-        const int fstart = f * p.hop - NFFT / 2;
-        c2 v[8];
+        const float* gn = p.gout + n * (long long)NFFT * p.F;
+        for (int f0 = flo; f0 <= fhi; f0 += BWD_WARPS) {
+            const int nf = fhi - f0 + 1 < BWD_WARPS ? fhi - f0 + 1 : BWD_WARPS;
+            if (warp < nf) {
+                const int f = f0 + warp;
+                const int fstart = f * hop - h;
+                c2 v[8];
 #pragma unroll
-        for (int q = 0; q < 8; ++q) {
-            const int nidx = lane + 32 * q;
-            v[q] = pscale(__ldg(z + bwd_reflect(fstart + nidx, T)), hann[nidx]);
+                for (int q = 0; q < 8; ++q) {
+                    const int nidx = lane + 32 * q;
+                    v[q] = pscale(__ldg(z + bwd_reflect(fstart + nidx, T)), hann[nidx]);
+                }
+                bwd_fft256(v, xch, tw1, tw2, lane);
+                // log-magnitude + fftshift backward: G = g X / (|X| (|X| + 1e-6)); park conj(G) by bin
+                const float* g = gn + f;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const int kbin = bwd_bin(lane, j);
+                    const int row = (kbin + NFFT / 2) & (NFFT - 1);
+                    const float a = sqrtf(v[j].x * v[j].x + v[j].y * v[j].y);
+                    const float s = a > 0.f ? __ldg(g + (size_t)row * p.F) / (a * (a + 1e-6f)) : 0.f;
+                    tr[kbin] = make_float2(s * v[j].x, -s * v[j].y);
+                }
+                __syncwarp();
+#pragma unroll
+                for (int q = 0; q < 8; ++q) v[q] = tr[lane + 32 * q];
+                bwd_fft256(v, xch, tw1, tw2, lane);
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {                        // the frame's contribution at padded position f hop + nidx
+                    const int nidx = bwd_bin(lane, j);
+                    const float w = hann[nidx];
+                    tr[nidx] = make_float2(w * v[j].x, -w * v[j].y);
+                }
+            }
+            __syncthreads();
+            // the samples this round reaches: direct t = u - 128 for u in [ulo, uhi], and the mirrors
+            const int ulo = f0 * hop, uhi = (f0 + nf - 1) * hop + NFFT - 1;
+            int tlo = ulo - h, thi = uhi - h;
+            if (ulo < h) thi = thi > h - ulo ? thi : h - ulo;
+            if (uhi >= T + h) { const int m = 2 * (T - 1) + h - (uhi < T + NFFT - 1 ? uhi : T + NFFT - 1); tlo = tlo < m ? tlo : m; }
+            tlo = tlo > s0 ? tlo : s0;
+            thi = thi < s1 - 1 ? thi : s1 - 1;
+            for (int t = tlo + tid; t <= thi; t += blockDim.x) {
+                float2 a = acc[t - s0];
+                const bool left = t >= 1 && t <= h, right = t >= T - 1 - h && t <= T - 2;
+                for (int w = 0; w < nf; ++w) {
+                    const int fb = (f0 + w) * hop;
+                    const float2* c = xch_all[w];
+                    int j = t + h - fb;
+                    if ((unsigned)j < (unsigned)NFFT) { a.x += c[j].x; a.y += c[j].y; }
+                    j = h - t - fb;
+                    if (left && (unsigned)j < (unsigned)NFFT) { a.x += c[j].x; a.y += c[j].y; }
+                    j = h + 2 * (T - 1) - t - fb;
+                    if (right && (unsigned)j < (unsigned)NFFT) { a.x += c[j].x; a.y += c[j].y; }
+                }
+                acc[t - s0] = a;
+            }
+            __syncthreads();
         }
-        bwd_fft256(v, xch, tw1, tw2, lane);
-        // log-magnitude + fftshift backward: G = g X / (|X| (|X| + 1e-6)); park conj(G) by bin
-        const float* g = p.gout + n * (long long)NFFT * p.F + f;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const int kbin = bwd_bin(lane, j);
-            const int row = (kbin + NFFT / 2) & (NFFT - 1);
-            const float a = sqrtf(v[j].x * v[j].x + v[j].y * v[j].y);
-            const float s = a > 0.f ? __ldg(g + (size_t)row * p.F) / (a * (a + 1e-6f)) : 0.f;
-            tr[kbin] = make_float2(s * v[j].x, -s * v[j].y);
-        }
-        __syncwarp();
-#pragma unroll
-        for (int q = 0; q < 8; ++q) v[q] = tr[lane + 32 * q];
-        bwd_fft256(v, xch, tw1, tw2, lane);
-        float* gz = p.gz + n * (long long)T * 2;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const int nidx = bwd_bin(lane, j);
-            const int t = bwd_reflect(fstart + nidx, T);
-            const float w = hann[nidx];
-            atomicAdd(gz + 2 * t, w * v[j].x);
-            atomicAdd(gz + 2 * t + 1, -w * v[j].y);
-        }
+        float2* gz = reinterpret_cast<float2*>(p.gz) + n * T;
+        for (int i = tid; i < s1 - s0; i += blockDim.x) gz[s0 + i] = acc[i];
     }
 }
 
@@ -241,10 +328,17 @@ __device__ __forceinline__ void synth_adjoint_body(const BwdParams& p, const Pos
     }
 }
 
-// block reduction of the four parameter gradients, then one float64 atomic per block and parameter
-__device__ __forceinline__ void synth_adjoint_reduce(const BwdParams& p, double g_lam, double g_lx, double g_ly, double g_lz) {
-    __shared__ double red[4][4];
-    double vals[4] = {g_lam, g_lx, g_ly, g_lz};
+// The parameter gradients' partial sums: PARAM_SLOTS slots of static memory, handed out round-robin per launch by the host
+// (like the forward's ticket pool), so that launches in flight on different streams do not share one.  A slot holds 4
+// partials per block and a counter of finished blocks.  Budget: PARAM_MAX_BLOCKS * 4 doubles per slot (80 KB),
+// PARAM_SLOTS slots (2.5 MB); the host caps the grid at PARAM_MAX_BLOCKS.
+constexpr int PARAM_SLOTS = 32;
+constexpr int PARAM_MAX_BLOCKS = 2560;
+__device__ double g_param_partials[PARAM_SLOTS][PARAM_MAX_BLOCKS * 4];
+__device__ unsigned g_param_count[PARAM_SLOTS];
+
+// sum over the block's 128 threads in a fixed order: warp shuffles, then the four warps' sums in pairs
+__device__ __forceinline__ void block_sum4(double (&vals)[4], double (&red)[4][4]) {
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         double v = vals[i];
@@ -252,10 +346,38 @@ __device__ __forceinline__ void synth_adjoint_reduce(const BwdParams& p, double 
         if ((threadIdx.x & 31) == 0) red[i][threadIdx.x >> 5] = v;
     }
     __syncthreads();
-    if (threadIdx.x < 4) {
-        const double v = (red[threadIdx.x][0] + red[threadIdx.x][1]) + (red[threadIdx.x][2] + red[threadIdx.x][3]);
-        if (v != 0.0) atomicAdd(p.gparams + threadIdx.x, v);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) vals[i] = (red[i][0] + red[i][1]) + (red[i][2] + red[i][3]);
+    __syncthreads();
+}
+
+// Block reduction of the four parameter gradients into the block's partials; the last block to finish adds the partials in
+// block order, adds the total to gparams and re-arms the counter.  No float atomics: the result depends only on the
+// inputs and the grid, and the grid only on (N, T, sm_count).  128 threads per block.
+__device__ __forceinline__ void synth_adjoint_reduce(const BwdParams& p, double g_lam, double g_lx, double g_ly, double g_lz) {
+    __shared__ double red[4][4];
+    __shared__ bool last;
+    double vals[4] = {g_lam, g_lx, g_ly, g_lz};
+    block_sum4(vals, red);
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        if (threadIdx.x == i) p.part[blockIdx.x * 4 + i] = vals[i];
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) last = atomicAdd(p.count, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    double acc[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int b = threadIdx.x; b < (int)gridDim.x; b += blockDim.x) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) acc[i] += __ldcg(p.part + b * 4 + i);
     }
+    block_sum4(acc, red);
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        if (threadIdx.x == i) p.gparams[i] += acc[i];
+    if (threadIdx.x == 0) *p.count = 0u;
 }
 
 __global__ void __launch_bounds__(128) vr_synth_adjoint_kernel(const __grid_constant__ BwdParams p) {

@@ -353,7 +353,11 @@ KernelFn pick_kernel(bool fma, int vm, int m, bool ups, bool park) {
 
 constexpr int TEAM_AUTO_WAVES = 3;      // automatic schedule: team-job kernel from this many jobs per team slot
 
-struct DeviceInfo { int sm_count = 0; bool attr_set = false; int* tickets = nullptr; unsigned next_slot = 0; };
+struct DeviceInfo {
+    int sm_count = 0; bool attr_set = false; int* tickets = nullptr; unsigned next_slot = 0;
+    double* param_partials = nullptr; unsigned* param_count = nullptr; unsigned next_param_slot = 0;
+    float* splitk_pool = nullptr; unsigned next_splitk_slot = 0;
+};
 std::mutex g_mu;
 DeviceInfo g_dev[64];
 
@@ -373,6 +377,10 @@ int device_setup(int& dev, int& sm_count) {
         for (int i = 0; i < kNumTeamVariants; ++i)
             CUDA_TRY(cudaFuncSetAttribute(kTeamVariants[i].fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
         CUDA_TRY(cudaGetSymbolAddress((void**)&d.tickets, vr::g_ticket_pool));
+        CUDA_TRY(cudaFuncSetAttribute(vr::vr_stft_adjoint_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, vr::ADJ_SEG_MAX * 8));
+        CUDA_TRY(cudaGetSymbolAddress((void**)&d.param_partials, vr::g_param_partials));
+        CUDA_TRY(cudaGetSymbolAddress((void**)&d.param_count, vr::g_param_count));
+        CUDA_TRY(cudaGetSymbolAddress((void**)&d.splitk_pool, vr::g_splitk_pool));
         d.attr_set = true;
     }
     sm_count = d.sm_count;
@@ -384,6 +392,22 @@ int* next_ticket_slot(int dev) {
     std::lock_guard<std::mutex> lk(g_mu);
     DeviceInfo& d = g_dev[dev];
     return d.tickets + 2 * (d.next_slot++ % vr::TICKET_SLOTS);
+}
+
+// a slot of the parameter-gradient partials for one synthesis-adjoint launch
+void next_param_slot(int dev, vr::BwdParams& p) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    DeviceInfo& d = g_dev[dev];
+    const unsigned s = d.next_param_slot++ % vr::PARAM_SLOTS;
+    p.part = d.param_partials + (size_t)s * vr::PARAM_MAX_BLOCKS * 4;
+    p.count = d.param_count + s;
+}
+
+// a slot of the kernel gradient's split-K partials for one launch
+float* next_splitk_slot(int dev) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    DeviceInfo& d = g_dev[dev];
+    return d.splitk_pool + (size_t)(d.next_splitk_slot++ % vr::G_SPLIT_SLOTS) * vr::G_SPLIT_SLOT_FLOATS;
 }
 
 // Plans depend only on shapes and the bone list; the last one is kept per host thread so that a
@@ -966,15 +990,15 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     p.ups_ratio = coef ? (double)(ups_T - 1) / (double)((long long)ups_K * ups_T - 1) : 0.0;
     cudaStream_t st = (cudaStream_t)stream;
     if (grad_x_dev) CUDA_TRY(cudaMemsetAsync(grad_x_dev, 0, (size_t)N * 3 * T * V * M * sizeof(float), st));
-    if (!synth_only) {
-        CUDA_TRY(cudaMemsetAsync(gz_work_dev, 0, (size_t)N * T * 2 * sizeof(float), st));
-        const long long frames = N * (long long)p.F;
-        const int grid1 = (int)std::min<long long>((frames + vr::BWD_WARPS - 1) / vr::BWD_WARPS, (long long)sm_count * 8);
-        vr::vr_stft_adjoint_kernel<<<grid1, vr::BWD_WARPS * 32, 0, st>>>(p);
+    if (!synth_only) {                                  // writes every sample of gz: no zero fill
+        vr::adjoint_plan(N, T, sm_count, p.seg_len, p.segs);
+        const int grid1 = (int)std::min<long long>(N * p.segs, (long long)sm_count * 8);
+        vr::vr_stft_adjoint_kernel<<<grid1, vr::BWD_WARPS * 32, (size_t)p.seg_len * 8, st>>>(p);
         CUDA_TRY(cudaGetLastError());
     }
     const long long steps = N * T;
-    const int grid2 = (int)std::min<long long>((steps + 127) / 128, (long long)sm_count * 16);
+    const int grid2 = (int)std::min<long long>(std::min<long long>((steps + 127) / 128, (long long)sm_count * 16), vr::PARAM_MAX_BLOCKS);
+    next_param_slot(dev, p);
     if (coef) vr::vr_synth_adjoint_ups_kernel<<<grid2, 128, 0, st>>>(p);
     else vr::vr_synth_adjoint_kernel<<<grid2, 128, 0, st>>>(p);
     CUDA_TRY(cudaGetLastError());
@@ -1063,6 +1087,30 @@ int vr_selftest_rounding(uint64_t n, float wavelength, uint64_t mismatches[3]) {
     return VR_OK;
 }
 
+int vr_plan_adjoint_stft(int64_t N, int64_t T, int32_t hop, int32_t sm_count, int64_t plan[4], int64_t* segments,
+                         int64_t max_segments) {
+    if (!plan) return fail(VR_ERR_ARG, "plan must not be null");
+    if (N <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, hop must be positive");
+    if (T <= vr::NFFT / 2) return fail(VR_ERR_SHAPE, "T=%lld must exceed n_fft/2=%d", (long long)T, vr::NFFT / 2);
+    if (T > (1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T=%lld too long", (long long)T);
+    const int sms = sm_count > 0 ? sm_count : 148;
+    int seg_len, segs;
+    vr::adjoint_plan(N, T, sms, seg_len, segs);
+    plan[0] = seg_len; plan[1] = segs; plan[2] = std::min<long long>(N * segs, (long long)sms * 8); plan[3] = (int64_t)seg_len * 8;
+    if (segments) {
+        if (max_segments < segs) return fail(VR_ERR_ARG, "segments holds %lld rows, the plan has %d", (long long)max_segments, segs);
+        const int F = (int)(T / hop) + 1;
+        for (int k = 0; k < segs; ++k) {
+            const long long s0 = (long long)k * seg_len, s1 = std::min<long long>(T, s0 + seg_len);
+            int lo, hi;
+            vr::adj_seg_frames(s0, s1, T, F, hop, lo, hi);
+            int64_t* r = segments + 4 * k;
+            r[0] = s0; r[1] = s1; r[2] = lo; r[3] = hi;
+        }
+    }
+    return VR_OK;
+}
+
 int vr_partition_edges(const int32_t* src_host, const int32_t* dst_host, int32_t E, int32_t V, int32_t* group_of_edge) {
     if (!group_of_edge) return fail(VR_ERR_ARG, "group_of_edge must not be null");
     Partition P;
@@ -1137,7 +1185,7 @@ int stft_forward_gemm(const float* P, long long Lp, int hop, int F, int64_t N, i
 // (kernel gradients, reduced over every frame of the batch)
 int stft_backward_gemm(const float* grad_out_dev, const float* P, long long Lp, int hop, int F, int64_t N, int n_fft,
                        const float* bt_work, const float* c_save, float* dc_work, float* da_work, float* dbt_work,
-                       float* grad_wsin_dev, float* grad_wcos_dev, int sm_count, cudaStream_t st) {
+                       float* grad_wsin_dev, float* grad_wcos_dev, int dev, int sm_count, cudaStream_t st) {
     const int nb = stft_nb(n_fft), K = 2 * n_fft;
     const long long M = N * (long long)F;
     const long long ldm = stft_ldm(M);
@@ -1157,18 +1205,18 @@ int stft_backward_gemm(const float* grad_out_dev, const float* P, long long Lp, 
         g.P = P; g.Lp = Lp; g.hop = hop; g.F = F; g.n_fft = n_fft;     // B'(n' = k, k' = m) = A[m][k], a view
         g.M = K; g.N = K; g.K = (int)M; g.C = dbt_work; g.ldc = K;
         // the reduction runs over all frames of the batch: split it over gridDim.z so that the (2 n_fft / 128)^2 output
-        // tiles fill the machine; the slices add into the zeroed result with float atomics
+        // tiles fill the machine; each slice writes its own K x K plane of a split-K pool slot, added in slice order below
         const int tiles = ((K + vr::GM - 1) / vr::GM) * ((K + vr::GN - 1) / vr::GN);
         const int kb_all = (int)((M + vr::GK - 1) / vr::GK);
         // one CTA per SM at a time (192 KB of stages): whole waves, i.e. splits * tiles <= a multiple of sm_count; one wave
-        // unless that leaves a slice fewer than 8 K blocks
-        int splits = std::max(1, std::min(sm_count / tiles, (kb_all + 7) / 8));
+        // unless that leaves a slice fewer than 8 K blocks; and no more planes than a pool slot holds
+        int splits = std::max(1, std::min(std::min(sm_count, vr::G_SPLIT_CTAS_MAX) / tiles, (kb_all + 7) / 8));
         g.kb_per_split = (kb_all + splits - 1) / splits;
         splits = (kb_all + g.kb_per_split - 1) / g.kb_per_split;
-        if (splits > 1) CUDA_TRY(cudaMemsetAsync(dbt_work, 0, (size_t)K * K * sizeof(float), st));
-        dim3 grid((unsigned)(((K + vr::GM - 1) / vr::GM) * ((K + vr::GN - 1) / vr::GN)), 1u, (unsigned)splits);
+        if (splits > 1) { g.C = next_splitk_slot(dev); g.c_split = (long long)K * K; }
+        dim3 grid((unsigned)tiles, 1u, (unsigned)splits);
         vr::vr_gemm_tf32x3_kernel<0, vr::G_STRIDED, vr::G_FRAME_COLS><<<grid, vr::G_THREADS, vr::G_SMEM_BYTES, st>>>(g);
-        vr::vr_stft_dw_kernel<<<(n_fft * n_fft + 255) / 256, 256, 0, st>>>(dbt_work, grad_wsin_dev, grad_wcos_dev, n_fft, nb);
+        vr::vr_stft_dw_kernel<<<(n_fft * n_fft + 255) / 256, 256, 0, st>>>(g.C, splits, g.c_split, grad_wsin_dev, grad_wcos_dev, n_fft, nb);
     }
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
@@ -1249,7 +1297,7 @@ int vr_stft_general_backward_f32(const float* grad_out_dev, const float* frames_
     cudaStream_t st = (cudaStream_t)stream;
     const int F = (int)(T / hop) + 1;
     rc = stft_backward_gemm(grad_out_dev, frames_work, stft_lp(T, n_fft), hop, F, N, n_fft, bt_work, c_save, dc_work, da_work,
-                            dbt_work, grad_wsin_dev, grad_wcos_dev, sm_count, st);
+                            dbt_work, grad_wsin_dev, grad_wcos_dev, dev, sm_count, st);
     if (rc || !da_work) return rc;
     vr::vr_stft_fold_kernel<<<(unsigned)std::min<long long>((N * T + 255) / 256, sm_count * 16ll), 256, 0, st>>>(da_work, grad_iq_dev, N, (int)T, F, n_fft, hop);
     CUDA_TRY(cudaGetLastError());
@@ -1291,7 +1339,7 @@ int vr_stft_general_frames_backward_f32(const float* grad_out_dev, const float* 
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     rc = stft_backward_gemm(grad_out_dev, frames_work, F_kept * (long long)n_fft, n_fft, (int)F_kept, N, n_fft, bt_work, c_save,
-                            dc_work, da_work, dbt_work, grad_wsin_dev, grad_wcos_dev, sm_count, st);
+                            dc_work, da_work, dbt_work, grad_wsin_dev, grad_wcos_dev, dev, sm_count, st);
     if (rc || !da_work) return rc;
     vr::vr_stft_fold_kept_kernel<<<(unsigned)std::min<long long>((N * T + 255) / 256, sm_count * 16ll), 256, 0, st>>>(da_work, frames_dev, grad_iq_dev, N, (int)T, (int)F_kept, n_fft, hop);
     CUDA_TRY(cudaGetLastError());

@@ -27,6 +27,9 @@
 // into the (N, n_fft, F) output, optionally saving Re/Im for the backward pass.
 // The same kernel does the backward GEMMs (operands are addressed through element strides, the frame view or the tiled
 // image, so transposes cost nothing): dA = dC . Bt (gradient of the frames) and dBt = dC^T . A (gradient of the kernels).
+// The kernel gradient's reduction runs over every frame of the batch and is split over gridDim.z; each slice stores its
+// partial dBt with plain stores into its own K x K plane of a static pool, and vr_stft_dw_kernel adds the planes in slice
+// order: no float atomics, no CTA waiting on another, the same bits on every run.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -62,8 +65,9 @@ struct GemmParams {
     const float* A; long long sAm, sAk;             // A(m, k) = A[m * sAm + k * sAk]
     const float* B; long long sBn, sBk;             // B(n, k) = B[n * sBn + k * sBk]    (C = A . B^T)
     int M, N, K;
-    int kb_per_split;                               // K blocks per gridDim.z slice (EPI 0 accumulates with atomics when gridDim.z > 1)
-    float* C; long long ldc;                        // EPI 0: C[m * ldc + n]
+    int kb_per_split;                               // K blocks per gridDim.z slice
+    float* C; long long ldc;                        // EPI 0: C[z * c_split + m * ldc + n], z = blockIdx.z (one plane per slice)
+    long long c_split;
     float* out; float* csave;                       // EPI 1: (sequences, n_fft, F) log-magnitude; optional raw C, column-major (N x ldc)
     int F, n_fft, nb;                               // frames per sequence; bins per column tile (re block | im block)
     // the frame matrix as a VIEW of the padded signal (operand modes 1 and 2): frame row m = (sequence s, frame f),
@@ -462,23 +466,21 @@ __global__ void __launch_bounds__(G_THREADS, 1) vr_gemm_tf32x3_kernel(const __gr
                 *reinterpret_cast<float4*>(tile + (tid & 127) * LDT + part * W + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
         }
         __syncthreads();
-        const bool vec = (p.ldc & 3) == 0 && (reinterpret_cast<uintptr_t>(p.C) & 15) == 0 && gridDim.z == 1;
+        float* const C = p.C + blockIdx.z * p.c_split;
+        const bool vec = (p.ldc & 3) == 0 && (p.c_split & 3) == 0 && (reinterpret_cast<uintptr_t>(p.C) & 15) == 0;
         if (KB > 0) {
             for (int i = tid; i < GM * (GN / 4); i += G_THREADS) {
                 const int r = i / (GN / 4), c = (i % (GN / 4)) * 4;
                 const int gm = m0 + r, gn = n0 + c;
                 if (gm >= p.M || gn >= p.N) continue;
                 const float4 v = *reinterpret_cast<const float4*>(tile + r * LDT + c);
-                float* dst = p.C + (long long)gm * p.ldc + gn;
+                float* dst = C + (long long)gm * p.ldc + gn;
                 if (vec && gn + 3 < p.N) *reinterpret_cast<float4*>(dst) = v;
                 else {
                     const float e[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
                     for (int j = 0; j < 4; ++j)
-                        if (gn + j < p.N) {
-                            if (gridDim.z > 1) atomicAdd(dst + j, e[j]);      // split K: C was zeroed by the host
-                            else dst[j] = e[j];
-                        }
+                        if (gn + j < p.N) dst[j] = e[j];
                 }
             }
         }
@@ -688,15 +690,29 @@ __global__ void vr_stft_fold_kept_kernel(const float* __restrict__ dA, const int
         reinterpret_cast<float2*>(giq)[i] = g;
     }
 }
-// dBt (2 n_fft, 2 n_fft) -> grad wsin / wcos
-__global__ void vr_stft_dw_kernel(const float* __restrict__ dBt, float* __restrict__ gsin, float* __restrict__ gcos, int n_fft, int nb) {
+// The split-K partials of the kernel gradient: at most G_SPLIT_PLANES_MAX tiles' worth of K x K planes per launch (the host
+// caps splits * tiles, which one wave already bounds by the SM count), G_SPLIT_SLOTS slots handed out round-robin per launch
+// so that launches in flight on other streams do not share one.  10 MB per slot, 40 MB in all.
+constexpr int G_SPLIT_CTAS_MAX = 160;
+constexpr int G_SPLIT_SLOTS = 4;
+constexpr long long G_SPLIT_SLOT_FLOATS = (long long)G_SPLIT_CTAS_MAX * GM * GN;
+__device__ float g_splitk_pool[G_SPLIT_SLOTS * G_SPLIT_SLOT_FLOATS];
+
+// dBt (2 n_fft, 2 n_fft), as `splits` partial planes `stride` floats apart added in slice order -> grad wsin / wcos
+__device__ __forceinline__ float stft_split_sum(const float* __restrict__ q, int splits, long long stride) {
+    float v = __ldg(q);
+    for (int z = 1; z < splits; ++z) v += __ldg(q + z * stride);
+    return v;
+}
+__global__ void vr_stft_dw_kernel(const float* __restrict__ dBt, int splits, long long stride, float* __restrict__ gsin,
+                                  float* __restrict__ gcos, int n_fft, int nb) {
     const int total = n_fft * n_fft;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         const int bin = i / n_fft, s = i - bin * n_fft;
         const float* re = dBt + (long long)stft_row_re(bin, nb) * 2 * n_fft;
         const float* im = dBt + (long long)stft_row_im(bin, nb) * 2 * n_fft;
-        gcos[i] = re[s] + im[n_fft + s];
-        gsin[i] = re[n_fft + s] - im[s];
+        gcos[i] = stft_split_sum(re + s, splits, stride) + stft_split_sum(im + n_fft + s, splits, stride);
+        gsin[i] = stft_split_sum(re + n_fft + s, splits, stride) - stft_split_sum(im + s, splits, stride);
     }
 }
 #endif  // __CUDACC__
