@@ -22,7 +22,7 @@ SYMBOLS = ("vr_abi_version", "vr_last_error", "vr_forward_f32", "vr_forward_debu
            "vr_stft_general_workspace_floats", "vr_stft_general_f32", "vr_stft_general_backward_f32",
            "vr_synth_f32", "vr_synth_upsampled_f32", "vr_synth_adjoint_upsampled_f32",
            "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32",
-           "vr_plan_adjoint_stft")
+           "vr_plan_adjoint_stft", "vr_plan_pad_frames")
 
 _lib = None
 
@@ -100,6 +100,8 @@ def lib():
     L.vr_stft_general_frames_backward_f32.restype = ctypes.c_int
     L.vr_plan_adjoint_stft.argtypes = [i64, i64, i32, i32, ctypes.POINTER(i64), ctypes.POINTER(i64), i64]
     L.vr_plan_adjoint_stft.restype = ctypes.c_int
+    L.vr_plan_pad_frames.argtypes = [i32, i64, i64, i32, i32, i32, f32, i32, ctypes.POINTER(i64)]
+    L.vr_plan_pad_frames.restype = ctypes.c_int
     L.vr_set_timeline_buffer.argtypes = [vp]
     L.vr_set_timeline_buffer.restype = ctypes.c_int
     L.vr_selftest_rounding.argtypes = [ctypes.c_uint64, f32, ctypes.POINTER(ctypes.c_uint64)]
@@ -175,6 +177,19 @@ def plan_adjoint_stft(N, T, hop=16, sm_count=148):
     rows = (ctypes.c_int64 * (4 * plan["segments"]))()
     check(lib().vr_plan_adjoint_stft(N, T, hop, sm_count, out, rows, plan["segments"]))
     return plan, [tuple(int(v) for v in rows[4 * k:4 * k + 4]) for k in range(plan["segments"])]
+
+
+PAD_PLAN_FIELDS = ("nc", "ncb", "units", "grid", "smem_bytes", "nrs", "rows_per_slice", "radius")
+PAD_KINDS = {"forward": 0, "backward": 1, "notebook": 2}
+
+
+def plan_pad_frames(kind, N, T, V, M_or_C, num_pad_frames, sigma, sm_count=148):
+    """Launch configuration of vr_pad_frames_f32 ("forward"), vr_pad_frames_backward_f32 ("backward") or
+    vr_pad_frames_joints ("notebook", M_or_C = C)."""
+    out = (ctypes.c_int64 * 8)()
+    check(lib().vr_plan_pad_frames(PAD_KINDS[kind], N, T, V, M_or_C, num_pad_frames, ctypes.c_float(float(sigma)),
+                                   sm_count, out))
+    return dict(zip(PAD_PLAN_FIELDS, [int(v) for v in out]))
 
 
 def set_schedule(mode):

@@ -672,6 +672,62 @@ int pad_check(int64_t N, int64_t T, int32_t V, int32_t M, int32_t num_pad_frames
     return VR_OK;
 }
 
+// the arguments vr_pad_frames_joints accepts
+int pad_joints_check(int64_t N, int64_t T, int32_t V, int32_t C, int32_t num_pad_frames, float sigma) {
+    if (N <= 0 || V <= 0 || C <= 0) return fail(VR_ERR_SHAPE, "N, V, C must be positive (got %lld, %d, %d)", (long long)N, V, C);
+    if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames (scipy interp1d raises ValueError)", (long long)T);
+    if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
+    if (!(sigma > 0.f)) return fail(VR_ERR_SHAPE, "sigma must be positive, got %g", (double)sigma);
+    if ((double)T * num_pad_frames > 2.0e9) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
+    return VR_OK;
+}
+
+// Launch configuration of the three up-sampling kernels (vr_plan_pad_frames): kind 0 vr_pad_frames_kernel, 1 its backward,
+// 2 the notebook variant (MC = C, the coordinates per joint).  One CTA of 1024 threads owns nc adjacent columns of one
+// (sequence, coordinate) plane -- of one sequence for kind 2 -- and, for kind 2, one of nrs slices of the output rows;
+// the grid strides over the units.  w (optional): the Gaussian weights, w[0] = centre.
+struct PadPlan { long long nc, ncb, units, grid, smem, nrs, rows_per_slice; int radius; };
+int pad_plan(int kind, int64_t N, int64_t T, int32_t V, int32_t MC, int32_t num_pad_frames, float sigma, int sm_count,
+             PadPlan& q, double* w) {
+    if (kind < 0 || kind > 2) return fail(VR_ERR_ARG, "kind must be 0 (forward), 1 (backward) or 2 (notebook), got %d", kind);
+    int rc = kind == 2 ? pad_joints_check(N, T, V, MC, num_pad_frames, sigma) : pad_check(N, T, V, MC, num_pad_frames, sigma);
+    if (rc) return rc;
+    double wbuf[vr::PF_MAX_RADIUS + 1];
+    rc = gaussian_weights(sigma, q.radius, w ? w : wbuf);
+    if (rc) return rc;
+    const long long cols = (long long)V * MC, KT = (long long)num_pad_frames * T;
+    long long nc;
+    if (kind == 0) {                 // 12 bytes per (frame, column) + 8 bytes per frame of shared memory
+        nc = (200 * 1024 - 8ll * T) / (12ll * T);
+        if (nc < 1) return fail(VR_ERR_UNSUPPORTED, "T=%lld too long for the shared-memory spline solve (max %d frames)", (long long)T, 200 * 1024 / 20);
+    } else if (kind == 1) {          // 16 bytes per (frame, column): dL/dys and dL/dM in float64
+        if (T > 200 * 1024 / 20)     // the forward's limit (vr_pad_frames_f32)
+            return fail(VR_ERR_UNSUPPORTED, "T=%lld too long for the shared-memory spline solve (max %d frames)", (long long)T, 200 * 1024 / 20);
+        nc = (200 * 1024) / (16ll * T);
+    } else {                         // 16 bytes per (frame, column) + 8 per frame
+        nc = (200 * 1024 - 8ll * T) / (16ll * T);
+        if (nc < 1) return fail(VR_ERR_UNSUPPORTED, "T=%lld too long for the shared-memory spline solve (max %d frames)", (long long)T, 200 * 1024 / 24);
+    }
+    nc = std::min<long long>(std::min<long long>(nc, cols), 1024);     // one thread per column solves its spline
+    q.ncb = (cols + nc - 1) / nc;
+    q.nc = (cols + q.ncb - 1) / q.ncb;                                   // even out the blocks
+    q.smem = kind == 0 ? T * q.nc * 12 + T * 8 + 16 : kind == 1 ? T * q.nc * 16 : T * q.nc * 16 + T * 8 + 16;
+    q.nrs = 1;
+    if (kind == 2) {
+        // row slices: only when the per-unit preamble (Gaussian + sequential spline solve, ~50 cycles per frame) is cheap next
+        // to the evaluation (a latency-bound chain of conversions and FP64 operations: ~500 cycles per value and thread were
+        // measured with one CTA per SM), and only up to one wave of CTAs
+        const double solve_cost = 50.0 * (double)T, eval_cost = 500.0 * (double)KT * q.nc / 1024.0;
+        long long nrs = std::min<long long>(std::max<long long>(1, sm_count / std::max<long long>(1, N * q.ncb)),
+                                            std::max<long long>(1, (long long)(eval_cost / (2.0 * solve_cost))));
+        q.nrs = std::min<long long>(nrs, std::max<long long>(1, KT / 1024));
+    }
+    q.rows_per_slice = (KT + q.nrs - 1) / q.nrs;
+    q.units = (kind == 2 ? N : N * 3) * q.ncb * q.nrs;
+    q.grid = std::min<long long>(q.units, (long long)sm_count * 4);
+    return VR_OK;
+}
+
 // Dataset.pad_frames on the device.  out_dev: the up-sampled batch, and/or coef_dev: only the spline
 // (per-interval cubics) for the fused radar kernel.
 int pad_launch(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M, int32_t num_pad_frames,
@@ -684,20 +740,14 @@ int pad_launch(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M, i
     if (rc) return rc;
     vr::PadParams p;
     memset(&p, 0, sizeof(p));
-    rc = gaussian_weights(sigma, p.radius, p.w);
+    PadPlan q;
+    rc = pad_plan(0, N, T, V, M, num_pad_frames, sigma, sm_count, q, p.w);
     if (rc) return rc;
+    p.radius = q.radius;
     p.x = x_dev; p.out = out_dev; p.coef = coef_dev;
     p.planes = N * 3; p.T = (int)T; p.VM = V * M; p.K = num_pad_frames;
     p.ratio = (double)(T - 1) / (double)((long long)num_pad_frames * T - 1);
-    // columns per CTA: 12 bytes per (frame, column) + 8 bytes per frame of shared memory
-    const long long budget = 200 * 1024 - 8ll * T;
-    long long nc = budget / (12ll * T);
-    if (nc < 1) return fail(VR_ERR_UNSUPPORTED, "T=%lld too long for the shared-memory spline solve (max %d frames)", (long long)T, 200 * 1024 / 20);
-    nc = std::min<long long>(nc, p.VM);
-    nc = std::min<long long>(nc, 1024);                          // one thread per column solves its spline (1024 threads per CTA)
-    p.ncb = (int)((p.VM + nc - 1) / nc);
-    p.nc = (int)((p.VM + p.ncb - 1) / p.ncb);                    // even out the blocks
-    const size_t smem = (size_t)p.T * p.nc * 12 + (size_t)p.T * 8 + 16;
+    p.nc = (int)q.nc; p.ncb = (int)q.ncb;
     static std::mutex mu;
     static bool attr_done[64] = {false};
     {
@@ -707,8 +757,8 @@ int pad_launch(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M, i
             attr_done[dev] = true;
         }
     }
-    const long long units = p.planes * p.ncb;
-    const int grid = (int)std::min<long long>(units, (long long)sm_count * 4);
+    const size_t smem = (size_t)q.smem;
+    const int grid = (int)q.grid;
     vr::vr_pad_frames_kernel<<<grid, 1024, smem, (cudaStream_t)stream>>>(p);
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
@@ -732,10 +782,10 @@ int vr_pad_frames_backward_f32(const float* grad_out_dev, int64_t N, int64_t T, 
     if (rc) return rc;
     vr::PadBwdParams p;
     memset(&p, 0, sizeof(p));
-    rc = gaussian_weights(sigma, p.radius, p.w);
+    PadPlan q;
+    rc = pad_plan(1, N, T, V, M, num_pad_frames, sigma, sm_count, q, p.w);
     if (rc) return rc;
-    if (T > 200 * 1024 / 20)                                     // the forward's limit (vr_pad_frames_f32)
-        return fail(VR_ERR_UNSUPPORTED, "T=%lld too long for the shared-memory spline solve (max %d frames)", (long long)T, 200 * 1024 / 20);
+    p.radius = q.radius;
     {
         double c = 0.0;                                          // the forward's Thomas recurrence, bit for bit
         for (int i = 2; i < vr::PF_CP_N; ++i) { c = 1.0 / (4.0 - c); p.cp[i] = c; }
@@ -744,12 +794,7 @@ int vr_pad_frames_backward_f32(const float* grad_out_dev, int64_t N, int64_t T, 
     p.g = grad_out_dev; p.gx = grad_x_dev;
     p.planes = N * 3; p.T = (int)T; p.VM = V * M; p.K = num_pad_frames;
     p.ratio = (double)(T - 1) / (double)((long long)num_pad_frames * T - 1);
-    // columns per CTA: 16 bytes per (frame, column) of shared memory (dL/dys and dL/dM in float64)
-    long long nc = (200 * 1024) / (16ll * T);
-    nc = std::min<long long>(std::min<long long>(nc, p.VM), 1024);
-    p.ncb = (int)((p.VM + nc - 1) / nc);
-    p.nc = (int)((p.VM + p.ncb - 1) / p.ncb);
-    const size_t smem = (size_t)p.T * p.nc * 16;
+    p.nc = (int)q.nc; p.ncb = (int)q.ncb;
     static std::mutex mu;
     static bool attr_done[64] = {false};
     {
@@ -759,8 +804,8 @@ int vr_pad_frames_backward_f32(const float* grad_out_dev, int64_t N, int64_t T, 
             attr_done[dev] = true;
         }
     }
-    const long long units = p.planes * p.ncb;
-    const int grid = (int)std::min<long long>(units, (long long)sm_count * 4);
+    const size_t smem = (size_t)q.smem;
+    const int grid = (int)q.grid;
     vr::vr_pad_frames_backward_kernel<<<grid, 1024, smem, (cudaStream_t)stream>>>(p);
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
@@ -769,28 +814,20 @@ int vr_pad_frames_backward_f32(const float* grad_out_dev, int64_t N, int64_t T, 
 int vr_pad_frames_joints(const void* x_dev, int32_t x_is_f64, int64_t N, int64_t T, int32_t V, int32_t C,
                          int32_t num_pad_frames, float sigma, int32_t planar_out, float* out_dev, void* stream) {
     if (!x_dev || !out_dev) return fail(VR_ERR_ARG, "x_dev and out_dev must not be null");
-    if (N <= 0 || V <= 0 || C <= 0) return fail(VR_ERR_SHAPE, "N, V, C must be positive (got %lld, %d, %d)", (long long)N, V, C);
-    if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames (scipy interp1d raises ValueError)", (long long)T);
-    if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
-    if (!(sigma > 0.f)) return fail(VR_ERR_SHAPE, "sigma must be positive, got %g", (double)sigma);
-    if ((double)T * num_pad_frames > 2.0e9) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
+    int rc = pad_joints_check(N, T, V, C, num_pad_frames, sigma);
+    if (rc) return rc;
     int dev, sm_count;
-    int rc = device_setup(dev, sm_count);
+    rc = device_setup(dev, sm_count);
     if (rc) return rc;
     vr::PadNbParams p;
     memset(&p, 0, sizeof(p));
-    rc = gaussian_weights(sigma, p.radius, p.w);
+    PadPlan q;
+    rc = pad_plan(2, N, T, V, C, num_pad_frames, sigma, sm_count, q, p.w);
     if (rc) return rc;
+    p.radius = q.radius;
     p.x = x_dev; p.out = out_dev; p.N = N; p.T = (int)T; p.V = V; p.C = C; p.K = num_pad_frames; p.planar = planar_out ? 1 : 0;
     p.ratio = (double)(T - 1) / (double)((long long)num_pad_frames * T - 1);
-    const long long VC = (long long)V * C;
-    const long long budget = 200 * 1024 - 8ll * T;               // 16 bytes per (frame, column) + 8 per frame
-    long long nc = budget / (16ll * T);
-    if (nc < 1) return fail(VR_ERR_UNSUPPORTED, "T=%lld too long for the shared-memory spline solve (max %d frames)", (long long)T, 200 * 1024 / 24);
-    nc = std::min<long long>(std::min<long long>(nc, VC), 1024);
-    p.ncb = (int)((VC + nc - 1) / nc);
-    p.nc = (int)((VC + p.ncb - 1) / p.ncb);
-    const size_t smem = (size_t)p.T * p.nc * 16 + (size_t)p.T * 8 + 16;
+    p.nc = (int)q.nc; p.ncb = (int)q.ncb; p.nrs = (int)q.nrs; p.rows_per_slice = q.rows_per_slice;
     static std::mutex mu;
     static bool attr_done[64] = {false};
     {
@@ -801,19 +838,8 @@ int vr_pad_frames_joints(const void* x_dev, int32_t x_is_f64, int64_t N, int64_t
             attr_done[dev] = true;
         }
     }
-    // row slices: only when the per-unit preamble (Gaussian + sequential spline solve, ~50 cycles per frame) is cheap next to
-    // the evaluation (a latency-bound chain of conversions and FP64 operations: ~500 cycles per value and thread were
-    // measured with one CTA per SM), and only up to one wave of CTAs
-    {
-        const long long KT = (long long)num_pad_frames * T;
-        const double solve_cost = 50.0 * (double)T, eval_cost = 500.0 * (double)KT * p.nc / 1024.0;
-        long long nrs = std::min<long long>(std::max<long long>(1, sm_count / std::max<long long>(1, N * p.ncb)),
-                                            std::max<long long>(1, (long long)(eval_cost / (2.0 * solve_cost))));
-        nrs = std::min<long long>(nrs, std::max<long long>(1, KT / 1024));
-        p.nrs = (int)nrs;
-        p.rows_per_slice = (KT + nrs - 1) / nrs;
-    }
-    const int grid = (int)std::min<long long>(N * p.ncb * p.nrs, (long long)sm_count * 4);
+    const size_t smem = (size_t)q.smem;
+    const int grid = (int)q.grid;
     if (x_is_f64) vr::vr_pad_frames_nb_kernel<double><<<grid, 1024, smem, (cudaStream_t)stream>>>(p);
     else vr::vr_pad_frames_nb_kernel<float><<<grid, 1024, smem, (cudaStream_t)stream>>>(p);
     CUDA_TRY(cudaGetLastError());
@@ -1108,6 +1134,17 @@ int vr_plan_adjoint_stft(int64_t N, int64_t T, int32_t hop, int32_t sm_count, in
             r[0] = s0; r[1] = s1; r[2] = lo; r[3] = hi;
         }
     }
+    return VR_OK;
+}
+
+int vr_plan_pad_frames(int32_t kind, int64_t N, int64_t T, int32_t V, int32_t M_or_C, int32_t num_pad_frames, float sigma,
+                       int32_t sm_count, int64_t plan[8]) {
+    if (!plan) return fail(VR_ERR_ARG, "plan must not be null");
+    PadPlan q;
+    int rc = pad_plan(kind, N, T, V, M_or_C, num_pad_frames, sigma, sm_count > 0 ? sm_count : 148, q, nullptr);
+    if (rc) return rc;
+    plan[0] = q.nc; plan[1] = q.ncb; plan[2] = q.units; plan[3] = q.grid; plan[4] = q.smem; plan[5] = q.nrs;
+    plan[6] = q.rows_per_slice; plan[7] = q.radius;
     return VR_OK;
 }
 
