@@ -22,7 +22,7 @@ SYMBOLS = ("vr_abi_version", "vr_last_error", "vr_forward_f32", "vr_forward_debu
            "vr_stft_general_workspace_floats", "vr_stft_general_f32", "vr_stft_general_backward_f32",
            "vr_synth_f32", "vr_synth_upsampled_f32", "vr_synth_adjoint_upsampled_f32",
            "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32",
-           "vr_plan_adjoint_stft", "vr_plan_pad_frames")
+           "vr_plan_adjoint_stft", "vr_plan_pad_frames", "vr_plan_stft_general")
 
 _lib = None
 
@@ -102,6 +102,8 @@ def lib():
     L.vr_plan_adjoint_stft.restype = ctypes.c_int
     L.vr_plan_pad_frames.argtypes = [i32, i64, i64, i32, i32, i32, f32, i32, ctypes.POINTER(i64)]
     L.vr_plan_pad_frames.restype = ctypes.c_int
+    L.vr_plan_stft_general.argtypes = [i64, i64, i32, i32, i64, i32, ctypes.POINTER(i64)]
+    L.vr_plan_stft_general.restype = ctypes.c_int
     L.vr_set_timeline_buffer.argtypes = [vp]
     L.vr_set_timeline_buffer.restype = ctypes.c_int
     L.vr_selftest_rounding.argtypes = [ctypes.c_uint64, f32, ctypes.POINTER(ctypes.c_uint64)]
@@ -190,6 +192,18 @@ def plan_pad_frames(kind, N, T, V, M_or_C, num_pad_frames, sigma, sm_count=148):
     check(lib().vr_plan_pad_frames(PAD_KINDS[kind], N, T, V, M_or_C, num_pad_frames, ctypes.c_float(float(sigma)),
                                    sm_count, out))
     return dict(zip(PAD_PLAN_FIELDS, [int(v) for v in out]))
+
+
+STFT_PLAN_FIELDS = ("nb", "F", "M", "ldm", "Lp", "row_tiles", "col_tiles", "kblocks", "dbt_tiles", "splits", "kb_per_split",
+                    "kb_last", "hop_view")
+
+
+def plan_stft_general(N, T, n_fft, hop, F_kept=0, sm_count=148):
+    """Launch configuration of the general-kernel STFT's GEMMs (vr_stft_general_f32 and its backward; F_kept > 0: the
+    kept-frames entries)."""
+    out = (ctypes.c_int64 * len(STFT_PLAN_FIELDS))()
+    check(lib().vr_plan_stft_general(N, T, n_fft, hop, F_kept, sm_count, out))
+    return dict(zip(STFT_PLAN_FIELDS, [int(v) for v in out]))
 
 
 def set_schedule(mode):

@@ -1196,64 +1196,89 @@ static long long stft_lp(long long T, int n_fft) { return (T + n_fft + 3) & ~3ll
 
 }  // extern "C"
 namespace {
-// The GEMM part of the forward, over a planar padded signal P (S, 2, Lp) whose frame f starts at P[.. + f hop]: the full
-// route passes the reflect-padded signal (hop, F = T / hop + 1), the kept-frames route its compact copy of the kept frames
-// (hop = n_fft, F = F_kept).  Each output column is one GEMM row with the same K order and B tiles in both.
-int stft_forward_gemm(const float* P, long long Lp, int hop, int F, int64_t N, int n_fft, const float* wsin_dev,
-                      const float* wcos_dev, float* bt_work, float* c_save, float* out_dev, cudaStream_t st) {
-    const int nb = stft_nb(n_fft), K = 2 * n_fft;
-    const long long M = N * (long long)F;
+// The launch configuration of the general-kernel STFT's GEMMs (vr_plan_stft_general; the launches below take every number
+// from it).  P (S, 2, Lp) is the planar signal the frame views read: the reflect-padded signal (hop, F = T / hop + 1) on the
+// full route, the compact copy of the kept frames (hop' = n_fft, F = F_kept) on the kept-frames route.
+struct StftPlan {
+    int nb, F, K, hop_view;                          // bins per column tile; frames per sequence; K = 2 n_fft; hop of the view
+    long long M, ldm, Lp;                            // GEMM rows (sequence, frame); leading dimension of C / dC; plane length
+    int row_tiles, col_tiles, kblocks;               // forward and dA GEMMs: M x K output, K = 2 n_fft reduction
+    int dbt_tiles, splits, kb_per_split, kb_last;    // kernel-gradient GEMM: K x K output, reduction over the M frames
+};
+int stft_plan(int64_t N, int64_t T, int n_fft, int hop, int64_t F_kept, int sm_count, StftPlan& q) {
+    int rc = stft_check(N, T, n_fft, hop);
+    if (rc) return rc;
+    if (F_kept < 0 || F_kept > T / hop + 1) return fail(VR_ERR_SHAPE, "F_kept=%lld outside [0, T/hop+1 = %lld] (0: all frames)", (long long)F_kept, (long long)(T / hop + 1));
+    q.nb = stft_nb(n_fft);
+    q.K = 2 * n_fft;
+    q.F = F_kept ? (int)F_kept : (int)(T / hop) + 1;
+    q.hop_view = F_kept ? n_fft : hop;
+    q.M = N * (long long)q.F;
+    q.ldm = stft_ldm(q.M);
+    q.Lp = F_kept ? F_kept * (long long)n_fft : stft_lp(T, n_fft);
+    q.row_tiles = (int)((q.M + vr::GM - 1) / vr::GM);
+    q.col_tiles = (q.K + vr::GN - 1) / vr::GN;
+    q.kblocks = (q.K + vr::GK - 1) / vr::GK;
+    // the kernel gradient's reduction runs over all frames of the batch: split it over gridDim.z so that the (2 n_fft / 128)^2
+    // output tiles fill the machine.  One CTA per SM at a time (192 KB of stages): whole waves, i.e. splits * tiles <= a
+    // multiple of sm_count; one wave unless that leaves a slice fewer than 8 K blocks; and no more planes than a pool slot holds
+    q.dbt_tiles = ((q.K + vr::GM - 1) / vr::GM) * ((q.K + vr::GN - 1) / vr::GN);
+    const int kb_all = (int)((q.M + vr::GK - 1) / vr::GK);
+    const int splits = std::max(1, std::min(std::min(sm_count, vr::G_SPLIT_CTAS_MAX) / q.dbt_tiles, (kb_all + 7) / 8));
+    q.kb_per_split = (kb_all + splits - 1) / splits;
+    q.splits = (kb_all + q.kb_per_split - 1) / q.kb_per_split;
+    q.kb_last = kb_all - (q.splits - 1) * q.kb_per_split;
+    return VR_OK;
+}
+
+// The GEMM part of the forward, over the planar signal P of the plan.  Each output column is one GEMM row with the same K
+// order and B tiles on both routes.
+int stft_forward_gemm(const StftPlan& q, const float* P, int n_fft, const float* wsin_dev, const float* wcos_dev,
+                      float* bt_work, float* c_save, float* out_dev, cudaStream_t st) {
+    const int K = q.K;
     const long long img = stft_bimg_floats(n_fft);
     if (K % vr::GN) CUDA_TRY(cudaMemsetAsync(bt_work, 0, (size_t)(2 * img) * sizeof(float), st));      // rows past K of the one tile
-    vr::vr_stft_bt_kernel<<<(n_fft * n_fft + 255) / 256, 256, 0, st>>>(wsin_dev, wcos_dev, bt_work, bt_work + img, n_fft, nb, (K + vr::GK - 1) / vr::GK);
+    vr::vr_stft_bt_kernel<<<(n_fft * n_fft + 255) / 256, 256, 0, st>>>(wsin_dev, wcos_dev, bt_work, bt_work + img, n_fft, q.nb, q.kblocks);
     vr::GemmParams g;
     memset(&g, 0, sizeof(g));
-    g.P = P; g.Lp = Lp; g.hop = hop;                 // A = the frames, read as views of the padded signal
+    g.P = P; g.Lp = q.Lp; g.hop = q.hop_view;        // A = the frames, read as views of the padded signal
     g.Bimg = bt_work;                                // B = the kernel matrix, pre-split and pre-tiled: bulk copies
-    g.M = (int)M; g.N = K; g.K = K; g.kb_per_split = (K + vr::GK - 1) / vr::GK;
-    g.out = out_dev; g.csave = c_save; g.ldc = stft_ldm(M); g.F = F; g.n_fft = n_fft; g.nb = nb;
-    dim3 grid((unsigned)(((M + vr::GM - 1) / vr::GM) * ((K + vr::GN - 1) / vr::GN)));
+    g.M = (int)q.M; g.N = K; g.K = K; g.kb_per_split = q.kblocks;
+    g.out = out_dev; g.csave = c_save; g.ldc = q.ldm; g.F = q.F; g.n_fft = n_fft; g.nb = q.nb;
+    dim3 grid((unsigned)((long long)q.row_tiles * q.col_tiles));
     vr::vr_gemm_tf32x3_kernel<1, vr::G_FRAME_ROWS, vr::G_TILED><<<grid, vr::G_THREADS, vr::G_SMEM_BYTES, st>>>(g);
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
 }
 
-// The GEMM part of the backward over the same (P, Lp, hop, F): dC, then dA (frame gradients, folded by the caller) and dBt
-// (kernel gradients, reduced over every frame of the batch)
-int stft_backward_gemm(const float* grad_out_dev, const float* P, long long Lp, int hop, int F, int64_t N, int n_fft,
+// The GEMM part of the backward over the same plan: dC, then dA (frame gradients, folded by the caller) and dBt (kernel
+// gradients, reduced over every frame of the batch)
+int stft_backward_gemm(const StftPlan& q, const float* grad_out_dev, const float* P, int n_fft,
                        const float* bt_work, const float* c_save, float* dc_work, float* da_work, float* dbt_work,
                        float* grad_wsin_dev, float* grad_wcos_dev, int dev, int sm_count, cudaStream_t st) {
-    const int nb = stft_nb(n_fft), K = 2 * n_fft;
-    const long long M = N * (long long)F;
-    const long long ldm = stft_ldm(M);
-    vr::vr_stft_dc_kernel<<<dim3((unsigned)std::min<long long>((M / 4 + 256) / 256, sm_count * 4ll), (unsigned)n_fft), 256, 0, st>>>(grad_out_dev, c_save, dc_work, (int)M, ldm, F, n_fft, nb);
+    const int K = q.K;
+    const long long M = q.M, ldm = q.ldm;
+    vr::vr_stft_dc_kernel<<<dim3((unsigned)std::min<long long>((M / 4 + 256) / 256, sm_count * 4ll), (unsigned)n_fft), 256, 0, st>>>(grad_out_dev, c_save, dc_work, (int)M, ldm, q.F, n_fft, q.nb);
     vr::GemmParams g;
     if (da_work) {                                   // dA[m, k] = sum_n dC[m, n] Bt[n, k]
         memset(&g, 0, sizeof(g));
         g.A = dc_work; g.sAm = 1; g.sAk = ldm;       // dC is column-major: dC(m, n) = dc[n * ldm + m]
         g.Bimg = bt_work + stft_bimg_floats(n_fft);  // B'(n' = k, k' = n) = Bt[n][k]: the transposed image
-        g.M = (int)M; g.N = K; g.K = K; g.C = da_work; g.ldc = K; g.kb_per_split = (K + vr::GK - 1) / vr::GK;
-        dim3 grid((unsigned)(((M + vr::GM - 1) / vr::GM) * ((K + vr::GN - 1) / vr::GN)));
+        g.M = (int)M; g.N = K; g.K = K; g.C = da_work; g.ldc = K; g.kb_per_split = q.kblocks;
+        dim3 grid((unsigned)((long long)q.row_tiles * q.col_tiles));
         vr::vr_gemm_tf32x3_kernel<0, vr::G_STRIDED, vr::G_TILED><<<grid, vr::G_THREADS, vr::G_SMEM_BYTES, st>>>(g);
     }
     if (dbt_work) {                                  // dBt[n, k] = sum_m dC[m, n] A[m, k]
         memset(&g, 0, sizeof(g));
         g.A = dc_work; g.sAm = ldm; g.sAk = 1;       // A'(m' = n, k' = m) = dC(m, n) = dc[n * ldm + m]: rows of 16-byte aligned chunks
-        g.P = P; g.Lp = Lp; g.hop = hop; g.F = F; g.n_fft = n_fft;     // B'(n' = k, k' = m) = A[m][k], a view
+        g.P = P; g.Lp = q.Lp; g.hop = q.hop_view; g.F = q.F; g.n_fft = n_fft;     // B'(n' = k, k' = m) = A[m][k], a view
         g.M = K; g.N = K; g.K = (int)M; g.C = dbt_work; g.ldc = K;
-        // the reduction runs over all frames of the batch: split it over gridDim.z so that the (2 n_fft / 128)^2 output
-        // tiles fill the machine; each slice writes its own K x K plane of a split-K pool slot, added in slice order below
-        const int tiles = ((K + vr::GM - 1) / vr::GM) * ((K + vr::GN - 1) / vr::GN);
-        const int kb_all = (int)((M + vr::GK - 1) / vr::GK);
-        // one CTA per SM at a time (192 KB of stages): whole waves, i.e. splits * tiles <= a multiple of sm_count; one wave
-        // unless that leaves a slice fewer than 8 K blocks; and no more planes than a pool slot holds
-        int splits = std::max(1, std::min(std::min(sm_count, vr::G_SPLIT_CTAS_MAX) / tiles, (kb_all + 7) / 8));
-        g.kb_per_split = (kb_all + splits - 1) / splits;
-        splits = (kb_all + g.kb_per_split - 1) / g.kb_per_split;
-        if (splits > 1) { g.C = next_splitk_slot(dev); g.c_split = (long long)K * K; }
-        dim3 grid((unsigned)tiles, 1u, (unsigned)splits);
+        // each slice writes its own K x K plane of a split-K pool slot, added in slice order below
+        g.kb_per_split = q.kb_per_split;
+        if (q.splits > 1) { g.C = next_splitk_slot(dev); g.c_split = (long long)K * K; }
+        dim3 grid((unsigned)q.dbt_tiles, 1u, (unsigned)q.splits);
         vr::vr_gemm_tf32x3_kernel<0, vr::G_STRIDED, vr::G_FRAME_COLS><<<grid, vr::G_THREADS, vr::G_SMEM_BYTES, st>>>(g);
-        vr::vr_stft_dw_kernel<<<(n_fft * n_fft + 255) / 256, 256, 0, st>>>(g.C, splits, g.c_split, grad_wsin_dev, grad_wcos_dev, n_fft, nb);
+        vr::vr_stft_dw_kernel<<<(n_fft * n_fft + 255) / 256, 256, 0, st>>>(g.C, q.splits, g.c_split, grad_wsin_dev, grad_wcos_dev, n_fft, q.nb);
     }
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
@@ -1317,10 +1342,12 @@ int vr_stft_general_f32(const float* iq_dev, int64_t N, int64_t T, int32_t n_fft
     int dev, sm_count;
     int rc = stft_forward_args(iq_dev, wsin_dev, wcos_dev, frames_work, bt_work, c_save, out_dev, N, T, n_fft, hop, dev, sm_count);
     if (rc) return rc;
+    StftPlan q;
+    rc = stft_plan(N, T, n_fft, hop, 0, sm_count, q);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    const long long Lp = stft_lp(T, n_fft);
-    vr::vr_stft_pad_kernel<<<(unsigned)std::min<long long>((N * Lp + 255) / 256, sm_count * 16ll), 256, 0, st>>>(iq_dev, frames_work, N, (int)T, Lp, n_fft);
-    return stft_forward_gemm(frames_work, Lp, hop, (int)(T / hop) + 1, N, n_fft, wsin_dev, wcos_dev, bt_work, c_save, out_dev, st);
+    vr::vr_stft_pad_kernel<<<(unsigned)std::min<long long>((N * q.Lp + 255) / 256, sm_count * 16ll), 256, 0, st>>>(iq_dev, frames_work, N, (int)T, q.Lp, n_fft);
+    return stft_forward_gemm(q, frames_work, n_fft, wsin_dev, wcos_dev, bt_work, c_save, out_dev, st);
 }
 
 int vr_stft_general_backward_f32(const float* grad_out_dev, const float* frames_work, const float* bt_work, const float* c_save,
@@ -1331,12 +1358,14 @@ int vr_stft_general_backward_f32(const float* grad_out_dev, const float* frames_
     int rc = stft_backward_args(grad_out_dev, frames_work, bt_work, c_save, dc_work, da_work, dbt_work, grad_iq_dev,
                                 grad_wsin_dev, grad_wcos_dev, N, T, n_fft, hop, dev, sm_count);
     if (rc) return rc;
+    StftPlan q;
+    rc = stft_plan(N, T, n_fft, hop, 0, sm_count, q);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    const int F = (int)(T / hop) + 1;
-    rc = stft_backward_gemm(grad_out_dev, frames_work, stft_lp(T, n_fft), hop, F, N, n_fft, bt_work, c_save, dc_work, da_work,
+    rc = stft_backward_gemm(q, grad_out_dev, frames_work, n_fft, bt_work, c_save, dc_work, da_work,
                             dbt_work, grad_wsin_dev, grad_wcos_dev, dev, sm_count, st);
     if (rc || !da_work) return rc;
-    vr::vr_stft_fold_kernel<<<(unsigned)std::min<long long>((N * T + 255) / 256, sm_count * 16ll), 256, 0, st>>>(da_work, grad_iq_dev, N, (int)T, F, n_fft, hop);
+    vr::vr_stft_fold_kernel<<<(unsigned)std::min<long long>((N * T + 255) / 256, sm_count * 16ll), 256, 0, st>>>(da_work, grad_iq_dev, N, (int)T, q.F, n_fft, hop);
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
 }
@@ -1358,10 +1387,12 @@ int vr_stft_general_frames_f32(const float* iq_dev, int64_t N, int64_t T, int32_
     if (rc) return rc;
     rc = stft_kept_check(frames_dev, N, T, hop, F_kept);
     if (rc) return rc;
+    StftPlan q;
+    rc = stft_plan(N, T, n_fft, hop, F_kept, sm_count, q);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    const long long Lp = F_kept * (long long)n_fft;
-    vr::vr_stft_gather_kernel<<<(unsigned)std::min<long long>((N * Lp + 255) / 256, sm_count * 16ll), 256, 0, st>>>(iq_dev, frames_dev, frames_work, N, (int)T, (int)F_kept, n_fft, hop);
-    return stft_forward_gemm(frames_work, Lp, n_fft, (int)F_kept, N, n_fft, wsin_dev, wcos_dev, bt_work, c_save, out_dev, st);
+    vr::vr_stft_gather_kernel<<<(unsigned)std::min<long long>((N * q.Lp + 255) / 256, sm_count * 16ll), 256, 0, st>>>(iq_dev, frames_dev, frames_work, N, (int)T, (int)F_kept, n_fft, hop);
+    return stft_forward_gemm(q, frames_work, n_fft, wsin_dev, wcos_dev, bt_work, c_save, out_dev, st);
 }
 
 int vr_stft_general_frames_backward_f32(const float* grad_out_dev, const float* frames_work, const float* bt_work, const float* c_save,
@@ -1374,12 +1405,26 @@ int vr_stft_general_frames_backward_f32(const float* grad_out_dev, const float* 
     if (rc) return rc;
     rc = stft_kept_check(frames_dev, N, T, hop, F_kept);
     if (rc) return rc;
+    StftPlan q;
+    rc = stft_plan(N, T, n_fft, hop, F_kept, sm_count, q);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    rc = stft_backward_gemm(grad_out_dev, frames_work, F_kept * (long long)n_fft, n_fft, (int)F_kept, N, n_fft, bt_work, c_save,
+    rc = stft_backward_gemm(q, grad_out_dev, frames_work, n_fft, bt_work, c_save,
                             dc_work, da_work, dbt_work, grad_wsin_dev, grad_wcos_dev, dev, sm_count, st);
     if (rc || !da_work) return rc;
     vr::vr_stft_fold_kept_kernel<<<(unsigned)std::min<long long>((N * T + 255) / 256, sm_count * 16ll), 256, 0, st>>>(da_work, frames_dev, grad_iq_dev, N, (int)T, (int)F_kept, n_fft, hop);
     CUDA_TRY(cudaGetLastError());
+    return VR_OK;
+}
+
+int vr_plan_stft_general(int64_t N, int64_t T, int32_t n_fft, int32_t hop, int64_t F_kept, int32_t sm_count, int64_t plan[13]) {
+    if (!plan) return fail(VR_ERR_ARG, "plan must not be null");
+    StftPlan q;
+    int rc = stft_plan(N, T, n_fft, hop, F_kept, sm_count > 0 ? sm_count : 148, q);
+    if (rc) return rc;
+    plan[0] = q.nb; plan[1] = q.F; plan[2] = q.M; plan[3] = q.ldm; plan[4] = q.Lp;
+    plan[5] = q.row_tiles; plan[6] = q.col_tiles; plan[7] = q.kblocks;
+    plan[8] = q.dbt_tiles; plan[9] = q.splits; plan[10] = q.kb_per_split; plan[11] = q.kb_last; plan[12] = q.hop_view;
     return VR_OK;
 }
 

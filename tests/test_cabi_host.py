@@ -143,6 +143,42 @@ def test_stft_general_rejects_misaligned_work_buffers(cabi):
     assert L.vr_stft_general_backward_f32(ok, ok, ok, ok, 2, 300, 256, 16, ok + 4, None, None, None, None, None, None) == cabi.VR_ERR_ARG
 
 
+def test_plan_stft_general(cabi):
+    """Host plan of the general-kernel STFT's GEMMs (vr_plan_stft_general): what the launches reject, and the split-K
+    kernel gradient's limits -- splits x tiles within one wave of min(SMs, 160) CTAs whenever it splits, and the slices'
+    K x K planes within one slot of the static pool (160 tiles of 128 x 128 floats)."""
+    L = cabi.lib()
+    assert L.vr_plan_stft_general(2, 300, 256, 16, 0, 148, None) == cabi.VR_ERR_ARG
+    for bad, exc in (((0, 300, 256, 16), ValueError), ((2, 300, 256, 0), ValueError), ((2, 128, 256, 16), ValueError),
+                     ((2, 300, 48, 16), NotImplementedError), ((2, 300, 8, 16), NotImplementedError),
+                     ((2, 3000, 2048, 16), NotImplementedError), ((1 << 27, 300, 256, 16), NotImplementedError)):
+        with pytest.raises(exc):
+            cabi.plan_stft_general(*bad)
+    with pytest.raises(ValueError, match="F_kept"):
+        cabi.plan_stft_general(2, 300, 256, 16, 20)                  # T / hop + 1 = 19 frames
+    with pytest.raises(ValueError, match="F_kept"):
+        cabi.plan_stft_general(2, 300, 256, 16, -1)
+    assert cabi.plan_stft_general(2, 300, 256, 16, 19)["F"] == 19
+    assert cabi.plan_stft_general(2, 300, 256, 16, 0, sm_count=0) == cabi.plan_stft_general(2, 300, 256, 16, 0, sm_count=148)
+    p = cabi.plan_stft_general(4096, 300, 256, 16)                   # the flagship batch with trainable kernels
+    assert (p["nb"], p["F"], p["M"], p["ldm"], p["Lp"]) == (64, 19, 77824, 77824, 556)
+    assert (p["row_tiles"], p["col_tiles"], p["kblocks"], p["dbt_tiles"], p["splits"]) == (608, 4, 16, 16, 9)
+    slot = 160 * 128 * 128
+    for n in (16, 32, 64, 128, 256, 512, 1024):
+        for N, T, hop in ((1, n // 2 + 1, 1), (3, 1000, 7), (64, 3000, 4), (4096, 300, 16), (20000, 2 * n, 1)):
+            T = max(T, n // 2 + 1)
+            for sms in (1, 16, 132, 148, 160, 1000):
+                p = cabi.plan_stft_general(N, T, n, hop, 0, sms)
+                K = 2 * n
+                assert p["dbt_tiles"] == (-(-K // 128)) ** 2 and p["kblocks"] == K // 32 and p["col_tiles"] == -(-K // 128)
+                kb_all = -(-p["M"] // 32)
+                assert (p["splits"] - 1) * p["kb_per_split"] + p["kb_last"] == kb_all
+                assert 1 <= p["kb_last"] <= p["kb_per_split"]
+                if p["splits"] > 1:
+                    assert p["splits"] * p["dbt_tiles"] <= min(sms, 160), (n, N, T, hop, sms, p)
+                    assert p["splits"] * K * K <= slot, (n, N, T, hop, sms, p)
+
+
 def test_module_surface_matches_reference():
     import torch
     from skeleton_action_recognition_b200 import VirtualRadar, edges

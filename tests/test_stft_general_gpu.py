@@ -156,7 +156,8 @@ def test_arbitrary_windows_hops_and_lengths(n_fft, hop, extra, N, seed):
         k64.wcos.copy_(k.wcos.detach().cpu().double())
     x64 = iq.double().requires_grad_(True)
     (k64._logmag_torch(x64) * go.double()).sum().backward()
-    for name, a, b in (("iq", x.grad.cpu().double(), x64.grad), ("wsin", k.wsin.grad.cpu().double(), k64.wsin.grad)):
+    for name, a, b in (("iq", x.grad.cpu().double(), x64.grad), ("wsin", k.wsin.grad.cpu().double(), k64.wsin.grad),
+                       ("wcos", k.wcos.grad.cpu().double(), k64.wcos.grad)):
         scale = float(b.square().mean().sqrt()) + 1e-30
         # bins with |X| ~ 0 make d ln|X| ill-conditioned in float32 (see test_backward_matches_float64_autograd): the bar is
         # on the bulk of the entries, the maximum only has to stay finite and of the right size
