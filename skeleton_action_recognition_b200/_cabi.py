@@ -10,6 +10,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libvirtual_radar_b200.so")
 VR_OK, VR_ERR_ARG, VR_ERR_SHAPE, VR_ERR_UNSUPPORTED, VR_ERR_CUDA = 0, -1, -2, -3, -4
 VR_FLAG_RANGE_FMA = 1
 VR_FLAG_INPUTS_READY = 2
+VR_FLAG_PER_SEQUENCE = 4
 ABI_VERSION = 1
 
 # every symbol include/virtual_radar_b200.h declares
@@ -22,7 +23,7 @@ SYMBOLS = ("vr_abi_version", "vr_last_error", "vr_forward_f32", "vr_forward_debu
            "vr_stft_general_workspace_floats", "vr_stft_general_f32", "vr_stft_general_backward_f32",
            "vr_synth_f32", "vr_synth_upsampled_f32", "vr_synth_adjoint_upsampled_f32",
            "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32",
-           "vr_plan_adjoint_stft", "vr_plan_pad_frames", "vr_plan_stft_general")
+           "vr_plan_adjoint_stft", "vr_plan_pad_frames", "vr_plan_stft_general", "vr_per_sequence_grad_doubles")
 
 _lib = None
 
@@ -104,6 +105,8 @@ def lib():
     L.vr_plan_pad_frames.restype = ctypes.c_int
     L.vr_plan_stft_general.argtypes = [i64, i64, i32, i32, i64, i32, ctypes.POINTER(i64)]
     L.vr_plan_stft_general.restype = ctypes.c_int
+    L.vr_per_sequence_grad_doubles.argtypes = [i64, i64]
+    L.vr_per_sequence_grad_doubles.restype = i64
     L.vr_set_timeline_buffer.argtypes = [vp]
     L.vr_set_timeline_buffer.restype = ctypes.c_int
     L.vr_selftest_rounding.argtypes = [ctypes.c_uint64, f32, ctypes.POINTER(ctypes.c_uint64)]
@@ -204,6 +207,13 @@ def plan_stft_general(N, T, n_fft, hop, F_kept=0, sm_count=148):
     out = (ctypes.c_int64 * len(STFT_PLAN_FIELDS))()
     check(lib().vr_plan_stft_general(N, T, n_fft, hop, F_kept, sm_count, out))
     return dict(zip(STFT_PLAN_FIELDS, [int(v) for v in out]))
+
+
+def per_sequence_grad_doubles(N, T):
+    """Length in float64 values of the gradient buffer of a backward call with VR_FLAG_PER_SEQUENCE: N x 4 per-sequence
+    gradients, then the scratch of the per-sequence reduction.  T: the steps the adjoint runs over (up-sampled length for
+    the _upsampled entries)."""
+    return int(lib().vr_per_sequence_grad_doubles(int(N), int(T)))
 
 
 def set_schedule(mode):

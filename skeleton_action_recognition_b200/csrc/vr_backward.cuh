@@ -34,8 +34,10 @@ struct BwdParams {
     unsigned* count;             // and its counter of finished blocks (0 between launches)
     int seg_len, segs;           // adjoint STFT: samples per segment, segments per sequence (adjoint_plan)
     float* gx;                   // optional dL/dx (N,3,T,V,M), zeroed before the launch; nullptr = not wanted
-    const float* lam_ptr;
+    const float* lam_ptr;        // 1 wavelength and 1 location, or (VR_FLAG_PER_SEQUENCE) N and N x 3
     const float* loc_ptr;
+    long long ps_segs;           // VR_FLAG_PER_SEQUENCE: segments per sequence of the per-sequence reduction (part = their
+                                 // partials, gparams = N x 4 gradients); 0 = one reduction over the batch
     long long N, T;
     int V, M, E, F, hop, VM;
     int fma_range;
@@ -84,6 +86,11 @@ inline void adjoint_plan(long long N, long long T, int sm_count, int& seg_len, i
     seg_len = (int)len;
     segs = (int)((T + len - 1) / len);
 }
+
+// Per-sequence parameter gradients (VR_FLAG_PER_SEQUENCE): steps per segment of the reduction (one per lane of a warp), and
+// the segments of a T-step sequence.  Depends on nothing but T.
+constexpr int PS_SEG = 32;
+inline long long ps_segments(long long T) { return (T + PS_SEG - 1) / PS_SEG; }
 
 #ifdef __CUDACC__
 // 256-point forward DFT (e^{-j...}) of one frame by one warp.  In: v[q] = sample lane + 32 q.  Out: v holds
@@ -380,6 +387,45 @@ __device__ __forceinline__ void synth_adjoint_reduce(const BwdParams& p, double 
     if (threadIdx.x == 0) *p.count = 0u;
 }
 
+// The adjoint of time step t of sequence n, joint positions read from x (and dL/dx written when p.gx is set).
+__device__ __forceinline__ void synth_adjoint_step(const BwdParams& p, long long n, int t, float lam, float lam_rcp,
+                                                   float Lx, float Ly, float Lz,
+                                                   double& g_lam, double& g_lx, double& g_ly, double& g_lz) {
+    const int T = (int)p.T;
+    const long long idx = n * T + t;
+    const double gI = (double)__ldg(p.gz + idx * 2), gQ = (double)__ldg(p.gz + idx * 2 + 1);
+    if (gI == 0.0 && gQ == 0.0) return;
+    const float* x0 = p.x + (n * 3 * T + t) * (long long)p.VM;       // x-plane row of this time step
+    const long long ps = (long long)T * p.VM;                         // floats between coordinate planes
+    const int M = p.M;
+    auto pos = [&](int v, int m, int c) { return __ldg(x0 + v * M + m + c * ps); };
+    float* gx0 = p.gx ? p.gx + (n * 3 * T + t) * (long long)p.VM : nullptr;   // this thread's own rows of dL/dx
+    for (int m = 0; m < p.M; ++m)
+        synth_adjoint_body(p, pos, m, gI, gQ, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz, gx0, ps);
+}
+
+// The same at up-sampled step i of sequence n (T = ups_K * ups_T): the joint positions come from the per-interval cubics
+// (pf_locate + pf_eval on p.coef), bit-identical to what vr_pad_frames_f32 writes.  Parameter gradients only.
+__device__ __forceinline__ void synth_adjoint_ups_step(const BwdParams& p, long long n, long long i, float lam, float lam_rcp,
+                                                       float Lx, float Ly, float Lz,
+                                                       double& g_lam, double& g_lx, double& g_ly, double& g_lz) {
+    const long long idx = n * p.T + i;
+    const double gI = (double)__ldg(p.gz + idx * 2), gQ = (double)__ldg(p.gz + idx * 2 + 1);
+    if (gI == 0.0 && gQ == 0.0) return;
+    const int C3 = 3 * p.VM;
+    int j;
+    double tt;
+    pf_locate(i, p.ups_ratio, p.ups_T, j, tt);
+    const double* cf = p.coef + ((size_t)n * (p.ups_T - 1) + j) * 4 * C3;   // a0..a3 of interval j, C3 apart
+    const int M = p.M, VM = p.VM;
+    auto pos = [&](int v, int m, int c) {
+        const double* a = cf + c * VM + v * M + m;
+        return pf_eval(tt, __ldg(a), __ldg(a + C3), __ldg(a + 2 * C3), __ldg(a + 3 * C3));
+    };
+    for (int m = 0; m < p.M; ++m)
+        synth_adjoint_body(p, pos, m, gI, gQ, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz, nullptr, 0);
+}
+
 __global__ void __launch_bounds__(128) vr_synth_adjoint_kernel(const __grid_constant__ BwdParams p) {
     const int T = (int)p.T;
     const long long total = p.N * (long long)T;
@@ -389,50 +435,73 @@ __global__ void __launch_bounds__(128) vr_synth_adjoint_kernel(const __grid_cons
     double g_lam = 0.0, g_lx = 0.0, g_ly = 0.0, g_lz = 0.0;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
         const long long n = idx / T;
-        const int t = (int)(idx - n * T);
-        const double gI = (double)__ldg(p.gz + idx * 2), gQ = (double)__ldg(p.gz + idx * 2 + 1);
-        if (gI == 0.0 && gQ == 0.0) continue;
-        const float* x0 = p.x + (n * 3 * T + t) * (long long)p.VM;       // x-plane row of this time step
-        const long long ps = (long long)T * p.VM;                         // floats between coordinate planes
-        const int M = p.M;
-        auto pos = [&](int v, int m, int c) { return __ldg(x0 + v * M + m + c * ps); };
-        float* gx0 = p.gx ? p.gx + (n * 3 * T + t) * (long long)p.VM : nullptr;   // this thread's own rows of dL/dx
-        for (int m = 0; m < p.M; ++m)
-            synth_adjoint_body(p, pos, m, gI, gQ, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz, gx0, ps);
+        synth_adjoint_step(p, n, (int)(idx - n * T), lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz);
     }
     synth_adjoint_reduce(p, g_lam, g_lx, g_ly, g_lz);
 }
 
-// The same adjoint at the up-sampled steps of vr_forward_upsampled_f32 (T = ups_K * ups_T): the joint positions of step
-// i come from the per-interval cubics (pf_locate + pf_eval on p.coef), bit-identical to what vr_pad_frames_f32 writes.
-// Parameter gradients only.  (Staging the positions of a block's steps in shared memory first was measured slower on a
-// B200: 54.7 vs 38.6 ms per fwd+bwd step at N = 256, k = 250 -- occupancy drops to two blocks per SM.)
+// The same adjoint at the up-sampled steps of vr_forward_upsampled_f32.  (Staging the positions of a block's steps in shared
+// memory first was measured slower on a B200: 54.7 vs 38.6 ms per fwd+bwd step at N = 256, k = 250 -- occupancy drops to
+// two blocks per SM.)
 __global__ void __launch_bounds__(128) vr_synth_adjoint_ups_kernel(const __grid_constant__ BwdParams p) {
     const long long KT = p.T;
     const long long total = p.N * KT;
     const float lam = __ldg(p.lam_ptr);
     const float Lx = __ldg(p.loc_ptr), Ly = __ldg(p.loc_ptr + 1), Lz = __ldg(p.loc_ptr + 2);
     const float lam_rcp = rcp_refined(lam);
-    const int C3 = 3 * p.VM;
     double g_lam = 0.0, g_lx = 0.0, g_ly = 0.0, g_lz = 0.0;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
         const long long n = idx / KT;
-        const long long i = idx - n * KT;
-        const double gI = (double)__ldg(p.gz + idx * 2), gQ = (double)__ldg(p.gz + idx * 2 + 1);
-        if (gI == 0.0 && gQ == 0.0) continue;
-        int j;
-        double tt;
-        pf_locate(i, p.ups_ratio, p.ups_T, j, tt);
-        const double* cf = p.coef + ((size_t)n * (p.ups_T - 1) + j) * 4 * C3;   // a0..a3 of interval j, C3 apart
-        const int M = p.M, VM = p.VM;
-        auto pos = [&](int v, int m, int c) {
-            const double* a = cf + c * VM + v * M + m;
-            return pf_eval(tt, __ldg(a), __ldg(a + C3), __ldg(a + 2 * C3), __ldg(a + 3 * C3));
-        };
-        for (int m = 0; m < p.M; ++m)
-            synth_adjoint_body(p, pos, m, gI, gQ, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz, nullptr, 0);
+        synth_adjoint_ups_step(p, n, idx - n * KT, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz);
     }
     synth_adjoint_reduce(p, g_lam, g_lx, g_ly, g_lz);
+}
+
+// ---- per-sequence parameter gradients (VR_FLAG_PER_SEQUENCE) ----------------------------------------------------------
+// Sequence n reads placement n.  Its steps are cut into PS_SEG-step segments; one warp at a time owns a (sequence,
+// segment) unit, lane k runs the per-step adjoint above for step k of the segment, the warp adds the four gradients with a
+// fixed butterfly of shuffles and lane 0 stores the unit's 4 partials (p.part, the scratch tail of the caller's gradient
+// buffer).  vr_param_fold_kernel then adds each sequence's partials in segment order into gparams[4 n ..].  The cut depends
+// on T alone and every sum runs in a fixed order, so a sequence's gradients are the same bits wherever it sits in the
+// batch, whatever the batch size, grid or SM count.  No atomics, no counters.  (A block of 128 threads per 256-step
+// segment, reduced with block_sum4, measured 1.19x the scalar path's forward + backward step at T = 300, N = 256 and 4096,
+// on a B200, against 1.01-1.02x for a warp per 32 steps: 300 = 256 + 44 steps, and the second segment leaves 84 of the 128
+// threads idle, where a warp per 32 steps idles at most 31 lanes per sequence; profiles/r03d_rejected_variants.md.)
+template <bool UPS>
+__global__ void __launch_bounds__(128) vr_synth_adjoint_ps_kernel(const __grid_constant__ BwdParams p) {
+    const int lane = threadIdx.x & 31;
+    const long long segs = p.ps_segs, units = p.N * segs;
+    const long long wstride = (long long)gridDim.x * (blockDim.x >> 5);
+    for (long long u = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); u < units; u += wstride) {
+        const long long n = u / segs;
+        const long long t = (u - n * segs) * PS_SEG + lane;
+        const float lam = __ldg(p.lam_ptr + n);
+        const float Lx = __ldg(p.loc_ptr + 3 * n), Ly = __ldg(p.loc_ptr + 3 * n + 1), Lz = __ldg(p.loc_ptr + 3 * n + 2);
+        const float lam_rcp = rcp_refined(lam);
+        double g[4] = {0.0, 0.0, 0.0, 0.0};
+        if (t < p.T) {
+            if (UPS) synth_adjoint_ups_step(p, n, t, lam, lam_rcp, Lx, Ly, Lz, g[0], g[1], g[2], g[3]);
+            else synth_adjoint_step(p, n, (int)t, lam, lam_rcp, Lx, Ly, Lz, g[0], g[1], g[2], g[3]);
+        }
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+            for (int o = 16; o > 0; o >>= 1) g[i] += __shfl_xor_sync(0xffffffffu, g[i], o);
+        if (lane == 0) {
+            double* q = p.part + u * 4;
+            q[0] = g[0]; q[1] = g[1]; q[2] = g[2]; q[3] = g[3];
+        }
+    }
+}
+
+// gparams[i] += the segment partials of sequence i / 4, component i % 4, added in segment order
+__global__ void __launch_bounds__(128) vr_param_fold_kernel(const double* __restrict__ part, double* __restrict__ gparams,
+                                                            long long N, long long segs) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= 4 * N) return;
+    const double* q = part + (i >> 2) * segs * 4 + (i & 3);
+    double a = 0.0;
+    for (long long s = 0; s < segs; ++s) a += q[s * 4];
+    gparams[i] += a;
 }
 #endif  // __CUDACC__
 

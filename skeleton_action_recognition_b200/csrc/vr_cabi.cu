@@ -312,15 +312,18 @@ bool make_team_plan(vr::Params& p, int sm_count, int& grid) {
 }
 
 typedef void (*KernelFn)(const vr::Params);
-struct TeamVariant { bool fma; int vm; int nb; KernelFn fn; };
-#define VR_TEAM_VARIANT(VM, NB) {false, VM, NB, vr::vr_team_kernel<false, VM, NB>}, {true, VM, NB, vr::vr_team_kernel<true, VM, NB>}
-const TeamVariant kTeamVariants[] = { VR_TEAM_VARIANT(0, 1), VR_TEAM_VARIANT(0, 2), VR_TEAM_VARIANT(50, 2) };
+// ps: per-sequence placements (VR_FLAG_PER_SEQUENCE); the scalar instantiations are the kernels without them
+struct TeamVariant { bool fma; int vm; int nb; bool ps; KernelFn fn; };
+#define VR_TEAM_VARIANT(VM, NB, PS) {false, VM, NB, PS, vr::vr_team_kernel<false, VM, NB, PS>}, \
+                                    {true, VM, NB, PS, vr::vr_team_kernel<true, VM, NB, PS>}
+const TeamVariant kTeamVariants[] = { VR_TEAM_VARIANT(0, 1, false), VR_TEAM_VARIANT(0, 2, false), VR_TEAM_VARIANT(50, 2, false),
+                                      VR_TEAM_VARIANT(0, 1, true), VR_TEAM_VARIANT(0, 2, true), VR_TEAM_VARIANT(50, 2, true) };
 const int kNumTeamVariants = sizeof(kTeamVariants) / sizeof(kTeamVariants[0]);
-KernelFn pick_team_kernel(bool fma, int vm, int m) {
+KernelFn pick_team_kernel(bool fma, int vm, int m, bool ps) {
     const int nb = (m % 2 == 0) ? 2 : 1;
     KernelFn generic = nullptr;
     for (int i = 0; i < kNumTeamVariants; ++i) {
-        if (kTeamVariants[i].fma != fma || kTeamVariants[i].nb != nb) continue;
+        if (kTeamVariants[i].fma != fma || kTeamVariants[i].nb != nb || kTeamVariants[i].ps != ps) continue;
         if (kTeamVariants[i].vm == vm) return kTeamVariants[i].fn;
         if (kTeamVariants[i].vm == 0) generic = kTeamVariants[i].fn;
     }
@@ -328,23 +331,24 @@ KernelFn pick_team_kernel(bool fma, int vm, int m) {
 }
 
 // kernel variants: range rounding mode x compile-time V*M (plane stride as an immediate); VM=0 is generic
-struct Variant { bool fma; int vm; int nb; bool ups; bool park; KernelFn fn; };
-#define VR_VARIANT(VM, NB, UPS, PARK) {false, VM, NB, UPS, PARK, vr::vr_fused_kernel<false, VM, NB, UPS, PARK>}, \
-                                      {true, VM, NB, UPS, PARK, vr::vr_fused_kernel<true, VM, NB, UPS, PARK>}
-const Variant kVariants[] = {
-    // short sequences (one job each, a z plane per bone group): generic V*M, one / two bodies at a time; NTU
-    VR_VARIANT(0, 1, false, false), VR_VARIANT(0, 2, false, false), VR_VARIANT(50, 2, false, false),
-    // long sequences (several jobs, parked partial sums)
-    VR_VARIANT(0, 1, false, true), VR_VARIANT(0, 2, false, true), VR_VARIANT(50, 2, false, true),
-    // fused temporal up-sampling (always long)
-    VR_VARIANT(0, 1, true, true), VR_VARIANT(0, 2, true, true), VR_VARIANT(50, 2, true, true),
-};
+struct Variant { bool fma; int vm; int nb; bool ups; bool park; bool ps; KernelFn fn; };
+#define VR_VARIANT(VM, NB, UPS, PARK, PS) {false, VM, NB, UPS, PARK, PS, vr::vr_fused_kernel<false, VM, NB, UPS, PARK, PS>}, \
+                                          {true, VM, NB, UPS, PARK, PS, vr::vr_fused_kernel<true, VM, NB, UPS, PARK, PS>}
+#define VR_VARIANTS(PS) \
+    /* short sequences (one job each, a z plane per bone group): generic V*M, one / two bodies at a time; NTU */ \
+    VR_VARIANT(0, 1, false, false, PS), VR_VARIANT(0, 2, false, false, PS), VR_VARIANT(50, 2, false, false, PS), \
+    /* long sequences (several jobs, parked partial sums) */ \
+    VR_VARIANT(0, 1, false, true, PS), VR_VARIANT(0, 2, false, true, PS), VR_VARIANT(50, 2, false, true, PS), \
+    /* fused temporal up-sampling (always long) */ \
+    VR_VARIANT(0, 1, true, true, PS), VR_VARIANT(0, 2, true, true, PS), VR_VARIANT(50, 2, true, true, PS)
+const Variant kVariants[] = { VR_VARIANTS(false), VR_VARIANTS(true) };
 const int kNumVariants = sizeof(kVariants) / sizeof(kVariants[0]);
-KernelFn pick_kernel(bool fma, int vm, int m, bool ups, bool park) {
+KernelFn pick_kernel(bool fma, int vm, int m, bool ups, bool park, bool ps) {
     const int nb = (m % 2 == 0) ? 2 : 1;
     KernelFn generic = nullptr;
     for (int i = 0; i < kNumVariants; ++i) {
-        if (kVariants[i].fma != fma || kVariants[i].nb != nb || kVariants[i].ups != ups || kVariants[i].park != park) continue;
+        if (kVariants[i].fma != fma || kVariants[i].nb != nb || kVariants[i].ups != ups || kVariants[i].park != park ||
+            kVariants[i].ps != ps) continue;
         if (kVariants[i].vm == vm) return kVariants[i].fn;
         if (kVariants[i].vm == 0) generic = kVariants[i].fn;
     }
@@ -454,7 +458,8 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
     const bool iq_only = out == nullptr;
     if (!x || (!out && !iq)) return fail(VR_ERR_ARG, "x and out (or iq) must not be null");
     if ((lam_dev == nullptr) != (loc_dev == nullptr)) return fail(VR_ERR_ARG, "wavelength and radar_location must both be device pointers or both be null");
-    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_INPUTS_READY)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
+    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_INPUTS_READY | VR_FLAG_PER_SEQUENCE)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
+    const bool per_seq = (flags & VR_FLAG_PER_SEQUENCE) != 0;   // (the entries reject it with host parameters or null pointers)
     int dev, sm_count;
     int rc = device_setup(dev, sm_count);
     if (rc) return rc;
@@ -497,8 +502,8 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = g_pdl ? 1 : 0;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    KernelFn fn = team ? pick_team_kernel((flags & VR_FLAG_RANGE_FMA) != 0, p.VM, p.M)
-                       : pick_kernel((flags & VR_FLAG_RANGE_FMA) != 0, p.VM, p.M, coef != nullptr, p.zpark != 0);
+    KernelFn fn = team ? pick_team_kernel((flags & VR_FLAG_RANGE_FMA) != 0, p.VM, p.M, per_seq)
+                       : pick_kernel((flags & VR_FLAG_RANGE_FMA) != 0, p.VM, p.M, coef != nullptr, p.zpark != 0, per_seq);
     CUDA_TRY(cudaLaunchKernelEx(&cfg, fn, p));
     return VR_OK;
 }
@@ -603,6 +608,8 @@ int vr_forward_host_f32(const float* x_host, int64_t N, int64_t T, int32_t V, in
                         float wavelength, const float* radar_loc_host,
                         int32_t n_fft, int32_t hop, uint32_t flags, float* out_host, int64_t sub_batch) {
     if (!x_host || !out_host || !radar_loc_host) return fail(VR_ERR_ARG, "host pointers must not be null");
+    if (flags & VR_FLAG_PER_SEQUENCE)
+        return fail(VR_ERR_ARG, "vr_forward_host_f32 takes one host placement for the batch; VR_FLAG_PER_SEQUENCE needs a device-pointer entry point");
     if (N <= 0 || T <= 0 || V <= 0 || M <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M, hop must be positive");
     int dev, sm_count;
     int rc = device_setup(dev, sm_count);
@@ -988,7 +995,10 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     // the up-sampling spline's (T = ups_K * ups_T steps, x_dev unused), parameter gradients only
     if ((!x_dev && !coef) || !gz_work_dev || !grad_params_dev || !wavelength_dev || !radar_loc_dev || (!synth_only && (!iq_dev || !grad_out_dev)))
         return fail(VR_ERR_ARG, "device pointers must not be null");
-    if (flags & ~VR_FLAG_RANGE_FMA) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
+    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_PER_SEQUENCE)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
+    const bool per_seq = (flags & VR_FLAG_PER_SEQUENCE) != 0;
+    if (per_seq && ((uintptr_t)grad_params_dev & 7) != 0)
+        return fail(VR_ERR_ARG, "grad_params_dev must be 8-byte aligned (float64 per-sequence gradients)");
     if (N <= 0 || T <= 0 || V <= 0 || M <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M, hop must be positive");
     if (n_fft != vr::NFFT) return fail(VR_ERR_UNSUPPORTED, "this ABI version implements n_fft=256 only (got %d)", n_fft);
     if (!synth_only && T <= n_fft / 2) return fail(VR_ERR_SHAPE, "T=%lld must exceed n_fft/2=%d", (long long)T, n_fft / 2);
@@ -1022,6 +1032,19 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
         vr::vr_stft_adjoint_kernel<<<grid1, vr::BWD_WARPS * 32, (size_t)p.seg_len * 8, st>>>(p);
         CUDA_TRY(cudaGetLastError());
     }
+    if (per_seq) {
+        // per-sequence gradients: (sequence, segment) units reduced block by block into the scratch tail of
+        // grad_params_dev (vr_per_sequence_grad_doubles), then folded per sequence in segment order
+        p.ps_segs = vr::ps_segments(T);
+        p.part = grad_params_dev + 4 * N;
+        const int grid2 = (int)std::min<long long>((N * p.ps_segs + 3) / 4, (long long)sm_count * 16);   // 4 warps per block
+        if (coef) vr::vr_synth_adjoint_ps_kernel<true><<<grid2, 128, 0, st>>>(p);
+        else vr::vr_synth_adjoint_ps_kernel<false><<<grid2, 128, 0, st>>>(p);
+        CUDA_TRY(cudaGetLastError());
+        vr::vr_param_fold_kernel<<<(unsigned)((4 * N + 127) / 128), 128, 0, st>>>(p.part, grad_params_dev, N, p.ps_segs);
+        CUDA_TRY(cudaGetLastError());
+        return VR_OK;
+    }
     const long long steps = N * T;
     const int grid2 = (int)std::min<long long>(std::min<long long>((steps + 127) / 128, (long long)sm_count * 16), vr::PARAM_MAX_BLOCKS);
     next_param_slot(dev, p);
@@ -1041,6 +1064,11 @@ int vr_synth_adjoint_upsampled_f32(const void* workspace_dev, const float* grad_
     // the second stage of vr_backward_upsampled_params_f32 alone: dL/d(iq) comes from the caller (a general STFT)
     return backward_ups_impl(workspace_dev, nullptr, nullptr, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev,
                              vr::NFFT, 16, flags, num_pad_frames, true, const_cast<float*>(grad_iq_dev), grad_params_dev, stream);
+}
+
+int64_t vr_per_sequence_grad_doubles(int64_t N, int64_t T) {
+    if (N <= 0 || T <= 0) return 0;
+    return 4 * N + 4 * N * vr::ps_segments(T);
 }
 
 int vr_release_host_staging(void) {

@@ -160,6 +160,23 @@ class _GeneralSTFTFunction(torch.autograd.Function):
         return (giq, gsin if ctx.needs_input_grad[1] else None, gcos if ctx.needs_input_grad[2] else None, None, None, None, None)
 
 
+def _param_grad_buffer(flags, N, T, device):
+    """float64 gradient buffer of a backward call: the 4 batch-summed gradients, or with VR_FLAG_PER_SEQUENCE N x 4
+    per-sequence gradients followed by the scratch of their reduction (T: the steps the adjoint runs over)."""
+    if flags & _cabi.VR_FLAG_PER_SEQUENCE:
+        return torch.zeros(_cabi.per_sequence_grad_doubles(N, T), dtype=torch.float64, device=device)
+    return torch.zeros(4, dtype=torch.float64, device=device)
+
+
+def _param_grads(ctx, gp, lam, loc):
+    """(dL/dwavelength, dL/dradar_location) in the shapes of `lam` and `loc` -- () and (3,), or (N,) and (N, 3) -- from the
+    buffer of _param_grad_buffer; None where no gradient is needed."""
+    g = gp[:4 * lam.numel()].view(-1, 4)
+    g_lam = g[:, 0].to(torch.float32).reshape(lam.shape) if ctx.needs_input_grad[0] else None
+    g_loc = g[:, 1:4].to(torch.float32).reshape(loc.shape) if ctx.needs_input_grad[1] else None
+    return g_lam, g_loc
+
+
 class _RadarFunction(torch.autograd.Function):
     """forward() with gradients for `wavelength`, `radar_location` and `x` (the reference gets them from
     PyTorch autograd over layers/virtual_radar.py:79-134; here: C ABI vr_backward_f32).  The
@@ -167,7 +184,7 @@ class _RadarFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, lam, loc, xc, layer, flags):
-        out, iq = layer._launch(xc, flags, want_iq=True)
+        out, iq = layer._launch(xc, flags, want_iq=True, lam=lam, loc=loc)
         ctx.save_for_backward(lam, loc, xc, iq)
         ctx.layer, ctx.flags = layer, flags
         return out
@@ -179,7 +196,7 @@ class _RadarFunction(torch.autograd.Function):
         N, _, T, V, M = xc.shape
         g = grad_out.contiguous().to(torch.float32)
         gz = torch.empty((N, T, 2), dtype=torch.float32, device=xc.device)
-        gp = torch.zeros(4, dtype=torch.float64, device=xc.device)
+        gp = _param_grad_buffer(ctx.flags, N, T, xc.device)
         gx = torch.empty_like(xc) if ctx.needs_input_grad[2] else None
         with torch.cuda.device(xc.device):
             stream = torch.cuda.current_stream(xc.device).cuda_stream
@@ -189,8 +206,7 @@ class _RadarFunction(torch.autograd.Function):
                                              ctx.flags, gz.data_ptr(), gp.data_ptr(),
                                              gx.data_ptr() if gx is not None else None, ctypes.c_void_p(stream))
         _cabi.check(rc)
-        g_lam = gp[0].to(torch.float32).reshape(lam.shape) if ctx.needs_input_grad[0] else None
-        g_loc = gp[1:4].to(torch.float32).reshape(loc.shape) if ctx.needs_input_grad[1] else None
+        g_lam, g_loc = _param_grads(ctx, gp, lam, loc)
         return g_lam, g_loc, gx, None, None
 
 
@@ -201,7 +217,7 @@ class _SynthFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, lam, loc, xc, layer, flags):
-        iq = layer._synth(xc, flags)
+        iq = layer._synth(xc, flags, lam, loc)
         ctx.save_for_backward(lam, loc, xc)
         ctx.layer, ctx.flags = layer, flags
         return iq
@@ -212,7 +228,7 @@ class _SynthFunction(torch.autograd.Function):
         layer = ctx.layer
         N, _, T, V, M = xc.shape
         g = grad_iq.contiguous().to(torch.float32)
-        gp = torch.zeros(4, dtype=torch.float64, device=xc.device)
+        gp = _param_grad_buffer(ctx.flags, N, T, xc.device)
         gx = torch.empty_like(xc) if ctx.needs_input_grad[2] else None
         with torch.cuda.device(xc.device):
             stream = torch.cuda.current_stream(xc.device).cuda_stream
@@ -220,8 +236,7 @@ class _SynthFunction(torch.autograd.Function):
                                                   len(layer.src), lam.data_ptr(), loc.data_ptr(), ctx.flags, gp.data_ptr(),
                                                   gx.data_ptr() if gx is not None else None, ctypes.c_void_p(stream))
         _cabi.check(rc)
-        g_lam = gp[0].to(torch.float32).reshape(lam.shape) if ctx.needs_input_grad[0] else None
-        g_loc = gp[1:4].to(torch.float32).reshape(loc.shape) if ctx.needs_input_grad[1] else None
+        g_lam, g_loc = _param_grads(ctx, gp, lam, loc)
         return g_lam, g_loc, gx, None, None
 
 
@@ -232,7 +247,7 @@ class _UpsampledRadarFunction(torch.autograd.Function):
     re-evaluates the joint positions of every up-sampled step."""
 
     @staticmethod
-    def forward(ctx, lam, loc, xc, layer, k, sigma):
+    def forward(ctx, lam, loc, xc, layer, k, sigma, flags=0):
         N, _, T, V, M = xc.shape
         L = _cabi.lib()
         nbytes = int(L.vr_upsampled_workspace_bytes(N, T, V, M))
@@ -242,12 +257,12 @@ class _UpsampledRadarFunction(torch.autograd.Function):
         with torch.cuda.device(xc.device):
             stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
             rc = L.vr_forward_upsampled_debug_f32(xc.data_ptr(), N, T, V, M, layer._src_c, layer._dst_c, len(layer.src),
-                                                  lam.data_ptr(), loc.data_ptr(), layer.n_fft, layer.hop_length, 0,
+                                                  lam.data_ptr(), loc.data_ptr(), layer.n_fft, layer.hop_length, flags,
                                                   k, ctypes.c_float(float(sigma)), work.data_ptr(), nbytes,
                                                   out.data_ptr(), iq.data_ptr(), stream)
         _cabi.check(rc)
         ctx.save_for_backward(lam, loc, work, iq)
-        ctx.layer, ctx.dims = layer, (N, T, V, M, k)
+        ctx.layer, ctx.dims, ctx.flags = layer, (N, T, V, M, k), flags
         return out
 
     @staticmethod
@@ -257,17 +272,16 @@ class _UpsampledRadarFunction(torch.autograd.Function):
         N, T, V, M, k = ctx.dims
         g = grad_out.contiguous().to(torch.float32)
         gz = torch.empty_like(iq)
-        gp = torch.zeros(4, dtype=torch.float64, device=iq.device)
+        gp = _param_grad_buffer(ctx.flags, N, k * T, iq.device)
         with torch.cuda.device(iq.device):
             stream = torch.cuda.current_stream(iq.device).cuda_stream
             rc = _cabi.lib().vr_backward_upsampled_params_f32(work.data_ptr(), iq.data_ptr(), g.data_ptr(), N, T, V, M,
                                                               layer._src_c, layer._dst_c, len(layer.src),
                                                               lam.data_ptr(), loc.data_ptr(), layer.n_fft, layer.hop_length,
-                                                              0, k, gz.data_ptr(), gp.data_ptr(), ctypes.c_void_p(stream))
+                                                              ctx.flags, k, gz.data_ptr(), gp.data_ptr(), ctypes.c_void_p(stream))
         _cabi.check(rc)
-        g_lam = gp[0].to(torch.float32).reshape(lam.shape) if ctx.needs_input_grad[0] else None
-        g_loc = gp[1:4].to(torch.float32).reshape(loc.shape) if ctx.needs_input_grad[1] else None
-        return g_lam, g_loc, None, None, None, None
+        g_lam, g_loc = _param_grads(ctx, gp, lam, loc)
+        return g_lam, g_loc, None, None, None, None, None
 
 
 class _UpsampledSynthFunction(torch.autograd.Function):
@@ -277,10 +291,10 @@ class _UpsampledSynthFunction(torch.autograd.Function):
     Used by forward_upsampled when the STFT is general and therefore runs outside the fused kernel."""
 
     @staticmethod
-    def forward(ctx, lam, loc, xc, layer, k, sigma):
-        iq, work = layer._synth_upsampled(xc, k, sigma)
+    def forward(ctx, lam, loc, xc, layer, k, sigma, flags=0):
+        iq, work = layer._synth_upsampled(xc, k, sigma, lam, loc, flags)
         ctx.save_for_backward(lam, loc, work)
-        ctx.layer, ctx.dims = layer, tuple(xc.shape) + (k,)
+        ctx.layer, ctx.dims, ctx.flags = layer, tuple(xc.shape) + (k,), flags
         return iq
 
     @staticmethod
@@ -289,16 +303,15 @@ class _UpsampledSynthFunction(torch.autograd.Function):
         layer = ctx.layer
         N, _, T, V, M, k = ctx.dims
         g = grad_iq.contiguous().to(torch.float32)
-        gp = torch.zeros(4, dtype=torch.float64, device=g.device)
+        gp = _param_grad_buffer(ctx.flags, N, k * T, g.device)
         with torch.cuda.device(g.device):
             stream = torch.cuda.current_stream(g.device).cuda_stream
             rc = _cabi.lib().vr_synth_adjoint_upsampled_f32(work.data_ptr(), g.data_ptr(), N, T, V, M, layer._src_c, layer._dst_c,
-                                                            len(layer.src), lam.data_ptr(), loc.data_ptr(), 0, k, gp.data_ptr(),
-                                                            ctypes.c_void_p(stream))
+                                                            len(layer.src), lam.data_ptr(), loc.data_ptr(), ctx.flags, k,
+                                                            gp.data_ptr(), ctypes.c_void_p(stream))
         _cabi.check(rc)
-        g_lam = gp[0].to(torch.float32).reshape(lam.shape) if ctx.needs_input_grad[0] else None
-        g_loc = gp[1:4].to(torch.float32).reshape(loc.shape) if ctx.needs_input_grad[1] else None
-        return g_lam, g_loc, None, None, None, None
+        g_lam, g_loc = _param_grads(ctx, gp, lam, loc)
+        return g_lam, g_loc, None, None, None, None, None
 
 
 def kept_frame_table(n_frames, image_size):
@@ -410,6 +423,34 @@ class VirtualRadar(torch.nn.Module):
             raise RuntimeError("module parameters are on %s but x is on %s; call .to(x.device)" % (lam.device, x.device))
         return lam, loc
 
+    def _placements(self, x, radar_location, wavelength):
+        """Per-sequence radar placements (the `radar_location=` / `wavelength=` keywords of forward, forward_image and
+        forward_upsampled) -> None when neither is given, else (wavelength (N,), radar_location (N, 3)): each keyword
+        expanded to the batch and made contiguous, the module parameter standing in for a keyword not given.  Autograd's
+        expand carries the per-sequence gradients back to whatever the caller passed (summed where it broadcast)."""
+        if radar_location is None and wavelength is None:
+            return None
+        N = x.shape[0]
+        out = []
+        for name, value, param, shape in (("wavelength", wavelength, self.wavelength, (N,)),
+                                          ("radar_location", radar_location, self.radar_location, (N, 3))):
+            if value is None:
+                value = param
+            elif not isinstance(value, torch.Tensor) or value.dtype != torch.float32:
+                raise ValueError("%s must be a float32 tensor that broadcasts to %s, got %s"
+                                 % (name, shape, value.dtype if isinstance(value, torch.Tensor) else type(value)))
+            elif not value.is_cuda or value.device != x.device:
+                raise RuntimeError("%s is on %s but x is on %s: per-sequence placements are read on x's device"
+                                   % (name, value.device, x.device))
+            if tuple(value.shape) != shape or not value.is_contiguous():   # (a full contiguous tensor is used as it is)
+                try:
+                    value = value.expand(shape)
+                except RuntimeError:
+                    raise ValueError("%s of shape %s does not broadcast to %s" % (name, tuple(value.shape), shape)) from None
+                value = value.contiguous()
+            out.append(value)
+        return tuple(out)
+
     def _prepare(self, x):
         """Pick the range rounding mode from the caller's strides BEFORE normalising the layout
         (SURVEY fact 6: ATen's CPU norm rounds differently when the coordinate axis is innermost)."""
@@ -418,8 +459,12 @@ class VirtualRadar(torch.nn.Module):
 
     _FUSED_N_FFT = 256      # the fused kernel's FFT size; other n_fft values go through the general-kernel path
 
-    def _launch(self, xc, flags, want_iq=False):
+    def _launch(self, xc, flags, want_iq=False, lam=None, loc=None):
+        """One fused launch.  lam / loc: the radar parameters to read (default: the module's; (N,) and (N, 3) with
+        VR_FLAG_PER_SEQUENCE in flags)."""
         N, _, T, V, M = xc.shape
+        lam = self.wavelength if lam is None else lam
+        loc = self.radar_location if loc is None else loc
         n_fft = self._FUSED_N_FFT if want_iq else self.n_fft       # iq does not depend on the STFT parameters
         if self.assume_inputs_ready:
             flags |= _cabi.VR_FLAG_INPUTS_READY
@@ -433,8 +478,8 @@ class VirtualRadar(torch.nn.Module):
         try:
             with torch.cuda.device(xc.device):
                 stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
-                args = (xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src), self.wavelength.data_ptr(),
-                        self.radar_location.data_ptr(), n_fft, self.hop_length, flags, out.data_ptr())
+                args = (xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src), lam.data_ptr(),
+                        loc.data_ptr(), n_fft, self.hop_length, flags, out.data_ptr())
                 rc = L.vr_forward_debug_f32(*args, iq.data_ptr(), stream) if want_iq else L.vr_forward_f32(*args, stream)
         finally:
             if self.nvtx_ranges:
@@ -442,10 +487,12 @@ class VirtualRadar(torch.nn.Module):
         _cabi.check(rc)
         return out, iq
 
-    def _synth(self, xc, flags):
+    def _synth(self, xc, flags, lam=None, loc=None):
         """Synthesis only (C ABI vr_synth_f32): the complex baseband signal (N,T,2) that the general-kernel STFT reads,
         bit for bit forward_debug's, without any STFT work."""
         N, _, T, V, M = xc.shape
+        lam = self.wavelength if lam is None else lam
+        loc = self.radar_location if loc is None else loc
         if self.assume_inputs_ready:
             flags |= _cabi.VR_FLAG_INPUTS_READY
         iq = torch.empty((N, T, 2), dtype=torch.float32, device=xc.device)
@@ -457,19 +504,20 @@ class VirtualRadar(torch.nn.Module):
             with torch.cuda.device(xc.device):
                 stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
                 rc = _cabi.lib().vr_synth_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
-                                              self.wavelength.data_ptr(), self.radar_location.data_ptr(), flags,
-                                              iq.data_ptr(), stream)
+                                              lam.data_ptr(), loc.data_ptr(), flags, iq.data_ptr(), stream)
         finally:
             if self.nvtx_ranges:
                 torch.cuda.nvtx.range_pop()
         _cabi.check(rc)
         return iq
 
-    def _synth_upsampled(self, xc, k, sigma):
+    def _synth_upsampled(self, xc, k, sigma, lam=None, loc=None, flags=0):
         """Synthesis of pad_frames(xc, k, sigma) without the up-sampled batch (C ABI vr_synth_upsampled_f32) -> iq
         (N, k*T, 2) and the workspace holding the spline's cubics.  The up-sampled tensor the reference's loader builds
-        is standard-contiguous: range rounding mode "seq" (flags 0)."""
+        is standard-contiguous: range rounding mode "seq" (no VR_FLAG_RANGE_FMA)."""
         N, _, T, V, M = xc.shape
+        lam = self.wavelength if lam is None else lam
+        loc = self.radar_location if loc is None else loc
         L = _cabi.lib()
         nbytes = int(L.vr_upsampled_workspace_bytes(N, T, V, M))
         work = torch.empty(max(nbytes, 8) // 8, dtype=torch.float64, device=xc.device)
@@ -479,7 +527,7 @@ class VirtualRadar(torch.nn.Module):
         with torch.cuda.device(xc.device):
             stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
             rc = L.vr_synth_upsampled_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
-                                          self.wavelength.data_ptr(), self.radar_location.data_ptr(), 0, k,
+                                          lam.data_ptr(), loc.data_ptr(), flags, k,
                                           ctypes.c_float(float(sigma)), work.data_ptr(), nbytes, iq.data_ptr(), stream)
         _cabi.check(rc)
         return iq, work
@@ -496,31 +544,49 @@ class VirtualRadar(torch.nn.Module):
         frames = _kept_frames_on(n_frames, image_size, iq.device) if n_frames > image_size else None
         return torch.nn.functional.interpolate(self.stft.logmag(iq, frames).unsqueeze(1), image_size)
 
-    def _needs_grad(self, x=None):
+    def _needs_grad(self, x=None, pl=None):
+        if pl is not None:      # per-sequence placements: whatever the caller passed (or the module parameters) decides
+            return torch.is_grad_enabled() and (pl[0].requires_grad or pl[1].requires_grad
+                                                or (x is not None and x.requires_grad))
         return torch.is_grad_enabled() and (self.wavelength.requires_grad or self.radar_location.requires_grad
                                             or (x is not None and x.requires_grad))
 
-    def forward(self, x):
+    def forward(self, x, radar_location=None, wavelength=None):
+        """x (N,3,T,V,M) -> (N, n_fft, T//hop+1).  `radar_location` / `wavelength` (optional): one radar placement per
+        sequence, float32 tensors on x's device that broadcast to (N, 3) and (N,) -- sequence n is seen from
+        radar_location[n] at wavelength[n] (C ABI VR_FLAG_PER_SEQUENCE); a keyword not given is the module parameter.
+        Differentiable per sequence: the gradients reach the tensors passed (through autograd's expand).  Under
+        torch.nn.DataParallel pass full (N, 3) / (N,) tensors: DataParallel splits every tensor argument along dim 0 like
+        the batch, so a broadcast-shaped one -- a (3,) location, a 0-d wavelength -- would reach the replicas cut apart
+        (expand it to the batch first, e.g. `loc.expand(len(x), 3)`)."""
         self._check_input(x)
         self._check_device(x)
+        pl = self._placements(x, radar_location, wavelength)
         xc, flags = self._prepare(x)
-        return self._run(x, xc, flags)
+        return self._run(x, xc, flags, pl)
 
-    def _run(self, x, xc, flags):
-        """forward() after the layout has been normalised: xc standard-contiguous, flags carry the range rounding mode."""
+    def _run(self, x, xc, flags, pl=None):
+        """forward() after the layout has been normalised: xc standard-contiguous, flags carry the range rounding mode;
+        pl: per-sequence placements (_placements) or None."""
         lam, loc = self.wavelength, self.radar_location
+        if pl is not None:
+            lam, loc = pl
+            flags |= _cabi.VR_FLAG_PER_SEQUENCE
         if self._general_stft():     # trained / trainable STFT kernels: synthesis on our kernels, STFT as a GEMM
             self._check_general_length(xc.shape[2])
             if xc.shape[0] == 0:
-                return self._launch(xc, flags)[0]
-            return self.stft.logmag(self._general_iq(x, xc, flags))
-        if self._needs_grad(x) and xc.shape[0] > 0:
+                return self._launch(xc, flags, lam=lam, loc=loc)[0]
+            return self.stft.logmag(self._general_iq(x, xc, flags, pl))
+        if self._needs_grad(x, pl) and xc.shape[0] > 0:
             return _RadarFunction.apply(lam, loc, xc, self, flags)
-        return self._launch(xc, flags)[0]
+        return self._launch(xc, flags, lam=lam, loc=loc)[0]
 
-    def _general_iq(self, x, xc, flags):
+    def _general_iq(self, x, xc, flags, pl=None):
         lam, loc = self.wavelength, self.radar_location
-        return _SynthFunction.apply(lam, loc, xc, self, flags) if self._needs_grad(x) else self._synth(xc, flags)
+        if pl is not None:
+            lam, loc = pl
+            flags |= _cabi.VR_FLAG_PER_SEQUENCE
+        return _SynthFunction.apply(lam, loc, xc, self, flags) if self._needs_grad(x, pl) else self._synth(xc, flags, lam, loc)
 
     def forward_notebook(self, data, num_pad_frames=1, sigma=3):
         """virtual_radar_example.ipynb cells 2-4 on the device: `data` is one body's (T, V, 3) array (or a batch
@@ -538,23 +604,28 @@ class VirtualRadar(torch.nn.Module):
         self._check_device(x)
         return self._run(x, x, _cabi.VR_FLAG_RANGE_FMA)
 
-    def forward_image(self, x, image_size=256):
+    def forward_image(self, x, image_size=256, radar_location=None, wavelength=None):
         """The layer fused with its consumer's input stage (reference models/resnet.py:24-26):
         equals `F.interpolate(self(x).unsqueeze(1), image_size)` (nearest) bit for bit, in one launch
         that writes (N, 1, image_size, image_size) directly and transforms only the frames the
-        resize keeps."""
+        resize keeps.  `radar_location` / `wavelength`: per-sequence placements, as in forward()."""
         self._check_input(x)
         lam, loc = self._check_device(x)
+        pl = self._placements(x, radar_location, wavelength)
         image_size = int(image_size)
         if image_size < 1:
             raise ValueError("image_size must be positive, got %d" % image_size)
         if self._general_stft():        # general STFT kernels: synthesis, then the STFT of the frames the resize keeps
             xc, flags = self._prepare(x)
             self._check_general_length(xc.shape[2])
-            return self._general_image(self._general_iq(x, xc, flags), image_size)
-        if self._needs_grad(x):         # gradients wanted: spectrogram, then torch's resize
-            return torch.nn.functional.interpolate(self.forward(x).unsqueeze(1), image_size)
+            return self._general_image(self._general_iq(x, xc, flags, pl), image_size)
+        if self._needs_grad(x, pl):     # gradients wanted: spectrogram, then torch's resize
+            spec = self.forward(x) if pl is None else self._run(x, *self._prepare(x), pl)
+            return torch.nn.functional.interpolate(spec.unsqueeze(1), image_size)
         xc, flags = self._prepare(x)
+        if pl is not None:
+            lam, loc = pl
+            flags |= _cabi.VR_FLAG_PER_SEQUENCE
         if self.assume_inputs_ready:
             flags |= _cabi.VR_FLAG_INPUTS_READY
         N, _, T, V, M = xc.shape
@@ -569,7 +640,7 @@ class VirtualRadar(torch.nn.Module):
         _cabi.check(rc)
         return out
 
-    def forward_upsampled(self, x, num_pad_frames=250, sigma=3, image_size=None):
+    def forward_upsampled(self, x, num_pad_frames=250, sigma=3, image_size=None, radar_location=None, wavelength=None):
         """The data loader's temporal up-sampling fused in front of the layer: x is the RAW
         (N,3,T,V,M) batch; the result equals `self(pad_frames(x, num_pad_frames, sigma))` -- or
         `self.forward_image(pad_frames(...), image_size)` when `image_size` is given -- bit for bit,
@@ -578,9 +649,15 @@ class VirtualRadar(torch.nn.Module):
         [+ models/resnet.py:24-26]).  Trainable `wavelength` / `radar_location` keep the fused path
         (vr_forward_upsampled_debug_f32 + vr_backward_upsampled_params_f32); with `image_size` the
         spectrogram is then resized by `F.interpolate`, as `forward_image` does under grad.  Gradients
-        with respect to x itself go through `self(pad_frames(x, num_pad_frames, sigma))`."""
+        with respect to x itself go through `self(pad_frames(x, num_pad_frames, sigma))`.  `radar_location` /
+        `wavelength`: per-sequence placements, as in forward()."""
         self._check_input(x)
         lam, loc = self._check_device(x)
+        pl = self._placements(x, radar_location, wavelength)
+        flags = 0
+        if pl is not None:
+            lam, loc = pl
+            flags = _cabi.VR_FLAG_PER_SEQUENCE
         xc = x.contiguous()
         N, _, T, V, M = xc.shape
         k = int(num_pad_frames)
@@ -591,14 +668,14 @@ class VirtualRadar(torch.nn.Module):
             raise NotImplementedError("forward_upsampled has no gradient with respect to x: detach x, or differentiate "
                                       "layer(pad_frames(x, num_pad_frames, sigma)), which materialises the up-sampled batch")
         if self._general_stft():      # general STFT kernels: synthesis without the up-sampled batch, then the GEMM STFT
-            if self._needs_grad() and N > 0:
-                iq = _UpsampledSynthFunction.apply(lam, loc, xc, self, k, sigma)
+            if self._needs_grad(None, pl) and N > 0:
+                iq = _UpsampledSynthFunction.apply(lam, loc, xc, self, k, sigma, flags)
             else:
-                iq = self._synth_upsampled(xc, k, sigma)[0]
+                iq = self._synth_upsampled(xc, k, sigma, lam, loc, flags)[0]
             self._check_general_length(k * T)
             return self._general_image(iq, img) if img else self.stft.logmag(iq)
-        if self._needs_grad() and N > 0:
-            out = _UpsampledRadarFunction.apply(lam, loc, xc, self, k, sigma)
+        if self._needs_grad(None, pl) and N > 0:
+            out = _UpsampledRadarFunction.apply(lam, loc, xc, self, k, sigma, flags)
             return torch.nn.functional.interpolate(out.unsqueeze(1), img) if img else out
         shape = (N, 1, img, img) if img else (N, self.n_fft, (k * T) // self.hop_length + 1)
         out = torch.empty(shape, dtype=torch.float32, device=x.device)
@@ -611,7 +688,7 @@ class VirtualRadar(torch.nn.Module):
             stream = torch.cuda.current_stream(x.device).cuda_stream
             # the up-sampled tensor the reference's loader builds is standard-contiguous: range rounding mode "seq"
             rc = L.vr_forward_upsampled_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
-                                            lam.data_ptr(), loc.data_ptr(), self.n_fft, self.hop_length, 0,
+                                            lam.data_ptr(), loc.data_ptr(), self.n_fft, self.hop_length, flags,
                                             k, ctypes.c_float(float(sigma)), img, work.data_ptr(), nbytes,
                                             out.data_ptr(), ctypes.c_void_p(stream))
         _cabi.check(rc)

@@ -82,10 +82,12 @@ class Model(nn.Module):
         self.num_pad_frames = num_pad_frames
         self.sigma = sigma
 
-    def spectrogram_image(self, x):
+    def spectrogram_image(self, x, radar_location=None, wavelength=None):
+        """radar_location / wavelength (optional): one radar placement per sequence (VirtualRadar.forward)."""
+        kw = dict(radar_location=radar_location, wavelength=wavelength)
         if self.num_pad_frames:       # raw sequences: up-sampling, radar and resize in one fused pass
-            return self.virtual_radar.forward_upsampled(x, self.num_pad_frames, self.sigma, self.image_size)
-        return self.virtual_radar.forward_image(x, self.image_size)
+            return self.virtual_radar.forward_upsampled(x, self.num_pad_frames, self.sigma, self.image_size, **kw)
+        return self.virtual_radar.forward_image(x, self.image_size, **kw)
 
-    def forward(self, x):
-        return self.base_model(self.spectrogram_image(x))
+    def forward(self, x, radar_location=None, wavelength=None):
+        return self.base_model(self.spectrogram_image(x, radar_location, wavelength))
