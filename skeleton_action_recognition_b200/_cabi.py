@@ -11,6 +11,8 @@ VR_OK, VR_ERR_ARG, VR_ERR_SHAPE, VR_ERR_UNSUPPORTED, VR_ERR_CUDA = 0, -1, -2, -3
 VR_FLAG_RANGE_FMA = 1
 VR_FLAG_INPUTS_READY = 2
 VR_FLAG_PER_SEQUENCE = 4
+VR_FLAG_VIEWS_SHIFT = 8         # VR_FLAG_VIEWS(R) = R << 8, R in [1, 255]: R radars per sequence (with VR_FLAG_PER_SEQUENCE)
+VR_FLAG_VIEWS_MASK = 0xff << VR_FLAG_VIEWS_SHIFT
 ABI_VERSION = 1
 
 # every symbol include/virtual_radar_b200.h declares
@@ -214,6 +216,19 @@ def per_sequence_grad_doubles(N, T):
     gradients, then the scratch of the per-sequence reduction.  T: the steps the adjoint runs over (up-sampled length for
     the _upsampled entries)."""
     return int(lib().vr_per_sequence_grad_doubles(int(N), int(T)))
+
+
+def views_flag(R):
+    """VR_FLAG_VIEWS(R): R radar views per sequence, x holding N / R sequences (add VR_FLAG_PER_SEQUENCE)."""
+    R = int(R)
+    if not 1 <= R <= 255:
+        raise ValueError("the number of views per sequence must be in [1, 255], got %d" % R)
+    return R << VR_FLAG_VIEWS_SHIFT
+
+
+def views_of(flags):
+    """R of the VR_FLAG_VIEWS field of `flags` (1 when the field is 0): outputs per x sequence."""
+    return ((int(flags) & VR_FLAG_VIEWS_MASK) >> VR_FLAG_VIEWS_SHIFT) or 1
 
 
 def set_schedule(mode):

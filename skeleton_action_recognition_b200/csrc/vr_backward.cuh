@@ -33,7 +33,7 @@ struct BwdParams {
     double* part;                // this launch's slot of g_param_partials: 4 partials per block
     unsigned* count;             // and its counter of finished blocks (0 between launches)
     int seg_len, segs;           // adjoint STFT: samples per segment, segments per sequence (adjoint_plan)
-    float* gx;                   // optional dL/dx (N,3,T,V,M), zeroed before the launch; nullptr = not wanted
+    float* gx;                   // optional dL/dx (N / views,3,T,V,M), zeroed before the launch; nullptr = not wanted
     const float* lam_ptr;        // 1 wavelength and 1 location, or (VR_FLAG_PER_SEQUENCE) N and N x 3
     const float* loc_ptr;
     long long ps_segs;           // VR_FLAG_PER_SEQUENCE: segments per sequence of the per-sequence reduction (part = their
@@ -46,6 +46,8 @@ struct BwdParams {
     double ups_ratio;
     int ups_T;
     uint16_t src[NG * MAX_EG], dst[NG * MAX_EG];
+    int views;                   // VR_FLAG_VIEWS: radars per sequence R (vr_synth_adjoint_ps_kernel); x and coef hold N / R
+                                 // sequences, output n reads sequence n / R.  (Last: the other fields keep their offsets.)
 };
 
 // ---- owner-form plan of the adjoint STFT -----------------------------------------------------------------------------
@@ -387,26 +389,28 @@ __device__ __forceinline__ void synth_adjoint_reduce(const BwdParams& p, double 
     if (threadIdx.x == 0) *p.count = 0u;
 }
 
-// The adjoint of time step t of sequence n, joint positions read from x (and dL/dx written when p.gx is set).
-__device__ __forceinline__ void synth_adjoint_step(const BwdParams& p, long long n, int t, float lam, float lam_rcp,
+// The adjoint of time step t of output n, joint positions read from x sequence xn (and dL/dx added to its row when p.gx is
+// set); xn = n but with VR_FLAG_VIEWS.
+__device__ __forceinline__ void synth_adjoint_step(const BwdParams& p, long long n, long long xn, int t, float lam, float lam_rcp,
                                                    float Lx, float Ly, float Lz,
                                                    double& g_lam, double& g_lx, double& g_ly, double& g_lz) {
     const int T = (int)p.T;
     const long long idx = n * T + t;
     const double gI = (double)__ldg(p.gz + idx * 2), gQ = (double)__ldg(p.gz + idx * 2 + 1);
     if (gI == 0.0 && gQ == 0.0) return;
-    const float* x0 = p.x + (n * 3 * T + t) * (long long)p.VM;       // x-plane row of this time step
+    const float* x0 = p.x + (xn * 3 * T + t) * (long long)p.VM;      // x-plane row of this time step
     const long long ps = (long long)T * p.VM;                         // floats between coordinate planes
     const int M = p.M;
     auto pos = [&](int v, int m, int c) { return __ldg(x0 + v * M + m + c * ps); };
-    float* gx0 = p.gx ? p.gx + (n * 3 * T + t) * (long long)p.VM : nullptr;   // this thread's own rows of dL/dx
+    float* gx0 = p.gx ? p.gx + (xn * 3 * T + t) * (long long)p.VM : nullptr;  // this thread's own rows of dL/dx
     for (int m = 0; m < p.M; ++m)
         synth_adjoint_body(p, pos, m, gI, gQ, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz, gx0, ps);
 }
 
-// The same at up-sampled step i of sequence n (T = ups_K * ups_T): the joint positions come from the per-interval cubics
-// (pf_locate + pf_eval on p.coef), bit-identical to what vr_pad_frames_f32 writes.  Parameter gradients only.
-__device__ __forceinline__ void synth_adjoint_ups_step(const BwdParams& p, long long n, long long i, float lam, float lam_rcp,
+// The same at up-sampled step i of output n (T = ups_K * ups_T): the joint positions come from the per-interval cubics of
+// raw sequence xn (pf_locate + pf_eval on p.coef), bit-identical to what vr_pad_frames_f32 writes.  Parameter gradients only.
+__device__ __forceinline__ void synth_adjoint_ups_step(const BwdParams& p, long long n, long long xn, long long i, float lam,
+                                                       float lam_rcp,
                                                        float Lx, float Ly, float Lz,
                                                        double& g_lam, double& g_lx, double& g_ly, double& g_lz) {
     const long long idx = n * p.T + i;
@@ -416,7 +420,7 @@ __device__ __forceinline__ void synth_adjoint_ups_step(const BwdParams& p, long 
     int j;
     double tt;
     pf_locate(i, p.ups_ratio, p.ups_T, j, tt);
-    const double* cf = p.coef + ((size_t)n * (p.ups_T - 1) + j) * 4 * C3;   // a0..a3 of interval j, C3 apart
+    const double* cf = p.coef + ((size_t)xn * (p.ups_T - 1) + j) * 4 * C3;  // a0..a3 of interval j, C3 apart
     const int M = p.M, VM = p.VM;
     auto pos = [&](int v, int m, int c) {
         const double* a = cf + c * VM + v * M + m;
@@ -435,7 +439,7 @@ __global__ void __launch_bounds__(128) vr_synth_adjoint_kernel(const __grid_cons
     double g_lam = 0.0, g_lx = 0.0, g_ly = 0.0, g_lz = 0.0;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
         const long long n = idx / T;
-        synth_adjoint_step(p, n, (int)(idx - n * T), lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz);
+        synth_adjoint_step(p, n, n, (int)(idx - n * T), lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz);
     }
     synth_adjoint_reduce(p, g_lam, g_lx, g_ly, g_lz);
 }
@@ -452,43 +456,60 @@ __global__ void __launch_bounds__(128) vr_synth_adjoint_ups_kernel(const __grid_
     double g_lam = 0.0, g_lx = 0.0, g_ly = 0.0, g_lz = 0.0;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
         const long long n = idx / KT;
-        synth_adjoint_ups_step(p, n, idx - n * KT, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz);
+        synth_adjoint_ups_step(p, n, n, idx - n * KT, lam, lam_rcp, Lx, Ly, Lz, g_lam, g_lx, g_ly, g_lz);
     }
     synth_adjoint_reduce(p, g_lam, g_lx, g_ly, g_lz);
 }
 
 // ---- per-sequence parameter gradients (VR_FLAG_PER_SEQUENCE) ----------------------------------------------------------
-// Sequence n reads placement n.  Its steps are cut into PS_SEG-step segments; one warp at a time owns a (sequence,
+// Output n reads placement n.  Its steps are cut into PS_SEG-step segments; one warp at a time owns an (x sequence,
 // segment) unit, lane k runs the per-step adjoint above for step k of the segment, the warp adds the four gradients with a
 // fixed butterfly of shuffles and lane 0 stores the unit's 4 partials (p.part, the scratch tail of the caller's gradient
-// buffer).  vr_param_fold_kernel then adds each sequence's partials in segment order into gparams[4 n ..].  The cut depends
-// on T alone and every sum runs in a fixed order, so a sequence's gradients are the same bits wherever it sits in the
+// buffer).  vr_param_fold_kernel then adds each output's partials in segment order into gparams[4 n ..].  The cut depends
+// on T alone and every sum runs in a fixed order, so an output's gradients are the same bits wherever it sits in the
 // batch, whatever the batch size, grid or SM count.  No atomics, no counters.  (A block of 128 threads per 256-step
 // segment, reduced with block_sum4, measured 1.19x the scalar path's forward + backward step at T = 300, N = 256 and 4096,
 // on a B200, against 1.01-1.02x for a warp per 32 steps: 300 = 256 + 44 steps, and the second segment leaves 84 of the 128
 // threads idle, where a warp per 32 steps idles at most 31 lanes per sequence; profiles/r03d_rejected_variants.md.)
-template <bool UPS>
+// VIEWS (VR_FLAG_VIEWS(R), R = p.views > 1 views per x sequence) selects how the views are spread:
+//   VIEWS_ROWS (dL/dx wanted): the unit is (x sequence xn, segment) and its warp runs the R views r = 0 .. R-1 in order, each
+//     with output xn R + r's dL/d(iq) row and placement on the positions of x sequence xn.  Lane k owns the dL/dx row of
+//     (xn, step k) and adds the views' contributions to it in view order: one owner per row, no atomics.
+//   VIEWS_OUTPUTS (parameter gradients only): the unit is (output n, segment), as without views, reading x sequence n / R;
+//     R times the units of VIEWS_ROWS, and no serial view loop.
+// Either way each view's partials go where the repeated batch's unit of that output would put them, so the parameter
+// gradients are its bits.  VIEWS_NONE is the plain per-sequence kernel, operation for operation (the same SASS as before
+// views existed): the view loop keeps its index and placement live and costs registers (128 / 48 against 122 / 40
+// without UPS), which R = 1 has no use for.
+constexpr int VIEWS_NONE = 0, VIEWS_OUTPUTS = 1, VIEWS_ROWS = 2;
+template <bool UPS, int VIEWS>
 __global__ void __launch_bounds__(128) vr_synth_adjoint_ps_kernel(const __grid_constant__ BwdParams p) {
     const int lane = threadIdx.x & 31;
-    const long long segs = p.ps_segs, units = p.N * segs;
+    const int R = VIEWS == VIEWS_ROWS ? p.views : 1;
+    const long long segs = p.ps_segs, units = (VIEWS == VIEWS_ROWS ? p.N / R : p.N) * segs;
     const long long wstride = (long long)gridDim.x * (blockDim.x >> 5);
     for (long long u = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); u < units; u += wstride) {
-        const long long n = u / segs;
-        const long long t = (u - n * segs) * PS_SEG + lane;
-        const float lam = __ldg(p.lam_ptr + n);
-        const float Lx = __ldg(p.loc_ptr + 3 * n), Ly = __ldg(p.loc_ptr + 3 * n + 1), Lz = __ldg(p.loc_ptr + 3 * n + 2);
-        const float lam_rcp = rcp_refined(lam);
-        double g[4] = {0.0, 0.0, 0.0, 0.0};
-        if (t < p.T) {
-            if (UPS) synth_adjoint_ups_step(p, n, t, lam, lam_rcp, Lx, Ly, Lz, g[0], g[1], g[2], g[3]);
-            else synth_adjoint_step(p, n, (int)t, lam, lam_rcp, Lx, Ly, Lz, g[0], g[1], g[2], g[3]);
-        }
+        const long long un = u / segs;                   // VIEWS_ROWS: the x sequence; otherwise the output
+        const long long s = u - un * segs;
+        const long long t = s * PS_SEG + lane;
+        for (int r = 0; r < R; ++r) {
+            const long long n = VIEWS == VIEWS_ROWS ? un * R + r : un;
+            const long long xn = VIEWS == VIEWS_OUTPUTS ? n / p.views : un;
+            const float lam = __ldg(p.lam_ptr + n);
+            const float Lx = __ldg(p.loc_ptr + 3 * n), Ly = __ldg(p.loc_ptr + 3 * n + 1), Lz = __ldg(p.loc_ptr + 3 * n + 2);
+            const float lam_rcp = rcp_refined(lam);
+            double g[4] = {0.0, 0.0, 0.0, 0.0};
+            if (t < p.T) {
+                if (UPS) synth_adjoint_ups_step(p, n, xn, t, lam, lam_rcp, Lx, Ly, Lz, g[0], g[1], g[2], g[3]);
+                else synth_adjoint_step(p, n, xn, (int)t, lam, lam_rcp, Lx, Ly, Lz, g[0], g[1], g[2], g[3]);
+            }
 #pragma unroll
-        for (int i = 0; i < 4; ++i)
-            for (int o = 16; o > 0; o >>= 1) g[i] += __shfl_xor_sync(0xffffffffu, g[i], o);
-        if (lane == 0) {
-            double* q = p.part + u * 4;
-            q[0] = g[0]; q[1] = g[1]; q[2] = g[2]; q[3] = g[3];
+            for (int i = 0; i < 4; ++i)
+                for (int o = 16; o > 0; o >>= 1) g[i] += __shfl_xor_sync(0xffffffffu, g[i], o);
+            if (lane == 0) {
+                double* q = p.part + (VIEWS == VIEWS_ROWS ? n * segs + s : u) * 4;
+                q[0] = g[0]; q[1] = g[1]; q[2] = g[2]; q[3] = g[3];
+            }
         }
     }
 }

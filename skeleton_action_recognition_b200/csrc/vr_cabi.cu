@@ -365,6 +365,17 @@ struct DeviceInfo {
 std::mutex g_mu;
 DeviceInfo g_dev[64];
 
+// VR_FLAG_VIEWS: R radars per x sequence (R = 1 without the field).  Valid only with VR_FLAG_PER_SEQUENCE (every view has
+// its own placement), and N -- the outputs -- must be a multiple of R.  Host-side, before anything touches the device.
+int views_of(uint32_t flags, int64_t N, int& R) {
+    R = (int)((flags & VR_FLAG_VIEWS_MASK) >> VR_FLAG_VIEWS_SHIFT);
+    if (R == 0) { R = 1; return VR_OK; }
+    if (!(flags & VR_FLAG_PER_SEQUENCE))
+        return fail(VR_ERR_ARG, "VR_FLAG_VIEWS(%d) needs VR_FLAG_PER_SEQUENCE: each view has its own placement", R);
+    if (N % R != 0) return fail(VR_ERR_SHAPE, "N=%lld outputs is not a multiple of the %d views per sequence", (long long)N, R);
+    return VR_OK;
+}
+
 int device_setup(int& dev, int& sm_count) {
     CUDA_TRY(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64) return fail(VR_ERR_CUDA, "device index %d out of range", dev);
@@ -458,10 +469,14 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
     const bool iq_only = out == nullptr;
     if (!x || (!out && !iq)) return fail(VR_ERR_ARG, "x and out (or iq) must not be null");
     if ((lam_dev == nullptr) != (loc_dev == nullptr)) return fail(VR_ERR_ARG, "wavelength and radar_location must both be device pointers or both be null");
-    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_INPUTS_READY | VR_FLAG_PER_SEQUENCE)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
+    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_INPUTS_READY | VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK))
+        return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
     const bool per_seq = (flags & VR_FLAG_PER_SEQUENCE) != 0;   // (the entries reject it with host parameters or null pointers)
+    int views;
+    int rc = views_of(flags, N, views);
+    if (rc) return rc;
     int dev, sm_count;
-    int rc = device_setup(dev, sm_count);
+    rc = device_setup(dev, sm_count);
     if (rc) return rc;
     vr::Params p;
     int grid, cps;
@@ -485,6 +500,7 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
     }
     const int job_slots = team ? grid * vr::TJ_TEAMS : grid;
     p.x = x; p.out = out; p.iq = iq; p.tl = g_timeline;
+    p.views = views;
     p.ticket = (g_dynamic && p.n_jobs > job_slots) ? next_ticket_slot(dev) : nullptr;
     p.early_reads = (g_pdl && !coef && (flags & VR_FLAG_INPUTS_READY)) ? 1 : 0;   // coef is written by the launch just before
     p.coef = coef; p.ups_T = ups_T; p.ups_K = ups_K;
@@ -608,8 +624,9 @@ int vr_forward_host_f32(const float* x_host, int64_t N, int64_t T, int32_t V, in
                         float wavelength, const float* radar_loc_host,
                         int32_t n_fft, int32_t hop, uint32_t flags, float* out_host, int64_t sub_batch) {
     if (!x_host || !out_host || !radar_loc_host) return fail(VR_ERR_ARG, "host pointers must not be null");
-    if (flags & VR_FLAG_PER_SEQUENCE)
-        return fail(VR_ERR_ARG, "vr_forward_host_f32 takes one host placement for the batch; VR_FLAG_PER_SEQUENCE needs a device-pointer entry point");
+    if (flags & (VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK))
+        return fail(VR_ERR_ARG, "vr_forward_host_f32 takes one host placement for the batch; VR_FLAG_PER_SEQUENCE and "
+                                "VR_FLAG_VIEWS need a device-pointer entry point");
     if (N <= 0 || T <= 0 || V <= 0 || M <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M, hop must be positive");
     int dev, sm_count;
     int rc = device_setup(dev, sm_count);
@@ -873,12 +890,16 @@ int upsampled_impl(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t 
     if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames (scipy interp1d raises ValueError)", (long long)T);
     if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
     if ((double)T * num_pad_frames > (double)(1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
-    if (workspace_bytes < vr_upsampled_workspace_bytes(N, T, V, M))
+    int views;                                            // VR_FLAG_VIEWS: the spline of the N / R raw sequences, once
+    int rc = views_of(flags, N, views);
+    if (rc) return rc;
+    const int64_t Nx = N / views;
+    if (workspace_bytes < vr_upsampled_workspace_bytes(Nx, T, V, M))
         return fail(VR_ERR_ARG, "workspace of %lld bytes is smaller than vr_upsampled_workspace_bytes = %lld",
-                    (long long)workspace_bytes, (long long)vr_upsampled_workspace_bytes(N, T, V, M));
+                    (long long)workspace_bytes, (long long)vr_upsampled_workspace_bytes(Nx, T, V, M));
     if (((uintptr_t)workspace_dev & 7) != 0) return fail(VR_ERR_ARG, "workspace_dev must be 8-byte aligned");
     double* coef = static_cast<double*>(workspace_dev);
-    int rc = pad_launch(x_dev, N, T, V, M, num_pad_frames, sigma, nullptr, coef, stream);
+    rc = pad_launch(x_dev, Nx, T, V, M, num_pad_frames, sigma, nullptr, coef, stream);
     if (rc) return rc;
     return launch(x_dev, N, T * num_pad_frames, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
                   n_fft, hop, flags, image_size, out_dev, iq_dev, (cudaStream_t)stream, coef, (int)T, num_pad_frames);
@@ -995,8 +1016,11 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     // the up-sampling spline's (T = ups_K * ups_T steps, x_dev unused), parameter gradients only
     if ((!x_dev && !coef) || !gz_work_dev || !grad_params_dev || !wavelength_dev || !radar_loc_dev || (!synth_only && (!iq_dev || !grad_out_dev)))
         return fail(VR_ERR_ARG, "device pointers must not be null");
-    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_PER_SEQUENCE)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
+    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
     const bool per_seq = (flags & VR_FLAG_PER_SEQUENCE) != 0;
+    int views;                                          // VR_FLAG_VIEWS: x (and coef) hold N / views sequences
+    int rc = views_of(flags, N, views);
+    if (rc) return rc;
     if (per_seq && ((uintptr_t)grad_params_dev & 7) != 0)
         return fail(VR_ERR_ARG, "grad_params_dev must be 8-byte aligned (float64 per-sequence gradients)");
     if (N <= 0 || T <= 0 || V <= 0 || M <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M, hop must be positive");
@@ -1007,7 +1031,7 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     if (E <= 0 || E > vr::NG * vr::MAX_EG) return fail(VR_ERR_UNSUPPORTED, "E=%d outside [1, %d]", E, vr::NG * vr::MAX_EG);
     if (V > 65535) return fail(VR_ERR_UNSUPPORTED, "V=%d too large", V);
     int dev, sm_count;
-    int rc = device_setup(dev, sm_count);
+    rc = device_setup(dev, sm_count);
     if (rc) return rc;
     vr::BwdParams p;
     memset(&p, 0, sizeof(p));
@@ -1024,8 +1048,9 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     p.inv_E = 1.0f / (float)E;
     p.coef = coef; p.ups_T = ups_T;
     p.ups_ratio = coef ? (double)(ups_T - 1) / (double)((long long)ups_K * ups_T - 1) : 0.0;
+    p.views = views;
     cudaStream_t st = (cudaStream_t)stream;
-    if (grad_x_dev) CUDA_TRY(cudaMemsetAsync(grad_x_dev, 0, (size_t)N * 3 * T * V * M * sizeof(float), st));
+    if (grad_x_dev) CUDA_TRY(cudaMemsetAsync(grad_x_dev, 0, (size_t)(N / views) * 3 * T * V * M * sizeof(float), st));
     if (!synth_only) {                                  // writes every sample of gz: no zero fill
         vr::adjoint_plan(N, T, sm_count, p.seg_len, p.segs);
         const int grid1 = (int)std::min<long long>(N * p.segs, (long long)sm_count * 8);
@@ -1033,13 +1058,25 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
         CUDA_TRY(cudaGetLastError());
     }
     if (per_seq) {
-        // per-sequence gradients: (sequence, segment) units reduced block by block into the scratch tail of
-        // grad_params_dev (vr_per_sequence_grad_doubles), then folded per sequence in segment order
+        // per-sequence gradients: (x sequence, segment) units, each running its views, reduced warp by warp into the scratch
+        // tail of grad_params_dev (vr_per_sequence_grad_doubles), then folded per output in segment order
         p.ps_segs = vr::ps_segments(T);
         p.part = grad_params_dev + 4 * N;
-        const int grid2 = (int)std::min<long long>((N * p.ps_segs + 3) / 4, (long long)sm_count * 16);   // 4 warps per block
-        if (coef) vr::vr_synth_adjoint_ps_kernel<true><<<grid2, 128, 0, st>>>(p);
-        else vr::vr_synth_adjoint_ps_kernel<false><<<grid2, 128, 0, st>>>(p);
+        // views: with dL/dx one warp runs a row's views in order (one owner per dL/dx row); without it the units are per
+        // output, as without views, for R times the parallelism.  R = 1: the plain per-sequence kernel
+        const int mode = views == 1 ? vr::VIEWS_NONE : grad_x_dev ? vr::VIEWS_ROWS : vr::VIEWS_OUTPUTS;
+        const long long units = (mode == vr::VIEWS_ROWS ? N / views : N) * p.ps_segs;
+        const int grid2 = (int)std::min<long long>((units + 3) / 4, (long long)sm_count * 16);   // 4 warps per block
+        if (mode == vr::VIEWS_ROWS) {
+            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_ROWS><<<grid2, 128, 0, st>>>(p);
+            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_ROWS><<<grid2, 128, 0, st>>>(p);
+        } else if (mode == vr::VIEWS_OUTPUTS) {
+            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_OUTPUTS><<<grid2, 128, 0, st>>>(p);
+            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_OUTPUTS><<<grid2, 128, 0, st>>>(p);
+        } else {
+            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_NONE><<<grid2, 128, 0, st>>>(p);
+            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_NONE><<<grid2, 128, 0, st>>>(p);
+        }
         CUDA_TRY(cudaGetLastError());
         vr::vr_param_fold_kernel<<<(unsigned)((4 * N + 127) / 128), 128, 0, st>>>(p.part, grad_params_dev, N, p.ps_segs);
         CUDA_TRY(cudaGetLastError());

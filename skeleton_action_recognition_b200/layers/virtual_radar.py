@@ -193,7 +193,8 @@ class _RadarFunction(torch.autograd.Function):
     def backward(ctx, grad_out):
         lam, loc, xc, iq = ctx.saved_tensors
         layer = ctx.layer
-        N, _, T, V, M = xc.shape
+        _, _, T, V, M = xc.shape
+        N = xc.shape[0] * _cabi.views_of(ctx.flags)        # outputs: R views of each x sequence (VR_FLAG_VIEWS)
         g = grad_out.contiguous().to(torch.float32)
         gz = torch.empty((N, T, 2), dtype=torch.float32, device=xc.device)
         gp = _param_grad_buffer(ctx.flags, N, T, xc.device)
@@ -226,7 +227,8 @@ class _SynthFunction(torch.autograd.Function):
     def backward(ctx, grad_iq):
         lam, loc, xc = ctx.saved_tensors
         layer = ctx.layer
-        N, _, T, V, M = xc.shape
+        _, _, T, V, M = xc.shape
+        N = xc.shape[0] * _cabi.views_of(ctx.flags)
         g = grad_iq.contiguous().to(torch.float32)
         gp = _param_grad_buffer(ctx.flags, N, T, xc.device)
         gx = torch.empty_like(xc) if ctx.needs_input_grad[2] else None
@@ -248,9 +250,10 @@ class _UpsampledRadarFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, lam, loc, xc, layer, k, sigma, flags=0):
-        N, _, T, V, M = xc.shape
+        _, _, T, V, M = xc.shape
+        N = xc.shape[0] * _cabi.views_of(flags)             # outputs; the spline is solved once per raw sequence
         L = _cabi.lib()
-        nbytes = int(L.vr_upsampled_workspace_bytes(N, T, V, M))
+        nbytes = int(L.vr_upsampled_workspace_bytes(xc.shape[0], T, V, M))
         work = torch.empty(max(nbytes, 8) // 8, dtype=torch.float64, device=xc.device)
         out = torch.empty((N, layer.n_fft, (k * T) // layer.hop_length + 1), dtype=torch.float32, device=xc.device)
         iq = torch.empty((N, k * T, 2), dtype=torch.float32, device=xc.device)
@@ -294,7 +297,7 @@ class _UpsampledSynthFunction(torch.autograd.Function):
     def forward(ctx, lam, loc, xc, layer, k, sigma, flags=0):
         iq, work = layer._synth_upsampled(xc, k, sigma, lam, loc, flags)
         ctx.save_for_backward(lam, loc, work)
-        ctx.layer, ctx.dims, ctx.flags = layer, tuple(xc.shape) + (k,), flags
+        ctx.layer, ctx.dims, ctx.flags = layer, (iq.shape[0],) + tuple(xc.shape[1:]) + (k,), flags
         return iq
 
     @staticmethod
@@ -425,31 +428,51 @@ class VirtualRadar(torch.nn.Module):
 
     def _placements(self, x, radar_location, wavelength):
         """Per-sequence radar placements (the `radar_location=` / `wavelength=` keywords of forward, forward_image and
-        forward_upsampled) -> None when neither is given, else (wavelength (N,), radar_location (N, 3)): each keyword
-        expanded to the batch and made contiguous, the module parameter standing in for a keyword not given.  Autograd's
-        expand carries the per-sequence gradients back to whatever the caller passed (summed where it broadcast)."""
+        forward_upsampled) -> None when neither is given, else (wavelength (N,), radar_location (N, 3), flags): each
+        keyword expanded to the batch and made contiguous, the module parameter standing in for a keyword not given.
+        Autograd's expand carries the per-sequence gradients back to whatever the caller passed (summed where it
+        broadcast).  flags: what the launch adds (VR_FLAG_PER_SEQUENCE)."""
         if radar_location is None and wavelength is None:
             return None
         N = x.shape[0]
-        out = []
-        for name, value, param, shape in (("wavelength", wavelength, self.wavelength, (N,)),
-                                          ("radar_location", radar_location, self.radar_location, (N, 3))):
-            if value is None:
-                value = param
-            elif not isinstance(value, torch.Tensor) or value.dtype != torch.float32:
-                raise ValueError("%s must be a float32 tensor that broadcasts to %s, got %s"
-                                 % (name, shape, value.dtype if isinstance(value, torch.Tensor) else type(value)))
-            elif not value.is_cuda or value.device != x.device:
-                raise RuntimeError("%s is on %s but x is on %s: per-sequence placements are read on x's device"
-                                   % (name, value.device, x.device))
-            if tuple(value.shape) != shape or not value.is_contiguous():   # (a full contiguous tensor is used as it is)
-                try:
-                    value = value.expand(shape)
-                except RuntimeError:
-                    raise ValueError("%s of shape %s does not broadcast to %s" % (name, tuple(value.shape), shape)) from None
-                value = value.contiguous()
-            out.append(value)
-        return tuple(out)
+        lam = self._expand_placement(x, "wavelength", wavelength, self.wavelength, (N,))
+        loc = self._expand_placement(x, "radar_location", radar_location, self.radar_location, (N, 3))
+        return lam, loc, _cabi.VR_FLAG_PER_SEQUENCE
+
+    def _view_placements(self, x, radar_location, wavelength):
+        """The placements of forward_views -> (wavelength (N R,), radar_location (N R, 3), flags): R from radar_location's
+        second-to-last dimension, each keyword expanded to (N, R[, 3]) and flattened view-minor (output n R + r is view r
+        of sequence n), the module's wavelength standing in for `wavelength=None`.  flags: VR_FLAG_PER_SEQUENCE |
+        VR_FLAG_VIEWS(R)."""
+        if not isinstance(radar_location, torch.Tensor) or radar_location.dim() < 2:
+            raise ValueError("radar_location must be a tensor of R placements, (R, 3) for every sequence or (N, R, 3), got %s"
+                             % (tuple(radar_location.shape) if isinstance(radar_location, torch.Tensor) else type(radar_location),))
+        N, R = x.shape[0], radar_location.shape[-2]
+        if not 1 <= R <= 255:
+            raise ValueError("forward_views takes 1 to 255 views per sequence, got R=%d (radar_location of shape %s)"
+                             % (R, tuple(radar_location.shape)))
+        lam = self._expand_placement(x, "wavelength", wavelength, self.wavelength, (N, R))
+        loc = self._expand_placement(x, "radar_location", radar_location, self.radar_location, (N, R, 3))
+        return lam.reshape(N * R), loc.reshape(N * R, 3), _cabi.VR_FLAG_PER_SEQUENCE | _cabi.views_flag(R)
+
+    @staticmethod
+    def _expand_placement(x, name, value, param, shape):
+        """One placement keyword checked (float32, on x's device) and expanded to `shape`, contiguous; `param` if None."""
+        if value is None:
+            value = param
+        elif not isinstance(value, torch.Tensor) or value.dtype != torch.float32:
+            raise ValueError("%s must be a float32 tensor that broadcasts to %s, got %s"
+                             % (name, shape, value.dtype if isinstance(value, torch.Tensor) else type(value)))
+        elif not value.is_cuda or value.device != x.device:
+            raise RuntimeError("%s is on %s but x is on %s: per-sequence placements are read on x's device"
+                               % (name, value.device, x.device))
+        if tuple(value.shape) != shape or not value.is_contiguous():   # (a full contiguous tensor is used as it is)
+            try:
+                value = value.expand(shape)
+            except RuntimeError:
+                raise ValueError("%s of shape %s does not broadcast to %s" % (name, tuple(value.shape), shape)) from None
+            value = value.contiguous()
+        return value
 
     def _prepare(self, x):
         """Pick the range rounding mode from the caller's strides BEFORE normalising the layout
@@ -461,8 +484,9 @@ class VirtualRadar(torch.nn.Module):
 
     def _launch(self, xc, flags, want_iq=False, lam=None, loc=None):
         """One fused launch.  lam / loc: the radar parameters to read (default: the module's; (N,) and (N, 3) with
-        VR_FLAG_PER_SEQUENCE in flags)."""
-        N, _, T, V, M = xc.shape
+        VR_FLAG_PER_SEQUENCE in flags, N = R x the rows of xc with VR_FLAG_VIEWS(R))."""
+        _, _, T, V, M = xc.shape
+        N = xc.shape[0] * _cabi.views_of(flags)
         lam = self.wavelength if lam is None else lam
         loc = self.radar_location if loc is None else loc
         n_fft = self._FUSED_N_FFT if want_iq else self.n_fft       # iq does not depend on the STFT parameters
@@ -490,7 +514,8 @@ class VirtualRadar(torch.nn.Module):
     def _synth(self, xc, flags, lam=None, loc=None):
         """Synthesis only (C ABI vr_synth_f32): the complex baseband signal (N,T,2) that the general-kernel STFT reads,
         bit for bit forward_debug's, without any STFT work."""
-        N, _, T, V, M = xc.shape
+        _, _, T, V, M = xc.shape
+        N = xc.shape[0] * _cabi.views_of(flags)
         lam = self.wavelength if lam is None else lam
         loc = self.radar_location if loc is None else loc
         if self.assume_inputs_ready:
@@ -515,11 +540,12 @@ class VirtualRadar(torch.nn.Module):
         """Synthesis of pad_frames(xc, k, sigma) without the up-sampled batch (C ABI vr_synth_upsampled_f32) -> iq
         (N, k*T, 2) and the workspace holding the spline's cubics.  The up-sampled tensor the reference's loader builds
         is standard-contiguous: range rounding mode "seq" (no VR_FLAG_RANGE_FMA)."""
-        N, _, T, V, M = xc.shape
+        _, _, T, V, M = xc.shape
+        N = xc.shape[0] * _cabi.views_of(flags)
         lam = self.wavelength if lam is None else lam
         loc = self.radar_location if loc is None else loc
         L = _cabi.lib()
-        nbytes = int(L.vr_upsampled_workspace_bytes(N, T, V, M))
+        nbytes = int(L.vr_upsampled_workspace_bytes(xc.shape[0], T, V, M))
         work = torch.empty(max(nbytes, 8) // 8, dtype=torch.float64, device=xc.device)
         iq = torch.empty((N, k * T, 2), dtype=torch.float32, device=xc.device)
         if N == 0:
@@ -567,11 +593,11 @@ class VirtualRadar(torch.nn.Module):
 
     def _run(self, x, xc, flags, pl=None):
         """forward() after the layout has been normalised: xc standard-contiguous, flags carry the range rounding mode;
-        pl: per-sequence placements (_placements) or None."""
+        pl: per-sequence placements (_placements, _view_placements) or None."""
         lam, loc = self.wavelength, self.radar_location
         if pl is not None:
-            lam, loc = pl
-            flags |= _cabi.VR_FLAG_PER_SEQUENCE
+            lam, loc, pflags = pl
+            flags |= pflags
         if self._general_stft():     # trained / trainable STFT kernels: synthesis on our kernels, STFT as a GEMM
             self._check_general_length(xc.shape[2])
             if xc.shape[0] == 0:
@@ -584,8 +610,8 @@ class VirtualRadar(torch.nn.Module):
     def _general_iq(self, x, xc, flags, pl=None):
         lam, loc = self.wavelength, self.radar_location
         if pl is not None:
-            lam, loc = pl
-            flags |= _cabi.VR_FLAG_PER_SEQUENCE
+            lam, loc, pflags = pl
+            flags |= pflags
         return _SynthFunction.apply(lam, loc, xc, self, flags) if self._needs_grad(x, pl) else self._synth(xc, flags, lam, loc)
 
     def forward_notebook(self, data, num_pad_frames=1, sigma=3):
@@ -610,8 +636,12 @@ class VirtualRadar(torch.nn.Module):
         that writes (N, 1, image_size, image_size) directly and transforms only the frames the
         resize keeps.  `radar_location` / `wavelength`: per-sequence placements, as in forward()."""
         self._check_input(x)
-        lam, loc = self._check_device(x)
-        pl = self._placements(x, radar_location, wavelength)
+        self._check_device(x)
+        return self._image(x, image_size, self._placements(x, radar_location, wavelength))
+
+    def _image(self, x, image_size, pl):
+        """forward_image after the input checks; pl: placements (_placements, _view_placements) or None."""
+        lam, loc = self.wavelength, self.radar_location
         image_size = int(image_size)
         if image_size < 1:
             raise ValueError("image_size must be positive, got %d" % image_size)
@@ -624,11 +654,12 @@ class VirtualRadar(torch.nn.Module):
             return torch.nn.functional.interpolate(spec.unsqueeze(1), image_size)
         xc, flags = self._prepare(x)
         if pl is not None:
-            lam, loc = pl
-            flags |= _cabi.VR_FLAG_PER_SEQUENCE
+            lam, loc, pflags = pl
+            flags |= pflags
         if self.assume_inputs_ready:
             flags |= _cabi.VR_FLAG_INPUTS_READY
-        N, _, T, V, M = xc.shape
+        _, _, T, V, M = xc.shape
+        N = xc.shape[0] * _cabi.views_of(flags)
         out = torch.empty((N, 1, image_size, image_size), dtype=torch.float32, device=x.device)
         if N == 0:
             return out
@@ -652,14 +683,18 @@ class VirtualRadar(torch.nn.Module):
         with respect to x itself go through `self(pad_frames(x, num_pad_frames, sigma))`.  `radar_location` /
         `wavelength`: per-sequence placements, as in forward()."""
         self._check_input(x)
-        lam, loc = self._check_device(x)
-        pl = self._placements(x, radar_location, wavelength)
+        self._check_device(x)
+        return self._upsampled(x, num_pad_frames, sigma, image_size, self._placements(x, radar_location, wavelength))
+
+    def _upsampled(self, x, num_pad_frames, sigma, image_size, pl):
+        """forward_upsampled after the input checks; pl: placements (_placements, _view_placements) or None."""
+        lam, loc = self.wavelength, self.radar_location
         flags = 0
         if pl is not None:
-            lam, loc = pl
-            flags = _cabi.VR_FLAG_PER_SEQUENCE
+            lam, loc, flags = pl
         xc = x.contiguous()
-        N, _, T, V, M = xc.shape
+        _, _, T, V, M = xc.shape
+        Nx, N = xc.shape[0], xc.shape[0] * _cabi.views_of(flags)     # raw sequences, outputs
         k = int(num_pad_frames)
         img = 0 if image_size is None else int(image_size)
         if image_size is not None and img < 1:
@@ -682,7 +717,7 @@ class VirtualRadar(torch.nn.Module):
         if N == 0:
             return out
         L = _cabi.lib()
-        nbytes = int(L.vr_upsampled_workspace_bytes(N, T, V, M))
+        nbytes = int(L.vr_upsampled_workspace_bytes(Nx, T, V, M))
         work = torch.empty(max(nbytes, 8) // 8, dtype=torch.float64, device=x.device)
         with torch.cuda.device(x.device):
             stream = torch.cuda.current_stream(x.device).cuda_stream
@@ -693,6 +728,33 @@ class VirtualRadar(torch.nn.Module):
                                             out.data_ptr(), ctypes.c_void_p(stream))
         _cabi.check(rc)
         return out
+
+    def forward_views(self, x, radar_location, wavelength=None, image_size=None, num_pad_frames=None, sigma=3):
+        """R radar views of every sequence in one launch from one copy of x (C ABI VR_FLAG_VIEWS(R)): a
+        multistatic array, a set of viewpoints for augmentation, one scene in several bands.  x (N,3,T,V,M);
+        `radar_location` float32 (R, 3), the same R placements for every sequence, or (N, R, 3); `wavelength` None (the
+        module parameter), 0-d, (R,) or (N, R).  -> (N, R, n_fft, T//hop+1), or (N, R, image_size, image_size) with
+        `image_size` (the forward_image fusion).  With `num_pad_frames` x is the RAW batch, up-sampled on the device as in
+        forward_upsampled (its spline solved once per sequence, not once per view).  Bit for bit
+
+            forward(x.repeat_interleave(R, 0), radar_location=loc.expand(N, R, 3).reshape(N*R, 3),
+                    wavelength=lam.expand(N, R).reshape(N*R)).view(N, R, ...)
+
+        (and likewise forward_image / forward_upsampled), without the R-times repeated batch.  Differentiable: the
+        placement gradients reach the tensors passed and are the repeated route's bits; dL/dx adds the R views'
+        contributions in view order, in float32, inside the kernel (deterministic; not the bits of autograd's
+        repeat_interleave backward for R > 1).  As in forward_upsampled, `num_pad_frames` has no gradient with respect to
+        x.  Under torch.nn.DataParallel pass full (N, R, 3) / (N, R) tensors, for the reason forward() gives."""
+        self._check_input(x)
+        self._check_device(x)
+        pl = self._view_placements(x, radar_location, wavelength)
+        if num_pad_frames is not None:
+            out = self._upsampled(x, num_pad_frames, sigma, image_size, pl)
+        elif image_size is not None:
+            out = self._image(x, image_size, pl)
+        else:
+            out = self._run(x, *self._prepare(x), pl)
+        return out.reshape(x.shape[0], _cabi.views_of(pl[2]), *out.shape[-2:])
 
     def forward_debug(self, x):
         """forward plus the intermediate complex baseband signal (N,T,2); for stage-level parity tests."""
