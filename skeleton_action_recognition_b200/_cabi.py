@@ -11,6 +11,7 @@ VR_OK, VR_ERR_ARG, VR_ERR_SHAPE, VR_ERR_UNSUPPORTED, VR_ERR_CUDA = 0, -1, -2, -3
 VR_FLAG_RANGE_FMA = 1
 VR_FLAG_INPUTS_READY = 2
 VR_FLAG_PER_SEQUENCE = 4
+VR_FLAG_NOISE = 8               # receiver noise from vr_set_noise (with VR_FLAG_PER_SEQUENCE); never passed to a backward entry
 VR_FLAG_VIEWS_SHIFT = 8         # VR_FLAG_VIEWS(R) = R << 8, R in [1, 255]: R radars per sequence (with VR_FLAG_PER_SEQUENCE)
 VR_FLAG_VIEWS_MASK = 0xff << VR_FLAG_VIEWS_SHIFT
 ABI_VERSION = 1
@@ -25,7 +26,8 @@ SYMBOLS = ("vr_abi_version", "vr_last_error", "vr_forward_f32", "vr_forward_debu
            "vr_stft_general_workspace_floats", "vr_stft_general_f32", "vr_stft_general_backward_f32",
            "vr_synth_f32", "vr_synth_upsampled_f32", "vr_synth_adjoint_upsampled_f32",
            "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32",
-           "vr_plan_adjoint_stft", "vr_plan_pad_frames", "vr_plan_stft_general", "vr_per_sequence_grad_doubles")
+           "vr_plan_adjoint_stft", "vr_plan_pad_frames", "vr_plan_stft_general", "vr_per_sequence_grad_doubles",
+           "vr_set_noise")
 
 _lib = None
 
@@ -109,6 +111,8 @@ def lib():
     L.vr_plan_stft_general.restype = ctypes.c_int
     L.vr_per_sequence_grad_doubles.argtypes = [i64, i64]
     L.vr_per_sequence_grad_doubles.restype = i64
+    L.vr_set_noise.argtypes = [vp, vp]
+    L.vr_set_noise.restype = ctypes.c_int
     L.vr_set_timeline_buffer.argtypes = [vp]
     L.vr_set_timeline_buffer.restype = ctypes.c_int
     L.vr_selftest_rounding.argtypes = [ctypes.c_uint64, f32, ctypes.POINTER(ctypes.c_uint64)]
@@ -229,6 +233,12 @@ def views_flag(R):
 def views_of(flags):
     """R of the VR_FLAG_VIEWS field of `flags` (1 when the field is 0): outputs per x sequence."""
     return ((int(flags) & VR_FLAG_VIEWS_MASK) >> VR_FLAG_VIEWS_SHIFT) or 1
+
+
+def set_noise(noise_std, seed):
+    """vr_set_noise for the next VR_FLAG_NOISE launch of this thread: noise_std (N,) float32 and seed, a 0-d int64 tensor
+    holding the 64 seed bits, both on the launch's device (contiguous)."""
+    check(lib().vr_set_noise(noise_std.data_ptr(), seed.data_ptr()))
 
 
 def set_schedule(mode):

@@ -376,6 +376,33 @@ int views_of(uint32_t flags, int64_t N, int& R) {
     return VR_OK;
 }
 
+// vr_set_noise's pending setting, consumed by the next entry call of the thread that carries VR_FLAG_NOISE
+struct NoiseSlot {
+    const float* std = nullptr;
+    const uint64_t* seed = nullptr;
+};
+thread_local NoiseSlot t_noise;
+
+// The noise of an entry call: consumes the thread's pending setting when the flags ask for noise (the slot is cleared
+// whether the call then succeeds or fails), nothing otherwise.  Host-side, before anything is enqueued.
+int take_noise(uint32_t flags, vr::NoiseParams& q) {
+    q.std = nullptr; q.seed = nullptr;
+    if (!(flags & VR_FLAG_NOISE)) return VR_OK;
+    const NoiseSlot s = t_noise;
+    t_noise = NoiseSlot{};
+    if (!(flags & VR_FLAG_PER_SEQUENCE))
+        return fail(VR_ERR_ARG, "VR_FLAG_NOISE needs VR_FLAG_PER_SEQUENCE: the noise level is one per output");
+    if (!s.std) return fail(VR_ERR_ARG, "VR_FLAG_NOISE without a pending vr_set_noise on this thread");
+    q.std = s.std; q.seed = reinterpret_cast<const unsigned long long*>(s.seed);
+    return VR_OK;
+}
+
+// The entries that do not take VR_FLAG_NOISE (the host entry, the backward entries) still consume a pending setting when
+// a call carries the flag, before rejecting it, so that a stale setting never reaches a later launch
+void drop_noise(uint32_t flags) {
+    if (flags & VR_FLAG_NOISE) t_noise = NoiseSlot{};
+}
+
 int device_setup(int& dev, int& sm_count) {
     CUDA_TRY(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64) return fail(VR_ERR_CUDA, "device index %d out of range", dev);
@@ -463,14 +490,17 @@ int cached_plan(int64_t N, int64_t T, int V, int M, const int32_t* src, const in
 int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* src, const int32_t* dst, int E,
            const float* lam_dev, const float* loc_dev, float lam_val, const float* loc_val,
            int n_fft, int hop, uint32_t flags, int img, float* out, float* iq, cudaStream_t stream,
-           const double* coef = nullptr, int ups_T = 0, int ups_K = 0) {
+           const double* coef = nullptr, int ups_T = 0, int ups_K = 0, const vr::NoiseParams& noise = vr::NoiseParams{}) {
     // coef != nullptr: fused temporal up-sampling; T is then the UP-SAMPLED length ups_K * ups_T and x is only
-    // used for its alignment (the kernel reads the spline coefficients instead).  out == nullptr: synthesis only (iq)
+    // used for its alignment (the kernel reads the spline coefficients instead).  out == nullptr: synthesis only (iq).
+    // noise: from take_noise (VR_FLAG_NOISE), read by the PS kernels only
     const bool iq_only = out == nullptr;
     if (!x || (!out && !iq)) return fail(VR_ERR_ARG, "x and out (or iq) must not be null");
     if ((lam_dev == nullptr) != (loc_dev == nullptr)) return fail(VR_ERR_ARG, "wavelength and radar_location must both be device pointers or both be null");
-    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_INPUTS_READY | VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK))
+    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_INPUTS_READY | VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK | VR_FLAG_NOISE))
         return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
+    if (((flags & VR_FLAG_NOISE) != 0) != (noise.std != nullptr))
+        return fail(VR_ERR_ARG, "VR_FLAG_NOISE needs a noise setting (vr_set_noise) and a noise setting needs the flag");
     const bool per_seq = (flags & VR_FLAG_PER_SEQUENCE) != 0;   // (the entries reject it with host parameters or null pointers)
     int views;
     int rc = views_of(flags, N, views);
@@ -501,6 +531,7 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
     const int job_slots = team ? grid * vr::TJ_TEAMS : grid;
     p.x = x; p.out = out; p.iq = iq; p.tl = g_timeline;
     p.views = views;
+    p.noise = noise;
     p.ticket = (g_dynamic && p.n_jobs > job_slots) ? next_ticket_slot(dev) : nullptr;
     p.early_reads = (g_pdl && !coef && (flags & VR_FLAG_INPUTS_READY)) ? 1 : 0;   // coef is written by the launch just before
     p.coef = coef; p.ups_T = ups_T; p.ups_K = ups_K;
@@ -554,32 +585,47 @@ int vr_set_schedule(int mode) {
     return VR_OK;
 }
 
+int vr_set_noise(const float* noise_std_dev, const uint64_t* seed_dev) {
+    t_noise = NoiseSlot{};
+    if (!noise_std_dev || !seed_dev) return fail(VR_ERR_ARG, "noise_std_dev and seed_dev must not be null");
+    if (((uintptr_t)noise_std_dev & 3) != 0 || ((uintptr_t)seed_dev & 7) != 0)
+        return fail(VR_ERR_ARG, "noise_std_dev must be 4-byte and seed_dev 8-byte aligned");
+    t_noise.std = noise_std_dev; t_noise.seed = seed_dev;
+    return VR_OK;
+}
+
 int vr_forward_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
                    const int32_t* src_host, const int32_t* dst_host, int32_t E,
                    const float* wavelength_dev, const float* radar_loc_dev,
                    int32_t n_fft, int32_t hop, uint32_t flags, float* out_dev, void* stream) {
+    vr::NoiseParams nz;
+    if (int rc = take_noise(flags, nz)) return rc;
     if (!wavelength_dev || !radar_loc_dev) return fail(VR_ERR_ARG, "wavelength_dev and radar_loc_dev must not be null");
     return launch(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
-                  n_fft, hop, flags, 0, out_dev, nullptr, (cudaStream_t)stream);
+                  n_fft, hop, flags, 0, out_dev, nullptr, (cudaStream_t)stream, nullptr, 0, 0, nz);
 }
 
 int vr_forward_debug_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
                          const int32_t* src_host, const int32_t* dst_host, int32_t E,
                          const float* wavelength_dev, const float* radar_loc_dev,
                          int32_t n_fft, int32_t hop, uint32_t flags, float* out_dev, float* iq_dev, void* stream) {
+    vr::NoiseParams nz;
+    if (int rc = take_noise(flags, nz)) return rc;
     if (!wavelength_dev || !radar_loc_dev) return fail(VR_ERR_ARG, "wavelength_dev and radar_loc_dev must not be null");
     if (!iq_dev) return fail(VR_ERR_ARG, "iq_dev must not be null");
     return launch(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
-                  n_fft, hop, flags, 0, out_dev, iq_dev, (cudaStream_t)stream);
+                  n_fft, hop, flags, 0, out_dev, iq_dev, (cudaStream_t)stream, nullptr, 0, 0, nz);
 }
 
 int vr_synth_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
                  const int32_t* src_host, const int32_t* dst_host, int32_t E,
                  const float* wavelength_dev, const float* radar_loc_dev, uint32_t flags, float* iq_dev, void* stream) {
+    vr::NoiseParams nz;
+    if (int rc = take_noise(flags, nz)) return rc;
     if (!wavelength_dev || !radar_loc_dev) return fail(VR_ERR_ARG, "wavelength_dev and radar_loc_dev must not be null");
     if (!iq_dev) return fail(VR_ERR_ARG, "iq_dev must not be null");
     return launch(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
-                  vr::NFFT, 1, flags, 0, nullptr, iq_dev, (cudaStream_t)stream);
+                  vr::NFFT, 1, flags, 0, nullptr, iq_dev, (cudaStream_t)stream, nullptr, 0, 0, nz);
 }
 
 int vr_forward_image_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
@@ -587,10 +633,12 @@ int vr_forward_image_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, in
                          const float* wavelength_dev, const float* radar_loc_dev,
                          int32_t n_fft, int32_t hop, uint32_t flags, int32_t image_size,
                          float* out_dev, void* stream) {
+    vr::NoiseParams nz;
+    if (int rc = take_noise(flags, nz)) return rc;
     if (!wavelength_dev || !radar_loc_dev) return fail(VR_ERR_ARG, "wavelength_dev and radar_loc_dev must not be null");
     if (image_size < 1) return fail(VR_ERR_SHAPE, "image_size must be positive, got %d", image_size);
     return launch(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
-                  n_fft, hop, flags, image_size, out_dev, nullptr, (cudaStream_t)stream);
+                  n_fft, hop, flags, image_size, out_dev, nullptr, (cudaStream_t)stream, nullptr, 0, 0, nz);
 }
 
 int vr_job_geometry(int64_t N, int64_t T, int32_t V, int32_t M, const int32_t* src_host, const int32_t* dst_host,
@@ -623,10 +671,11 @@ int vr_forward_host_f32(const float* x_host, int64_t N, int64_t T, int32_t V, in
                         const int32_t* src_host, const int32_t* dst_host, int32_t E,
                         float wavelength, const float* radar_loc_host,
                         int32_t n_fft, int32_t hop, uint32_t flags, float* out_host, int64_t sub_batch) {
+    drop_noise(flags);
     if (!x_host || !out_host || !radar_loc_host) return fail(VR_ERR_ARG, "host pointers must not be null");
-    if (flags & (VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK))
-        return fail(VR_ERR_ARG, "vr_forward_host_f32 takes one host placement for the batch; VR_FLAG_PER_SEQUENCE and "
-                                "VR_FLAG_VIEWS need a device-pointer entry point");
+    if (flags & (VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK | VR_FLAG_NOISE))
+        return fail(VR_ERR_ARG, "vr_forward_host_f32 takes one host placement for the batch; VR_FLAG_PER_SEQUENCE, "
+                                "VR_FLAG_VIEWS and VR_FLAG_NOISE need a device-pointer entry point");
     if (N <= 0 || T <= 0 || V <= 0 || M <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M, hop must be positive");
     int dev, sm_count;
     int rc = device_setup(dev, sm_count);
@@ -882,7 +931,8 @@ int upsampled_impl(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t 
                    const float* wavelength_dev, const float* radar_loc_dev,
                    int32_t n_fft, int32_t hop, uint32_t flags,
                    int32_t num_pad_frames, float sigma, int32_t image_size,
-                   void* workspace_dev, int64_t workspace_bytes, float* out_dev, float* iq_dev, void* stream) {
+                   void* workspace_dev, int64_t workspace_bytes, float* out_dev, float* iq_dev, void* stream,
+                   const vr::NoiseParams& noise) {
     if (!wavelength_dev || !radar_loc_dev) return fail(VR_ERR_ARG, "wavelength_dev and radar_loc_dev must not be null");
     if (!x_dev || (!out_dev && !iq_dev) || !workspace_dev) return fail(VR_ERR_ARG, "x_dev, out_dev and workspace_dev must not be null");
     if (image_size < 0) return fail(VR_ERR_SHAPE, "image_size must be >= 0, got %d", image_size);
@@ -902,7 +952,7 @@ int upsampled_impl(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t 
     rc = pad_launch(x_dev, Nx, T, V, M, num_pad_frames, sigma, nullptr, coef, stream);
     if (rc) return rc;
     return launch(x_dev, N, T * num_pad_frames, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, 0.f, nullptr,
-                  n_fft, hop, flags, image_size, out_dev, iq_dev, (cudaStream_t)stream, coef, (int)T, num_pad_frames);
+                  n_fft, hop, flags, image_size, out_dev, iq_dev, (cudaStream_t)stream, coef, (int)T, num_pad_frames, noise);
 }
 }  // namespace
 extern "C" {
@@ -913,8 +963,10 @@ int vr_forward_upsampled_f32(const float* x_dev, int64_t N, int64_t T, int32_t V
                              int32_t n_fft, int32_t hop, uint32_t flags,
                              int32_t num_pad_frames, float sigma, int32_t image_size,
                              void* workspace_dev, int64_t workspace_bytes, float* out_dev, void* stream) {
+    vr::NoiseParams nz;
+    if (int rc = take_noise(flags, nz)) return rc;
     return upsampled_impl(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, n_fft, hop, flags,
-                          num_pad_frames, sigma, image_size, workspace_dev, workspace_bytes, out_dev, nullptr, stream);
+                          num_pad_frames, sigma, image_size, workspace_dev, workspace_bytes, out_dev, nullptr, stream, nz);
 }
 
 int vr_forward_upsampled_debug_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
@@ -922,9 +974,11 @@ int vr_forward_upsampled_debug_f32(const float* x_dev, int64_t N, int64_t T, int
                                    const float* wavelength_dev, const float* radar_loc_dev,
                                    int32_t n_fft, int32_t hop, uint32_t flags, int32_t num_pad_frames, float sigma,
                                    void* workspace_dev, int64_t workspace_bytes, float* out_dev, float* iq_dev, void* stream) {
+    vr::NoiseParams nz;
+    if (int rc = take_noise(flags, nz)) return rc;
     if (!iq_dev) return fail(VR_ERR_ARG, "iq_dev must not be null");
     return upsampled_impl(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, n_fft, hop, flags,
-                          num_pad_frames, sigma, 0, workspace_dev, workspace_bytes, out_dev, iq_dev, stream);
+                          num_pad_frames, sigma, 0, workspace_dev, workspace_bytes, out_dev, iq_dev, stream, nz);
 }
 
 int vr_synth_upsampled_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, int32_t M,
@@ -932,9 +986,11 @@ int vr_synth_upsampled_f32(const float* x_dev, int64_t N, int64_t T, int32_t V, 
                            const float* wavelength_dev, const float* radar_loc_dev, uint32_t flags,
                            int32_t num_pad_frames, float sigma, void* workspace_dev, int64_t workspace_bytes,
                            float* iq_dev, void* stream) {
+    vr::NoiseParams nz;
+    if (int rc = take_noise(flags, nz)) return rc;
     if (!iq_dev) return fail(VR_ERR_ARG, "iq_dev must not be null");
     return upsampled_impl(x_dev, N, T, V, M, src_host, dst_host, E, wavelength_dev, radar_loc_dev, vr::NFFT, 1, flags,
-                          num_pad_frames, sigma, 0, workspace_dev, workspace_bytes, nullptr, iq_dev, stream);
+                          num_pad_frames, sigma, 0, workspace_dev, workspace_bytes, nullptr, iq_dev, stream, nz);
 }
 
 int vr_backward_params_f32(const float* x_dev, const float* iq_dev, const float* grad_out_dev,
@@ -962,6 +1018,7 @@ int backward_ups_impl(const void* workspace_dev, const float* iq_dev, const floa
                       int64_t N, int64_t T, int32_t V, int32_t M, const int32_t* src_host, const int32_t* dst_host, int32_t E,
                       const float* wavelength_dev, const float* radar_loc_dev, int32_t n_fft, int32_t hop, uint32_t flags,
                       int32_t num_pad_frames, bool synth_only, float* gz_work_dev, double* grad_params_dev, void* stream) {
+    drop_noise(flags);
     if (!workspace_dev) return fail(VR_ERR_ARG, "workspace_dev must not be null");
     if (((uintptr_t)workspace_dev & 7) != 0) return fail(VR_ERR_ARG, "workspace_dev must be 8-byte aligned");
     if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames", (long long)T);
@@ -1012,6 +1069,7 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
                   int32_t n_fft, int32_t hop, uint32_t flags, bool synth_only,
                   float* gz_work_dev, double* grad_params_dev, float* grad_x_dev, void* stream,
                   const double* coef, int ups_T, int ups_K) {
+    drop_noise(flags);                                   // VR_FLAG_NOISE is rejected below as an unknown flag
     // synth_only: gz_work_dev already holds dL/d(iq); the adjoint STFT is skipped.  coef != nullptr: the joint positions are
     // the up-sampling spline's (T = ups_K * ups_T steps, x_dev unused), parameter gradients only
     if ((!x_dev && !coef) || !gz_work_dev || !grad_params_dev || !wavelength_dev || !radar_loc_dev || (!synth_only && (!iq_dev || !grad_out_dev)))

@@ -16,6 +16,7 @@ kernels do not cover raises.
 import ctypes
 import functools
 import math
+import numbers
 
 import numpy as np
 import torch
@@ -183,10 +184,10 @@ class _RadarFunction(torch.autograd.Function):
     forward launch is the same fused kernel, asked to also save the complex baseband signal."""
 
     @staticmethod
-    def forward(ctx, lam, loc, xc, layer, flags):
-        out, iq = layer._launch(xc, flags, want_iq=True, lam=lam, loc=loc)
-        ctx.save_for_backward(lam, loc, xc, iq)
-        ctx.layer, ctx.flags = layer, flags
+    def forward(ctx, lam, loc, xc, layer, flags, noise=None):
+        out, iq = layer._launch(xc, flags, want_iq=True, lam=lam, loc=loc, noise=noise)
+        ctx.save_for_backward(lam, loc, xc, iq)      # iq carries the receiver noise: the STFT adjoint reads log|z + xi|
+        ctx.layer, ctx.flags = layer, flags & ~_cabi.VR_FLAG_NOISE
         return out
 
     @staticmethod
@@ -208,7 +209,7 @@ class _RadarFunction(torch.autograd.Function):
                                              gx.data_ptr() if gx is not None else None, ctypes.c_void_p(stream))
         _cabi.check(rc)
         g_lam, g_loc = _param_grads(ctx, gp, lam, loc)
-        return g_lam, g_loc, gx, None, None
+        return g_lam, g_loc, gx, None, None, None
 
 
 class _SynthFunction(torch.autograd.Function):
@@ -217,10 +218,10 @@ class _SynthFunction(torch.autograd.Function):
     trainable kernel pair and therefore runs outside the fused kernel."""
 
     @staticmethod
-    def forward(ctx, lam, loc, xc, layer, flags):
-        iq = layer._synth(xc, flags, lam, loc)
+    def forward(ctx, lam, loc, xc, layer, flags, noise=None):
+        iq = layer._synth(xc, flags, lam, loc, noise)
         ctx.save_for_backward(lam, loc, xc)
-        ctx.layer, ctx.flags = layer, flags
+        ctx.layer, ctx.flags = layer, flags & ~_cabi.VR_FLAG_NOISE     # d(z + xi)/d(theta) = dz/d(theta)
         return iq
 
     @staticmethod
@@ -239,7 +240,7 @@ class _SynthFunction(torch.autograd.Function):
                                                   gx.data_ptr() if gx is not None else None, ctypes.c_void_p(stream))
         _cabi.check(rc)
         g_lam, g_loc = _param_grads(ctx, gp, lam, loc)
-        return g_lam, g_loc, gx, None, None
+        return g_lam, g_loc, gx, None, None, None
 
 
 class _UpsampledRadarFunction(torch.autograd.Function):
@@ -249,7 +250,7 @@ class _UpsampledRadarFunction(torch.autograd.Function):
     re-evaluates the joint positions of every up-sampled step."""
 
     @staticmethod
-    def forward(ctx, lam, loc, xc, layer, k, sigma, flags=0):
+    def forward(ctx, lam, loc, xc, layer, k, sigma, flags=0, noise=None):
         _, _, T, V, M = xc.shape
         N = xc.shape[0] * _cabi.views_of(flags)             # outputs; the spline is solved once per raw sequence
         L = _cabi.lib()
@@ -259,13 +260,14 @@ class _UpsampledRadarFunction(torch.autograd.Function):
         iq = torch.empty((N, k * T, 2), dtype=torch.float32, device=xc.device)
         with torch.cuda.device(xc.device):
             stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
+            _set_noise(noise)
             rc = L.vr_forward_upsampled_debug_f32(xc.data_ptr(), N, T, V, M, layer._src_c, layer._dst_c, len(layer.src),
                                                   lam.data_ptr(), loc.data_ptr(), layer.n_fft, layer.hop_length, flags,
                                                   k, ctypes.c_float(float(sigma)), work.data_ptr(), nbytes,
                                                   out.data_ptr(), iq.data_ptr(), stream)
         _cabi.check(rc)
-        ctx.save_for_backward(lam, loc, work, iq)
-        ctx.layer, ctx.dims, ctx.flags = layer, (N, T, V, M, k), flags
+        ctx.save_for_backward(lam, loc, work, iq)      # iq carries the receiver noise, as in _RadarFunction
+        ctx.layer, ctx.dims, ctx.flags = layer, (N, T, V, M, k), flags & ~_cabi.VR_FLAG_NOISE
         return out
 
     @staticmethod
@@ -284,7 +286,7 @@ class _UpsampledRadarFunction(torch.autograd.Function):
                                                               ctx.flags, k, gz.data_ptr(), gp.data_ptr(), ctypes.c_void_p(stream))
         _cabi.check(rc)
         g_lam, g_loc = _param_grads(ctx, gp, lam, loc)
-        return g_lam, g_loc, None, None, None, None, None
+        return g_lam, g_loc, None, None, None, None, None, None
 
 
 class _UpsampledSynthFunction(torch.autograd.Function):
@@ -294,10 +296,10 @@ class _UpsampledSynthFunction(torch.autograd.Function):
     Used by forward_upsampled when the STFT is general and therefore runs outside the fused kernel."""
 
     @staticmethod
-    def forward(ctx, lam, loc, xc, layer, k, sigma, flags=0):
-        iq, work = layer._synth_upsampled(xc, k, sigma, lam, loc, flags)
+    def forward(ctx, lam, loc, xc, layer, k, sigma, flags=0, noise=None):
+        iq, work = layer._synth_upsampled(xc, k, sigma, lam, loc, flags, noise)
         ctx.save_for_backward(lam, loc, work)
-        ctx.layer, ctx.dims, ctx.flags = layer, (iq.shape[0],) + tuple(xc.shape[1:]) + (k,), flags
+        ctx.layer, ctx.dims, ctx.flags = layer, (iq.shape[0],) + tuple(xc.shape[1:]) + (k,), flags & ~_cabi.VR_FLAG_NOISE
         return iq
 
     @staticmethod
@@ -314,7 +316,13 @@ class _UpsampledSynthFunction(torch.autograd.Function):
                                                             gp.data_ptr(), ctypes.c_void_p(stream))
         _cabi.check(rc)
         g_lam, g_loc = _param_grads(ctx, gp, lam, loc)
-        return g_lam, g_loc, None, None, None, None, None
+        return g_lam, g_loc, None, None, None, None, None, None
+
+
+def _set_noise(noise):
+    """vr_set_noise right before a launch that carries VR_FLAG_NOISE; noise: (std, seed) of _noise, or None."""
+    if noise is not None:
+        _cabi.set_noise(*noise)
 
 
 def kept_frame_table(n_frames, image_size):
@@ -426,24 +434,26 @@ class VirtualRadar(torch.nn.Module):
             raise RuntimeError("module parameters are on %s but x is on %s; call .to(x.device)" % (lam.device, x.device))
         return lam, loc
 
-    def _placements(self, x, radar_location, wavelength):
+    def _placements(self, x, radar_location, wavelength, noise_std=None, noise_seed=None):
         """Per-sequence radar placements (the `radar_location=` / `wavelength=` keywords of forward, forward_image and
-        forward_upsampled) -> None when neither is given, else (wavelength (N,), radar_location (N, 3), flags): each
-        keyword expanded to the batch and made contiguous, the module parameter standing in for a keyword not given.
-        Autograd's expand carries the per-sequence gradients back to whatever the caller passed (summed where it
-        broadcast).  flags: what the launch adds (VR_FLAG_PER_SEQUENCE)."""
-        if radar_location is None and wavelength is None:
+        forward_upsampled) and receiver noise (`noise_std=` / `noise_seed=`) -> None when none is given, else
+        (wavelength (N,), radar_location (N, 3), flags, noise): each placement keyword expanded to the batch and made
+        contiguous, the module parameter standing in for a keyword not given.  Autograd's expand carries the
+        per-sequence gradients back to whatever the caller passed (summed where it broadcast).  flags: what the launch
+        adds (VR_FLAG_PER_SEQUENCE, and VR_FLAG_NOISE with noise); noise: (std (N,), seed) of _noise, or None."""
+        noise = self._noise(x, noise_std, noise_seed, (x.shape[0],))
+        if radar_location is None and wavelength is None and noise is None:
             return None
         N = x.shape[0]
         lam = self._expand_placement(x, "wavelength", wavelength, self.wavelength, (N,))
         loc = self._expand_placement(x, "radar_location", radar_location, self.radar_location, (N, 3))
-        return lam, loc, _cabi.VR_FLAG_PER_SEQUENCE
+        return lam, loc, _cabi.VR_FLAG_PER_SEQUENCE | (_cabi.VR_FLAG_NOISE if noise is not None else 0), noise
 
-    def _view_placements(self, x, radar_location, wavelength):
-        """The placements of forward_views -> (wavelength (N R,), radar_location (N R, 3), flags): R from radar_location's
-        second-to-last dimension, each keyword expanded to (N, R[, 3]) and flattened view-minor (output n R + r is view r
-        of sequence n), the module's wavelength standing in for `wavelength=None`.  flags: VR_FLAG_PER_SEQUENCE |
-        VR_FLAG_VIEWS(R)."""
+    def _view_placements(self, x, radar_location, wavelength, noise_std=None, noise_seed=None):
+        """The placements of forward_views -> (wavelength (N R,), radar_location (N R, 3), flags, noise): R from
+        radar_location's second-to-last dimension, each keyword expanded to (N, R[, 3]) and flattened view-minor (output
+        n R + r is view r of sequence n), the module's wavelength standing in for `wavelength=None`; noise_std likewise
+        from (N, R).  flags: VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS(R) [| VR_FLAG_NOISE]."""
         if not isinstance(radar_location, torch.Tensor) or radar_location.dim() < 2:
             raise ValueError("radar_location must be a tensor of R placements, (R, 3) for every sequence or (N, R, 3), got %s"
                              % (tuple(radar_location.shape) if isinstance(radar_location, torch.Tensor) else type(radar_location),))
@@ -453,7 +463,54 @@ class VirtualRadar(torch.nn.Module):
                              % (R, tuple(radar_location.shape)))
         lam = self._expand_placement(x, "wavelength", wavelength, self.wavelength, (N, R))
         loc = self._expand_placement(x, "radar_location", radar_location, self.radar_location, (N, R, 3))
-        return lam.reshape(N * R), loc.reshape(N * R, 3), _cabi.VR_FLAG_PER_SEQUENCE | _cabi.views_flag(R)
+        noise = self._noise(x, noise_std, noise_seed, (N, R))
+        flags = _cabi.VR_FLAG_PER_SEQUENCE | _cabi.views_flag(R) | (_cabi.VR_FLAG_NOISE if noise is not None else 0)
+        return lam.reshape(N * R), loc.reshape(N * R, 3), flags, noise
+
+    @staticmethod
+    def _noise(x, noise_std, noise_seed, shape):
+        """The receiver-noise keywords -> None without `noise_std`, else (std, seed): std the float32 noise standard
+        deviations broadcast to `shape` and flattened (one per output), seed a 0-d int64 tensor on x's device holding the
+        64 seed bits -- `noise_seed` itself when it is such a tensor (what a CUDA graph should pass: the launch reads it
+        at replay time), a Python int in [0, 2**64) copied to the device, or None: drawn from torch's CUDA generator, so
+        every call has fresh noise and torch.manual_seed makes the sequence of calls reproducible.  A float level must be
+        finite and non-negative; a tensor's values are not checked (that would synchronise with the device): a negative
+        level gives noise of its magnitude, a NaN level NaN outputs."""
+        if noise_std is None:
+            if noise_seed is not None:
+                raise ValueError("noise_seed needs noise_std: the noise level of every output")
+            return None
+        if isinstance(noise_std, torch.Tensor):
+            if noise_std.requires_grad:
+                raise ValueError("noise_std must not require grad: the layer has no gradient with respect to the noise level")
+            std = VirtualRadar._expand_placement(x, "noise_std", noise_std, None, shape)
+        elif isinstance(noise_std, numbers.Real) and not isinstance(noise_std, bool):
+            v = float(noise_std)
+            if not (math.isfinite(v) and v >= 0):
+                raise ValueError("noise_std must be a finite non-negative noise standard deviation, got %r" % (noise_std,))
+            std = torch.full(shape, v, dtype=torch.float32, device=x.device)
+        else:
+            raise ValueError("noise_std must be a float or a float32 tensor that broadcasts to %s, got %s"
+                             % (shape, type(noise_std)))
+        if noise_seed is None:
+            seed = torch.randint(0, 2 ** 63 - 1, (), dtype=torch.int64, device=x.device)
+        elif isinstance(noise_seed, torch.Tensor):
+            if noise_seed.dtype != torch.int64 or noise_seed.dim() != 0:
+                raise ValueError("noise_seed must be an int or a 0-d int64 tensor, got a %s tensor of shape %s"
+                                 % (noise_seed.dtype, tuple(noise_seed.shape)))
+            if noise_seed.device != x.device:
+                raise RuntimeError("noise_seed is on %s but x is on %s: the seed is read on x's device"
+                                   % (noise_seed.device, x.device))
+            seed = noise_seed
+        elif isinstance(noise_seed, numbers.Integral) and not isinstance(noise_seed, bool):
+            s = int(noise_seed)
+            if not 0 <= s < 2 ** 64:
+                raise ValueError("noise_seed must be in [0, 2**64), got %d" % s)
+            # a fill kernel, not a pageable host-to-device copy: no stream synchronisation per call
+            seed = torch.full((), s - 2 ** 64 if s >= 2 ** 63 else s, dtype=torch.int64, device=x.device)
+        else:
+            raise ValueError("noise_seed must be an int or a 0-d int64 tensor, got %s" % type(noise_seed))
+        return std.reshape(-1), seed
 
     @staticmethod
     def _expand_placement(x, name, value, param, shape):
@@ -482,9 +539,9 @@ class VirtualRadar(torch.nn.Module):
 
     _FUSED_N_FFT = 256      # the fused kernel's FFT size; other n_fft values go through the general-kernel path
 
-    def _launch(self, xc, flags, want_iq=False, lam=None, loc=None):
+    def _launch(self, xc, flags, want_iq=False, lam=None, loc=None, noise=None):
         """One fused launch.  lam / loc: the radar parameters to read (default: the module's; (N,) and (N, 3) with
-        VR_FLAG_PER_SEQUENCE in flags, N = R x the rows of xc with VR_FLAG_VIEWS(R))."""
+        VR_FLAG_PER_SEQUENCE in flags, N = R x the rows of xc with VR_FLAG_VIEWS(R)); noise: with VR_FLAG_NOISE."""
         _, _, T, V, M = xc.shape
         N = xc.shape[0] * _cabi.views_of(flags)
         lam = self.wavelength if lam is None else lam
@@ -504,6 +561,7 @@ class VirtualRadar(torch.nn.Module):
                 stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
                 args = (xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src), lam.data_ptr(),
                         loc.data_ptr(), n_fft, self.hop_length, flags, out.data_ptr())
+                _set_noise(noise)
                 rc = L.vr_forward_debug_f32(*args, iq.data_ptr(), stream) if want_iq else L.vr_forward_f32(*args, stream)
         finally:
             if self.nvtx_ranges:
@@ -511,7 +569,7 @@ class VirtualRadar(torch.nn.Module):
         _cabi.check(rc)
         return out, iq
 
-    def _synth(self, xc, flags, lam=None, loc=None):
+    def _synth(self, xc, flags, lam=None, loc=None, noise=None):
         """Synthesis only (C ABI vr_synth_f32): the complex baseband signal (N,T,2) that the general-kernel STFT reads,
         bit for bit forward_debug's, without any STFT work."""
         _, _, T, V, M = xc.shape
@@ -528,6 +586,7 @@ class VirtualRadar(torch.nn.Module):
         try:
             with torch.cuda.device(xc.device):
                 stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
+                _set_noise(noise)
                 rc = _cabi.lib().vr_synth_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
                                               lam.data_ptr(), loc.data_ptr(), flags, iq.data_ptr(), stream)
         finally:
@@ -536,7 +595,7 @@ class VirtualRadar(torch.nn.Module):
         _cabi.check(rc)
         return iq
 
-    def _synth_upsampled(self, xc, k, sigma, lam=None, loc=None, flags=0):
+    def _synth_upsampled(self, xc, k, sigma, lam=None, loc=None, flags=0, noise=None):
         """Synthesis of pad_frames(xc, k, sigma) without the up-sampled batch (C ABI vr_synth_upsampled_f32) -> iq
         (N, k*T, 2) and the workspace holding the spline's cubics.  The up-sampled tensor the reference's loader builds
         is standard-contiguous: range rounding mode "seq" (no VR_FLAG_RANGE_FMA)."""
@@ -552,6 +611,7 @@ class VirtualRadar(torch.nn.Module):
             return iq, work
         with torch.cuda.device(xc.device):
             stream = ctypes.c_void_p(torch.cuda.current_stream(xc.device).cuda_stream)
+            _set_noise(noise)
             rc = L.vr_synth_upsampled_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
                                           lam.data_ptr(), loc.data_ptr(), flags, k,
                                           ctypes.c_float(float(sigma)), work.data_ptr(), nbytes, iq.data_ptr(), stream)
@@ -577,42 +637,53 @@ class VirtualRadar(torch.nn.Module):
         return torch.is_grad_enabled() and (self.wavelength.requires_grad or self.radar_location.requires_grad
                                             or (x is not None and x.requires_grad))
 
-    def forward(self, x, radar_location=None, wavelength=None):
+    def forward(self, x, radar_location=None, wavelength=None, noise_std=None, noise_seed=None):
         """x (N,3,T,V,M) -> (N, n_fft, T//hop+1).  `radar_location` / `wavelength` (optional): one radar placement per
         sequence, float32 tensors on x's device that broadcast to (N, 3) and (N,) -- sequence n is seen from
         radar_location[n] at wavelength[n] (C ABI VR_FLAG_PER_SEQUENCE); a keyword not given is the module parameter.
         Differentiable per sequence: the gradients reach the tensors passed (through autograd's expand).  Under
         torch.nn.DataParallel pass full (N, 3) / (N,) tensors: DataParallel splits every tensor argument along dim 0 like
         the batch, so a broadcast-shaped one -- a (3,) location, a 0-d wavelength -- would reach the replicas cut apart
-        (expand it to the batch first, e.g. `loc.expand(len(x), 3)`)."""
+        (expand it to the batch first, e.g. `loc.expand(len(x), 3)`).
+
+        `noise_std` / `noise_seed` (optional): receiver noise (C ABI VR_FLAG_NOISE, DESIGN §3i), a complex Gaussian
+        sample xi[n, t] with E|xi|^2 = noise_std[n]^2 added to the baseband of sequence n at every step t before the STFT.
+        `noise_std`: a float or a float32 tensor on x's device that broadcasts to (N,), in the units of the I/Q (an
+        absolute level, not an SNR); it has no gradient, and a tensor's values are not checked.  `noise_seed`: an int in [0, 2**64), a 0-d int64 CUDA tensor
+        (for CUDA graphs: the seed is read when the graph replays), or None (drawn from torch's CUDA generator).  xi
+        depends only on (seed, n, t), n the position in this call's batch: a DataParallel replica or a sharded_forward
+        rank numbers its own shard from 0, so its noise differs from a single-device call with the same seed.  The
+        gradients with respect to x and the placements are those of the noisy spectrogram."""
         self._check_input(x)
         self._check_device(x)
-        pl = self._placements(x, radar_location, wavelength)
+        pl = self._placements(x, radar_location, wavelength, noise_std, noise_seed)
         xc, flags = self._prepare(x)
         return self._run(x, xc, flags, pl)
 
     def _run(self, x, xc, flags, pl=None):
         """forward() after the layout has been normalised: xc standard-contiguous, flags carry the range rounding mode;
         pl: per-sequence placements (_placements, _view_placements) or None."""
-        lam, loc = self.wavelength, self.radar_location
+        lam, loc, noise = self.wavelength, self.radar_location, None
         if pl is not None:
-            lam, loc, pflags = pl
+            lam, loc, pflags, noise = pl
             flags |= pflags
         if self._general_stft():     # trained / trainable STFT kernels: synthesis on our kernels, STFT as a GEMM
             self._check_general_length(xc.shape[2])
             if xc.shape[0] == 0:
-                return self._launch(xc, flags, lam=lam, loc=loc)[0]
+                return self._launch(xc, flags, lam=lam, loc=loc, noise=noise)[0]
             return self.stft.logmag(self._general_iq(x, xc, flags, pl))
         if self._needs_grad(x, pl) and xc.shape[0] > 0:
-            return _RadarFunction.apply(lam, loc, xc, self, flags)
-        return self._launch(xc, flags, lam=lam, loc=loc)[0]
+            return _RadarFunction.apply(lam, loc, xc, self, flags, noise)
+        return self._launch(xc, flags, lam=lam, loc=loc, noise=noise)[0]
 
     def _general_iq(self, x, xc, flags, pl=None):
-        lam, loc = self.wavelength, self.radar_location
+        lam, loc, noise = self.wavelength, self.radar_location, None
         if pl is not None:
-            lam, loc, pflags = pl
+            lam, loc, pflags, noise = pl
             flags |= pflags
-        return _SynthFunction.apply(lam, loc, xc, self, flags) if self._needs_grad(x, pl) else self._synth(xc, flags, lam, loc)
+        if self._needs_grad(x, pl):
+            return _SynthFunction.apply(lam, loc, xc, self, flags, noise)
+        return self._synth(xc, flags, lam, loc, noise)
 
     def forward_notebook(self, data, num_pad_frames=1, sigma=3):
         """virtual_radar_example.ipynb cells 2-4 on the device: `data` is one body's (T, V, 3) array (or a batch
@@ -630,14 +701,15 @@ class VirtualRadar(torch.nn.Module):
         self._check_device(x)
         return self._run(x, x, _cabi.VR_FLAG_RANGE_FMA)
 
-    def forward_image(self, x, image_size=256, radar_location=None, wavelength=None):
+    def forward_image(self, x, image_size=256, radar_location=None, wavelength=None, noise_std=None, noise_seed=None):
         """The layer fused with its consumer's input stage (reference models/resnet.py:24-26):
         equals `F.interpolate(self(x).unsqueeze(1), image_size)` (nearest) bit for bit, in one launch
         that writes (N, 1, image_size, image_size) directly and transforms only the frames the
-        resize keeps.  `radar_location` / `wavelength`: per-sequence placements, as in forward()."""
+        resize keeps.  `radar_location` / `wavelength`: per-sequence placements, and `noise_std` / `noise_seed`
+        receiver noise, as in forward()."""
         self._check_input(x)
         self._check_device(x)
-        return self._image(x, image_size, self._placements(x, radar_location, wavelength))
+        return self._image(x, image_size, self._placements(x, radar_location, wavelength, noise_std, noise_seed))
 
     def _image(self, x, image_size, pl):
         """forward_image after the input checks; pl: placements (_placements, _view_placements) or None."""
@@ -653,8 +725,9 @@ class VirtualRadar(torch.nn.Module):
             spec = self.forward(x) if pl is None else self._run(x, *self._prepare(x), pl)
             return torch.nn.functional.interpolate(spec.unsqueeze(1), image_size)
         xc, flags = self._prepare(x)
+        noise = None
         if pl is not None:
-            lam, loc, pflags = pl
+            lam, loc, pflags, noise = pl
             flags |= pflags
         if self.assume_inputs_ready:
             flags |= _cabi.VR_FLAG_INPUTS_READY
@@ -665,13 +738,15 @@ class VirtualRadar(torch.nn.Module):
             return out
         with torch.cuda.device(x.device):
             stream = torch.cuda.current_stream(x.device).cuda_stream
+            _set_noise(noise)
             rc = _cabi.lib().vr_forward_image_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
                                                   lam.data_ptr(), loc.data_ptr(), self.n_fft, self.hop_length,
                                                   flags, image_size, out.data_ptr(), ctypes.c_void_p(stream))
         _cabi.check(rc)
         return out
 
-    def forward_upsampled(self, x, num_pad_frames=250, sigma=3, image_size=None, radar_location=None, wavelength=None):
+    def forward_upsampled(self, x, num_pad_frames=250, sigma=3, image_size=None, radar_location=None, wavelength=None,
+                          noise_std=None, noise_seed=None):
         """The data loader's temporal up-sampling fused in front of the layer: x is the RAW
         (N,3,T,V,M) batch; the result equals `self(pad_frames(x, num_pad_frames, sigma))` -- or
         `self.forward_image(pad_frames(...), image_size)` when `image_size` is given -- bit for bit,
@@ -681,17 +756,19 @@ class VirtualRadar(torch.nn.Module):
         (vr_forward_upsampled_debug_f32 + vr_backward_upsampled_params_f32); with `image_size` the
         spectrogram is then resized by `F.interpolate`, as `forward_image` does under grad.  Gradients
         with respect to x itself go through `self(pad_frames(x, num_pad_frames, sigma))`.  `radar_location` /
-        `wavelength`: per-sequence placements, as in forward()."""
+        `wavelength`: per-sequence placements, and `noise_std` / `noise_seed` receiver noise, as in forward(); the noise
+        is keyed by the up-sampled step, so the result equals `self(pad_frames(x, ...), noise_std=..., noise_seed=...)`."""
         self._check_input(x)
         self._check_device(x)
-        return self._upsampled(x, num_pad_frames, sigma, image_size, self._placements(x, radar_location, wavelength))
+        pl = self._placements(x, radar_location, wavelength, noise_std, noise_seed)
+        return self._upsampled(x, num_pad_frames, sigma, image_size, pl)
 
     def _upsampled(self, x, num_pad_frames, sigma, image_size, pl):
         """forward_upsampled after the input checks; pl: placements (_placements, _view_placements) or None."""
-        lam, loc = self.wavelength, self.radar_location
+        lam, loc, noise = self.wavelength, self.radar_location, None
         flags = 0
         if pl is not None:
-            lam, loc, flags = pl
+            lam, loc, flags, noise = pl
         xc = x.contiguous()
         _, _, T, V, M = xc.shape
         Nx, N = xc.shape[0], xc.shape[0] * _cabi.views_of(flags)     # raw sequences, outputs
@@ -704,13 +781,13 @@ class VirtualRadar(torch.nn.Module):
                                       "layer(pad_frames(x, num_pad_frames, sigma)), which materialises the up-sampled batch")
         if self._general_stft():      # general STFT kernels: synthesis without the up-sampled batch, then the GEMM STFT
             if self._needs_grad(None, pl) and N > 0:
-                iq = _UpsampledSynthFunction.apply(lam, loc, xc, self, k, sigma, flags)
+                iq = _UpsampledSynthFunction.apply(lam, loc, xc, self, k, sigma, flags, noise)
             else:
-                iq = self._synth_upsampled(xc, k, sigma, lam, loc, flags)[0]
+                iq = self._synth_upsampled(xc, k, sigma, lam, loc, flags, noise)[0]
             self._check_general_length(k * T)
             return self._general_image(iq, img) if img else self.stft.logmag(iq)
         if self._needs_grad(None, pl) and N > 0:
-            out = _UpsampledRadarFunction.apply(lam, loc, xc, self, k, sigma, flags)
+            out = _UpsampledRadarFunction.apply(lam, loc, xc, self, k, sigma, flags, noise)
             return torch.nn.functional.interpolate(out.unsqueeze(1), img) if img else out
         shape = (N, 1, img, img) if img else (N, self.n_fft, (k * T) // self.hop_length + 1)
         out = torch.empty(shape, dtype=torch.float32, device=x.device)
@@ -722,6 +799,7 @@ class VirtualRadar(torch.nn.Module):
         with torch.cuda.device(x.device):
             stream = torch.cuda.current_stream(x.device).cuda_stream
             # the up-sampled tensor the reference's loader builds is standard-contiguous: range rounding mode "seq"
+            _set_noise(noise)
             rc = L.vr_forward_upsampled_f32(xc.data_ptr(), N, T, V, M, self._src_c, self._dst_c, len(self.src),
                                             lam.data_ptr(), loc.data_ptr(), self.n_fft, self.hop_length, flags,
                                             k, ctypes.c_float(float(sigma)), img, work.data_ptr(), nbytes,
@@ -729,7 +807,8 @@ class VirtualRadar(torch.nn.Module):
         _cabi.check(rc)
         return out
 
-    def forward_views(self, x, radar_location, wavelength=None, image_size=None, num_pad_frames=None, sigma=3):
+    def forward_views(self, x, radar_location, wavelength=None, image_size=None, num_pad_frames=None, sigma=3,
+                      noise_std=None, noise_seed=None):
         """R radar views of every sequence in one launch from one copy of x (C ABI VR_FLAG_VIEWS(R)): a
         multistatic array, a set of viewpoints for augmentation, one scene in several bands.  x (N,3,T,V,M);
         `radar_location` float32 (R, 3), the same R placements for every sequence, or (N, R, 3); `wavelength` None (the
@@ -744,10 +823,12 @@ class VirtualRadar(torch.nn.Module):
         placement gradients reach the tensors passed and are the repeated route's bits; dL/dx adds the R views'
         contributions in view order, in float32, inside the kernel (deterministic; not the bits of autograd's
         repeat_interleave backward for R > 1).  As in forward_upsampled, `num_pad_frames` has no gradient with respect to
-        x.  Under torch.nn.DataParallel pass full (N, R, 3) / (N, R) tensors, for the reason forward() gives."""
+        x.  Under torch.nn.DataParallel pass full (N, R, 3) / (N, R) tensors, for the reason forward() gives.
+        `noise_std` (a float or a float32 tensor that broadcasts to (N, R)) / `noise_seed`: receiver noise as in forward(),
+        output n R + r keyed as output n R + r of the repeated route, so the identity above holds with the same keywords."""
         self._check_input(x)
         self._check_device(x)
-        pl = self._view_placements(x, radar_location, wavelength)
+        pl = self._view_placements(x, radar_location, wavelength, noise_std, noise_seed)
         if num_pad_frames is not None:
             out = self._upsampled(x, num_pad_frames, sigma, image_size, pl)
         elif image_size is not None:

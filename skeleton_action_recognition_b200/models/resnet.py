@@ -82,12 +82,13 @@ class Model(nn.Module):
         self.num_pad_frames = num_pad_frames
         self.sigma = sigma
 
-    def spectrogram_image(self, x, radar_location=None, wavelength=None):
-        """radar_location / wavelength (optional): one radar placement per sequence (VirtualRadar.forward)."""
-        kw = dict(radar_location=radar_location, wavelength=wavelength)
+    def spectrogram_image(self, x, radar_location=None, wavelength=None, noise_std=None, noise_seed=None):
+        """radar_location / wavelength (optional): one radar placement per sequence; noise_std / noise_seed (optional):
+        receiver noise (VirtualRadar.forward)."""
+        kw = dict(radar_location=radar_location, wavelength=wavelength, noise_std=noise_std, noise_seed=noise_seed)
         if self.num_pad_frames:       # raw sequences: up-sampling, radar and resize in one fused pass
             return self.virtual_radar.forward_upsampled(x, self.num_pad_frames, self.sigma, self.image_size, **kw)
         return self.virtual_radar.forward_image(x, self.image_size, **kw)
 
-    def forward(self, x, radar_location=None, wavelength=None):
-        return self.base_model(self.spectrogram_image(x, radar_location, wavelength))
+    def forward(self, x, radar_location=None, wavelength=None, noise_std=None, noise_seed=None):
+        return self.base_model(self.spectrogram_image(x, radar_location, wavelength, noise_std, noise_seed))
