@@ -27,7 +27,7 @@ SYMBOLS = ("vr_abi_version", "vr_last_error", "vr_forward_f32", "vr_forward_debu
            "vr_synth_f32", "vr_synth_upsampled_f32", "vr_synth_adjoint_upsampled_f32",
            "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32",
            "vr_plan_adjoint_stft", "vr_plan_pad_frames", "vr_plan_stft_general", "vr_per_sequence_grad_doubles",
-           "vr_set_noise")
+           "vr_set_noise", "vr_plan_launch")
 
 _lib = None
 
@@ -111,6 +111,9 @@ def lib():
     L.vr_plan_stft_general.restype = ctypes.c_int
     L.vr_per_sequence_grad_doubles.argtypes = [i64, i64]
     L.vr_per_sequence_grad_doubles.restype = i64
+    L.vr_plan_launch.argtypes = [i32, i64, i64, i32, i32, c_i32p, c_i32p, i32, i32, i32, i32, i32, u32, i32, i32, i32,
+                                 ctypes.POINTER(i64)]
+    L.vr_plan_launch.restype = ctypes.c_int
     L.vr_set_noise.argtypes = [vp, vp]
     L.vr_set_noise.restype = ctypes.c_int
     L.vr_set_timeline_buffer.argtypes = [vp]
@@ -174,6 +177,24 @@ def plan_team(N, T, V, M, src, dst, n_fft=256, hop=16, sm_count=148):
     out = (ctypes.c_int64 * 8)()
     check(lib().vr_plan_team(N, T, V, M, i32_array(src), i32_array(dst), len(src), n_fft, hop, sm_count, out))
     return dict(zip(TEAM_PLAN_FIELDS, [int(v) for v in out]))
+
+
+LAUNCH_PLAN_FIELDS = ("team", "grid", "block", "smem_bytes", "ring_stages", "columns_per_job", "jobs_per_seq", "jobs",
+                      "columns_per_tile", "tile_stride", "tma_loads", "tma_bulk_store", "chunks_per_job", "z_capacity",
+                      "parked_sums", "sparse_frames", "columns", "ctas_per_sm", "ticket", "bodies_per_pass", "compiled_vm",
+                      "max_bones_per_group", "max_sources_per_group", "iq_fill")
+LAUNCH_MODES = {"spectrogram": 0, "debug": 1, "synth": 2}
+
+
+def plan_launch(mode, N, T, V, M, src, dst, hop=16, image_size=0, num_pad_frames=0, flags=0, x_aligned=True, schedule=-1,
+                sm_count=148, n_fft=256):
+    """Configuration of one fused forward launch (vr_plan_launch): mode "spectrogram" (vr_forward_f32, _image_f32 with
+    image_size, _upsampled_f32 with num_pad_frames and T raw), "debug" (the entries that write iq as well) or "synth"
+    (synthesis only); schedule as set_schedule."""
+    out = (ctypes.c_int64 * len(LAUNCH_PLAN_FIELDS))()
+    check(lib().vr_plan_launch(LAUNCH_MODES[mode], N, T, V, M, i32_array(src), i32_array(dst), len(src), n_fft, hop,
+                               image_size, num_pad_frames, flags, 1 if x_aligned else 0, schedule, sm_count, out))
+    return dict(zip(LAUNCH_PLAN_FIELDS, [int(v) for v in out]))
 
 
 ADJOINT_PLAN_FIELDS = ("segment_length", "segments", "grid", "smem_bytes")

@@ -319,12 +319,14 @@ struct TeamVariant { bool fma; int vm; int nb; bool ps; KernelFn fn; };
 const TeamVariant kTeamVariants[] = { VR_TEAM_VARIANT(0, 1, false), VR_TEAM_VARIANT(0, 2, false), VR_TEAM_VARIANT(50, 2, false),
                                       VR_TEAM_VARIANT(0, 1, true), VR_TEAM_VARIANT(0, 2, true), VR_TEAM_VARIANT(50, 2, true) };
 const int kNumTeamVariants = sizeof(kTeamVariants) / sizeof(kTeamVariants[0]);
-KernelFn pick_team_kernel(bool fma, int vm, int m, bool ps) {
+// vmc (optional): the compile-time V*M of the instantiation picked, 0 for the generic one
+KernelFn pick_team_kernel(bool fma, int vm, int m, bool ps, int* vmc = nullptr) {
     const int nb = (m % 2 == 0) ? 2 : 1;
     KernelFn generic = nullptr;
+    if (vmc) *vmc = 0;
     for (int i = 0; i < kNumTeamVariants; ++i) {
         if (kTeamVariants[i].fma != fma || kTeamVariants[i].nb != nb || kTeamVariants[i].ps != ps) continue;
-        if (kTeamVariants[i].vm == vm) return kTeamVariants[i].fn;
+        if (kTeamVariants[i].vm == vm) { if (vmc) *vmc = vm; return kTeamVariants[i].fn; }
         if (kTeamVariants[i].vm == 0) generic = kTeamVariants[i].fn;
     }
     return generic;
@@ -343,13 +345,14 @@ struct Variant { bool fma; int vm; int nb; bool ups; bool park; bool ps; KernelF
     VR_VARIANT(0, 1, true, true, PS), VR_VARIANT(0, 2, true, true, PS), VR_VARIANT(50, 2, true, true, PS)
 const Variant kVariants[] = { VR_VARIANTS(false), VR_VARIANTS(true) };
 const int kNumVariants = sizeof(kVariants) / sizeof(kVariants[0]);
-KernelFn pick_kernel(bool fma, int vm, int m, bool ups, bool park, bool ps) {
+KernelFn pick_kernel(bool fma, int vm, int m, bool ups, bool park, bool ps, int* vmc = nullptr) {
     const int nb = (m % 2 == 0) ? 2 : 1;
     KernelFn generic = nullptr;
+    if (vmc) *vmc = 0;
     for (int i = 0; i < kNumVariants; ++i) {
         if (kVariants[i].fma != fma || kVariants[i].nb != nb || kVariants[i].ups != ups || kVariants[i].park != park ||
             kVariants[i].ps != ps) continue;
-        if (kVariants[i].vm == vm) return kVariants[i].fn;
+        if (kVariants[i].vm == vm) { if (vmc) *vmc = vm; return kVariants[i].fn; }
         if (kVariants[i].vm == 0) generic = kVariants[i].fn;
     }
     return generic;
@@ -487,6 +490,59 @@ int cached_plan(int64_t N, int64_t T, int V, int M, const int32_t* src, const in
     return VR_OK;
 }
 
+// Samples of a sequence that no job of a spectrogram plan synthesises.  A job covers the samples its frames' windows reach
+// (job_geom), so with hop > n_fft / 2 the samples between two frames' windows and after the last window belong to no job:
+// the spectrogram never reads them, but a debug launch must still write them to iq (launch fills them in).
+bool iq_gaps(const vr::Params& p) {
+    if (p.iq_only) return false;
+    int next = 0;
+    for (int j = 0; j < p.jobs_per_seq; ++j) {
+        const vr::JobGeom g = vr::job_geom(j, p.jobs_per_seq, p.FJ, p.ncols, p.img, p.cscale, p.F, p.hop, (int)p.T);
+        if (g.lo > next) return true;
+        next = std::max(next, g.hi + 1);
+    }
+    return next < (int)p.T;
+}
+
+// The configuration of one fused launch: the plan, the schedule and the kernel instantiation.  launch() runs exactly
+// this; vr_plan_launch reports it without a GPU.  debug: iq is written as well as out (never the team-job kernel);
+// schedule: vr_set_schedule's mode.
+struct LaunchPlan {
+    vr::Params p;
+    int grid = 0, cps = 0, vmc = 0;
+    bool team = false, ticket = false;
+    KernelFn fn = nullptr;
+};
+int plan_launch(int64_t N, int64_t T, int V, int M, const int32_t* src, const int32_t* dst, int E, int n_fft, int hop, int img,
+                bool ups, bool iq_only, bool debug, uint32_t flags, bool aligned, int schedule, int sm_count, bool cached,
+                LaunchPlan& L) {
+    int rc = cached ? cached_plan(N, T, V, M, src, dst, E, n_fft, hop, img, ups, iq_only, sm_count, aligned, L.p, L.grid, L.cps)
+                    : make_plan(N, T, V, M, src, dst, E, n_fft, hop, img, ups, sm_count, aligned, L.p, L.grid, L.cps, iq_only);
+    if (rc) return rc;
+    // schedule: batches with several sequences per team slot take the team-job kernel (no CTA-wide barriers, a double
+    // buffer per team); small batches keep the cooperative kernel, whose latency per sequence is half
+    L.team = false;
+    if (!ups && !iq_only && !debug && !g_timeline && schedule != 0) {
+        vr::Params q = L.p;
+        int tg = 0;
+        // automatic: from TEAM_AUTO_WAVES jobs per team slot in plain stream order (below that the cooperative kernel's
+        // shorter latency per sequence wins: N = 1024 66 vs 74 us, N = 4096 248 vs 228 us); always when the caller has
+        // declared the batches independent -- consecutive launches then overlap and only throughput counts
+        // (N = 256: 14.8 vs 16.3 us per launch)
+        const bool overlapped = g_pdl && (flags & VR_FLAG_INPUTS_READY);
+        if (make_team_plan(q, sm_count, tg) &&
+            (schedule == 1 || overlapped || q.n_jobs >= (long long)TEAM_AUTO_WAVES * sm_count * 2 * vr::TJ_TEAMS)) {
+            L.p = q; L.grid = tg; L.team = true;
+        }
+    }
+    const int job_slots = L.team ? L.grid * vr::TJ_TEAMS : L.grid;
+    L.ticket = g_dynamic && L.p.n_jobs > job_slots;
+    const bool fma = (flags & VR_FLAG_RANGE_FMA) != 0, per_seq = (flags & VR_FLAG_PER_SEQUENCE) != 0;
+    L.fn = L.team ? pick_team_kernel(fma, L.p.VM, L.p.M, per_seq, &L.vmc)
+                  : pick_kernel(fma, L.p.VM, L.p.M, ups, L.p.zpark != 0, per_seq, &L.vmc);
+    return VR_OK;
+}
+
 int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* src, const int32_t* dst, int E,
            const float* lam_dev, const float* loc_dev, float lam_val, const float* loc_val,
            int n_fft, int hop, uint32_t flags, int img, float* out, float* iq, cudaStream_t stream,
@@ -501,38 +557,21 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
         return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
     if (((flags & VR_FLAG_NOISE) != 0) != (noise.std != nullptr))
         return fail(VR_ERR_ARG, "VR_FLAG_NOISE needs a noise setting (vr_set_noise) and a noise setting needs the flag");
-    const bool per_seq = (flags & VR_FLAG_PER_SEQUENCE) != 0;   // (the entries reject it with host parameters or null pointers)
     int views;
     int rc = views_of(flags, N, views);
     if (rc) return rc;
     int dev, sm_count;
     rc = device_setup(dev, sm_count);
     if (rc) return rc;
-    vr::Params p;
-    int grid, cps;
-    rc = cached_plan(N, T, V, M, src, dst, E, n_fft, hop, img, coef != nullptr, iq_only, sm_count, ((uintptr_t)x & 15) == 0, p, grid, cps);
+    LaunchPlan L;
+    rc = plan_launch(N, T, V, M, src, dst, E, n_fft, hop, img, coef != nullptr, iq_only, iq != nullptr, flags,
+                     ((uintptr_t)x & 15) == 0, g_schedule, sm_count, true, L);
     if (rc) return rc;
-    // schedule: batches with several sequences per team slot take the team-job kernel (no CTA-wide barriers, a double
-    // buffer per team); small batches keep the cooperative kernel, whose latency per sequence is half
-    bool team = false;
-    if (!coef && !iq && !g_timeline && g_schedule != 0) {
-        vr::Params q = p;
-        int tg = 0;
-        // automatic: from TEAM_AUTO_WAVES jobs per team slot in plain stream order (below that the cooperative kernel's
-        // shorter latency per sequence wins: N = 1024 66 vs 74 us, N = 4096 248 vs 228 us); always when the caller has
-        // declared the batches independent -- consecutive launches then overlap and only throughput counts
-        // (N = 256: 14.8 vs 16.3 us per launch)
-        const bool overlapped = g_pdl && (flags & VR_FLAG_INPUTS_READY);
-        if (make_team_plan(q, sm_count, tg) &&
-            (g_schedule == 1 || overlapped || q.n_jobs >= (long long)TEAM_AUTO_WAVES * sm_count * 2 * vr::TJ_TEAMS)) {
-            p = q; grid = tg; team = true;
-        }
-    }
-    const int job_slots = team ? grid * vr::TJ_TEAMS : grid;
+    vr::Params& p = L.p;
     p.x = x; p.out = out; p.iq = iq; p.tl = g_timeline;
     p.views = views;
     p.noise = noise;
-    p.ticket = (g_dynamic && p.n_jobs > job_slots) ? next_ticket_slot(dev) : nullptr;
+    p.ticket = L.ticket ? next_ticket_slot(dev) : nullptr;
     p.early_reads = (g_pdl && !coef && (flags & VR_FLAG_INPUTS_READY)) ? 1 : 0;   // coef is written by the launch just before
     p.coef = coef; p.ups_T = ups_T; p.ups_K = ups_K;
     p.ups_ratio = coef ? (double)(ups_T - 1) / (double)((long long)ups_K * ups_T - 1) : 0.0;
@@ -543,15 +582,20 @@ int launch(const float* x, int64_t N, int64_t T, int V, int M, const int32_t* sr
     // the tail of the previous kernel in the stream; the kernel executes griddepcontrol.wait before
     // its first global-memory access, so stream order is preserved.
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(team ? (unsigned)vr::TJ_THREADS : (unsigned)(p.W + 1) * 32);
+    cfg.gridDim = dim3((unsigned)L.grid); cfg.blockDim = dim3(L.team ? (unsigned)vr::TJ_THREADS : (unsigned)(p.W + 1) * 32);
     cfg.dynamicSmemBytes = (size_t)p.smem_bytes; cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = g_pdl ? 1 : 0;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    KernelFn fn = team ? pick_team_kernel((flags & VR_FLAG_RANGE_FMA) != 0, p.VM, p.M, per_seq)
-                       : pick_kernel((flags & VR_FLAG_RANGE_FMA) != 0, p.VM, p.M, coef != nullptr, p.zpark != 0, per_seq);
-    CUDA_TRY(cudaLaunchKernelEx(&cfg, fn, p));
+    CUDA_TRY(cudaLaunchKernelEx(&cfg, L.fn, p));
+    // A debug launch writes every sample of iq: where its plan leaves samples to no job (hop > n_fft / 2), the
+    // synthesis-only launch follows on the stream and writes all of iq again -- the same bits where both write (the two
+    // launches fold each chunk's partial sums in the same fixed order, and the noise is keyed by (seed, n, t)).  Its
+    // stores wait for this launch to complete (griddepcontrol.wait), so the order of the two writes is the stream's.
+    if (iq && out && iq_gaps(p))
+        return launch(x, N, T, V, M, src, dst, E, lam_dev, loc_dev, lam_val, loc_val, n_fft, hop, flags, img, nullptr, iq,
+                      stream, coef, ups_T, ups_K, noise);
     return VR_OK;
 }
 
@@ -1217,6 +1261,28 @@ int vr_plan_team(int64_t N, int64_t T, int32_t V, int32_t M, const int32_t* src_
     plan[0] = grid; plan[1] = vr::TJ_THREADS; plan[2] = p.smem_bytes; plan[3] = vr::TJ_RS; plan[4] = vr::TJ_TEAMS;
     plan[5] = p.stage_bytes; plan[6] = p.z_stride;
     plan[7] = (p.n_jobs >= (long long)TEAM_AUTO_WAVES * sms * 2 * vr::TJ_TEAMS) ? 1 : 0;
+    return VR_OK;
+}
+
+int vr_plan_launch(int32_t mode, int64_t N, int64_t T, int32_t V, int32_t M, const int32_t* src_host, const int32_t* dst_host,
+                   int32_t E, int32_t n_fft, int32_t hop, int32_t image_size, int32_t num_pad_frames, uint32_t flags,
+                   int32_t x_aligned, int32_t schedule, int32_t sm_count, int64_t plan[24]) {
+    if (!plan) return fail(VR_ERR_ARG, "plan must not be null");
+    if (mode < 0 || mode > 2) return fail(VR_ERR_ARG, "mode must be 0 (spectrogram), 1 (debug: iq too) or 2 (synthesis only), got %d", mode);
+    if (schedule < -1 || schedule > 1) return fail(VR_ERR_ARG, "schedule must be -1, 0 or 1, got %d", schedule);
+    if (num_pad_frames < 0) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 0, got %d", num_pad_frames);
+    if (mode != 0 && image_size != 0) return fail(VR_ERR_ARG, "the debug and synthesis-only entries take no image_size");
+    const bool ups = num_pad_frames > 0;
+    LaunchPlan L;
+    int rc = plan_launch(N, ups ? T * num_pad_frames : T, V, M, src_host, dst_host, E, n_fft, hop, image_size, ups, mode == 2,
+                         mode == 1, flags, x_aligned != 0, schedule, sm_count > 0 ? sm_count : 148, false, L);
+    if (rc) return rc;
+    const vr::Params& p = L.p;
+    plan[0] = L.team; plan[1] = L.grid; plan[2] = L.team ? vr::TJ_THREADS : (p.W + 1) * 32; plan[3] = p.smem_bytes;
+    plan[4] = p.S; plan[5] = p.FJ; plan[6] = p.jobs_per_seq; plan[7] = p.n_jobs; plan[8] = p.FB; plan[9] = p.ostride;
+    plan[10] = p.tma_in; plan[11] = p.bulk_out; plan[12] = p.cmax; plan[13] = p.zcap; plan[14] = p.zpark; plan[15] = p.sparse;
+    plan[16] = p.ncols; plan[17] = L.cps; plan[18] = L.ticket; plan[19] = (p.M % 2 == 0) ? 2 : 1; plan[20] = L.vmc;
+    plan[21] = p.eg_max; plan[22] = p.sg_max; plan[23] = mode == 1 && iq_gaps(p);
     return VR_OK;
 }
 

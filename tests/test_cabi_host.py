@@ -93,6 +93,45 @@ def test_plan_image(cabi):
         cabi.plan_image(1, 300, 25, 2, src, dst, 5000)
 
 
+@pytest.mark.parametrize("N,T,V,M,hop,image", [(256, 300, 25, 2, 16, 0), (65536, 300, 25, 2, 16, 0), (1, 165000, 25, 1, 16, 0),
+                                              (2, 301, 25, 1, 16, 0), (3, 1800, 25, 2, 16, 0), (1, 5000, 25, 2, 300, 0),
+                                              (2, 399, 25, 2, 200, 0), (256, 300, 25, 2, 16, 256), (4, 75000, 25, 2, 16, 256),
+                                              (2, 3000, 25, 2, 16, 77), (16384, 300, 25, 2, 16, 0), (7, 300, 25, 1, 16, 0)])
+def test_plan_launch_agrees_with_the_plan_calls(cabi, N, T, V, M, hop, image):
+    """vr_plan_launch reports the plan of vr_plan / vr_plan_image and, under the team-job schedule, of vr_plan_team"""
+    from skeleton_action_recognition_b200 import edges
+    src, dst = map(list, zip(*edges))
+    q = cabi.plan_launch("spectrogram", N, T, V, M, src, dst, hop=hop, image_size=image, schedule=0)
+    p = cabi.plan_image(N, T, V, M, src, dst, image, hop=hop) if image else cabi.plan(N, T, V, M, src, dst, hop=hop)
+    assert q["team"] == 0 and q["jobs"] == N * q["jobs_per_seq"]
+    for k in ("grid", "block", "smem_bytes", "ring_stages", "jobs_per_seq", "tma_loads", "tma_bulk_store", "chunks_per_job",
+              "z_capacity", "ctas_per_sm"):
+        assert q[k] == p[k], k
+    assert q["columns_per_job"] == p["columns_per_job" if image else "frames_per_job"]
+    assert q["columns_per_tile"] == p["frames_per_tile"] and q["ticket"] == (q["jobs"] > q["grid"])
+    if image:
+        assert (q["sparse_frames"], q["columns"]) == (p["sparse_frames"], p["columns"])
+    else:
+        assert (q["max_bones_per_group"], q["max_sources_per_group"]) == (p["max_bones_per_group"], p["max_sources_per_group"])
+        assert q["compiled_vm"] == (50 if M % 2 == 0 else 0) and q["bodies_per_pass"] == (2 if M % 2 == 0 else 1)
+    try:
+        t = None if image else cabi.plan_team(N, T, V, M, src, dst, hop=hop)      # images never take the team-job kernel
+    except NotImplementedError:
+        t = None
+    forced = cabi.plan_launch("spectrogram", N, T, V, M, src, dst, hop=hop, image_size=image, schedule=1)
+    auto = cabi.plan_launch("spectrogram", N, T, V, M, src, dst, hop=hop, image_size=image)
+    assert forced["team"] == (t is not None) and auto["team"] == (t is not None and t["automatic"] == 1)
+    if t is not None:
+        assert (forced["grid"], forced["block"], forced["smem_bytes"], forced["ring_stages"]) == \
+            (t["grid"], t["block"], t["smem_bytes"], t["ring_stages_per_team"])
+    # the debug entries never take the team-job kernel; they fill in iq exactly where frames leave samples to no job
+    dbg = cabi.plan_launch("debug", N, T, V, M, src, dst, hop=hop, schedule=1) if not image else None
+    if dbg is not None:
+        assert dbg["team"] == 0 and dbg["iq_fill"] == ((T - 1) - (T // hop) * hop > 127 or hop > 256)
+    with pytest.raises(ValueError):
+        cabi.plan_launch("debug", N, T, V, M, src, dst, hop=hop, image_size=64)
+
+
 def test_partition_keeps_sources_together_and_balances(cabi):
     from skeleton_action_recognition_b200 import edges
     src, dst = map(list, zip(*edges))

@@ -131,6 +131,41 @@ def test_synth_iq_equals_the_debug_launch(N, T, V, M, fma, E):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("N,T,hop,K", [(2, 399, 200, 0), (1, 5000, 300, 0), (3, 700, 257, 0), (2, 133, 200, 3), (1, 300, 130, 0)])
+def test_debug_iq_is_written_where_no_frame_reaches(N, T, hop, K):
+    """hop > n_fft / 2 leaves samples outside every frame's window (after the last one, between frames); the debug launches
+    still write every sample of iq, with the bits of the synthesis-only launch"""
+    from skeleton_action_recognition_b200 import _cabi
+    layer = _layer(wavelength=1e-3, radar_location=[0.3, -0.2, 1.5])
+    x = fx.s3_smooth(N, T=T).cuda()
+    L = _cabi.lib()
+    args = (x.data_ptr(), N, T, 25, 2, layer._src_c, layer._dst_c, len(layer.src), layer.wavelength.data_ptr(),
+            layer.radar_location.data_ptr())
+    Tu = K * T if K else T
+    out = torch.empty(N, 256, Tu // hop + 1, device="cuda")
+    iq = torch.full((N, Tu, 2), float("nan"), device="cuda")
+    if K:
+        nbytes = int(L.vr_upsampled_workspace_bytes(N, T, 25, 2))
+        work = torch.empty(nbytes // 8, dtype=torch.float64, device="cuda")
+        _cabi.check(L.vr_forward_upsampled_debug_f32(*args, 256, hop, 0, K, ctypes.c_float(3.0), work.data_ptr(), nbytes,
+                                                     out.data_ptr(), iq.data_ptr(), _stream()))
+        want = _synth_upsampled(layer, x, K, 3.0, debug=False)
+    else:
+        _cabi.check(L.vr_forward_debug_f32(*args, 256, hop, 0, out.data_ptr(), iq.data_ptr(), _stream()))
+        want = _synth(layer, x, 0)
+    assert not torch.isnan(want).any()
+    assert torch.equal(iq, want)
+    # the spectrogram is the launch without iq
+    out2 = torch.empty_like(out)
+    if K:
+        _cabi.check(L.vr_forward_upsampled_f32(*args, 256, hop, 0, K, ctypes.c_float(3.0), 0, work.data_ptr(), nbytes,
+                                               out2.data_ptr(), _stream()))
+    else:
+        _cabi.check(L.vr_forward_f32(*args, 256, hop, 0, out2.data_ptr(), _stream()))
+    assert torch.equal(out, out2)
+
+
+@pytest.mark.gpu
 def test_synth_needs_no_stft_length():
     """T <= n_fft/2 is fine for the synthesis alone: it equals the first samples of a longer sequence's synthesis."""
     layer = _layer(wavelength=1e-3)
