@@ -27,7 +27,7 @@ SYMBOLS = ("vr_abi_version", "vr_last_error", "vr_forward_f32", "vr_forward_debu
            "vr_synth_f32", "vr_synth_upsampled_f32", "vr_synth_adjoint_upsampled_f32",
            "vr_stft_general_frames_workspace_floats", "vr_stft_general_frames_f32", "vr_stft_general_frames_backward_f32",
            "vr_plan_adjoint_stft", "vr_plan_pad_frames", "vr_plan_stft_general", "vr_per_sequence_grad_doubles",
-           "vr_set_noise", "vr_plan_launch")
+           "vr_set_noise", "vr_plan_launch", "vr_plan_backward")
 
 _lib = None
 
@@ -114,6 +114,9 @@ def lib():
     L.vr_plan_launch.argtypes = [i32, i64, i64, i32, i32, c_i32p, c_i32p, i32, i32, i32, i32, i32, u32, i32, i32, i32,
                                  ctypes.POINTER(i64)]
     L.vr_plan_launch.restype = ctypes.c_int
+    L.vr_plan_backward.argtypes = [i32, i64, i64, i32, i32, c_i32p, c_i32p, i32, i32, i32, u32, i32, i32, i32,
+                                   ctypes.POINTER(i64)]
+    L.vr_plan_backward.restype = ctypes.c_int
     L.vr_set_noise.argtypes = [vp, vp]
     L.vr_set_noise.restype = ctypes.c_int
     L.vr_set_timeline_buffer.argtypes = [vp]
@@ -209,6 +212,28 @@ def plan_adjoint_stft(N, T, hop=16, sm_count=148):
     rows = (ctypes.c_int64 * (4 * plan["segments"]))()
     check(lib().vr_plan_adjoint_stft(N, T, hop, sm_count, out, rows, plan["segments"]))
     return plan, [tuple(int(v) for v in rows[4 * k:4 * k + 4]) for k in range(plan["segments"])]
+
+
+BACKWARD_PLAN_FIELDS = ("stft", "segment_length", "segments", "stft_grid", "stft_smem_bytes", "synth_kernel", "ups",
+                        "views_mode", "views", "grid", "units", "ps_segments", "fold_grid", "scratch_tail", "grad_x_fill",
+                        "grid_cap")
+BACKWARD_ENTRIES = {"backward": 0, "backward_params": 1, "synth_adjoint": 2, "backward_upsampled_params": 3,
+                    "synth_adjoint_upsampled": 4}
+SYNTH_KERNELS = ("scalar", "scalar_ups", "ps")
+VIEWS_MODES = ("none", "outputs", "rows")
+
+
+def plan_backward(entry, N, T, V, M, src, dst, hop=16, flags=0, grad_x=False, num_pad_frames=0, sm_count=148, n_fft=256):
+    """Configuration of one backward call (vr_plan_backward): entry "backward" (vr_backward_f32), "backward_params",
+    "synth_adjoint", "backward_upsampled_params" or "synth_adjoint_upsampled" (T raw, with num_pad_frames); grad_x: a
+    dL/dx buffer is passed.  synth_kernel and views_mode come back as names."""
+    out = (ctypes.c_int64 * len(BACKWARD_PLAN_FIELDS))()
+    check(lib().vr_plan_backward(BACKWARD_ENTRIES[entry], N, T, V, M, i32_array(src), i32_array(dst), len(src), n_fft, hop,
+                                 flags, 1 if grad_x else 0, num_pad_frames, sm_count, out))
+    plan = dict(zip(BACKWARD_PLAN_FIELDS, [int(v) for v in out]))
+    plan["synth_kernel"] = SYNTH_KERNELS[plan["synth_kernel"]]
+    plan["views_mode"] = VIEWS_MODES[plan["views_mode"]]
+    return plan
 
 
 PAD_PLAN_FIELDS = ("nc", "ncb", "units", "grid", "smem_bytes", "nrs", "rows_per_slice", "radius")

@@ -1049,6 +1049,81 @@ int vr_backward_params_f32(const float* x_dev, const float* iq_dev, const float*
 
 }  // extern "C"
 namespace {
+// The backward entries' checks of everything but the device pointers, before the device is touched.  T: the steps the
+// adjoint runs over (up-sampled length for the _upsampled entries).
+int backward_args(int64_t N, int64_t T, int V, int M, const int32_t* src_host, const int32_t* dst_host, int E, int n_fft,
+                  int hop, uint32_t flags, bool synth_only) {
+    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
+    int views;
+    int rc = views_of(flags, N, views);
+    if (rc) return rc;
+    if (N <= 0 || T <= 0 || V <= 0 || M <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M, hop must be positive");
+    if (n_fft != vr::NFFT) return fail(VR_ERR_UNSUPPORTED, "this ABI version implements n_fft=256 only (got %d)", n_fft);
+    if (!synth_only && T <= n_fft / 2) return fail(VR_ERR_SHAPE, "T=%lld must exceed n_fft/2=%d", (long long)T, n_fft / 2);
+    if (T > (1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T=%lld too long", (long long)T);
+    if (!src_host || !dst_host) return fail(VR_ERR_ARG, "edge arrays must not be null");
+    if (E <= 0 || E > vr::NG * vr::MAX_EG) return fail(VR_ERR_UNSUPPORTED, "E=%d outside [1, %d]", E, vr::NG * vr::MAX_EG);
+    if (V > 65535) return fail(VR_ERR_UNSUPPORTED, "V=%d too large", V);
+    for (int e = 0; e < E; ++e)
+        if (src_host[e] < 0 || src_host[e] >= V || dst_host[e] < 0 || dst_host[e] >= V)
+            return fail(VR_ERR_SHAPE, "edge %d = (%d,%d) indexes a joint outside [0,%d)", e, src_host[e], dst_host[e], V);
+    return VR_OK;
+}
+
+// the _upsampled backward entries' checks of the raw length and the factor
+int backward_ups_args(int64_t T, int num_pad_frames) {
+    if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames", (long long)T);
+    if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
+    if ((double)T * num_pad_frames > (double)(1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
+    return VR_OK;
+}
+
+// The configuration of one backward call: the adjoint STFT (unless the entry is synthesis only), then the synthesis
+// adjoint -- the scalar kernels with a slot of the static partials (g_param_partials), or the per-sequence kernel
+// vr_synth_adjoint_ps_kernel<ups, views_mode> with the scratch tail of the caller's gradient buffer and the fold.
+// backward_impl launches exactly this; vr_plan_backward reports it without a GPU.
+constexpr int BWD_SYNTH_SCALAR = 0, BWD_SYNTH_SCALAR_UPS = 1, BWD_SYNTH_PS = 2;
+struct BackwardPlan {
+    bool stft = false;
+    int seg_len = 0, segs = 0, stft_grid = 0;
+    long long stft_smem = 0;
+    int synth = BWD_SYNTH_SCALAR, views_mode = vr::VIEWS_NONE, views = 1, grid = 0, fold_grid = 0;
+    bool ups = false;
+    long long units = 0, ps_segs = 0;   // per-sequence: warp units and segments per sequence; scalar: units = steps
+    long long gx_floats = 0;            // extent of the dL/dx zero fill (0: not wanted)
+};
+int plan_backward(int64_t N, int64_t T, int V, int M, const int32_t* src_host, const int32_t* dst_host, int E, int n_fft,
+                  int hop, uint32_t flags, bool synth_only, bool ups, bool want_gx, int sm_count, BackwardPlan& B) {
+    int rc = backward_args(N, T, V, M, src_host, dst_host, E, n_fft, hop, flags, synth_only);
+    if (rc) return rc;
+    if (ups && want_gx) return fail(VR_ERR_ARG, "the _upsampled backward entries take no dL/dx");
+    B = BackwardPlan{};
+    views_of(flags, N, B.views);
+    B.ups = ups;
+    B.gx_floats = want_gx ? (N / B.views) * 3 * T * V * M : 0;
+    B.stft = !synth_only;
+    if (B.stft) {
+        vr::adjoint_plan(N, T, sm_count, B.seg_len, B.segs);
+        B.stft_grid = (int)std::min<long long>(N * B.segs, (long long)sm_count * 8);
+        B.stft_smem = (long long)B.seg_len * 8;
+    }
+    if (flags & VR_FLAG_PER_SEQUENCE) {
+        // views: with dL/dx one warp runs a row's views in order (one owner per dL/dx row); without it the units are per
+        // output, as without views, for R times the parallelism.  R = 1: the plain per-sequence kernel
+        B.synth = BWD_SYNTH_PS;
+        B.views_mode = B.views == 1 ? vr::VIEWS_NONE : want_gx ? vr::VIEWS_ROWS : vr::VIEWS_OUTPUTS;
+        B.ps_segs = vr::ps_segments(T);
+        B.units = (B.views_mode == vr::VIEWS_ROWS ? N / B.views : N) * B.ps_segs;
+        B.grid = (int)std::min<long long>((B.units + 3) / 4, (long long)sm_count * 16);   // 4 warps per block
+        B.fold_grid = (int)((4 * N + 127) / 128);
+        return VR_OK;
+    }
+    B.synth = ups ? BWD_SYNTH_SCALAR_UPS : BWD_SYNTH_SCALAR;
+    B.units = N * T;
+    B.grid = (int)std::min<long long>(std::min<long long>((B.units + 127) / 128, (long long)sm_count * 16), vr::PARAM_MAX_BLOCKS);
+    return VR_OK;
+}
+
 int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out_dev,
                   int64_t N, int64_t T, int32_t V, int32_t M,
                   const int32_t* src_host, const int32_t* dst_host, int32_t E,
@@ -1065,9 +1140,7 @@ int backward_ups_impl(const void* workspace_dev, const float* iq_dev, const floa
     drop_noise(flags);
     if (!workspace_dev) return fail(VR_ERR_ARG, "workspace_dev must not be null");
     if (((uintptr_t)workspace_dev & 7) != 0) return fail(VR_ERR_ARG, "workspace_dev must be 8-byte aligned");
-    if (T < 4) return fail(VR_ERR_SHAPE, "T=%lld: cubic interpolation needs at least 4 frames", (long long)T);
-    if (num_pad_frames < 1) return fail(VR_ERR_SHAPE, "num_pad_frames must be >= 1, got %d", num_pad_frames);
-    if ((double)T * num_pad_frames > (double)(1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T*num_pad_frames too large");
+    if (int rc = backward_ups_args(T, num_pad_frames)) return rc;
     return backward_impl(nullptr, iq_dev, grad_out_dev, N, T * num_pad_frames, V, M, src_host, dst_host, E, wavelength_dev,
                          radar_loc_dev, n_fft, hop, flags, synth_only, gz_work_dev, grad_params_dev, nullptr, stream,
                          static_cast<const double*>(workspace_dev), (int)T, num_pad_frames);
@@ -1118,30 +1191,20 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     // the up-sampling spline's (T = ups_K * ups_T steps, x_dev unused), parameter gradients only
     if ((!x_dev && !coef) || !gz_work_dev || !grad_params_dev || !wavelength_dev || !radar_loc_dev || (!synth_only && (!iq_dev || !grad_out_dev)))
         return fail(VR_ERR_ARG, "device pointers must not be null");
-    if (flags & ~(VR_FLAG_RANGE_FMA | VR_FLAG_PER_SEQUENCE | VR_FLAG_VIEWS_MASK)) return fail(VR_ERR_ARG, "unknown flags 0x%x", flags);
-    const bool per_seq = (flags & VR_FLAG_PER_SEQUENCE) != 0;
-    int views;                                          // VR_FLAG_VIEWS: x (and coef) hold N / views sequences
-    int rc = views_of(flags, N, views);
+    int rc = backward_args(N, T, V, M, src_host, dst_host, E, n_fft, hop, flags, synth_only);
     if (rc) return rc;
-    if (per_seq && ((uintptr_t)grad_params_dev & 7) != 0)
+    if ((flags & VR_FLAG_PER_SEQUENCE) && ((uintptr_t)grad_params_dev & 7) != 0)
         return fail(VR_ERR_ARG, "grad_params_dev must be 8-byte aligned (float64 per-sequence gradients)");
-    if (N <= 0 || T <= 0 || V <= 0 || M <= 0 || hop <= 0) return fail(VR_ERR_SHAPE, "N, T, V, M, hop must be positive");
-    if (n_fft != vr::NFFT) return fail(VR_ERR_UNSUPPORTED, "this ABI version implements n_fft=256 only (got %d)", n_fft);
-    if (!synth_only && T <= n_fft / 2) return fail(VR_ERR_SHAPE, "T=%lld must exceed n_fft/2=%d", (long long)T, n_fft / 2);
-    if (T > (1ll << 30)) return fail(VR_ERR_UNSUPPORTED, "T=%lld too long", (long long)T);
-    if (!src_host || !dst_host) return fail(VR_ERR_ARG, "edge arrays must not be null");
-    if (E <= 0 || E > vr::NG * vr::MAX_EG) return fail(VR_ERR_UNSUPPORTED, "E=%d outside [1, %d]", E, vr::NG * vr::MAX_EG);
-    if (V > 65535) return fail(VR_ERR_UNSUPPORTED, "V=%d too large", V);
     int dev, sm_count;
     rc = device_setup(dev, sm_count);
     if (rc) return rc;
+    BackwardPlan B;
+    rc = plan_backward(N, T, V, M, src_host, dst_host, E, n_fft, hop, flags, synth_only, coef != nullptr, grad_x_dev != nullptr,
+                       sm_count, B);
+    if (rc) return rc;
     vr::BwdParams p;
     memset(&p, 0, sizeof(p));
-    for (int e = 0; e < E; ++e) {
-        if (src_host[e] < 0 || src_host[e] >= V || dst_host[e] < 0 || dst_host[e] >= V)
-            return fail(VR_ERR_SHAPE, "edge %d = (%d,%d) indexes a joint outside [0,%d)", e, src_host[e], dst_host[e], V);
-        p.src[e] = (uint16_t)src_host[e]; p.dst[e] = (uint16_t)dst_host[e];
-    }
+    for (int e = 0; e < E; ++e) { p.src[e] = (uint16_t)src_host[e]; p.dst[e] = (uint16_t)dst_host[e]; }
     p.x = x_dev; p.iq = iq_dev; p.gout = grad_out_dev; p.gz = gz_work_dev; p.gparams = grad_params_dev; p.gx = grad_x_dev;
     p.lam_ptr = wavelength_dev; p.loc_ptr = radar_loc_dev;
     p.N = N; p.T = T; p.V = V; p.M = M; p.E = E; p.hop = hop; p.VM = V * M;
@@ -1150,45 +1213,37 @@ int backward_impl(const float* x_dev, const float* iq_dev, const float* grad_out
     p.inv_E = 1.0f / (float)E;
     p.coef = coef; p.ups_T = ups_T;
     p.ups_ratio = coef ? (double)(ups_T - 1) / (double)((long long)ups_K * ups_T - 1) : 0.0;
-    p.views = views;
+    p.views = B.views;
+    p.seg_len = B.seg_len; p.segs = B.segs;
     cudaStream_t st = (cudaStream_t)stream;
-    if (grad_x_dev) CUDA_TRY(cudaMemsetAsync(grad_x_dev, 0, (size_t)(N / views) * 3 * T * V * M * sizeof(float), st));
-    if (!synth_only) {                                  // writes every sample of gz: no zero fill
-        vr::adjoint_plan(N, T, sm_count, p.seg_len, p.segs);
-        const int grid1 = (int)std::min<long long>(N * p.segs, (long long)sm_count * 8);
-        vr::vr_stft_adjoint_kernel<<<grid1, vr::BWD_WARPS * 32, (size_t)p.seg_len * 8, st>>>(p);
+    if (grad_x_dev) CUDA_TRY(cudaMemsetAsync(grad_x_dev, 0, (size_t)B.gx_floats * sizeof(float), st));
+    if (B.stft) {                                       // writes every sample of gz: no zero fill
+        vr::vr_stft_adjoint_kernel<<<B.stft_grid, vr::BWD_WARPS * 32, (size_t)B.stft_smem, st>>>(p);
         CUDA_TRY(cudaGetLastError());
     }
-    if (per_seq) {
+    if (B.synth == BWD_SYNTH_PS) {
         // per-sequence gradients: (x sequence, segment) units, each running its views, reduced warp by warp into the scratch
         // tail of grad_params_dev (vr_per_sequence_grad_doubles), then folded per output in segment order
-        p.ps_segs = vr::ps_segments(T);
+        p.ps_segs = B.ps_segs;
         p.part = grad_params_dev + 4 * N;
-        // views: with dL/dx one warp runs a row's views in order (one owner per dL/dx row); without it the units are per
-        // output, as without views, for R times the parallelism.  R = 1: the plain per-sequence kernel
-        const int mode = views == 1 ? vr::VIEWS_NONE : grad_x_dev ? vr::VIEWS_ROWS : vr::VIEWS_OUTPUTS;
-        const long long units = (mode == vr::VIEWS_ROWS ? N / views : N) * p.ps_segs;
-        const int grid2 = (int)std::min<long long>((units + 3) / 4, (long long)sm_count * 16);   // 4 warps per block
-        if (mode == vr::VIEWS_ROWS) {
-            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_ROWS><<<grid2, 128, 0, st>>>(p);
-            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_ROWS><<<grid2, 128, 0, st>>>(p);
-        } else if (mode == vr::VIEWS_OUTPUTS) {
-            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_OUTPUTS><<<grid2, 128, 0, st>>>(p);
-            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_OUTPUTS><<<grid2, 128, 0, st>>>(p);
+        if (B.views_mode == vr::VIEWS_ROWS) {
+            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_ROWS><<<B.grid, 128, 0, st>>>(p);
+            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_ROWS><<<B.grid, 128, 0, st>>>(p);
+        } else if (B.views_mode == vr::VIEWS_OUTPUTS) {
+            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_OUTPUTS><<<B.grid, 128, 0, st>>>(p);
+            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_OUTPUTS><<<B.grid, 128, 0, st>>>(p);
         } else {
-            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_NONE><<<grid2, 128, 0, st>>>(p);
-            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_NONE><<<grid2, 128, 0, st>>>(p);
+            if (coef) vr::vr_synth_adjoint_ps_kernel<true, vr::VIEWS_NONE><<<B.grid, 128, 0, st>>>(p);
+            else vr::vr_synth_adjoint_ps_kernel<false, vr::VIEWS_NONE><<<B.grid, 128, 0, st>>>(p);
         }
         CUDA_TRY(cudaGetLastError());
-        vr::vr_param_fold_kernel<<<(unsigned)((4 * N + 127) / 128), 128, 0, st>>>(p.part, grad_params_dev, N, p.ps_segs);
+        vr::vr_param_fold_kernel<<<(unsigned)B.fold_grid, 128, 0, st>>>(p.part, grad_params_dev, N, p.ps_segs);
         CUDA_TRY(cudaGetLastError());
         return VR_OK;
     }
-    const long long steps = N * T;
-    const int grid2 = (int)std::min<long long>(std::min<long long>((steps + 127) / 128, (long long)sm_count * 16), vr::PARAM_MAX_BLOCKS);
     next_param_slot(dev, p);
-    if (coef) vr::vr_synth_adjoint_ups_kernel<<<grid2, 128, 0, st>>>(p);
-    else vr::vr_synth_adjoint_kernel<<<grid2, 128, 0, st>>>(p);
+    if (B.synth == BWD_SYNTH_SCALAR_UPS) vr::vr_synth_adjoint_ups_kernel<<<B.grid, 128, 0, st>>>(p);
+    else vr::vr_synth_adjoint_kernel<<<B.grid, 128, 0, st>>>(p);
     CUDA_TRY(cudaGetLastError());
     return VR_OK;
 }
@@ -1323,6 +1378,32 @@ int vr_plan_adjoint_stft(int64_t N, int64_t T, int32_t hop, int32_t sm_count, in
             r[0] = s0; r[1] = s1; r[2] = lo; r[3] = hi;
         }
     }
+    return VR_OK;
+}
+
+int vr_plan_backward(int32_t entry, int64_t N, int64_t T, int32_t V, int32_t M, const int32_t* src_host,
+                     const int32_t* dst_host, int32_t E, int32_t n_fft, int32_t hop, uint32_t flags, int32_t want_grad_x,
+                     int32_t num_pad_frames, int32_t sm_count, int64_t plan[16]) {
+    if (!plan) return fail(VR_ERR_ARG, "plan must not be null");
+    if (entry < 0 || entry > 4)
+        return fail(VR_ERR_ARG, "entry must be 0 (backward), 1 (backward_params), 2 (synth_adjoint), 3 (backward_upsampled_params) "
+                                "or 4 (synth_adjoint_upsampled), got %d", entry);
+    drop_noise(flags);
+    const bool ups = entry >= 3, synth_only = entry == 2 || entry == 4;
+    if (want_grad_x && entry != 0 && entry != 2) return fail(VR_ERR_ARG, "only vr_backward_f32 and vr_synth_adjoint_f32 take dL/dx");
+    if (ups) {
+        if (int rc = backward_ups_args(T, num_pad_frames)) return rc;
+        T *= num_pad_frames;
+    }
+    if (synth_only) { n_fft = vr::NFFT; hop = 16; }        // what the synthesis-only entries pass: they run no STFT
+    BackwardPlan B;
+    int rc = plan_backward(N, T, V, M, src_host, dst_host, E, n_fft, hop, flags, synth_only, ups, want_grad_x != 0,
+                           sm_count > 0 ? sm_count : 148, B);
+    if (rc) return rc;
+    const bool ps = B.synth == BWD_SYNTH_PS;
+    plan[0] = B.stft; plan[1] = B.seg_len; plan[2] = B.segs; plan[3] = B.stft_grid; plan[4] = B.stft_smem; plan[5] = B.synth;
+    plan[6] = B.ups; plan[7] = B.views_mode; plan[8] = B.views; plan[9] = B.grid; plan[10] = B.units; plan[11] = B.ps_segs;
+    plan[12] = B.fold_grid; plan[13] = ps ? 1 : 0; plan[14] = B.gx_floats; plan[15] = ps ? 0 : vr::PARAM_MAX_BLOCKS;
     return VR_OK;
 }
 

@@ -174,8 +174,9 @@ def stft_adjoint_tolerance(iq, go, hop, n_fft=256):
     """Per-sample bound on the float32 error of the adjoint STFT (vr_stft_adjoint_kernel), from the conditioning of each
     frame: the radix FFT of the windowed frame zp errs by at most eps_X = 2 u log2(n) sum |zp| per bin, and
     G = g X / |X|^2 turns that into |g| eps_X / |X|^2 (large where a bin nearly vanishes); the inverse FFT adds
-    2 u log2(n) sum |G|, the window and the float32 overlap-add atomics u * (frames + 2) * sum |y|.  The stage-1 error
-    of the module test is this loose bound's business; stage 2 propagates the error actually measured."""
+    2 u log2(n) sum |G|, the window and the float32 overlap-add, in the owner form's fixed frame order,
+    u * (frames + 2) * sum |y|.  A coarse bound for these end-to-end cases; tests/test_backward_oracle_gpu.py holds the
+    kernel to a bound derived from its instructions.  Stage 2 propagates the error actually measured."""
     iq = np.asarray(iq, np.float64)
     g = np.asarray(go, np.float64)
     N, T, _ = iq.shape
